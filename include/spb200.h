@@ -355,8 +355,6 @@ int spb_dmma_peak(spb_context *ctx, int iters, double *tflops_host, double *ms_h
  * the environment variables SPB_NO_TMA / SPB_NO_CLUSTER set the defaults at spb_create):
  *   "cholesky_tma"     1 | 0   operand ring of the batched Cholesky fed by TMA | by cp.async
  *   "cholesky_cluster" 1 | 0   few matrices: one matrix per thread-block cluster | per CTA
- *   "cholesky_tile"    64 | 128  rows per CTA tile of the batched Cholesky (4 warps, 3 CTAs per SM |
- *                              8 warps, 2 CTAs per SM)
  *   "moments_syrk_i8"  1 | 0   the FP64 GEMMs with an INT8-tensor-core form -- the second-moment SYRK of
  *                              spb_ylm_moments* (contrast.py:21-33) and, for nt >= 1024, the product
  *                              (A Sigma) A^T of spb_flux_conditional_lower (flux.py:335-343) -- on the INT8

@@ -22,18 +22,15 @@ print("design", float(gp2.design_matrix(t, i=[10.0, 80.0]).sum()))
 print("sample_ylm", float(gp2.sample_ylm(nsamples=3).sum()))
 torch.cuda.synchronize()
 print("done")
-# round 2: uniform spot-size prior, gradient (tangent kernels), alternative Cholesky geometries
+# round 2: uniform spot-size prior, gradient (tangent kernels)
 gd = spb.StarryProcess(r=[15.0, 20.0], dr=[5.0, 3.0], mu=30.0, sigma=5.0, c=0.1, n=10.0)
 print("dr lnlike", gd.log_likelihood(t, f, 1e-6, u=[0.4, 0.26]).cpu().numpy())
 gg = spb.StarryProcess(r=[12.0, 20.0], a=[0.4, 0.5], b=[0.27, 0.2], c=0.1, n=10.0)
 ll, g = gg.log_likelihood(t[:120], f[:120], 1e-6, u=[0.4, 0.26], return_grad=True)
 print("grad", {k: v.cpu().numpy() for k, v in g.items()})
 ctx = spb.get_context(0)
-for tile in (64, 163, 164):
-    ctx.set_option("cholesky_tile", tile)
-    ctx.set_option("cholesky_cluster", 0)
-    print("tile", tile, gg.log_likelihood(t, f, 1e-6, u=[0.4, 0.26]).cpu().numpy())
-ctx.set_option("cholesky_tile", 0)
+ctx.set_option("cholesky_cluster", 0)   # few matrices: the one-CTA-per-matrix kernel instead of clusters
+print("batch kernel", gg.log_likelihood(t, f, 1e-6, u=[0.4, 0.26]).cpu().numpy())
 ctx.set_option("cholesky_cluster", 1)
 torch.cuda.synchronize()
 print("done round 2")

@@ -28,7 +28,6 @@ struct spb_context {
   int opt_no_tma;         // Cholesky operand ring: cp.async instead of TMA
   int opt_no_cluster;     // Cholesky: never use the one-matrix-per-cluster kernel
   int opt_syrk_i8;        // second-moment SYRK of the Ylm moments on the INT8 tensor cores (syrk_i8.cu)
-  int opt_chol_tile;      // Cholesky batch kernel: rows per tile, 64 (4 warps, 3 CTAs/SM) or 128
   int max_active_clusters[3];   // cudaOccupancyMaxActiveClusters for cluster sizes 8, 4, 2 (-1: unknown)
   // ring of work counters for kernels that claim their work items dynamically (one per launch,
   // zeroed in-stream before the launch, so that concurrent streams never share one)
@@ -193,12 +192,6 @@ __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.comm
 template <int N>
 __device__ __forceinline__ void bulk_wait_read() {
   asm volatile("cp.async.bulk.wait_group.read %0;\n" ::"n"(N) : "memory");
-}
-
-// ---- 32-byte global store (STG.E.256, sm_100+): one full DRAM sector per lane ------------------
-__device__ __forceinline__ void st_global_256(double *p, double a, double b, double c, double d) {
-  asm volatile("st.global.v4.f64 [%0], {%1, %2, %3, %4};\n" ::"l"(p), "d"(a), "d"(b), "d"(c), "d"(d)
-               : "memory");
 }
 
 __device__ __forceinline__ double warp_sum(double v) {

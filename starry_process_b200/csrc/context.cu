@@ -61,7 +61,6 @@ extern "C" int spb_create(int device, const double *tables_host, size_t tables_c
   ctx->opt_no_tma = getenv("SPB_NO_TMA") != nullptr;          // defaults of the A/B switches
   ctx->opt_no_cluster = getenv("SPB_NO_CLUSTER") != nullptr;
   ctx->opt_syrk_i8 = getenv("SPB_SYRK_I8") ? atoi(getenv("SPB_SYRK_I8")) : 1;   // default: INT8 tensor cores
-  ctx->opt_chol_tile = getenv("SPB_CHOL_TILE") ? atoi(getenv("SPB_CHOL_TILE")) : 0;   // 0: automatic
   for (int k = 0; k < 3; ++k) ctx->max_active_clusters[k] = -1;
   SPB_CHECK_CUDA(cudaMalloc(&ctx->d_counters, SPB_NUM_COUNTERS * sizeof(unsigned int)));
   SPB_CHECK_CUDA(cudaMemset(ctx->d_counters, 0, SPB_NUM_COUNTERS * sizeof(unsigned int)));
@@ -92,12 +91,6 @@ extern "C" int spb_set_option(spb_context *ctx, const char *name, int value) {
   }
   if (key == "cholesky_tma") ctx->opt_no_tma = value ? 0 : 1;
   else if (key == "cholesky_cluster") ctx->opt_no_cluster = value ? 0 : 1;
-  else if (key == "cholesky_tile") {
-    SPB_REQUIRE(value == 0 || value == 64 || value == 128 || value == 645 || value == 644 || value == 1286 ||
-                    value == 163 || value == 164 || value == 165,
-                "spb_set_option: cholesky_tile must be 64 or 128");
-    ctx->opt_chol_tile = value;
-  }
   else SPB_REQUIRE(false, "spb_set_option: unknown option");
   return 0;
 }

@@ -47,25 +47,16 @@ namespace {
 
 constexpr int NB = 64;         // panel width
 constexpr int KC = 16;         // k-chunk per pipeline stage (one 128-byte row segment)
-constexpr int LS = NB + 4;     // smem stride of the unpacked diagonal block: 68
+constexpr int LS = NB + 4;     // smem stride of the diagonal block: 68
 constexpr int DS = 12;         // smem stride of the 8x8 diagonal-inverse blocks
 
-// Tile geometry.  A CTA of TM / 16 warps owns TM rows of a panel at a time (16 rows x 64 columns per
-// warp).  Two instantiations:
-//   TM = 128: 8 warps, 2 CTAs per SM (the round-1 kernel; still used by the cluster kernel);
-//   TM =  64: 4 warps, 3 CTAs per SM.  Finer tiles waste fewer warp slots on the partly filled last
-//             tile of a panel and on the triangular diagonal tile (k-loop slot efficiency at
-//             nt = 1000: 0.94 against 0.82), and three independent matrices per SM overlap one
-//             another's latency-bound phases (diagonal block, TRSM chains, prologues) better than
-//             two.  L_jj is kept PACKED (its 36 lower 8x8 tiles, 18 KB instead of 35 KB) so that
-//             three CTAs fit the shared memory of an SM.
-template <int TM_>
-struct Geo {
-  static constexpr int TM = TM_;
-  static constexpr int NTHREADS = 2 * TM_;
-  static constexpr int NWARPS = TM_ / 16;
-  static constexpr bool PACKED = (TM_ != 128);
-};
+// Tile geometry of the FP64 kernels: a CTA of 8 warps owns TM = 128 rows of a panel at a time (16 rows
+// x 64 columns per warp) and streams its operands through a ring of STAGES chunks.  The alternatives
+// measured against it (4-warp tiles, deeper rings, a producer warp) lost inside the bench step:
+// DESIGN.md section 4.1 (ii).
+constexpr int TM = 128;
+constexpr int NTHREADS = 2 * TM;
+constexpr int STAGES = 3;      // operand ring depth (look-ahead = STAGES - 1 chunks)
 
 enum { KIND_NONE = 0, KIND_DIAG = 1, KIND_PAD = 2, KIND_BELOW = 3, KIND_RHS = 4 };
 enum { MODE_FACTOR = 1, MODE_SOLVE = 0 };
@@ -131,39 +122,17 @@ struct RowMap {
 // k = 4 kk + tg) every half-warp then touches 16 distinct 8-byte banks: conflict-free LDS.64
 // without the 25 % padding, which is what lets three stages fit beside the diagonal block at
 // two CTAs per SM.
-// L_jj storage.  Unpacked: row stride 68 (conflict-free for the m8n8k4 fragment pattern).  Packed:
-// lower 8x8 tiles only, tile (ib, jb) at (ib (ib + 1) / 2 + jb) * 64, element (r, c) of a tile at
-// r * 8 + (c ^ ((r & 2) << 1)): the XOR moves columns 0-3 / 4-7 of rows 2, 3, 6, 7 so that the 16
-// lanes of a half-warp (rows g..g+3, columns 4 q + tg) hit 16 distinct 8-byte banks, and keeps the
-// (2 tg, 2 tg + 1) pairs of the accumulator layout adjacent and 16-byte aligned.
-template <bool PACKED>
-struct LdStore;
-template <>
-struct LdStore<false> {
+// L_jj storage: row stride 68 (conflict-free for the m8n8k4 fragment pattern).
+struct LdStore {
   double v[NB * LS];
   __device__ __forceinline__ double &at(int i, int j) { return v[i * LS + j]; }
   __device__ __forceinline__ const double &at(int i, int j) const { return v[i * LS + j]; }
 };
-template <>
-struct LdStore<true> {
-  double v[36 * 64];
-  static __device__ __forceinline__ int idx(int i, int j) {
-    const int ib = i >> 3, jb = j >> 3, r = i & 7, c = j & 7;
-    return ((ib * (ib + 1)) / 2 + jb) * 64 + r * 8 + (c ^ ((r & 2) << 1));
-  }
-  __device__ __forceinline__ double &at(int i, int j) { return v[idx(i, j)]; }
-  __device__ __forceinline__ const double &at(int i, int j) const { return v[idx(i, j)]; }
-};
 
-template <int TM_, int STAGES_>
 struct Smem {
-  using G = Geo<TM_>;
-  static constexpr int TM = TM_;
-  static constexpr int STAGES = STAGES_;   // operand ring depth (look-ahead = STAGES - 1 chunks)
-  static constexpr int NTHREADS = G::NTHREADS;
-  double As[STAGES][TM_][KC];
+  double As[STAGES][TM][KC];
   double Bs[STAGES][NB][KC];
-  LdStore<G::PACKED> Ld;   // diagonal block L_jj (lower), valid after potf2
+  LdStore Ld;   // diagonal block L_jj (lower), valid after potf2
   double Dv[NB][DS];   // the 8 inverses of the 8x8 diagonal blocks of L_jj: Dv[8*nb + r][c]
   double red[NTHREADS / 32];
   double dpiv[NB];         // pivots L_ii^2 of the current diagonal block
@@ -194,10 +163,8 @@ __device__ __forceinline__ unsigned long long gtimer() {
 #define PROF_MARK(sm, k)
 #endif
 
-using SmemCluster = Smem<128, 3>;
-static_assert(offsetof(SmemCluster, Dv) == offsetof(SmemCluster, Ld) + sizeof(double) * NB * LS,
+static_assert(offsetof(Smem, Dv) == offsetof(Smem, Ld) + sizeof(double) * NB * LS,
               "Ld and Dv must be adjacent (copied as one block by the cluster kernel)");
-static_assert(sizeof(Smem<64, 3>) <= 75 * 1024, "three 4-warp CTAs must fit the shared memory of an SM");
 
 // element index inside a stage row: the TMA 128-byte swizzle (16-byte chunk index XOR row mod 8),
 // used by the cp.async path as well so that both fill the ring in the same layout
@@ -358,47 +325,22 @@ __device__ __forceinline__ void init_acc(const SM &sm, const RM &rm, const AffRo
 // Warps whose 16 rows are all beyond the last virtual row keep feeding the ring but issue no
 // tensor work.
 // ------------------------------------------------------------------------------------------
-// nt_lim < 8 (rows of the diagonal block): only the first nt_lim 8-column groups reach the
+// lim0 < 8 (warp w of the diagonal block): only the first lim0 = 2 w + 2 8-column groups reach the
 // diagonal, the rest of the warp tile is never consumed and is not multiplied.
 // `init` loads (and, on the fused path, transforms) the accumulators; it runs AFTER the first two
 // chunks have been requested so that its global-load latency -- and the dependent affine FMAs --
 // overlap the cp.async prologue instead of preceding it.
-// Rows of the DIAGONAL tile are dealt to warps 0-3 in 8-row blocks (w, 7 - w) instead of
-// (2 w, 2 w + 1): block b only needs its first b + 1 column groups, so every warp multiplies
-// (w + 1) + (8 - w) = 9 groups per k-step instead of 4 ... 16 -- the k-loop of the diagonal tile is
-// balanced and finishes in 9/16 of the time of its slowest warp under the natural order.
-// (Only the 4-warp geometry does this: with 8 warps the four warps below the diagonal block set the
-// pace of the tile anyway, and the natural order keeps the round-1 code path.)
-template <bool BAL>
-__device__ __forceinline__ int diag_block(int warp, int mt) {
-  return BAL ? (mt == 0 ? warp : 7 - warp) : 2 * warp + mt;
-}
-
-// Virtual row (RowMap) of m-tile mt, row g of this warp in the tile starting at v0.
-template <bool BAL>
-__device__ __forceinline__ int tile_vrow(bool diag_tile, int v0, int warp, int mt, int g) {
-  return (BAL && diag_tile && warp < 4) ? 8 * diag_block<BAL>(warp, mt) + g
-                                        : v0 + warp * 16 + mt * 8 + g;
-}
-
-template <class SM, class Init>
-__device__ __forceinline__ void gemm_tile(SM &sm, const RowMap &rm, int v0, int c0, int nvirt,
+template <class Init>
+__device__ __forceinline__ void gemm_tile(Smem &sm, const RowMap &rm, int v0, int c0, int nvirt,
                                           bool diag_tile, unsigned &it, double (&acc)[2][8][2],
                                           Init init, const CUtensorMap *tmK = nullptr,
                                           int item = 0) {
-  constexpr int TM = SM::TM, NTHREADS = SM::NTHREADS, STAGES = SM::STAGES, LA = SM::STAGES - 1;
-  constexpr bool BAL = SM::G::PACKED;   // 4-warp geometry
+  constexpr int LA = STAGES - 1;
   constexpr int RPP = NTHREADS / 8;      // rows covered by one pass of the per-thread copies
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, tg = lane & 3;
   const int nchunks = c0 / KC;
   const bool diag_warp = diag_tile && warp < 4;
-  // balanced geometry: tile-relative rows of this warp's two m-tiles and how many 8-column groups
-  // each one needs; natural order (8-warp geometry, the round-1 code path): rows 16 w + 8 mt, and both
-  // m-tiles of a diagonal warp stop at group 2 w + 1
-  const int ar0 = BAL ? tile_vrow<BAL>(diag_tile, v0, warp, 0, 0) - v0 : warp * 16;
-  const int ar1 = BAL ? tile_vrow<BAL>(diag_tile, v0, warp, 1, 0) - v0 : warp * 16 + 8;
-  const int lim0 = diag_warp ? (BAL ? diag_block<BAL>(warp, 0) + 1 : 2 * warp + 2) : 8;
-  const int lim1 = BAL ? (diag_warp ? diag_block<BAL>(warp, 1) + 1 : 8) : lim0;
+  const int lim0 = diag_warp ? 2 * warp + 2 : 8;
   PROF_DECL;
   if (nchunks == 0) {
     init();
@@ -486,68 +428,32 @@ __device__ __forceinline__ void gemm_tile(SM &sm, const RowMap &rm, int v0, int 
 #endif
     if (warp_live) {
       const double *Bw = &sm.Bs[st][g][0];
-      if constexpr (!BAL) {
-        // ---- 8-warp geometry: the round-1 inner loops, verbatim
-        const double *Aw = &sm.As[st][warp * 16 + g][0];
-        if (lim0 >= 8) {
+      const double *Aw = &sm.As[st][warp * 16 + g][0];
+      if (lim0 >= 8) {
 #pragma unroll
-          for (int kk = 0; kk < KC / 4; ++kk) {
-            double a[2], b[8];
+        for (int kk = 0; kk < KC / 4; ++kk) {
+          double a[2], b[8];
 #pragma unroll
-            for (int mt = 0; mt < 2; ++mt) a[mt] = negate(Aw[mt * 8 * KC + koff[kk]]);
+          for (int mt = 0; mt < 2; ++mt) a[mt] = negate(Aw[mt * 8 * KC + koff[kk]]);
 #pragma unroll
-            for (int nt = 0; nt < 8; ++nt) b[nt] = Bw[nt * 8 * KC + koff[kk]];
+          for (int nt = 0; nt < 8; ++nt) b[nt] = Bw[nt * 8 * KC + koff[kk]];
 #pragma unroll
-            for (int mt = 0; mt < 2; ++mt)
+          for (int mt = 0; mt < 2; ++mt)
 #pragma unroll
-              for (int nt = 0; nt < 8; ++nt) dmma_m8n8k4(acc[mt][nt][0], acc[mt][nt][1], a[mt], b[nt]);
-          }
-        } else {
-#pragma unroll
-          for (int kk = 0; kk < KC / 4; ++kk) {
-            double a[2];
-#pragma unroll
-            for (int mt = 0; mt < 2; ++mt) a[mt] = negate(Aw[mt * 8 * KC + koff[kk]]);
-#pragma unroll
-            for (int nt = 0; nt < 8; ++nt) {
-              if (nt < lim0) {
-                const double b = Bw[nt * 8 * KC + koff[kk]];
-#pragma unroll
-                for (int mt = 0; mt < 2; ++mt) dmma_m8n8k4(acc[mt][nt][0], acc[mt][nt][1], a[mt], b);
-              }
-            }
-          }
+            for (int nt = 0; nt < 8; ++nt) dmma_m8n8k4(acc[mt][nt][0], acc[mt][nt][1], a[mt], b[nt]);
         }
       } else {
-        const double *Aw0 = &sm.As[st][ar0 + g][0];
-        const double *Aw1 = &sm.As[st][ar1 + g][0];
-        if (!diag_warp) {
 #pragma unroll
-          for (int kk = 0; kk < KC / 4; ++kk) {
-            double a[2], b[8];
-            a[0] = negate(Aw0[koff[kk]]);
-            a[1] = negate(Aw1[koff[kk]]);
+        for (int kk = 0; kk < KC / 4; ++kk) {
+          double a[2];
 #pragma unroll
-            for (int nt = 0; nt < 8; ++nt) b[nt] = Bw[nt * 8 * KC + koff[kk]];
+          for (int mt = 0; mt < 2; ++mt) a[mt] = negate(Aw[mt * 8 * KC + koff[kk]]);
 #pragma unroll
-            for (int mt = 0; mt < 2; ++mt)
+          for (int nt = 0; nt < 8; ++nt) {
+            if (nt < lim0) {
+              const double b = Bw[nt * 8 * KC + koff[kk]];
 #pragma unroll
-              for (int nt = 0; nt < 8; ++nt) dmma_m8n8k4(acc[mt][nt][0], acc[mt][nt][1], a[mt], b[nt]);
-          }
-        } else {
-          // rows of the diagonal block: m-tile mt only reaches the diagonal in its first lim_mt
-          // 8-column groups; the rest of the warp tile is never consumed and is not multiplied
-#pragma unroll
-          for (int kk = 0; kk < KC / 4; ++kk) {
-            const double a0 = negate(Aw0[koff[kk]]);
-            const double a1 = negate(Aw1[koff[kk]]);
-#pragma unroll
-            for (int nt = 0; nt < 8; ++nt) {
-              if (nt < lim0 || nt < lim1) {   // warp-uniform
-                const double b = Bw[nt * 8 * KC + koff[kk]];
-                if (nt < lim0) dmma_m8n8k4(acc[0][nt][0], acc[0][nt][1], a0, b);
-                if (nt < lim1) dmma_m8n8k4(acc[1][nt][0], acc[1][nt][1], a1, b);
-              }
+              for (int mt = 0; mt < 2; ++mt) dmma_m8n8k4(acc[mt][nt][0], acc[mt][nt][1], a[mt], b);
             }
           }
         }
@@ -752,21 +658,18 @@ __device__ __forceinline__ double potf2_tile8(double &v0, double &v1, double &w0
 template <class SM>
 __device__ __forceinline__ void potf2_regs(SM &sm, double (&acc)[2][8][2], int warp, int lane) {
   const int g = lane >> 2, tg = lane & 3;
-  // 8-row blocks of the diagonal tile held by this warp (see diag_block): m-tile 0 -> block warp,
-  // m-tile 1 -> block 7 - warp; block b lives in columns 0 .. 8 b + 7
-  constexpr bool BAL = SM::G::PACKED;
-  const int rb[2] = {diag_block<BAL>(warp, 0), diag_block<BAL>(warp, 1)};
+  // 8-row blocks of the diagonal tile held by this warp: m-tile mt -> block 2 warp + mt; block b lives
+  // in columns 0 .. 8 b + 7
+  const int rb[2] = {2 * warp, 2 * warp + 1};
   bool bad = false;
   PROF_DECL;
 #pragma unroll
   for (int s = 0; s < 8; ++s) {
     PROF_MARK(sm, 14);
-    // owner of diagonal tile s.  balanced: warp s (m-tile 0) for s < 4, warp 7 - s (m-tile 1) for
-    // s >= 4; natural: warp s / 2, m-tile s % 2
-    if (warp == (BAL ? ((s < 4) ? s : 7 - s) : (s >> 1))) {
+    // owner of diagonal tile s: warp s / 2, m-tile s % 2
+    if (warp == (s >> 1)) {
       double w0, w1;
-      const int omt = BAL ? (s < 4 ? 0 : 1) : (s & 1);   // compile-time after unrolling
-      double &t0 = acc[omt][s][0], &t1 = acc[omt][s][1];
+      double &t0 = acc[s & 1][s][0], &t1 = acc[s & 1][s][1];
       const double dg = potf2_tile8(t0, t1, w0, w1, lane, bad);
       *reinterpret_cast<double2 *>(&sm.Ld.at(8 * s + g, 8 * s + 2 * tg)) = make_double2(t0, t1);
       *reinterpret_cast<double2 *>(&sm.Dv[8 * s + g][2 * tg]) = make_double2(w0, w1);
@@ -830,9 +733,7 @@ __device__ __forceinline__ void potf2_regs(SM &sm, double (&acc)[2][8][2], int w
   PROF_MARK(sm, 14);
 }
 
-template <class SM>
-__device__ __forceinline__ double block_sum(SM &sm, double v) {
-  constexpr int NTHREADS = SM::NTHREADS;
+__device__ __forceinline__ double block_sum(Smem &sm, double v) {
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   v = warp_sum(v);
   __syncthreads();
@@ -845,12 +746,10 @@ __device__ __forceinline__ double block_sum(SM &sm, double v) {
   return t;
 }
 
-template <int TM, int STAGES, int MIN_CTAS>
-__global__ void __launch_bounds__(Geo<TM>::NTHREADS, MIN_CTAS)
+__global__ void __launch_bounds__(NTHREADS, 2)
     potrf_lnlike_kernel(PotrfParams p, const __grid_constant__ CUtensorMap tmK) {
-  constexpr int NTHREADS = Geo<TM>::NTHREADS;
   extern __shared__ __align__(1024) unsigned char smem_raw[];   // TMA 128-byte swizzle: 1 KB aligned
-  Smem<TM, STAGES> &sm = *reinterpret_cast<Smem<TM, STAGES> *>(smem_raw);
+  Smem &sm = *reinterpret_cast<Smem *>(smem_raw);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, tg = lane & 3;
 
   int nitems;
@@ -959,14 +858,13 @@ __global__ void __launch_bounds__(Geo<TM>::NTHREADS, MIN_CTAS)
         diag_inverses(sm);
       }
       for (int v0 = 0; v0 < nvirt; v0 += TM) {
-        // MODE_FACTOR, first tile: rows 0..63 are the diagonal block (warps 0-3, 8-row blocks dealt
-        // as (w, 7 - w): tile_vrow); with TM = 128 rows 64..127 are the first rows below it (warps 4-7)
+        // MODE_FACTOR, first tile: rows 0..63 are the diagonal block (warps 0-3), rows 64..127 the
+        // first rows below it (warps 4-7)
         const bool diag_tile = (p.mode == MODE_FACTOR) && (v0 == 0);
         gemm_tile(sm, rm, v0, c0, nvirt, diag_tile, it, acc, [&]() {
 #pragma unroll
           for (int mt = 0; mt < 2; ++mt)
-            init_acc(sm, rm, af, p.aff_on != 0, tile_vrow<Geo<TM>::PACKED>(diag_tile, v0, warp, mt, g),
-                     c0, tg, full_panel, acc[mt]);
+            init_acc(sm, rm, af, p.aff_on != 0, v0 + warp * 16 + mt * 8 + g, c0, tg, full_panel, acc[mt]);
         }, p.use_tma ? &tmK : nullptr, item);   // acc = K - L L^T = P
 #ifdef SPB_POTRF_PROF
         _pt = clock64();
@@ -1037,338 +935,6 @@ __global__ void __launch_bounds__(Geo<TM>::NTHREADS, MIN_CTAS)
 #include "potrf_i8.cuh"
 
 // ------------------------------------------------------------------------------------------
-// Warp-specialised batch kernel: 4 COMPUTE warps (one 64-row tile at a time, 16 rows x 64 columns
-// per warp, exactly the arithmetic of potrf_lnlike_kernel<64, ...>) + 1 PRODUCER warp that does
-// nothing but feed the operand ring.
-//
-// Why (scripts/micro/ring_micro.cu, measured on B200): with the copies requested from inside the
-// compute warps -- whichever thread does it -- the k-loop of a lone CTA reaches 78 % of the DMMA
-// peak (88 % with two CTAs per SM): the issuing warp waits for the slowest sibling to release a
-// slot, pays the TMA issue latency, and everyone then waits for that warp.  With a dedicated
-// producer warp the same loop reaches 91 % (93 %).  The producer walks the same sequence of
-// (panel, tile, chunk) as the consumers, bounded only by the empty[] barriers, so the ring never
-// drains between tiles or panels; the only true dependence -- chunks that read columns written
-// during the previous panel -- is an mbarrier (`panel`) the compute warps arrive on after their
-// stores and fence.proxy.async.  Tiles that mix matrix rows with appended right-hand-side rows (and
-// every tile of MODE_SOLVE) are copied by the 32 producer lanes with cp.async into the same swizzle.
-// ------------------------------------------------------------------------------------------
-constexpr int WS_TM = 64;
-constexpr int WS_NCT = 128;              // compute threads
-constexpr int WS_NTHREADS = WS_NCT + 32;
-
-template <int STAGES_>
-struct SmemWS : Smem<WS_TM, STAGES_> {
-  uint64_t panel;   // panel complete (its global stores fenced): 1 arrival (compute thread 0)
-};
-
-__device__ __forceinline__ void cbar() {  // the 128 compute threads (named barrier 2)
-  asm volatile("bar.sync 2, 128;\n" ::: "memory");
-}
-
-template <class SM>
-__device__ __forceinline__ double block_sum_ws(SM &sm, double v) {
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  v = warp_sum(v);
-  cbar();
-  if (lane == 0) sm.red[warp] = v;
-  cbar();
-  double t = 0.0;
-#pragma unroll
-  for (int w = 0; w < WS_NCT / 32; ++w) t += sm.red[w];
-  cbar();
-  return t;
-}
-
-template <int STAGES, int MIN_CTAS>
-__global__ void __launch_bounds__(WS_NTHREADS, MIN_CTAS)
-    potrf_ws_kernel(PotrfParams p, const __grid_constant__ CUtensorMap tmK) {
-  constexpr int TM = WS_TM;
-  extern __shared__ __align__(1024) unsigned char smem_raw[];
-  using SM = SmemWS<STAGES>;
-  SM &sm = *reinterpret_cast<SM *>(smem_raw);
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, tg = lane & 3;
-  const bool producer = (warp == WS_NCT / 32);
-
-  const int nitems = (p.mode == MODE_FACTOR) ? p.B : (p.M + p.rows_per_cta - 1) / p.rows_per_cta;
-  if (tid == 0) {
-#pragma unroll
-    for (int st = 0; st < STAGES; ++st) {
-      mbar_init(&sm.full[st], 32);          // the 32 producer lanes (lane 0 carries the TMA bytes)
-      mbar_init(&sm.empty[st], WS_NCT / 32);  // one arrival per compute warp
-    }
-    mbar_init(&sm.panel, 1);
-  }
-  __syncthreads();
-  unsigned it = 0;       // running k-chunk count (ring slot / phase), identical in both roles
-  unsigned npanel = 0;   // running count of completed panels (phase of sm.panel)
-
-  for (int item = blockIdx.x; item < nitems;) {
-    RowMap rm;
-    rm.n = p.n;
-    rm.ld = p.ld;
-    rm.ldr = p.ldr;
-    rm.mode = p.mode;
-    double *quad_out;
-    if (p.mode == MODE_FACTOR) {
-      rm.Kb = p.K + (size_t)item * p.strideK;
-      rm.Rb = p.R ? p.R + (size_t)item * p.strideR : nullptr;
-      rm.M = p.R ? p.M : 0;
-      rm.rb = 0;
-      rm.nrhs = rm.M;
-      quad_out = p.quad ? p.quad + (size_t)item * p.M : nullptr;
-    } else {
-      rm.Kb = p.K;
-      rm.Rb = p.R;
-      rm.M = p.M;
-      rm.rb = item * p.rows_per_cta;
-      rm.nrhs = min(p.rows_per_cta, p.M - rm.rb);
-      quad_out = p.quad;
-    }
-
-    if (producer) {
-      // ================================ producer warp ================================
-      for (int c0 = 0; c0 < p.n; c0 += NB) {
-        rm.c0 = c0;
-        rm.nbelow = max(0, p.n - c0 - NB);
-        const int nvirt = (p.mode == MODE_FACTOR) ? NB + rm.nbelow + rm.M : rm.nrhs;
-        const int nchunks = c0 / KC;
-        // chunks >= dep read columns that the PREVIOUS panel of this matrix wrote
-        const int dep = (p.mode == MODE_FACTOR && c0 >= NB) ? (c0 - NB) / KC : nchunks;
-        bool waited = false;
-        for (int v0 = 0; v0 < nvirt; v0 += TM) {
-          const bool tma_tile = p.use_tma && p.mode == MODE_FACTOR && (c0 + v0 + TM <= p.n);
-          // rows copied by this lane on the cp.async path: A rows lane, lane + 32; B rows likewise
-          const double *arow[TM / 32], *brow[NB / 32];
-          int abytes[TM / 32], bbytes[NB / 32];
-          if (!tma_tile) {
-#pragma unroll
-            for (int i = 0; i < TM / 32; ++i) {
-              int kind;
-              double *q = rm.row(v0 + lane + 32 * i, kind);
-              arow[i] = q ? q : rm.Kb;
-              abytes[i] = q ? 16 : 0;
-            }
-#pragma unroll
-            for (int i = 0; i < NB / 32; ++i) {
-              const int r = c0 + lane + 32 * i;
-              brow[i] = (r < rm.n) ? rm.Kb + (size_t)r * rm.ld : rm.Kb;
-              bbytes[i] = (r < rm.n) ? 16 : 0;
-            }
-          }
-          for (int ch = 0; ch < nchunks; ++ch) {
-            if (!waited && ch >= dep) {
-              // previous panel complete and visible to the async proxy (npanel panels done so far)
-              mbar_wait(&sm.panel, (npanel + 1u) & 1u);
-              waited = true;
-            }
-            const unsigned x = it + ch;
-            const unsigned st = x % STAGES;
-            mbar_wait(&sm.empty[st], ((x / STAGES) + 1u) & 1u);   // slot released by every warp
-            if (tma_tile) {
-              if (lane == 0) {
-                mbar_arrive_expect_tx(&sm.full[st], (TM + NB) * KC * (unsigned)sizeof(double));
-                tma_load_3d(&sm.As[st][0][0], &tmK, &sm.full[st], ch * KC, c0 + v0, item);
-                tma_load_3d(&sm.Bs[st][0][0], &tmK, &sm.full[st], ch * KC, c0, item);
-              } else {
-                mbar_arrive(&sm.full[st]);
-              }
-            } else {
-#pragma unroll
-              for (int i = 0; i < TM / 32; ++i) {
-                const int r = lane + 32 * i;
-#pragma unroll
-                for (int sg = 0; sg < 8; ++sg)
-                  cp_async16(&sm.As[st][r][(sg ^ (r & 7)) << 1], arow[i] + ch * KC + 2 * sg, abytes[i]);
-              }
-#pragma unroll
-              for (int i = 0; i < NB / 32; ++i) {
-                const int r = lane + 32 * i;
-#pragma unroll
-                for (int sg = 0; sg < 8; ++sg)
-                  cp_async16(&sm.Bs[st][r][(sg ^ (r & 7)) << 1], brow[i] + ch * KC + 2 * sg, bbytes[i]);
-              }
-              mbar_cp_async_arrive(&sm.full[st]);
-            }
-          }
-          it += nchunks;
-        }
-        if (p.mode == MODE_FACTOR && c0 >= NB && !waited) {   // (nchunks > dep always: defensive)
-          mbar_wait(&sm.panel, (npanel + 1u) & 1u);
-        }
-        if (p.mode == MODE_FACTOR) npanel += 1;
-      }
-    } else {
-      // ================================ compute warps ================================
-      AffRow af;
-      af.q = nullptr;
-      af.dg = nullptr;
-      af.dg_vec = 0;
-      af.norm = false;
-      if (p.aff_on && p.mode == MODE_FACTOR) {
-        af.norm = (p.aff.scal != nullptr) && (p.aff.q != nullptr);
-        if (af.norm) af.q = p.aff.q + (size_t)item * p.n;
-        if (p.aff.diag) {
-          af.dg = p.aff.diag + (size_t)item * p.aff.diag_stride;
-          af.dg_vec = (p.aff.diag_kind == 1);
-        }
-        if (tid == 0) {
-          sm.af[0] = af.norm ? p.aff.scal[4 * (size_t)item + 0] : 1.0;
-          sm.af[1] = af.norm ? p.aff.scal[4 * (size_t)item + 1] : 0.0;
-          sm.af[2] = af.norm ? p.aff.scal[4 * (size_t)item + 2] : 0.0;
-          sm.af[3] = p.aff.offset ? p.aff.offset[(size_t)item * p.aff.offset_stride] : 0.0;
-        }
-      }
-      if (tid == 0) sm.bad = 0;
-      if (quad_out) {
-        if (p.mode == MODE_FACTOR) {
-          for (int m = tid; m < rm.M; m += WS_NCT) quad_out[m] = 0.0;
-        } else {
-          for (int m = tid; m < rm.nrhs; m += WS_NCT) quad_out[rm.rb + m] = 0.0;
-        }
-      }
-      cbar();
-
-      double logdet_part = 0.0, quad_part = 0.0;
-      double acc[2][8][2];
-      int koff[KC / 4];
-#pragma unroll
-      for (int kk = 0; kk < KC / 4; ++kk) koff[kk] = swz(g, kk * 4 + tg);
-
-      for (int c0 = 0; c0 < p.n; c0 += NB) {
-        rm.c0 = c0;
-        rm.nbelow = max(0, p.n - c0 - NB);
-        const int nvirt = (p.mode == MODE_FACTOR) ? NB + rm.nbelow + rm.M : rm.nrhs;
-        const int nchunks = c0 / KC;
-        const bool full_panel = (c0 + NB <= p.n);
-        if (p.mode == MODE_SOLVE) {
-          // fetch L_jj (identity-padded) and invert its 8x8 diagonal blocks
-          for (int idx = tid; idx < NB * NB; idx += WS_NCT) {
-            const int i = idx >> 6, j = idx & 63;
-            double v = 0.0;
-            if (j <= i) {
-              if (c0 + i < p.n) v = rm.Kb[(size_t)(c0 + i) * p.ld + c0 + j];
-              else v = (i == j) ? 1.0 : 0.0;
-            }
-            sm.Ld.at(i, j) = v;
-          }
-          cbar();
-          if (tid < 64) {
-            const int blk = tid >> 3, c = tid & 7, o = blk * 8;
-            double xs[8];
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-              double sacc = (i == c) ? 1.0 : 0.0;
-#pragma unroll
-              for (int k = 0; k < 8; ++k)
-                if (k < i && k >= c) sacc -= sm.Ld.at(o + i, o + k) * xs[k];
-              xs[i] = (i >= c) ? sacc / sm.Ld.at(o + i, o + i) : 0.0;
-            }
-#pragma unroll
-            for (int i = 0; i < 8; ++i) sm.Dv[o + i][c] = xs[i];
-          }
-          cbar();
-        }
-        for (int v0 = 0; v0 < nvirt; v0 += TM) {
-          const bool diag_tile = (p.mode == MODE_FACTOR) && (v0 == 0);
-          const bool warp_live = diag_tile || (v0 + warp * 16) < nvirt;
-          // accumulators <- K (or residual) rows: the loads overlap the wait for the first chunk
-#pragma unroll
-          for (int mt = 0; mt < 2; ++mt)
-            init_acc(sm, rm, af, p.aff_on != 0, tile_vrow<true>(diag_tile, v0, warp, mt, g), c0, tg,
-                     full_panel, acc[mt]);
-          // ---- k-loop: acc -= A[rows][k] L[c0 + cols][k], operands from the ring
-          const int ar0 = tile_vrow<true>(diag_tile, v0, warp, 0, 0) - v0;
-          const int ar1 = tile_vrow<true>(diag_tile, v0, warp, 1, 0) - v0;
-          const int lim0 = diag_tile ? diag_block<true>(warp, 0) + 1 : 8;
-          const int lim1 = diag_tile ? diag_block<true>(warp, 1) + 1 : 8;
-          for (int ch = 0; ch < nchunks; ++ch) {
-            const unsigned x = it + ch;
-            const unsigned st = x % STAGES;
-            mbar_wait(&sm.full[st], (x / STAGES) & 1u);
-            if (warp_live) {
-              const double *Aw0 = &sm.As[st][ar0 + g][0];
-              const double *Aw1 = &sm.As[st][ar1 + g][0];
-              const double *Bw = &sm.Bs[st][g][0];
-              if (!diag_tile) {
-#pragma unroll
-                for (int kk = 0; kk < KC / 4; ++kk) {
-                  double a[2], b[8];
-                  a[0] = negate(Aw0[koff[kk]]);
-                  a[1] = negate(Aw1[koff[kk]]);
-#pragma unroll
-                  for (int nt = 0; nt < 8; ++nt) b[nt] = Bw[nt * 8 * KC + koff[kk]];
-#pragma unroll
-                  for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-                    for (int nt = 0; nt < 8; ++nt)
-                      dmma_m8n8k4(acc[mt][nt][0], acc[mt][nt][1], a[mt], b[nt]);
-                }
-              } else {
-#pragma unroll
-                for (int kk = 0; kk < KC / 4; ++kk) {
-                  const double a0 = negate(Aw0[koff[kk]]);
-                  const double a1 = negate(Aw1[koff[kk]]);
-#pragma unroll
-                  for (int nt = 0; nt < 8; ++nt) {
-                    if (nt < lim0 || nt < lim1) {   // warp-uniform
-                      const double b = Bw[nt * 8 * KC + koff[kk]];
-                      if (nt < lim0) dmma_m8n8k4(acc[0][nt][0], acc[0][nt][1], a0, b);
-                      if (nt < lim1) dmma_m8n8k4(acc[1][nt][0], acc[1][nt][1], a1, b);
-                    }
-                  }
-                }
-              }
-            }
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&sm.empty[st]);
-          }
-          it += nchunks;
-          if (diag_tile) {
-            potf2_regs(sm, acc, warp, lane);
-            cbar();  // L_jj and the inverses of its diagonal tiles are in shared memory
-            if (tid < min(NB, p.n - c0)) logdet_part += 0.5 * log(sm.dpiv[tid]);
-            for (int idx = tid; idx < NB * NB; idx += WS_NCT) {
-              const int i = idx >> 6, j = idx & 63;
-              if (j <= i && c0 + i < p.n) rm.Kb[(size_t)(c0 + i) * p.ld + c0 + j] = sm.Ld.at(i, j);
-            }
-          } else if ((v0 + warp * 16) < nvirt) {
-            trsm_warp(sm, acc, lane);
-#pragma unroll
-            for (int mt = 0; mt < 2; ++mt)
-              store_rows(rm, v0 + warp * 16 + mt * 8 + g, c0, tg, acc[mt], quad_part, quad_out);
-          }
-        }
-        // this thread's st.global of the panel must be visible to the async proxy (TMA) before the
-        // producer is told that the panel is complete
-        fence_proxy_async_global();
-        cbar();  // Ld/Dv are rewritten by the next panel; every thread's stores + fence are done
-        if (p.mode == MODE_FACTOR && tid == 0) mbar_arrive(&sm.panel);
-      }
-
-      // ---- reductions -> lnlike
-      const double quad = block_sum_ws(sm, quad_part);
-      const double logdet = block_sum_ws(sm, logdet_part);
-      if (p.mode == MODE_FACTOR && tid == 0) {
-        const bool bad = sm.bad != 0;
-        double ll = -0.5 * quad - (double)rm.M * logdet -
-                    0.5 * (double)p.n * (double)rm.M * 1.8378770664093453;  // log(2 pi)
-        const int prev = p.info ? (p.info[item] & ~SPB_INFO_NOT_PD) : 0;
-        if (bad || (prev & (SPB_INFO_Z_RANGE | SPB_INFO_BOUNDS)) || ll != ll) ll = -INFINITY;
-        if (p.lnlike) p.lnlike[item] = ll;
-        if (p.logdet) p.logdet[item] = bad ? NAN : logdet;
-        if (p.info) p.info[item] = prev | (bad ? SPB_INFO_NOT_PD : 0);
-      }
-      if (tid == 0) sm.next_item = (int)gridDim.x + (int)atomicAdd(p.counter, 1u);
-    }
-    // both roles: the producer has requested every chunk of this matrix, the compute warps have
-    // consumed them; the next work item is published
-    __syncthreads();
-    // (both roles advanced `it` identically: they walk the same panels / tiles / chunks)
-    item = sm.next_item;   // rewritten only at the end of the next matrix, long after this read
-  }
-}
-
-// ------------------------------------------------------------------------------------------
 // Small batches (B <= #SM / 2): ONE MATRIX PER THREAD-BLOCK CLUSTER of 8, 4 or 2 CTAs (SMs).
 //
 // A lone CTA needs 2.3 ms for a 1000 x 1000 matrix (one SM's tensor pipe, every serial phase
@@ -1395,10 +961,9 @@ __device__ __forceinline__ void cluster_barrier() {
 }
 
 template <int CLUSTER>
-__global__ void __launch_bounds__(Geo<128>::NTHREADS, 1) potrf_cluster_kernel(PotrfParams p) {
-  constexpr int TM = 128, NTHREADS = Geo<128>::NTHREADS, STAGES = 3;
+__global__ void __launch_bounds__(NTHREADS, 1) potrf_cluster_kernel(PotrfParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  Smem<128, 3> &sm = *reinterpret_cast<Smem<128, 3> *>(smem_raw);
+  Smem &sm = *reinterpret_cast<Smem *>(smem_raw);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, tg = lane & 3;
   const int rank = (int)cluster_rank();
   const int item = blockIdx.x / CLUSTER;
@@ -1465,8 +1030,7 @@ __global__ void __launch_bounds__(Geo<128>::NTHREADS, 1) potrf_cluster_kernel(Po
       gemm_tile(sm, rm, v0, c0, nvirt, rank == 0, it, acc, [&]() {
 #pragma unroll
         for (int mt = 0; mt < 2; ++mt)
-          init_acc(sm, rm, af, p.aff_on != 0, tile_vrow<false>(rank == 0, v0, warp, mt, g), c0, tg,
-                   full_panel, acc[mt]);
+          init_acc(sm, rm, af, p.aff_on != 0, v0 + warp * 16 + mt * 8 + g, c0, tg, full_panel, acc[mt]);
       });
     }
     if (rank == 0) {
@@ -1565,41 +1129,14 @@ static int potrf_launch(spb_context *ctx, PotrfParams &p, void *stream) {
   }
   SPB_CHECK_CUDA(cudaSetDevice(ctx->device));
   p.scratch = nullptr;
-  const size_t smem = sizeof(Smem<128, 3>);   // cluster kernel and the TM = 128 batch kernel
-  // 0 = default: the 8-warp / 2-CTAs-per-SM geometry.  Measured inside the bench step on B200
-  // (profiles/r02_potrf_geometries.log): 55.9 ms per 4096 matrices against 57.5 ms for the 4-warp /
-  // 3-CTAs-per-SM geometry and 61.1 ms for the warp-specialised kernel -- the finer geometries win
-  // the k-loop (micro-benchmarks: 93 % of the DMMA peak with a producer warp against 88 %) but lose
-  // it again in the latency-bound phases, which stretch under two siblings instead of one.
-  int tile = ctx->opt_chol_tile;
-  if (tile == 0) tile = 128;
+  const size_t smem = sizeof(Smem);   // batch and cluster kernel
   static spb_once_flag attr_once;
   {
     const int st = spb_once_per_device(attr_once, ctx->device, [&]() -> int {
-#define SPB_POTRF_ATTR(TM_, S_, C_)                                                              \
-  SPB_CHECK_CUDA(cudaFuncSetAttribute(potrf_lnlike_kernel<TM_, S_, C_>,                          \
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize,               \
-                                      (int)sizeof(Smem<TM_, S_>)));                              \
-  SPB_CHECK_CUDA(cudaFuncSetAttribute(potrf_lnlike_kernel<TM_, S_, C_>,                          \
-                                      cudaFuncAttributePreferredSharedMemoryCarveout,            \
-                                      cudaSharedmemCarveoutMaxShared))
-      SPB_POTRF_ATTR(128, 3, 2);
-      SPB_POTRF_ATTR(64, 3, 3);
-      SPB_POTRF_ATTR(64, 5, 2);
-      SPB_POTRF_ATTR(64, 4, 2);
-      SPB_POTRF_ATTR(128, 6, 1);
-#undef SPB_POTRF_ATTR
-#define SPB_WS_ATTR(S_, C_)                                                                      \
-  SPB_CHECK_CUDA(cudaFuncSetAttribute(potrf_ws_kernel<S_, C_>,                                   \
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize,               \
-                                      (int)sizeof(SmemWS<S_>)));                                 \
-  SPB_CHECK_CUDA(cudaFuncSetAttribute(potrf_ws_kernel<S_, C_>,                                   \
-                                      cudaFuncAttributePreferredSharedMemoryCarveout,            \
-                                      cudaSharedmemCarveoutMaxShared))
-      SPB_WS_ATTR(3, 3);
-      SPB_WS_ATTR(4, 2);
-      SPB_WS_ATTR(5, 2);
-#undef SPB_WS_ATTR
+      SPB_CHECK_CUDA(cudaFuncSetAttribute(potrf_lnlike_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                          (int)smem));
+      SPB_CHECK_CUDA(cudaFuncSetAttribute(potrf_lnlike_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
+                                          cudaSharedmemCarveoutMaxShared));
       SPB_CHECK_CUDA(cudaFuncSetAttribute(potrf_cluster_kernel<8>,
                                           cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       SPB_CHECK_CUDA(cudaFuncSetAttribute(potrf_cluster_kernel<4>,
@@ -1625,7 +1162,7 @@ static int potrf_launch(spb_context *ctx, PotrfParams &p, void *stream) {
           const int c = 8 >> k;
           cudaLaunchConfig_t q = {};
           q.gridDim = dim3((unsigned)(c * ctx->num_sms));
-          q.blockDim = dim3(Geo<128>::NTHREADS);
+          q.blockDim = dim3(NTHREADS);
           q.dynamicSmemBytes = smem;
           cudaLaunchAttribute a[1];
           a[0].id = cudaLaunchAttributeClusterDimension;
@@ -1654,7 +1191,7 @@ static int potrf_launch(spb_context *ctx, PotrfParams &p, void *stream) {
     p.counter = nullptr;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)(p.B * cs));
-    cfg.blockDim = dim3(Geo<128>::NTHREADS);
+    cfg.blockDim = dim3(NTHREADS);
     cfg.dynamicSmemBytes = smem;
     cfg.stream = (cudaStream_t)stream;
     cudaLaunchAttribute attr[1];
@@ -1670,20 +1207,13 @@ static int potrf_launch(spb_context *ctx, PotrfParams &p, void *stream) {
     SPB_LAUNCH_CHECK(ctx);
     return 0;
   }
-  // geometry variants (spb_set_option "cholesky_tile"): 128 -> TM 128, 3 stages, 2 CTAs/SM;
-  // 64 -> TM 64, 3 stages, 3 CTAs/SM; experiments: 645 -> TM 64, 5 stages, 2 CTAs/SM;
-  // 644 -> TM 64, 4 stages, 2 CTAs/SM; 1286 -> TM 128, 6 stages, 1 CTA/SM
-  // warp-specialised kernel (producer warp): 163 -> 3 stages, 3 CTAs/SM; 164 -> 4 stages, 2 CTAs/SM;
-  // 165 -> 5 stages, 2 CTAs/SM
-  const int per_sm = (tile == 64 || tile == 163) ? 3 : (tile == 1286) ? 1 : 2;
-  const int tm_rows = (tile == 128 || tile == 1286) ? 128 : 64;
-  int grid = nitems < per_sm * ctx->num_sms ? nitems : per_sm * ctx->num_sms;
+  int grid = nitems < 2 * ctx->num_sms ? nitems : 2 * ctx->num_sms;   // 2 CTAs per SM
   // tensor map of the batch of matrices for the TMA-fed operand ring: (columns, rows, matrix),
   // boxes of 16 columns x 64 rows, 128-byte swizzle
   CUtensorMap tmK;
   memset(&tmK, 0, sizeof(tmK));
   p.use_tma = 0;
-  if (!ctx->opt_no_tma && p.mode == MODE_FACTOR && p.n >= tm_rows + NB) {
+  if (!ctx->opt_no_tma && p.mode == MODE_FACTOR && p.n >= TM + NB) {
     const unsigned long long sk = p.strideK > 0 ? (unsigned long long)p.strideK : (unsigned long long)p.n * p.ld;
     int st = spb_encode_tmap_3d_f64(&tmK, p.K, (unsigned long long)p.ld, (unsigned long long)p.n,
                                     (unsigned long long)p.B, (unsigned long long)p.ld * 8, sk * 8, KC,
@@ -1693,20 +1223,7 @@ static int potrf_launch(spb_context *ctx, PotrfParams &p, void *stream) {
   p.counter = ctx->d_counters +
       (__atomic_fetch_add(&ctx->counter_next, 1u, __ATOMIC_RELAXED) % SPB_NUM_COUNTERS);
   SPB_CHECK_CUDA(cudaMemsetAsync(p.counter, 0, sizeof(unsigned int), (cudaStream_t)stream));
-#define SPB_POTRF_GO(TM_, S_, C_)                                                               \
-  potrf_lnlike_kernel<TM_, S_, C_><<<grid, Geo<TM_>::NTHREADS, sizeof(Smem<TM_, S_>), (cudaStream_t)stream>>>(p, tmK)
-  if (tile == 163)
-    potrf_ws_kernel<3, 3><<<grid, WS_NTHREADS, sizeof(SmemWS<3>), (cudaStream_t)stream>>>(p, tmK);
-  else if (tile == 164)
-    potrf_ws_kernel<4, 2><<<grid, WS_NTHREADS, sizeof(SmemWS<4>), (cudaStream_t)stream>>>(p, tmK);
-  else if (tile == 165)
-    potrf_ws_kernel<5, 2><<<grid, WS_NTHREADS, sizeof(SmemWS<5>), (cudaStream_t)stream>>>(p, tmK);
-  else if (tile == 128) SPB_POTRF_GO(128, 3, 2);
-  else if (tile == 645) SPB_POTRF_GO(64, 5, 2);
-  else if (tile == 644) SPB_POTRF_GO(64, 4, 2);
-  else if (tile == 1286) SPB_POTRF_GO(128, 6, 1);
-  else SPB_POTRF_GO(64, 3, 3);
-#undef SPB_POTRF_GO
+  potrf_lnlike_kernel<<<grid, NTHREADS, smem, (cudaStream_t)stream>>>(p, tmK);
   SPB_LAUNCH_CHECK(ctx);
   return 0;
 }
@@ -1845,10 +1362,6 @@ extern "C" int spb_cholesky_lnlike_i8(spb_context *ctx, int B, int nt, double *K
   ip.LDQ = n64;
   ip.store_factor = 0;
   ip.lambda_min = lambda_min;
-  {
-    const char *e = getenv("SPB_I8_GATE");
-    ip.gate = e ? atoi(e) : 0;   // experiments only (bit 0: hold the MMA stream back during potf2 / TRSM)
-  }
   uintptr_t w = ((uintptr_t)workspace + 255) & ~(uintptr_t)255;
   ip.Q = reinterpret_cast<uint8_t *>(w);
   ip.strideQ = (long long)planes * ip.NR * ip.LDQ;
@@ -1884,9 +1397,8 @@ extern "C" int spb_cholesky_lnlike_i8(spb_context *ctx, int B, int nt, double *K
       SPB_I8_ATTR(7, 2, 7, true);
       SPB_I8_ATTR(7, 2, 8, true);
 #undef SPB_I8_ATTR
-      SPB_CHECK_CUDA(cudaFuncSetAttribute(potrf_lnlike_kernel<128, 3, 2>,
-                                          cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                          (int)sizeof(Smem<128, 3>)));
+      SPB_CHECK_CUDA(cudaFuncSetAttribute(potrf_lnlike_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                          (int)sizeof(Smem)));
       return 0;
     });
     if (st) return st;
@@ -1897,7 +1409,7 @@ extern "C" int spb_cholesky_lnlike_i8(spb_context *ctx, int B, int nt, double *K
   SPB_CHECK_CUDA(cudaMemsetAsync(p.counter, 0, sizeof(unsigned int), (cudaStream_t)stream));
   // 7-plane kernels, nt <= 1536: two ring stages + the cp.async prefetch of the next K tile (the per-tile
   // chain dominates there); larger nt: three ring stages (the MMA stream dominates, -8 % with two)
-  const bool kpre = (planes == 7) && nt <= 1536 && !getenv("SPB_I8_NO_KPRE");
+  const bool kpre = (planes == 7) && nt <= 1536;
 #define SPB_I8_GO(S_, ST_, RB_, KP_)                                                                    \
   potrf_i8_kernel<S_, ST_, RB_, KP_><<<grid, I8_NTHREADS, sizeof(SmemI8<S_, ST_, KP_>), (cudaStream_t)stream>>>(p, ip, tmA, tmB)
   if (planes == 8) SPB_I8_GO(8, 3, 7, false);
@@ -1917,7 +1429,7 @@ extern "C" int spb_cholesky_lnlike_i8(spb_context *ctx, int B, int nt, double *K
     CUtensorMap tmK;
     memset(&tmK, 0, sizeof(tmK));
     const int g2 = B < 2 * ctx->num_sms ? B : 2 * ctx->num_sms;
-    potrf_lnlike_kernel<128, 3, 2><<<g2, Geo<128>::NTHREADS, sizeof(Smem<128, 3>), (cudaStream_t)stream>>>(f, tmK);
+    potrf_lnlike_kernel<<<g2, NTHREADS, sizeof(Smem), (cudaStream_t)stream>>>(f, tmK);
     SPB_LAUNCH_CHECK(ctx);
   }
   return 0;
@@ -1945,13 +1457,9 @@ extern "C" int spb_cholesky_solve_rows(spb_context *ctx, int nt, const double *L
   p.aff = spb_affine{};
   p.aff_on = 0;
   p.mode = MODE_SOLVE;
-  // spread the RHS rows over the whole GPU in multiples of 16 rows (one warp's share)
   // one full 128-row tile per work item (a tile costs the same DMMA time however many of its
   // rows are live, so smaller items would only replicate the streaming of L)
-  {
-    const int tile = ctx->opt_chol_tile ? ctx->opt_chol_tile : 128;
-    p.rows_per_cta = (tile == 128 || tile == 1286) ? 128 : 64;
-  }
+  p.rows_per_cta = TM;
   return potrf_launch(ctx, p, stream);
 }
 

@@ -66,7 +66,6 @@ struct I8Params {
   int NR, LDQ;
   int store_factor;      // also write L (fp64) over K like the DMMA kernel
   double lambda_min;     // > 0: lower bound of the smallest eigenvalue of K' (else min(aff.diag))
-  int gate;              // pause the MMA stream while warps are in the shuffle / shared-memory bound phases
 };
 
 // Virtual rows of a panel for this kernel.  A tile's A operand must be ONE box of 128 consecutive plane
@@ -113,16 +112,14 @@ struct RowMapI8 {
 
 template <int S_, int STAGES_, bool KPRE_ = false>
 struct SmemI8 {
-  using G = Geo<128>;
   static constexpr int S = S_;
   static constexpr int STAGES = STAGES_;
-  static constexpr int NTHREADS = I8_NCT;
   uint8_t A[STAGES_][S_][I8_TM][I8_KCH];   // 4 KB per plane
   uint8_t B[STAGES_][S_][NB][I8_KCH];      // 2 KB per plane; planes t0..t1 form one N = 64 (t1 - t0 + 1) operand
   // KPRE: the 128 x 64 K tile of the NEXT tile, copied by cp.async while the current one is processed; chunk c
   // (of 16) of thread t at [(c * 256 + t)]: every thread reads back what it copied, conflict-free both ways
   double2 Kpre[KPRE_ ? 16 * I8_NCT : 1];
-  LdStore<false> Ld;
+  LdStore Ld;
   double Dv[NB][DS];
   double red[I8_NCT / 32];
   double dpiv[NB];
@@ -132,7 +129,6 @@ struct SmemI8 {
   unsigned first[I8_MAXP + 1];   // sequence number of the first tile of every panel of this matrix
   uint32_t tmem_base;
   volatile unsigned stored;      // tiles whose planes are in global memory (monotone over the launch)
-  int quiet;                     // number of warps inside potf2 / TRSM (the issuer holds back while > 0)
   int bad;
   int bad_range;
   int next_item;
@@ -197,15 +193,6 @@ __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.
 // warp on the same scheduler (measured: the shuffle-bound 8x8 pivot chain ran 3.5x slower next to one).
 __device__ __forceinline__ void mbar_wait_sleep(uint64_t *bar, unsigned parity, unsigned ns) {
   while (!mbar_test(bar, parity)) __nanosleep(ns);
-}
-// The tensor core reads its operands through the same shared-memory datapath the warps' SHFL / LDS use:
-// while the MMA stream runs, the shuffle-bound pivot chain of potf2 and the in-register TRSM run 2.5x
-// slower (measured with phase timers).  Warps announce those phases; the issuer holds back meanwhile.
-__device__ __forceinline__ void quiet_enter(int *q, int lane, bool on) {
-  if (on && lane == 0) atomicAdd(q, 1);
-}
-__device__ __forceinline__ void quiet_leave(int *q, int lane, bool on) {
-  if (on && lane == 0) atomicSub(q, 1);
 }
 __device__ __forceinline__ void cbar256() { asm volatile("bar.sync 2, 256;\n" ::: "memory"); }
 
@@ -304,7 +291,6 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
     mbar_init(&sm.tmem_full, 1);
     mbar_init(&sm.tmem_empty, I8_NCT / 32);
     sm.stored = 0;
-    sm.quiet = 0;
     asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
   }
 #ifdef SPB_POTRF_PROF
@@ -546,7 +532,6 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
           const int lw = warp;
           if (diag_tile) {
             if (lw < 4) {
-              quiet_enter(&sm.quiet, lane, (ip.gate & 1) != 0);
 #ifdef SPB_POTRF_PROF
               const unsigned long long t8_before = sm.prof[0][11];
 #endif
@@ -554,7 +539,6 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
 #ifdef SPB_POTRF_PROF
               if (tid == 0 && c0 == 0) sm.prof[0][15] += sm.prof[0][11] - t8_before;   // pivot chains of panel 0
 #endif
-              quiet_leave(&sm.quiet, lane, (ip.gate & 1) != 0);
             }
             cbar256();   // L_jj and the inverses of its diagonal tiles are in shared memory
             if (tid < min(NB, p.n - c0)) logdet_part += 0.5 * log(sm.dpiv[tid]);
@@ -571,9 +555,7 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
           const bool already_bad = (*(volatile int *)&sm.bad) != 0;
           const int vr2 = v0 + lw * 16;             // first tile row of this warp from here on
           if (!(diag_tile && lw < 4) && vr2 < nvirt) {
-            quiet_enter(&sm.quiet, lane, (ip.gate & 1) != 0);
             trsm_warp(sm, acc, lane);
-            quiet_leave(&sm.quiet, lane, (ip.gate & 1) != 0);
             I8_PROF(sm, 4);
 #pragma unroll
             for (int mt = 0; mt < 2; ++mt) {
@@ -750,8 +732,6 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
               const unsigned st = xchunk % STAGES;
               I8_PROF(sm, 2);
               mbar_wait_sleep(&sm.full[st], (xchunk / STAGES) & 1u, 50);
-              if (ip.gate & 1)
-                while (*(volatile int *)&sm.quiet > 0) __nanosleep(40);
               tc_fence_after();
               I8_PROF(sm, 1);
 #pragma unroll

@@ -11,7 +11,6 @@
 // multiply/add sequence as the reference's `g++ -O2` build, but PARALLEL over the (m', m) entries
 // of each degree (the reference walks them serially): one CTA per angle, the complex matrices
 // D[l] for all l kept in shared memory (43.6 KB).
-#include <stdlib.h>
 #include <string.h>
 
 #include "common.cuh"
@@ -206,9 +205,8 @@ __global__ void __launch_bounds__(256) tensordotRz_kernel(int K, const double *M
 //                     recurrences in registers; the row is produced degree by degree by the
 //                     fully unrolled body of design_gen.inc, which visits only the 1372
 //                     structurally non-zero entries of Rx(pi/2) (of 5456) and fetches their values
-//                     as warp-uniform 16-byte shared-memory broadcasts; four finished columns leave
-//                     with one 32-byte store (STG.256: a full DRAM sector per lane, no
-//                     shared-memory transposition).  2048 B written + 8 B read per row: the kernel
+//                     as warp-uniform 16-byte shared-memory broadcasts; finished columns leave
+//                     through TMA tensor stores.  2048 B written + 8 B read per row: the kernel
 //                     is bound by HBM writes (DESIGN.md "design matrix").
 // ------------------------------------------------------------------------------------------
 constexpr int DM_THREADS = 128;
@@ -243,33 +241,27 @@ __global__ void __launch_bounds__(256) design_v_kernel(int I, const double *rTA1
   *out = make_double2(acc, m < 0 ? -vb : vb);
 }
 
-// Store path variants (DESIGN.md records the measured choice):
-//   STORE_TMA = false  four finished columns leave with one 32-byte STG.256 per lane (a full DRAM
-//                      sector); simple, but a warp-wide store touches 32 different lines and costs
-//                      ~45 LSU data-pipe wavefronts, which makes the LSU the limiter;
-//   STORE_TMA = true   the warp collects a (32 timestamps x 16 columns) tile in shared memory --
-//                      128-byte rows in the TMA 128B-swizzle layout, so the lanes' 16-byte stores
-//                      are conflict-free -- and one elected lane hands it to the TMA engine
-//                      (cp.async.bulk.tensor.3d shared -> global through a tensor map of A, which
-//                      also clips the rows past nt); double-buffered per warp, the LSU only sees
-//                      the STS.128.
+// Store path: the warp collects a (32 timestamps x 16 columns) tile in shared memory -- 128-byte rows
+// in the TMA 128B-swizzle layout, so the lanes' 16-byte stores are conflict-free -- and one elected
+// lane hands it to the TMA engine (cp.async.bulk.tensor.3d shared -> global through a tensor map of A,
+// which also clips the rows past nt); double-buffered per warp, the LSU only sees the STS.128.
+// (DESIGN.md section 4.2 records it against direct 32-byte global stores.)
 // The 1372 coefficients come from shared memory as warp-uniform broadcasts.  (A constant-bank
 // variant -- LDCU into uniform registers -- measured 13 % slower: profiles/r01_time_design_variants.log.)
 constexpr int DM_CW = 16;                        // columns per TMA box (128 bytes)
 constexpr int DM_BOX_BYTES = 32 * DM_CW * 8;     // 32 rows x 128 B = 4096
 constexpr int DM_STAGE_BYTES = (DM_THREADS / 32) * 2 * DM_BOX_BYTES;
 
-template <bool STORE_TMA>
 __global__ void __launch_bounds__(DM_THREADS, 3)
     design_rows_kernel(DesignParams p, const __grid_constant__ CUtensorMap tmapA) {
   extern __shared__ __align__(1024) unsigned char dm_smem[];
   // the swizzle pattern is a function of the shared-memory ADDRESS: align the tiles to its 1 KB atom
   unsigned char *stage = dm_smem;                                          // [warp][2][4096]
-  if (STORE_TMA) {
+  {
     const unsigned a = (unsigned)__cvta_generic_to_shared(dm_smem);
     stage += (1024u - (a & 1023u)) & 1023u;
   }
-  double2 *Rs2 = reinterpret_cast<double2 *>(stage + (STORE_TMA ? DM_STAGE_BYTES : 0));
+  double2 *Rs2 = reinterpret_cast<double2 *>(stage + DM_STAGE_BYTES);
   double2 *Vs2 = Rs2 + RX90_NZ / 2;                                        // 256
   const int tid = threadIdx.x, ii = blockIdx.y, warp = tid >> 5, lane = tid & 31;
   for (int k = tid; k < RX90_NZ / 2; k += DM_THREADS)
@@ -282,8 +274,7 @@ __global__ void __launch_bounds__(DM_THREADS, 3)
   const int ntiles = (p.nt + DM_THREADS - 1) / DM_THREADS;
   for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
     const int t = tile * DM_THREADS + tid;
-    if (!STORE_TMA && t >= p.nt) continue;
-    // TMA path: rows past nt are computed on a clamped timestamp and clipped by the tensor map
+    // rows past nt are computed on a clamped timestamp and clipped by the tensor map
     const double x = p.t[t < p.nt ? t : p.nt - 1] / per;
     const double theta = 2.0 * 3.14159265358979323846 * (x - floor(x));  // tt.mod(t/p, 1)
     double cs[16], sn[16];
@@ -296,13 +287,11 @@ __global__ void __launch_bounds__(DM_THREADS, 3)
       cs[k] = 2.0 * cs[k - 1] * cs[1] - cs[k - 2];
       sn[k] = 2.0 * sn[k - 1] * cs[1] - sn[k - 2];
     }
-    double *Arow = p.A + ((size_t)ii * p.nt + t) * 256;
     const int trow0 = tile * DM_THREADS + warp * 32;   // first timestamp of this warp's tile
     double o0, o1, o2, o3;
 #define RS2(q) Rs2[q]
-    if (STORE_TMA) {
-      // chunk q uses buffer q & 1; before refilling it, the store issued two chunks ago must have
-      // finished reading shared memory (at most the most recent store may still be in flight)
+    // chunk q uses buffer q & 1; before refilling it, the store issued two chunks ago must have
+    // finished reading shared memory (at most the most recent store may still be in flight)
 #define DM_BEGIN(q)                                                                 \
   do {                                                                              \
     if (lane == 0) bulk_wait_read<1>();                                             \
@@ -328,18 +317,9 @@ __global__ void __launch_bounds__(DM_THREADS, 3)
 #undef DM_BEGIN
 #undef DM_STORE4
 #undef DM_FLUSH
-    } else {
-#define DM_BEGIN(q)
-#define DM_STORE4(c, a, b, cc, d) st_global_256(Arow + (c), a, b, cc, d)
-#define DM_FLUSH(q)
-#include "design_gen.inc"
-#undef DM_BEGIN
-#undef DM_STORE4
-#undef DM_FLUSH
-    }
 #undef RS2
   }
-  if (STORE_TMA && lane == 0) bulk_wait_read<0>();  // TMA must be done reading this CTA's shared memory
+  if (lane == 0) bulk_wait_read<0>();  // TMA must be done reading this CTA's shared memory
 }
 
 }  // namespace
@@ -411,28 +391,22 @@ extern "C" int spb_design_matrix(spb_context *ctx, int I, int nt, const double *
     if (gx > ntiles) gx = ntiles;
   }
   dim3 grid(gx, I);
-  static const int variant = getenv("SPB_DESIGN_VARIANT") ? atoi(getenv("SPB_DESIGN_VARIANT")) : 0;
-  const size_t smem_base = (RX90_NZ / 2 + 256) * sizeof(double2);
-  const size_t smem_tma = smem_base + DM_STAGE_BYTES + 1024;
+  const size_t smem = (RX90_NZ / 2 + 256) * sizeof(double2) + DM_STAGE_BYTES + 1024;
   CUtensorMap tmap;
   memset(&tmap, 0, sizeof(tmap));
-  if (variant != 1) {
-    // 3-D view of A: (256 columns, nt timestamps, I inclinations), box = 16 columns x 32 timestamps,
-    // 128-byte swizzle (matches the kernel's shared-memory tile layout)
-    int st = spb_encode_tmap_3d_f64(&tmap, A, 256, (unsigned long long)nt, (unsigned long long)I,
-                                    256ull * 8, (unsigned long long)nt * 256 * 8, DM_CW, 32, 1);
-    if (st) return st;
-    static spb_once_flag attr_once;
-    st = spb_once_per_device(attr_once, ctx->device, [&]() -> int {
-      SPB_CHECK_CUDA(cudaFuncSetAttribute(design_rows_kernel<true>,
-                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_tma));
-      return 0;
-    });
-    if (st) return st;
-    design_rows_kernel<true><<<grid, DM_THREADS, smem_tma, stream>>>(p, tmap);
-  } else {
-    design_rows_kernel<false><<<grid, DM_THREADS, smem_base, stream>>>(p, tmap);
-  }
+  // 3-D view of A: (256 columns, nt timestamps, I inclinations), box = 16 columns x 32 timestamps,
+  // 128-byte swizzle (matches the kernel's shared-memory tile layout)
+  int st = spb_encode_tmap_3d_f64(&tmap, A, 256, (unsigned long long)nt, (unsigned long long)I,
+                                  256ull * 8, (unsigned long long)nt * 256 * 8, DM_CW, 32, 1);
+  if (st) return st;
+  static spb_once_flag attr_once;
+  st = spb_once_per_device(attr_once, ctx->device, [&]() -> int {
+    SPB_CHECK_CUDA(cudaFuncSetAttribute(design_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                        (int)smem));
+    return 0;
+  });
+  if (st) return st;
+  design_rows_kernel<<<grid, DM_THREADS, smem, stream>>>(p, tmap);
   SPB_LAUNCH_CHECK(ctx);
   return 0;
 }

@@ -268,66 +268,44 @@ def test_full_step_is_deterministic_run_to_run(spb, golden):
             assert torch.equal(ll, first), "run %d differs from run 0" % rep
 
 
-@pytest.mark.parametrize("tile", [64, 163, 164])
-def test_cholesky_alternative_geometries_bitwise(spb, tile):
-    """The 4-warp / 3-CTAs-per-SM geometry (packed L_jj, balanced diagonal tile) and the
-    warp-specialised kernels (producer warp feeding the ring) perform the same arithmetic per tile as
-    the default 8-warp kernel: identical factors and solved rows, bit for bit, with and without
-    TMA, incl. ragged sizes, many right-hand-side rows and a non positive-definite element."""
+@pytest.mark.parametrize("B, n, M", [(5, 1, 1), (3, 70, 2), (4, 257, 140), (300, 333, 1), (40, 1000, 3)])
+def test_cholesky_rings_bitwise_ragged_shapes(spb, B, n, M):
+    """The batch kernel with its operand ring fed by TMA and by cp.async: identical factors, solved rows
+    and info, bit for bit, and the same lnlike, on ragged sizes (partial last panel), many right-hand-side
+    rows and a non positive-definite element (flagged, lnlike = -inf, the other matrices unaffected)."""
     ctx = spb.get_context(0)
+    ld = n + (n & 1)
+    gen = torch.Generator(device="cuda").manual_seed(n)
+    A = torch.randn(B, n, 24, dtype=torch.float64, device="cuda", generator=gen)
+    K0 = torch.zeros(B, n, ld, dtype=torch.float64, device="cuda")
+    K0[:, :, :n] = torch.bmm(A, A.transpose(1, 2)) / 24 + 0.7 * torch.eye(n, dtype=torch.float64, device="cuda")
+    if n > 50:
+        K0[1, 40, 40] = -3.0
+    R0 = torch.zeros(B, M, ld, dtype=torch.float64, device="cuda")
+    R0[:, :, :n] = torch.randn(B, M, n, dtype=torch.float64, device="cuda", generator=gen)
+    outs = {}
     try:
-        for (B, n, M) in [(5, 1, 1), (3, 70, 2), (4, 257, 140), (300, 333, 1), (40, 1000, 3)]:
-            ld = n + (n & 1)
-            gen = torch.Generator(device="cuda").manual_seed(n)
-            A = torch.randn(B, n, 24, dtype=torch.float64, device="cuda", generator=gen)
-            K0 = torch.zeros(B, n, ld, dtype=torch.float64, device="cuda")
-            K0[:, :, :n] = torch.bmm(A, A.transpose(1, 2)) / 24 + 0.7 * torch.eye(
-                n, dtype=torch.float64, device="cuda")
-            if n > 50:
-                K0[1, 40, 40] = -3.0
-            R0 = torch.zeros(B, M, ld, dtype=torch.float64, device="cuda")
-            R0[:, :, :n] = torch.randn(B, M, n, dtype=torch.float64, device="cuda", generator=gen)
-            outs = {}
-            for t_, tma in ((128, 1), (tile, 1), (tile, 0)):
-                ctx.set_option("cholesky_tile", t_)
-                ctx.set_option("cholesky_tma", tma)
-                ctx.set_option("cholesky_cluster", 0)
-                K, R = K0.clone(), R0.clone()
-                ll = torch.zeros(B, dtype=torch.float64, device="cuda")
-                info = torch.zeros(B, dtype=torch.int32, device="cuda")
-                assert ctx.lib.spb_cholesky_lnlike(ctx.handle, B, n, P(K), ld, n * ld, M, P(R), ld,
-                                                   M * ld, P(ll), None, None, P(info), None) == 0
-                torch.cuda.synchronize()
-                outs[(t_, tma)] = (torch.tril(K[:, :, :n]), R, ll, info)
-            ref = outs[(128, 1)]
-            ok = [b for b in range(B) if not (n > 50 and b == 1)]
-            for key, o in outs.items():
-                assert torch.equal(o[3], ref[3]), key
-                assert torch.equal(o[0][ok], ref[0][ok]) and torch.equal(o[1][ok], ref[1][ok]), key
-                assert float((o[2][ok] - ref[2][ok]).abs().max()) <= 1e-13 * float(
-                    ref[2][ok].abs().max()), key
-            if n > 50:
-                assert int(ref[3][1]) == 1 and bool(torch.isneginf(ref[2][1]))
-        # the many-right-hand-side solve (MODE_SOLVE) under the alternative geometry
-        n, M = 1000, 300
-        gen = torch.Generator(device="cuda").manual_seed(9)
-        A = torch.randn(n, 50, dtype=torch.float64, device="cuda", generator=gen)
-        L = torch.linalg.cholesky(A @ A.T / 50 + 0.5 * torch.eye(n, dtype=torch.float64, device="cuda"))
-        R0 = torch.randn(M, n, dtype=torch.float64, device="cuda", generator=gen)
-        res = {}
-        for t_ in (128, tile):
-            ctx.set_option("cholesky_tile", t_)
-            R = R0.clone()
-            quad = torch.zeros(M, dtype=torch.float64, device="cuda")
-            assert ctx.lib.spb_cholesky_solve_rows(ctx.handle, n, P(L), n, M, P(R), n, P(quad), None) == 0
+        ctx.set_option("cholesky_cluster", 0)
+        for tma in (1, 0):
+            ctx.set_option("cholesky_tma", tma)
+            K, R = K0.clone(), R0.clone()
+            ll = torch.zeros(B, dtype=torch.float64, device="cuda")
+            info = torch.zeros(B, dtype=torch.int32, device="cuda")
+            assert ctx.lib.spb_cholesky_lnlike(ctx.handle, B, n, P(K), ld, n * ld, M, P(R), ld, M * ld, P(ll),
+                                               None, None, P(info), None) == 0
             torch.cuda.synchronize()
-            res[t_] = (R, quad)
-        assert torch.equal(res[tile][0], res[128][0])
-        assert float((res[tile][1] - res[128][1]).abs().max()) <= 1e-12 * float(res[128][1].abs().max())
+            outs[tma] = (torch.tril(K[:, :, :n]), R, ll, info)
     finally:
-        ctx.set_option("cholesky_tile", 0)
         ctx.set_option("cholesky_tma", 1)
         ctx.set_option("cholesky_cluster", 1)
+    ref, o = outs[1], outs[0]
+    ok = [b for b in range(B) if not (n > 50 and b == 1)]
+    assert torch.equal(o[3], ref[3])
+    assert torch.equal(o[0][ok], ref[0][ok]) and torch.equal(o[1][ok], ref[1][ok])
+    assert float((o[2][ok] - ref[2][ok]).abs().max()) <= 1e-13 * float(ref[2][ok].abs().max())
+    assert int(ref[3][ok].abs().sum()) == 0 and bool(torch.isfinite(ref[2][ok]).all())
+    if n > 50:
+        assert int(ref[3][1]) == 1 and bool(torch.isneginf(ref[2][1]))
 
 
 # ------------------------------------------------------------------------- uniform spot-size prior

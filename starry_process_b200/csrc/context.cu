@@ -113,22 +113,28 @@ typedef CUresult (*spb_encode_fn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t
                                   const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
+// The driver's cuTensorMapEncodeTiled, looked up once (thread-safe).
+static int spb_encode_fn_get(spb_encode_fn *out) {
+  static spb_encode_fn fn = nullptr;
+  static std::mutex mu;
+  std::lock_guard<std::mutex> lock(mu);
+  if (!fn) {
+    void *ptr = nullptr;
+    cudaDriverEntryPointQueryResult qres;
+    SPB_CHECK_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &qres));
+    SPB_REQUIRE(ptr != nullptr && qres == cudaDriverEntryPointSuccess,
+                "cuTensorMapEncodeTiled is not available in this driver");
+    fn = reinterpret_cast<spb_encode_fn>(ptr);
+  }
+  *out = fn;
+  return 0;
+}
+
 int spb_encode_tmap_3d_f64(CUtensorMap *out, void *base, unsigned long long d0,
                            unsigned long long d1, unsigned long long d2, unsigned long long s1,
                            unsigned long long s2, unsigned b0, unsigned b1, unsigned b2) {
-  static spb_encode_fn fn = nullptr;
-  static std::mutex mu;
-  {
-    std::lock_guard<std::mutex> lock(mu);
-    if (!fn) {
-      void *ptr = nullptr;
-      cudaDriverEntryPointQueryResult qres;
-      SPB_CHECK_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &qres));
-      SPB_REQUIRE(ptr != nullptr && qres == cudaDriverEntryPointSuccess,
-                  "cuTensorMapEncodeTiled is not available in this driver");
-      fn = reinterpret_cast<spb_encode_fn>(ptr);
-    }
-  }
+  spb_encode_fn fn;
+  if (const int st = spb_encode_fn_get(&fn)) return st;
   cuuint64_t dims[3] = {d0, d1, d2};
   cuuint64_t strides[2] = {s1, s2};
   cuuint32_t box[3] = {b0, b1, b2};
@@ -143,19 +149,8 @@ int spb_encode_tmap_3d_f64(CUtensorMap *out, void *base, unsigned long long d0,
 // 4-D tensor map of bytes (digit planes of the INT8 Cholesky path), 32-byte swizzle.
 int spb_encode_tmap_u8_4d(CUtensorMap *out, void *base, const unsigned long long dims_[4],
                           const unsigned long long strides_[3], const unsigned box_[4]) {
-  static spb_encode_fn fn = nullptr;
-  static std::mutex mu;
-  {
-    std::lock_guard<std::mutex> lock(mu);
-    if (!fn) {
-      void *ptr = nullptr;
-      cudaDriverEntryPointQueryResult qres;
-      SPB_CHECK_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &qres));
-      SPB_REQUIRE(ptr != nullptr && qres == cudaDriverEntryPointSuccess,
-                  "cuTensorMapEncodeTiled is not available in this driver");
-      fn = reinterpret_cast<spb_encode_fn>(ptr);
-    }
-  }
+  spb_encode_fn fn;
+  if (const int st = spb_encode_fn_get(&fn)) return st;
   cuuint64_t dims[4] = {dims_[0], dims_[1], dims_[2], dims_[3]};
   cuuint64_t strides[3] = {strides_[0], strides_[1], strides_[2]};
   cuuint32_t box[4] = {box_[0], box_[1], box_[2], box_[3]};

@@ -40,6 +40,7 @@
 #include <string.h>
 
 #include "common.cuh"
+#include "i8_planes.cuh"
 
 namespace cg = cooperative_groups;
 

@@ -2,26 +2,18 @@
 // Included by potrf.cu inside its anonymous namespace (shares RowMap, init_acc, potf2_regs, trsm_warp).
 //
 // FP64 has no tcgen05 form, but the panel update  P = K - L L^T  is a sum of products of numbers whose
-// magnitude is known in advance (|L_ik| <= sqrt(K_ii)), so it can be evaluated EXACTLY in integer
-// arithmetic (Ozaki-style error-free slicing; accuracy study: oracle/study/ozaki_cholesky.py,
-// micro-benchmark: scripts/micro/i8_emul_micro.cu):
+// magnitude is known in advance (|L_ik| <= sqrt(K_ii)), so it is evaluated exactly on INT8 digit planes
+// (i8_planes.cuh: digit format, MMA stream, TMEM read-back):
 //
-//   * every stored row of L (and of the appended right-hand sides y = L^-1 r) is scaled by a power of
-//     two 2^-e_i fixed before the factorisation starts, rounded to S x RB bits and cut into S signed
-//     RB-bit digits  L_ik 2^-e_i = sum_s d_s(i,k) 2^{-RB (s+1)};  the digits are stored as S int8 PLANES
-//     next to K.  Default: S = 7 planes of balanced RB = 8-bit digits (55 bits per row, 28 plane
-//     products); S = 8 x RB = 7 (56 bits, 36 products) and S = 7 x RB = 7 (49 bits) are kept;
-//   * for a 128 x 64 tile of the panel, one thread issues  tcgen05.mma.kind::i8  products of digit plane
-//     A_s (128 x 32 bytes of k) with the concatenated planes B_0 .. B_{D-s} (N up to 256) into TMEM:
-//     pairs with s + t = d accumulate EXACTLY (int32) in the 64-column block d, all 512 columns of an SM
-//     hold the D + 1 = S blocks of the tile; operands arrive by TMA (32-byte swizzle) in a shared
-//     memory ring; the tensor core runs from smem descriptors, so no warp touches the operands;
-//   * the 8 compute warps read the S blocks back with fragment-shaped tcgen05.ld (16x256b: the same
-//     (row g, columns 2 tg) layout as the DMMA accumulators), combine them in fp64
-//     (Horner in 2^-RB), apply the row scales and subtract from the K values of the tile (copied to
-//     shared memory by cp.async during the previous tile when nt <= 1536, loaded directly otherwise);
-//     from there on the tile is the round-1 kernel's: in-register potf2 of the diagonal block, in-register
-//     TRSM on DMMA, |y|^2 and log-determinant reductions;
+//   * every stored row of L (and of the appended right-hand sides y = L^-1 r) gets its scale 2^e_i before
+//     the factorisation starts; its digits are stored as S int8 planes next to K.  Default: S = 7 planes of
+//     balanced RB = 8-bit digits (55 bits per row); S = 8 x RB = 7 (56 bits) and S = 7 x RB = 7 (49 bits)
+//     are kept;
+//   * for a 128 x 64 tile of the panel the MMA stream accumulates the plane products of the already factored
+//     columns in TMEM; the 8 compute warps combine the S blocks in fp64, apply the row scales and subtract
+//     from the K values of the tile (copied to shared memory by cp.async during the previous tile when
+//     nt <= 1536, loaded directly otherwise); from there on the tile is the round-1 kernel's: in-register
+//     potf2 of the diagonal block, in-register TRSM on DMMA, |y|^2 and log-determinant reductions;
 //   * the new rows of L are cut into digit planes straight from the accumulator registers and stored;
 //     the producer thread waits for exactly the tiles a k-chunk needs (a monotone counter of stored
 //     tiles), so the MMA stream of the next tile -- and of the next PANEL, up to its last two k-chunks --
@@ -44,20 +36,8 @@
 #define I8_PROF(sm, k)
 #endif
 
-constexpr int I8_KCH = 32;           // bytes of k per ring stage = K of one tcgen05.mma.kind::i8
-// digit width RB (template parameter): 7 -> digits in [-64, 63] except the leading one, which uses the whole
-// int8 range (|x| <= 0.99); 8 -> balanced base-256 digits in [-128, 127], all planes use the whole range, the
-// rows are scaled to |x| <= 1/2: 7 planes then carry 55 bits -- one bit less than 8 planes of 7 bits with 28
-// instead of 36 plane products and 7/8 of the operand traffic
-constexpr int I8_NCT = 256;          // compute threads (warps 0-7)
-#ifndef I8_ROLE_WARP0
-#define I8_ROLE_WARP0 8
-#endif
-constexpr int I8_PRODUCER_WARP = I8_ROLE_WARP0;        // TMA producer (one thread)
-constexpr int I8_ISSUER_WARP = I8_ROLE_WARP0 + 1;      // MMA issuer (one thread)
-constexpr int I8_NTHREADS = 32 * (I8_ROLE_WARP0 + 2);
 constexpr int I8_MAXP = 256;         // panels per matrix (nt <= 16384)
-constexpr int I8_TM = 128;
+static_assert(NB == I8_TN, "a panel is one TMEM block wide");
 
 struct I8Params {
   uint8_t *Q;            // (B, S, NR, LDQ) digit planes
@@ -137,72 +117,7 @@ struct SmemI8 {
 #endif
 };
 
-__device__ __forceinline__ void tma_load_4d(void *sdst, const void *tmap, uint64_t *bar, int c0, int c1,
-                                            int c2, int c3) {
-  unsigned s = (unsigned)__cvta_generic_to_shared(sdst);
-  unsigned b = (unsigned)__cvta_generic_to_shared(bar);
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];\n" ::"r"(s),
-      "l"(tmap), "r"(b), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-      : "memory");
-}
-__device__ __forceinline__ uint64_t i8_smem_desc(const void *p) {
-  // K-major operand, 32-byte swizzle: rows of 32 B, 8-row groups 256 B apart, descriptor version 1
-  const uint32_t a = (uint32_t)__cvta_generic_to_shared(p);
-  uint64_t d = (uint64_t)((a >> 4) & 0x3FFF);
-  d |= (uint64_t)1 << 16;
-  d |= (uint64_t)(256 >> 4) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)6 << 61;
-  return d;
-}
-__device__ __forceinline__ uint32_t i8_idesc(int n) {
-  // D = s32, A = B = signed 8 bit, both K-major, M = 128
-  return (2u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(I8_TM >> 4) << 24);
-}
-__device__ __forceinline__ void i8_mma(uint32_t tmem_d, uint64_t da, uint64_t db, uint32_t idesc,
-                                       uint32_t accumulate) {
-  asm volatile(
-      "{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\n"
-      "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n}\n" ::"r"(tmem_d),
-      "l"(da), "l"(db), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void i8_commit(uint64_t *bar) {
-  const uint32_t a = (uint32_t)__cvta_generic_to_shared(bar);
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];\n" ::"r"(a)
-               : "memory");
-}
-__device__ __forceinline__ void tc_fence_before() {
-  asm volatile("tcgen05.fence::before_thread_sync;\n" ::: "memory");
-}
-__device__ __forceinline__ void tc_fence_after() {
-  asm volatile("tcgen05.fence::after_thread_sync;\n" ::: "memory");
-}
-// 16 lanes x 256 bit, x2 = 16 columns: for each 8-column block b, v[4 b], v[4 b + 1] = (row T/4,
-// columns 2 (T%4), +1) and v[4 b + 2], v[4 b + 3] = (row T/4 + 8, same columns): the DMMA C layout
-__device__ __forceinline__ void tmem_ld_frag16(uint32_t taddr, uint32_t (&v)[8]) {
-  asm volatile("tcgen05.ld.sync.aligned.16x256b.x2.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];\n"
-               : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
-               : "r"(taddr)
-               : "memory");
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;\n" ::: "memory"); }
-// Waits of the two single-thread roles: poll with a sleep in between.  A tight try_wait loop keeps the
-// warp permanently eligible and its barrier probes share the LSU path with the SHFL / LDS of the compute
-// warp on the same scheduler (measured: the shuffle-bound 8x8 pivot chain ran 3.5x slower next to one).
-__device__ __forceinline__ void mbar_wait_sleep(uint64_t *bar, unsigned parity, unsigned ns) {
-  while (!mbar_test(bar, parity)) __nanosleep(ns);
-}
 __device__ __forceinline__ void cbar256() { asm volatile("bar.sync 2, 256;\n" ::: "memory"); }
-
-// smallest power of two 2^e with 1.0101 x < 2^e  (x / 2^e <= 0.99: the leading digit fits int8)
-__device__ __forceinline__ double pow2_above(double x) {
-  if (!(x > 0.0) || !(x < 1e300)) return 1.0;
-  int ex;
-  (void)frexp(x * 1.0101, &ex);
-  return ldexp(1.0, ex);
-}
 
 // The fused affine map (spb_affine) of one accumulator row that holds RAW values of a full panel (the
 // arithmetic half of init_acc; used when the values come from the cp.async prefetch buffer).
@@ -251,13 +166,6 @@ __device__ __forceinline__ double block_min_i8(SM &sm, double v) {
   return t;
 }
 
-// sum_{j < S} 64 128^j: makes every base-128 digit of a signed S-digit number non-negative
-__host__ __device__ constexpr long long i8_bias(int S, int RB) {
-  long long b = 0;
-  for (int j = 0; j < S; ++j) b = (b << RB) + (1ll << (RB - 1));
-  return b;
-}
-
 // number of 128-row tiles of the panel starting at column c0 (NR = nt + M virtual rows in total)
 __device__ __forceinline__ int i8_nbel(int n, int n64, bool gap, int c0) {
   return gap ? ((c0 + NB <= n) ? n - c0 - NB : 0) : n64 - c0 - NB;
@@ -271,7 +179,6 @@ template <int S, int STAGES, int RB, bool KPRE>
 __global__ void __launch_bounds__(I8_NTHREADS, 1)
     potrf_i8_kernel(PotrfParams p, I8Params ip, const __grid_constant__ CUtensorMap tmA,
                     const __grid_constant__ CUtensorMap tmB) {
-  constexpr int D = S - 1;
   extern __shared__ __align__(1024) unsigned char smem_raw[];
   using SM = SmemI8<S, STAGES, KPRE>;
   SM &sm = *reinterpret_cast<SM *>(smem_raw);
@@ -283,25 +190,14 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
   const int NR = ip.NR;
 
   if (tid == 0) {
-#pragma unroll
-    for (int s = 0; s < STAGES; ++s) {
-      mbar_init(&sm.full[s], 1);
-      mbar_init(&sm.empty[s], 1);
-    }
-    mbar_init(&sm.tmem_full, 1);
-    mbar_init(&sm.tmem_empty, I8_NCT / 32);
+    i8_ring_init(sm);
     sm.stored = 0;
-    asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
+    fence_mbarrier_init();
   }
 #ifdef SPB_POTRF_PROF
   if (tid < 32) sm.prof[tid / 16][tid % 16] = 0;
 #endif
-  if (pw == I8_ISSUER_WARP) {
-    const uint32_t a = (uint32_t)__cvta_generic_to_shared(&sm.tmem_base);
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;\n" ::"r"(a), "r"(512u)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;\n" ::: "memory");
-  }
+  if (pw == I8_ISSUER_WARP) i8_tmem_alloc(&sm.tmem_base);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -376,6 +272,11 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
         }
       }
       dgm = block_min_i8(sm, dgm);
+      // 2^e (x 2 for balanced 8-bit digits); 1 (2) for a row without a finite positive bound
+      const auto row_scale = [](double x) {
+        int e;
+        return (i8_scale_exp(x, e) ? ldexp(1.0, e) : 1.0) * (RB == 8 ? 2.0 : 1.0);
+      };
       for (int r = tid; r < p.n; r += I8_NCT) {
         double kd = rm.Kb[(size_t)r * p.ld + r];
         if (p.aff_on) {
@@ -388,7 +289,7 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
           }
           kd = aff_apply(sm, af, kd, Ci, Di, true, r, r);
         }
-        Eb[r] = pow2_above(sqrt(kd)) * (RB == 8 ? 2.0 : 1.0);
+        Eb[r] = row_scale(sqrt(kd));
       }
       for (int m = pw; m < rm.M; m += I8_NCT / 32) {
         const double *rr = rm.Rb + (size_t)m * p.ldr;
@@ -397,7 +298,7 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, o));
         if (lane == 0)
-          Eb[n64 + m] = pow2_above(4.0 * sqrt((double)p.n) * mx * rsqrt(dgm)) * (RB == 8 ? 2.0 : 1.0);
+          Eb[n64 + m] = row_scale(4.0 * sqrt((double)p.n) * mx * rsqrt(dgm));
       }
       for (int r = p.n + tid; r < n64; r += I8_NCT) Eb[r] = 1.0;
       __threadfence_block();
@@ -501,9 +402,7 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
 #pragma unroll
             for (int cq = 0; cq < 4; ++cq) {
               uint32_t v[S][8];
-#pragma unroll
-              for (int d = 0; d < S; ++d) tmem_ld_frag16(tw + (uint32_t)(NB * d + 16 * cq), v[d]);
-              tmem_ld_wait();
+              i8_tmem_ld<S>(tw, 16 * cq, v);
 #pragma unroll
               for (int b = 0; b < 2; ++b) {
                 const int nt = 2 * cq + b;
@@ -514,10 +413,7 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
                 for (int mt = 0; mt < 2; ++mt) {
 #pragma unroll
                   for (int e = 0; e < 2; ++e) {
-                    double t = (double)(int)v[D][4 * b + 2 * mt + e];
-#pragma unroll
-                    for (int d = D - 1; d >= 0; --d)
-                      t = fma(t, RB == 8 ? 0.00390625 : 0.0078125, (double)(int)v[d][4 * b + 2 * mt + e]);
+                    const double t = i8_horner<S, RB>(v, 4 * b + 2 * mt + e);
                     acc[mt][nt][e] = fma(si[mt] * (e ? sj1 : sj0), t, acc[mt][nt][e]);
                   }
                 }
@@ -595,17 +491,16 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
               // (column 8 nt + 2 tg + e): a dot product over k does not care about the order as long
               // as both operands use the same one, and this one makes the 16 entries a thread holds of
               // a row contiguous -- one 16-byte store per (row, plane), no shuffles.
-              // Digits: X = rint(x 2^(7S - e)), Xb = X + sum_j 64 128^j has base-128 digits u_j in
-              // [0, 127] (plain bit fields, no carry chain), d_j = u_j - 64; the top digit keeps the sign.
               if (need_planes && live) {
                 const int mrhs = v - NB - rm.nbel;                      // right-hand-side index (KIND_RHS)
                 const int pr = (kind == KIND_RHS) ? n64 + mrhs : c0 + v;   // plane row == row of the scale table
                 const double sinv = ldexp(1.0 / Eb[pr], RB * S);   // 2^(RB S - e): exact
                 uint8_t *qrow = Qb + (size_t)pr * ip.LDQ + c0 + 16 * tg;
                 const size_t pstride = (size_t)NR * ip.LDQ;
+                // The cut of i8_cut, written out: 16 entries per thread in 4 words per plane, the range check
+                // between the lower digits and the top digit (i8_cut's order changes this kernel's schedule).
                 constexpr long long BIAS = i8_bias(S, RB);
                 constexpr unsigned FMASK = (1u << RB) - 1u;
-                constexpr unsigned HALF4 = (RB == 8) ? 0x80808080u : 0x40404040u;
                 uint32_t W[S][4];
 #pragma unroll
                 for (int s = 0; s < S; ++s)
@@ -628,10 +523,10 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
 #pragma unroll
                 for (int s = 0; s < S; ++s) {
                   uint4 o;
-                  o.x = (s == 0) ? W[s][0] : __vsub4(W[s][0], HALF4);
-                  o.y = (s == 0) ? W[s][1] : __vsub4(W[s][1], HALF4);
-                  o.z = (s == 0) ? W[s][2] : __vsub4(W[s][2], HALF4);
-                  o.w = (s == 0) ? W[s][3] : __vsub4(W[s][3], HALF4);
+                  o.x = i8_recentre<RB>(s, W[s][0]);
+                  o.y = i8_recentre<RB>(s, W[s][1]);
+                  o.z = i8_recentre<RB>(s, W[s][2]);
+                  o.w = i8_recentre<RB>(s, W[s][3]);
                   *reinterpret_cast<uint4 *>(qrow + (size_t)s * pstride) = o;
                   // "gap" layout: second copy of a right-hand-side row, read by the full panels
                   if (gap && kind == KIND_RHS && n64 != p.n)
@@ -734,20 +629,9 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
               mbar_wait_sleep(&sm.full[st], (xchunk / STAGES) & 1u, 50);
               tc_fence_after();
               I8_PROF(sm, 1);
-#pragma unroll
-              for (int s = 0; s < S; ++s) {
-                const uint64_t da = i8_smem_desc(&sm.A[st][s][0][0]);
-                const int nt = D - s + 1;                 // planes B_0 .. B_{nt-1}
-#pragma unroll
-                for (int t0 = 0; t0 < nt; t0 += 4) {
-                  const int np = nt - t0 < 4 ? nt - t0 : 4;
-                  // blocks 0 .. D are first written by s = 0 (accumulate = 0 on the first chunk)
 #ifndef SPB_I8_NOMMA
-                  i8_mma(tmem + (uint32_t)(NB * (s + t0)), da, i8_smem_desc(&sm.B[st][t0][0][0]),
-                         i8_idesc(NB * np), (ch > 0 || s > 0) ? 1u : 0u);
+              i8_issue_chunk<S>(tmem, sm.A[st], sm.B[st], ch > 0);
 #endif
-                }
-              }
               i8_commit(&sm.empty[st]);
             }
             i8_commit(&sm.tmem_full);
@@ -764,7 +648,5 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
 #ifdef SPB_POTRF_PROF
   if (tid < 32) atomicAdd(&g_potrf_prof[tid / 16][tid % 16], sm.prof[tid / 16][tid % 16]);
 #endif
-  if (pw == I8_ISSUER_WARP) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;\n" ::"r"(tmem), "r"(512u) : "memory");
-  }
+  if (pw == I8_ISSUER_WARP) i8_tmem_dealloc(tmem);
 }

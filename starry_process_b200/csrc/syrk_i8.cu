@@ -1,30 +1,29 @@
-// FP64 GEMMs of the path evaluated on the INT8 tensor cores (tcgen05 + TMEM): the second-moment SYRK of the Ylm
-// moments (this header) and the lower triangle of the conditional flux covariance (A Sigma) A^T (end of the file).
+// FP64 GEMMs of the path evaluated exactly on the INT8 tensor cores (tcgen05 + TMEM), on the digit planes of
+// i8_planes.cuh: the second-moment SYRK of the Ylm moments and the lower triangle of the conditional flux
+// covariance (A Sigma) A^T (end of the file).
 //
 //     cov_ylm[b] = scale_b ( ldeg_b o (X_b X_b^T) - mom1_b mom1_b^T ) + diag(lambda)      (contrast.py:21-33,
 //                                                                  size.py:116-125 for the ldeg factor)
 //
-// with X_b = sqrtC_lon (256 x 31 rk) -- the same product gemm_nt<EPI_SYRK_COV> evaluates on DMMA, here as an
-// error-free digit-plane emulation of the FP64 products (see potrf_i8.cuh for the scheme):
+// with X_b = sqrtC_lon (256 x 31 rk) -- the same product gemm_nt<EPI_SYRK_COV> evaluates on DMMA:
 //   1. slice_rows_kernel: every row of X_b is scaled by a power of two taken from its largest entry, rounded to
 //      55 bits and cut into 7 balanced 8-bit digits; the kept eigen-columns (the first rk4 of every 32-wide
 //      group) are packed contiguously, zero-padded to a multiple of 32 -> planes (B, 7, 256, 1024) int8;
-//   2. syrk_i8_kernel: persistent, one CTA per SM; per 128 x 64 tile of the lower triangle one thread streams
-//      the plane chunks by 4-D TMA into a 3-stage ring, one thread issues tcgen05.mma.kind::i8 (A_s against the
-//      concatenated planes B_0..B_{6-s}; pairs with s + t = d accumulate exactly in TMEM block d), 8 warps read
-//      the 7 blocks back in the DMMA fragment layout, combine them in fp64, apply the covariance epilogue and
-//      store the tile and its mirror image.
+//   2. syrk_i8_kernel: per 128 x 64 tile of the lower triangle, the 7 TMEM blocks combined in fp64, the
+//      covariance epilogue applied and the tile and its mirror image stored.
+// Both GEMMs run on one pipeline (i8_gemm): persistent, one CTA per SM; one thread streams the plane chunks
+// of a tile by 4-D TMA into a 5-stage ring, one thread issues the MMAs, 8 warps read the blocks back and run
+// the GEMM's epilogue.
 #include <stdlib.h>
 #include <string.h>
 
 #include "common.cuh"
+#include "i8_planes.cuh"
 
 namespace {
 
-constexpr int SY_S = 7, SY_D = 6, SY_RB = 8;   // 7 planes of 8-bit digits, plane pairs s + t <= 6
-constexpr int SY_KCH = 32, SY_TM = 128, SY_TN = 64, SY_STAGES = 5;
-constexpr int SY_LDQ = 1024;                   // bytes per plane row (31 x 32 = 992 entries at most)
-constexpr int SY_NCT = 256, SY_NTHREADS = 320;
+constexpr int SY_S = 7, SY_RB = 8;   // 7 planes of balanced 8-bit digits
+constexpr int SY_LDQ = 1024;         // bytes per plane row (31 x 32 = 992 entries at most)
 
 struct SyrkParams {
   const double *X;        // (B, 256, 992)
@@ -39,21 +38,9 @@ struct SyrkParams {
   int B;
 };
 
-struct SmemSy {
-  uint8_t A[SY_STAGES][SY_S][SY_TM][SY_KCH];
-  uint8_t B[SY_STAGES][SY_S][SY_TN][SY_KCH];
-  uint64_t full[SY_STAGES], empty[SY_STAGES], tmem_full, tmem_empty;
-  uint32_t tmem_base;
-};
-
-__host__ __device__ constexpr long long sy_bias() {
-  long long b = 0;
-  for (int j = 0; j < SY_S; ++j) b = (b << SY_RB) + (1ll << (SY_RB - 1));
-  return b;
-}
 __device__ __forceinline__ int sy_chunks(int rkeep) {   // k-chunks of 32 packed entries
   const int rk4 = (rkeep + 3) & ~3;
-  return (31 * rk4 + SY_KCH - 1) / SY_KCH;
+  return (31 * rk4 + I8_KCH - 1) / I8_KCH;
 }
 
 // ---- 1. digit planes of X ------------------------------------------------------------------------
@@ -61,7 +48,7 @@ __global__ void __launch_bounds__(256) slice_rows_kernel(SyrkParams p) {
   const int b = blockIdx.y, row = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
   const int rk4 = (p.rkeep[b] + 3) & ~3;
   const int KQ = 31 * rk4 / 4;                       // quads of packed entries (rk4 % 4 == 0)
-  const int KPQ = sy_chunks(p.rkeep[b]) * (SY_KCH / 4);   // quads incl. the zero padding
+  const int KPQ = sy_chunks(p.rkeep[b]) * (I8_KCH / 4);   // quads incl. the zero padding
   const double *xr = p.X + ((size_t)b * 256 + row) * 992;
   // pass 1: the largest entry of the row; the kept entries are parked in shared memory (8 KB per warp) so
   // that pass 2 neither re-reads them from DRAM (ncu: the second read missed L2) nor holds them in 64 registers
@@ -81,17 +68,12 @@ __global__ void __launch_bounds__(256) slice_rows_kernel(SyrkParams p) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, o));
   // 2^e > 2.02 max: balanced base-256 digits need |x| <= 1/2
-  double E = 1.0;
-  if (mx > 0.0 && mx < 1e300) {
-    int ex;
-    (void)frexp(mx * 1.0101, &ex);
-    E = ldexp(1.0, ex + 1);
-  }
+  int ex;
+  const double E = i8_scale_exp(mx, ex) ? ldexp(1.0, ex + 1) : 1.0;
   if (lane == 0) p.E[(size_t)b * 256 + row] = E;
   const double sinv = ldexp(1.0 / E, SY_RB * SY_S);
   uint8_t *qrow = p.Q + ((size_t)b * SY_S * 256 + row) * SY_LDQ;
   const size_t pstride = (size_t)256 * SY_LDQ;
-  constexpr long long BIAS = sy_bias();
 #pragma unroll
   for (int j = 0; j < 8; ++j) {
     const int q = lane + 32 * j;
@@ -105,222 +87,174 @@ __global__ void __launch_bounds__(256) slice_rows_kernel(SyrkParams p) {
 #pragma unroll
     for (int s = 0; s < SY_S; ++s) W[s] = 0u;
 #pragma unroll
-    for (int c = 0; c < 4; ++c) {
-      const long long Xb = __double2ll_rn(v4[c] * sinv) + BIAS;
-#pragma unroll
-      for (int jd = 0; jd < SY_S - 1; ++jd) W[SY_S - 1 - jd] |= ((uint32_t)(Xb >> (SY_RB * jd)) & 255u) << (8 * c);
-      const int top = (int)(Xb >> (SY_RB * (SY_S - 1))) - 128;
-      W[0] |= ((uint32_t)top & 255u) << (8 * c);
-    }
+    for (int c = 0; c < 4; ++c) (void)i8_cut<SY_S, SY_RB>(v4[c] * sinv, 8 * c, W);
 #pragma unroll
     for (int s = 0; s < SY_S; ++s)
-      *reinterpret_cast<uint32_t *>(qrow + (size_t)s * pstride + 4 * q) = (s == 0) ? W[s] : __vsub4(W[s], 0x80808080u);
+      *reinterpret_cast<uint32_t *>(qrow + (size_t)s * pstride + 4 * q) = i8_recentre<SY_RB>(s, W[s]);
   }
 }
 
-// ---- tcgen05 / TMA helpers (same conventions as potrf_i8.cuh) -----------------------------------------
-__device__ __forceinline__ void sy_tma_load_4d(void *sdst, const void *tmap, uint64_t *bar, int c0, int c1, int c2,
-                                               int c3) {
-  unsigned s = (unsigned)__cvta_generic_to_shared(sdst);
-  unsigned b = (unsigned)__cvta_generic_to_shared(bar);
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];\n" ::"r"(s),
-      "l"(tmap), "r"(b), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-      : "memory");
-}
-__device__ __forceinline__ uint64_t sy_desc(const void *p) {   // K-major, 32-byte swizzle, version 1
-  const uint32_t a = (uint32_t)__cvta_generic_to_shared(p);
-  uint64_t d = (uint64_t)((a >> 4) & 0x3FFF);
-  d |= (uint64_t)1 << 16;
-  d |= (uint64_t)(256 >> 4) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)6 << 61;
-  return d;
-}
-__device__ __forceinline__ uint32_t sy_idesc(int n) {
-  return (2u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(SY_TM >> 4) << 24);
-}
-__device__ __forceinline__ void sy_mma(uint32_t tmem_d, uint64_t da, uint64_t db, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\n"
-      "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n}\n" ::"r"(tmem_d),
-      "l"(da), "l"(db), "r"(idesc), "r"(acc)
-      : "memory");
-}
-__device__ __forceinline__ void sy_commit(uint64_t *bar) {
-  const uint32_t a = (uint32_t)__cvta_generic_to_shared(bar);
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];\n" ::"r"(a) : "memory");
-}
-__device__ __forceinline__ void sy_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;\n" ::: "memory"); }
-__device__ __forceinline__ void sy_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;\n" ::: "memory"); }
-__device__ __forceinline__ void sy_ld_frag16(uint32_t taddr, uint32_t (&v)[8]) {
-  asm volatile("tcgen05.ld.sync.aligned.16x256b.x2.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];\n"
-               : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
-               : "r"(taddr)
-               : "memory");
-}
-__device__ __forceinline__ void sy_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;\n" ::: "memory"); }
-__device__ __forceinline__ void sy_wait_sleep(uint64_t *bar, unsigned parity, unsigned ns) {
-  while (!mbar_test(bar, parity)) __nanosleep(ns);
-}
+// ---- the pipeline of both GEMMs ----------------------------------------------------------------------
+struct SmemGemm {
+  static constexpr int STAGES = 5;
+  uint8_t A[STAGES][SY_S][I8_TM][I8_KCH];
+  uint8_t B[STAGES][SY_S][I8_TN][I8_KCH];
+  uint64_t full[STAGES], empty[STAGES], tmem_full, tmem_empty;
+  uint32_t tmem_base;
+};
 
-// lower-triangle tiles of the 256 x 256 output: (row block of 128, column block of 64)
-__device__ __forceinline__ void sy_tile(int t, int &tm, int &tn) {
-  tm = (t < 2) ? 0 : 1;
-  tn = (t < 2) ? t : t - 2;
-}
-
-// ---- 2. the SYRK ------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(SY_NTHREADS, 1)
-    syrk_i8_kernel(SyrkParams p, const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB) {
+// Persistent loop over the work items of a Job, 128 x 64 output tiles:
+//   Job::Item                            integer type of the item index
+//   nitems()                             number of items
+//   tile(item, b, tm, tn, bB)            A rows tm * 128.. of batch b against B rows tn * 64.. of batch bB
+//   chunks(item)                         k-chunks of 32 bytes
+//   epilogue(item, wrow, lane, tw, wait) one draining warp (tile rows wrow .. wrow + 15, TMEM address tw):
+//                                        loads what it needs, calls wait() and then reads TMEM
+template <class Job>
+__device__ __forceinline__ void i8_gemm(const Job &job, const CUtensorMap &tmA, const CUtensorMap &tmB) {
+  using Item = typename Job::Item;
+  constexpr int STAGES = SmemGemm::STAGES;
   extern __shared__ __align__(1024) unsigned char smem_raw[];
-  SmemSy &sm = *reinterpret_cast<SmemSy *>(smem_raw);
-  const int tid = threadIdx.x, pw = tid >> 5, lane = tid & 31, g = lane >> 2, tg = lane & 3;
+  SmemGemm &sm = *reinterpret_cast<SmemGemm *>(smem_raw);
+  const int tid = threadIdx.x, pw = tid >> 5, lane = tid & 31;
   if (tid == 0) {
-#pragma unroll
-    for (int s = 0; s < SY_STAGES; ++s) {
-      mbar_init(&sm.full[s], 1);
-      mbar_init(&sm.empty[s], 1);
-    }
-    mbar_init(&sm.tmem_full, 1);
-    mbar_init(&sm.tmem_empty, SY_NCT / 32);
-    asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
+    i8_ring_init(sm);
+    fence_mbarrier_init();
   }
-  if (pw == 9) {
-    const uint32_t a = (uint32_t)__cvta_generic_to_shared(&sm.tmem_base);
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;\n" ::"r"(a), "r"(512u) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;\n" ::: "memory");
-  }
-  sy_fence_before();
+  if (pw == I8_ISSUER_WARP) i8_tmem_alloc(&sm.tmem_base);
+  tc_fence_before();
   __syncthreads();
-  sy_fence_after();
+  tc_fence_after();
   const uint32_t tmem = sm.tmem_base;
-  const int nitems = 6 * p.B;
+  const Item nitems = job.nitems();
 
-  if (pw == 8) {
-    // ================================================================ TMA producer (one thread)
+  if (pw == I8_PRODUCER_WARP) {
     if (lane == 0) {
       unsigned x = 0;
-      for (int item = blockIdx.x; item < nitems; item += gridDim.x) {
-        const int b = item / 6;
-        int tm, tn;
-        sy_tile(item - 6 * b, tm, tn);
-        const int nch = sy_chunks(p.rkeep[b]);
+      for (Item item = blockIdx.x; item < nitems; item += gridDim.x) {
+        int b, tm, tn, bB;
+        job.tile(item, b, tm, tn, bB);
+        const int nch = job.chunks(item);
         for (int ch = 0; ch < nch; ++ch, ++x) {
-          const unsigned st = x % SY_STAGES;
-          if (x >= (unsigned)SY_STAGES) sy_wait_sleep(&sm.empty[st], ((x / SY_STAGES) + 1u) & 1u, 60);
-          mbar_arrive_expect_tx(&sm.full[st], (unsigned)(SY_S * (SY_TM + SY_TN) * SY_KCH));
-          sy_tma_load_4d(&sm.A[st][0][0][0], &tmA, &sm.full[st], ch * SY_KCH, tm * SY_TM, 0, b);
-          sy_tma_load_4d(&sm.B[st][0][0][0], &tmB, &sm.full[st], ch * SY_KCH, tn * SY_TN, 0, b);
+          const unsigned st = x % STAGES;
+          if (x >= (unsigned)STAGES) mbar_wait_sleep(&sm.empty[st], ((x / STAGES) + 1u) & 1u, 60);
+          mbar_arrive_expect_tx(&sm.full[st], (unsigned)(SY_S * (I8_TM + I8_TN) * I8_KCH));
+          tma_load_4d(&sm.A[st][0][0][0], &tmA, &sm.full[st], ch * I8_KCH, tm * I8_TM, 0, b);
+          tma_load_4d(&sm.B[st][0][0][0], &tmB, &sm.full[st], ch * I8_KCH, tn * I8_TN, 0, bB);
         }
       }
     }
-  } else if (pw == 9) {
-    // ================================================================ MMA issuer (one thread)
+  } else if (pw == I8_ISSUER_WARP) {
     if (lane == 0) {
       unsigned x = 0, tq = 0;
-      for (int item = blockIdx.x; item < nitems; item += gridDim.x, ++tq) {
-        const int b = item / 6;
-        const int nch = sy_chunks(p.rkeep[b]);
-        if (tq > 0) sy_wait_sleep(&sm.tmem_empty, (tq + 1u) & 1u, 60);
-        sy_fence_after();
+      for (Item item = blockIdx.x; item < nitems; item += gridDim.x, ++tq) {
+        const int nch = job.chunks(item);
+        if (tq > 0) mbar_wait_sleep(&sm.tmem_empty, (tq + 1u) & 1u, 60);
+        tc_fence_after();
         for (int ch = 0; ch < nch; ++ch, ++x) {
-          const unsigned st = x % SY_STAGES;
-          sy_wait_sleep(&sm.full[st], (x / SY_STAGES) & 1u, 40);
-          sy_fence_after();
-#pragma unroll
-          for (int s = 0; s < SY_S; ++s) {
-            const uint64_t da = sy_desc(&sm.A[st][s][0][0]);
-            const int nt = SY_D - s + 1;
-#pragma unroll
-            for (int t0 = 0; t0 < nt; t0 += 4) {
-              const int np = nt - t0 < 4 ? nt - t0 : 4;
-              sy_mma(tmem + (uint32_t)(SY_TN * (s + t0)), da, sy_desc(&sm.B[st][t0][0][0]), sy_idesc(SY_TN * np),
-                     (ch > 0 || s > 0) ? 1u : 0u);
-            }
-          }
-          sy_commit(&sm.empty[st]);
+          const unsigned st = x % STAGES;
+          mbar_wait_sleep(&sm.full[st], (x / STAGES) & 1u, 40);
+          tc_fence_after();
+          i8_issue_chunk<SY_S>(tmem, sm.A[st], sm.B[st], ch > 0);
+          i8_commit(&sm.empty[st]);
         }
-        sy_commit(&sm.tmem_full);
+        i8_commit(&sm.tmem_full);
       }
     }
   } else {
-    // ================================================================ epilogue warps
     // TMEM lane rule: warp pw reads lanes 32 (pw % 4) + 16 (pw / 4) .. + 15 = its 16 tile rows
     const int wrow = 32 * (pw & 3) + 16 * ((pw >> 2) & 1);
     const uint32_t tw = tmem + ((uint32_t)wrow << 16);
     unsigned tq = 0;
-    for (int item = blockIdx.x; item < nitems; item += gridDim.x, ++tq) {
-      const int b = item / 6;
-      int tm, tn;
-      sy_tile(item - 6 * b, tm, tn);
-      const int nch = sy_chunks(p.rkeep[b]);
-      const int m0 = tm * SY_TM + wrow, n0 = tn * SY_TN;
-      const double *Eb = p.E + (size_t)b * 256;
-      const double *vb = p.vec + (size_t)b * 256;
-      const double sc = p.scale[b];
-      double *Cb = p.C + (size_t)b * 65536;
-      double em[2], vm[2];
-      int lm[2];
-#pragma unroll
-      for (int mt = 0; mt < 2; ++mt) {
-        const int m = m0 + mt * 8 + g;
-        em[mt] = ldexp(Eb[m], -2 * SY_RB);
-        vm[mt] = vb[m];
-        lm[mt] = (int)sqrt((double)m);
-      }
-      sy_wait_sleep(&sm.tmem_full, tq & 1u, 40);
-      sy_fence_after();
-#pragma unroll
-      for (int cq = 0; cq < 4; ++cq) {
-        uint32_t v[SY_S][8];
-#pragma unroll
-        for (int d = 0; d < SY_S; ++d) sy_ld_frag16(tw + (uint32_t)(SY_TN * d + 16 * cq), v[d]);
-        sy_ld_wait();
-#pragma unroll
-        for (int bl = 0; bl < 2; ++bl) {
-#pragma unroll
-          for (int e = 0; e < 2; ++e) {
-            const int n = n0 + 16 * cq + 8 * bl + 2 * tg + e;
-            const double en = Eb[n], vn = vb[n];
-            const int ln = p.ldeg ? (int)sqrt((double)n) : 0;
-#pragma unroll
-            for (int mt = 0; mt < 2; ++mt) {
-              const int m = m0 + mt * 8 + g;
-              if (n > m) continue;
-              double t = 0.0;
-              if (nch > 0) {
-                t = (double)(int)v[SY_D][4 * bl + 2 * mt + e];
-#pragma unroll
-                for (int d = SY_D - 1; d >= 0; --d) t = fma(t, 0.00390625, (double)(int)v[d][4 * bl + 2 * mt + e]);
-              }
-              double val = em[mt] * en * t;
-              if (p.ldeg) val *= p.ldeg[(size_t)b * 256 + lm[mt] * 16 + ln];
-              val = sc * (val - vm[mt] * vn);
-              if (m == n) val += p.diag[m];
-              Cb[(size_t)m * 256 + n] = val;
-              Cb[(size_t)n * 256 + m] = val;
-            }
-          }
-        }
-      }
-      sy_fence_before();
+    for (Item item = blockIdx.x; item < nitems; item += gridDim.x, ++tq) {
+      job.epilogue(item, wrow, lane, tw, [&] {
+        mbar_wait_sleep(&sm.tmem_full, tq & 1u, 40);
+        tc_fence_after();
+      });
+      tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&sm.tmem_empty);
     }
   }
-  sy_fence_before();
+  tc_fence_before();
   __syncthreads();
-  if (pw == 9) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;\n" ::"r"(tmem), "r"(512u) : "memory");
+  if (pw == I8_ISSUER_WARP) i8_tmem_dealloc(tmem);
+}
+
+// ---- 2. the SYRK ------------------------------------------------------------------------------------
+struct SyrkJob {
+  using Item = int;
+  SyrkParams p;
+  __device__ __forceinline__ Item nitems() const { return 6 * p.B; }
+  // lower-triangle tiles of the 256 x 256 output: (row block of 128, column block of 64), 6 per sample
+  __device__ __forceinline__ void tile(Item item, int &b, int &tm, int &tn, int &bB) const {
+    b = item / 6;
+    const int t = item - 6 * b;
+    tm = (t < 2) ? 0 : 1;
+    tn = (t < 2) ? t : t - 2;
+    bB = b;
   }
+  __device__ __forceinline__ int chunks(Item item) const { return sy_chunks(p.rkeep[item / 6]); }
+  template <class Wait>
+  __device__ __forceinline__ void epilogue(Item item, int wrow, int lane, uint32_t tw, Wait wait) const {
+    const int g = lane >> 2, tg = lane & 3;
+    int b, tm, tn, bB;
+    tile(item, b, tm, tn, bB);
+    const int nch = chunks(item);
+    const int m0 = tm * I8_TM + wrow, n0 = tn * I8_TN;
+    const double *Eb = p.E + (size_t)b * 256;
+    const double *vb = p.vec + (size_t)b * 256;
+    const double sc = p.scale[b];
+    double *Cb = p.C + (size_t)b * 65536;
+    double em[2], vm[2];
+    int lm[2];
+#pragma unroll
+    for (int mt = 0; mt < 2; ++mt) {
+      const int m = m0 + mt * 8 + g;
+      em[mt] = ldexp(Eb[m], -2 * SY_RB);
+      vm[mt] = vb[m];
+      lm[mt] = (int)sqrt((double)m);
+    }
+    wait();
+#pragma unroll
+    for (int cq = 0; cq < 4; ++cq) {
+      uint32_t v[SY_S][8];
+      i8_tmem_ld<SY_S>(tw, 16 * cq, v);
+#pragma unroll
+      for (int bl = 0; bl < 2; ++bl) {
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+          const int n = n0 + 16 * cq + 8 * bl + 2 * tg + e;
+          const double en = Eb[n], vn = vb[n];
+          const int ln = p.ldeg ? (int)sqrt((double)n) : 0;
+#pragma unroll
+          for (int mt = 0; mt < 2; ++mt) {
+            const int m = m0 + mt * 8 + g;
+            if (n > m) continue;
+            const double t = (nch > 0) ? i8_horner<SY_S, SY_RB>(v, 4 * bl + 2 * mt + e) : 0.0;
+            double val = em[mt] * en * t;
+            if (p.ldeg) val *= p.ldeg[(size_t)b * 256 + lm[mt] * 16 + ln];
+            val = sc * (val - vm[mt] * vn);
+            if (m == n) val += p.diag[m];
+            Cb[(size_t)m * 256 + n] = val;
+            Cb[(size_t)n * 256 + m] = val;
+          }
+        }
+      }
+    }
+  }
+};
+
+__global__ void __launch_bounds__(I8_NTHREADS, 1)
+    syrk_i8_kernel(SyrkParams p, const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB) {
+  i8_gemm(SyrkJob{p}, tmA, tmB);
 }
 
 
 // =====================================================================================================
 // Lower triangle of  C[b] = T[b] A[b]^T  with 256-wide rows (the conditional flux covariance
-// K = (A Sigma) A^T of flux.py:335-343 for long light curves): the same digit-plane scheme, planes of the rows
-// of T (per sample) and of A (shared or per sample), K = 256 = 8 chunks per 128 x 64 tile.
+// K = (A Sigma) A^T of flux.py:335-343 for long light curves): planes of the rows of T (per sample) and of
+// A (shared or per sample), K = 256 = 8 chunks per 128 x 64 tile.
 // =====================================================================================================
 struct GemmLParams {
   const uint8_t *QT, *QA;   // planes (B, 7, nt, 256), (nA, 7, nt, 256)
@@ -346,181 +280,88 @@ __global__ void __launch_bounds__(256) slice256_kernel(const double *src, long l
   }
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-  double Ev = 1.0;
-  if (mx > 0.0 && mx < 1e300) {
-    int ex;
-    (void)frexp(mx * 1.0101, &ex);
-    Ev = ldexp(1.0, ex + 1);
-  }
+  int ex;
+  const double Ev = i8_scale_exp(mx, ex) ? ldexp(1.0, ex + 1) : 1.0;
   if (lane == 0) E[(size_t)b * rows + row] = Ev;
   const double sinv = ldexp(1.0 / Ev, SY_RB * SY_S);
   uint8_t *qrow = Q + ((size_t)b * SY_S * rows + row) * 256;
   const size_t pstride = (size_t)rows * 256;
-  constexpr long long BIAS = sy_bias();
 #pragma unroll
   for (int j = 0; j < 2; ++j) {
     uint32_t W[SY_S];
 #pragma unroll
     for (int s = 0; s < SY_S; ++s) W[s] = 0u;
 #pragma unroll
-    for (int c = 0; c < 4; ++c) {
-      const long long Xb = __double2ll_rn(v[j][c] * sinv) + BIAS;
-#pragma unroll
-      for (int jd = 0; jd < SY_S - 1; ++jd) W[SY_S - 1 - jd] |= ((uint32_t)(Xb >> (SY_RB * jd)) & 255u) << (8 * c);
-      const int top = (int)(Xb >> (SY_RB * (SY_S - 1))) - 128;
-      W[0] |= ((uint32_t)top & 255u) << (8 * c);
-    }
+    for (int c = 0; c < 4; ++c) (void)i8_cut<SY_S, SY_RB>(v[j][c] * sinv, 8 * c, W);
 #pragma unroll
     for (int s = 0; s < SY_S; ++s)
-      *reinterpret_cast<uint32_t *>(qrow + (size_t)s * pstride + 4 * (lane + 32 * j)) =
-          (s == 0) ? W[s] : __vsub4(W[s], 0x80808080u);
+      *reinterpret_cast<uint32_t *>(qrow + (size_t)s * pstride + 4 * (lane + 32 * j)) = i8_recentre<SY_RB>(s, W[s]);
   }
 }
 
-// tile r of a sample (row-block-major over the lower triangle): row block tm has min(2 tm + 2, tilesN) tiles
-__device__ __forceinline__ void gl_tile(int r, int tilesN, int &tm, int &tn) {
-  tm = (int)((sqrt(4.0 * (double)r + 1.0) - 1.0) * 0.5);
-  while (tm * (tm + 1) > r) --tm;
-  while ((tm + 1) * (tm + 2) <= r) ++tm;
-  tn = r - tm * (tm + 1);
-  (void)tilesN;
-}
-
-constexpr int GL_SY_TN = 64, GL_STAGES = 5, GL_NCH = 256 / SY_KCH;
-struct SmemGl {
-  uint8_t A[GL_STAGES][SY_S][SY_TM][SY_KCH];
-  uint8_t B[GL_STAGES][SY_S][GL_SY_TN][SY_KCH];
-  uint64_t full[GL_STAGES], empty[GL_STAGES], tmem_full, tmem_empty;
-  uint32_t tmem_base;
+struct GemmLowerJob {
+  using Item = long long;
+  GemmLParams p;
+  __device__ __forceinline__ Item nitems() const { return (long long)p.ntile * p.B; }
+  // tile r of a sample (row-block-major over the lower triangle): row block tm has min(2 tm + 2, tilesN) tiles
+  __device__ __forceinline__ void tile(Item item, int &b, int &tm, int &tn, int &bB) const {
+    b = (int)(item / p.ntile);
+    const int r = (int)(item - (long long)b * p.ntile);
+    tm = (int)((sqrt(4.0 * (double)r + 1.0) - 1.0) * 0.5);
+    while (tm * (tm + 1) > r) --tm;
+    while ((tm + 1) * (tm + 2) <= r) ++tm;
+    tn = r - tm * (tm + 1);
+    bB = (p.nA == 1) ? 0 : b;
+  }
+  __device__ __forceinline__ int chunks(Item) const { return 256 / I8_KCH; }
+  template <class Wait>
+  __device__ __forceinline__ void epilogue(Item item, int wrow, int lane, uint32_t tw, Wait wait) const {
+    const int g = lane >> 2, tg = lane & 3;
+    int b, tm, tn, ba;
+    tile(item, b, tm, tn, ba);
+    const int m0 = tm * I8_TM + wrow, n0 = tn * I8_TN;
+    const double *Et = p.ET + (size_t)b * p.nt;
+    const double *Ea = p.EA + (size_t)ba * p.nt;
+    double *Cb = p.C + (size_t)b * p.strideC;
+    double em[2];
+#pragma unroll
+    for (int mt = 0; mt < 2; ++mt) {
+      const int m = m0 + mt * 8 + g;
+      em[mt] = (m < p.nt) ? ldexp(Et[m], -2 * SY_RB) : 0.0;
+    }
+    wait();
+#pragma unroll
+    for (int cq = 0; cq < 4; ++cq) {
+      uint32_t v[SY_S][8];
+      i8_tmem_ld<SY_S>(tw, 16 * cq, v);
+#pragma unroll
+      for (int bl = 0; bl < 2; ++bl) {
+        const int n = n0 + 16 * cq + 8 * bl + 2 * tg;
+        if (n >= p.nt) continue;
+        const double en0 = Ea[n], en1 = (n + 1 < p.nt) ? Ea[n + 1] : 0.0;
+#pragma unroll
+        for (int mt = 0; mt < 2; ++mt) {
+          const int m = m0 + mt * 8 + g;
+          if (m >= p.nt) continue;
+          // both columns in one loop (not two i8_horner calls: that order changes this kernel's schedule)
+          double t0 = (double)(int)v[SY_S - 1][4 * bl + 2 * mt], t1 = (double)(int)v[SY_S - 1][4 * bl + 2 * mt + 1];
+#pragma unroll
+          for (int d = SY_S - 2; d >= 0; --d) {
+            t0 = fma(t0, 0.00390625, (double)(int)v[d][4 * bl + 2 * mt]);
+            t1 = fma(t1, 0.00390625, (double)(int)v[d][4 * bl + 2 * mt + 1]);
+          }
+          double *c = Cb + (size_t)m * p.ldc + n;
+          if (n + 1 < p.nt) *reinterpret_cast<double2 *>(c) = make_double2(em[mt] * en0 * t0, em[mt] * en1 * t1);
+          else *c = em[mt] * en0 * t0;
+        }
+      }
+    }
+  }
 };
 
-__global__ void __launch_bounds__(SY_NTHREADS, 1)
+__global__ void __launch_bounds__(I8_NTHREADS, 1)
     gemm_i8_lower_kernel(GemmLParams p, const __grid_constant__ CUtensorMap tmT, const __grid_constant__ CUtensorMap tmA) {
-  extern __shared__ __align__(1024) unsigned char smem_raw[];
-  SmemGl &sm = *reinterpret_cast<SmemGl *>(smem_raw);
-  const int tid = threadIdx.x, pw = tid >> 5, lane = tid & 31, g = lane >> 2, tg = lane & 3;
-  if (tid == 0) {
-#pragma unroll
-    for (int s = 0; s < GL_STAGES; ++s) {
-      mbar_init(&sm.full[s], 1);
-      mbar_init(&sm.empty[s], 1);
-    }
-    mbar_init(&sm.tmem_full, 1);
-    mbar_init(&sm.tmem_empty, SY_NCT / 32);
-    asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
-  }
-  if (pw == 9) {
-    const uint32_t a = (uint32_t)__cvta_generic_to_shared(&sm.tmem_base);
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;\n" ::"r"(a), "r"(512u) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;\n" ::: "memory");
-  }
-  sy_fence_before();
-  __syncthreads();
-  sy_fence_after();
-  const uint32_t tmem = sm.tmem_base;
-  const long long nitems = (long long)p.ntile * p.B;
-
-  if (pw == 8) {
-    if (lane == 0) {
-      unsigned x = 0;
-      for (long long item = blockIdx.x; item < nitems; item += gridDim.x) {
-        const int b = (int)(item / p.ntile);
-        int tm, tn;
-        gl_tile((int)(item - (long long)b * p.ntile), p.tilesN, tm, tn);
-        const int ba = (p.nA == 1) ? 0 : b;
-        for (int ch = 0; ch < GL_NCH; ++ch, ++x) {
-          const unsigned st = x % GL_STAGES;
-          if (x >= (unsigned)GL_STAGES) sy_wait_sleep(&sm.empty[st], ((x / GL_STAGES) + 1u) & 1u, 60);
-          mbar_arrive_expect_tx(&sm.full[st], (unsigned)(SY_S * (SY_TM + GL_SY_TN) * SY_KCH));
-          sy_tma_load_4d(&sm.A[st][0][0][0], &tmT, &sm.full[st], ch * SY_KCH, tm * SY_TM, 0, b);
-          sy_tma_load_4d(&sm.B[st][0][0][0], &tmA, &sm.full[st], ch * SY_KCH, tn * GL_SY_TN, 0, ba);
-        }
-      }
-    }
-  } else if (pw == 9) {
-    if (lane == 0) {
-      unsigned x = 0, tq = 0;
-      for (long long item = blockIdx.x; item < nitems; item += gridDim.x, ++tq) {
-        if (tq > 0) sy_wait_sleep(&sm.tmem_empty, (tq + 1u) & 1u, 60);
-        sy_fence_after();
-        for (int ch = 0; ch < GL_NCH; ++ch, ++x) {
-          const unsigned st = x % GL_STAGES;
-          sy_wait_sleep(&sm.full[st], (x / GL_STAGES) & 1u, 40);
-          sy_fence_after();
-#pragma unroll
-          for (int s = 0; s < SY_S; ++s) {
-            const uint64_t da = sy_desc(&sm.A[st][s][0][0]);
-            const int nt = SY_D - s + 1;
-#pragma unroll
-            for (int t0 = 0; t0 < nt; t0 += 4) {
-              const int np = nt - t0 < 4 ? nt - t0 : 4;
-              sy_mma(tmem + (uint32_t)(GL_SY_TN * (s + t0)), da, sy_desc(&sm.B[st][t0][0][0]), sy_idesc(GL_SY_TN * np),
-                     (ch > 0 || s > 0) ? 1u : 0u);
-            }
-          }
-          sy_commit(&sm.empty[st]);
-        }
-        sy_commit(&sm.tmem_full);
-      }
-    }
-  } else {
-    const int wrow = 32 * (pw & 3) + 16 * ((pw >> 2) & 1);
-    const uint32_t tw = tmem + ((uint32_t)wrow << 16);
-    unsigned tq = 0;
-    for (long long item = blockIdx.x; item < nitems; item += gridDim.x, ++tq) {
-      const int b = (int)(item / p.ntile);
-      int tm, tn;
-      gl_tile((int)(item - (long long)b * p.ntile), p.tilesN, tm, tn);
-      const int ba = (p.nA == 1) ? 0 : b;
-      const int m0 = tm * SY_TM + wrow, n0 = tn * GL_SY_TN;
-      const double *Et = p.ET + (size_t)b * p.nt;
-      const double *Ea = p.EA + (size_t)ba * p.nt;
-      double *Cb = p.C + (size_t)b * p.strideC;
-      double em[2];
-#pragma unroll
-      for (int mt = 0; mt < 2; ++mt) {
-        const int m = m0 + mt * 8 + g;
-        em[mt] = (m < p.nt) ? ldexp(Et[m], -2 * SY_RB) : 0.0;
-      }
-      sy_wait_sleep(&sm.tmem_full, tq & 1u, 40);
-      sy_fence_after();
-#pragma unroll
-      for (int cq = 0; cq < 4; ++cq) {
-        uint32_t v[SY_S][8];
-#pragma unroll
-        for (int d = 0; d < SY_S; ++d) sy_ld_frag16(tw + (uint32_t)(GL_SY_TN * d + 16 * cq), v[d]);
-        sy_ld_wait();
-#pragma unroll
-        for (int bl = 0; bl < 2; ++bl) {
-          const int n = n0 + 16 * cq + 8 * bl + 2 * tg;
-          if (n >= p.nt) continue;
-          const double en0 = Ea[n], en1 = (n + 1 < p.nt) ? Ea[n + 1] : 0.0;
-#pragma unroll
-          for (int mt = 0; mt < 2; ++mt) {
-            const int m = m0 + mt * 8 + g;
-            if (m >= p.nt) continue;
-            double t0 = (double)(int)v[SY_D][4 * bl + 2 * mt], t1 = (double)(int)v[SY_D][4 * bl + 2 * mt + 1];
-#pragma unroll
-            for (int d = SY_D - 1; d >= 0; --d) {
-              t0 = fma(t0, 0.00390625, (double)(int)v[d][4 * bl + 2 * mt]);
-              t1 = fma(t1, 0.00390625, (double)(int)v[d][4 * bl + 2 * mt + 1]);
-            }
-            double *c = Cb + (size_t)m * p.ldc + n;
-            if (n + 1 < p.nt) *reinterpret_cast<double2 *>(c) = make_double2(em[mt] * en0 * t0, em[mt] * en1 * t1);
-            else *c = em[mt] * en0 * t0;
-          }
-        }
-      }
-      sy_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&sm.tmem_empty);
-    }
-  }
-  sy_fence_before();
-  __syncthreads();
-  if (pw == 9) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;\n" ::"r"(tmem), "r"(512u) : "memory");
-  }
+  i8_gemm(GemmLowerJob{p}, tmT, tmA);
 }
 
 }  // namespace
@@ -551,8 +392,8 @@ int spb_syrk_i8(spb_context *ctx, int Bc, const double *X, const int *rkeep, con
   {
     const unsigned long long dims[4] = {SY_LDQ, 256, SY_S, (unsigned long long)Bc};
     const unsigned long long strides[3] = {SY_LDQ, 256ull * SY_LDQ, (unsigned long long)SY_S * 256 * SY_LDQ};
-    const unsigned boxA[4] = {SY_KCH, SY_TM, SY_S, 1};
-    const unsigned boxB[4] = {SY_KCH, SY_TN, SY_S, 1};
+    const unsigned boxA[4] = {I8_KCH, I8_TM, SY_S, 1};
+    const unsigned boxB[4] = {I8_KCH, I8_TN, SY_S, 1};
     int st = spb_encode_tmap_u8_4d(&tmA, p.Q, dims, strides, boxA);
     if (st) return st;
     st = spb_encode_tmap_u8_4d(&tmB, p.Q, dims, strides, boxB);
@@ -562,7 +403,7 @@ int spb_syrk_i8(spb_context *ctx, int Bc, const double *X, const int *rkeep, con
   {
     const int st = spb_once_per_device(attr_once, ctx->device, [&]() -> int {
       SPB_CHECK_CUDA(cudaFuncSetAttribute(syrk_i8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                          (int)sizeof(SmemSy)));
+                                          (int)sizeof(SmemGemm)));
       SPB_CHECK_CUDA(cudaFuncSetAttribute(slice_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                           (int)(8 * 992 * sizeof(double))));
       return 0;
@@ -573,7 +414,7 @@ int spb_syrk_i8(spb_context *ctx, int Bc, const double *X, const int *rkeep, con
   slice_rows_kernel<<<gs, 256, 8 * 992 * sizeof(double), stream>>>(p);
   SPB_LAUNCH_CHECK(ctx);
   const int grid = 6 * Bc < ctx->num_sms ? 6 * Bc : ctx->num_sms;
-  syrk_i8_kernel<<<grid, SY_NTHREADS, sizeof(SmemSy), stream>>>(p, tmA, tmB);
+  syrk_i8_kernel<<<grid, I8_NTHREADS, sizeof(SmemGemm), stream>>>(p, tmA, tmB);
   SPB_LAUNCH_CHECK(ctx);
   return 0;
 }
@@ -611,8 +452,8 @@ int spb_gemm_i8_lower(spb_context *ctx, int Bc, int nt, const double *T, const d
   p.B = Bc;
   p.nt = nt;
   p.nA = nA;
-  p.tilesM = (nt + SY_TM - 1) / SY_TM;
-  p.tilesN = (nt + GL_SY_TN - 1) / GL_SY_TN;
+  p.tilesM = (nt + I8_TM - 1) / I8_TM;
+  p.tilesN = (nt + I8_TN - 1) / I8_TN;
   // every row block keeps its 2 tm + 2 column blocks (the last ones may lie wholly beyond nt: their loads are
   // zero-filled by TMA and their stores masked)
   p.ntile = p.tilesM * (p.tilesM + 1);
@@ -623,8 +464,8 @@ int spb_gemm_i8_lower(spb_context *ctx, int Bc, int nt, const double *T, const d
     const unsigned long long dT[4] = {256, (unsigned long long)nt, SY_S, (unsigned long long)Bc};
     const unsigned long long dA[4] = {256, (unsigned long long)nt, SY_S, (unsigned long long)nA};
     const unsigned long long st[3] = {256, 256ull * nt, (unsigned long long)SY_S * 256 * nt};
-    const unsigned boxA[4] = {SY_KCH, SY_TM, SY_S, 1};
-    const unsigned boxB[4] = {SY_KCH, GL_SY_TN, SY_S, 1};
+    const unsigned boxA[4] = {I8_KCH, I8_TM, SY_S, 1};
+    const unsigned boxB[4] = {I8_KCH, I8_TN, SY_S, 1};
     int e = spb_encode_tmap_u8_4d(&tmT, QT, dT, st, boxA);
     if (e) return e;
     e = spb_encode_tmap_u8_4d(&tmA, QA, dA, st, boxB);
@@ -634,12 +475,12 @@ int spb_gemm_i8_lower(spb_context *ctx, int Bc, int nt, const double *T, const d
   {
     const int e = spb_once_per_device(attr_once, ctx->device, [&]() -> int {
       SPB_CHECK_CUDA(cudaFuncSetAttribute(gemm_i8_lower_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                          (int)sizeof(SmemGl)));
+                                          (int)sizeof(SmemGemm)));
       return 0;
     });
     if (e) return e;
   }
-  gemm_i8_lower_kernel<<<ctx->num_sms, SY_NTHREADS, sizeof(SmemGl), stream>>>(p, tmT, tmA);
+  gemm_i8_lower_kernel<<<ctx->num_sms, I8_NTHREADS, sizeof(SmemGemm), stream>>>(p, tmT, tmA);
   SPB_LAUNCH_CHECK(ctx);
   return 0;
 }

@@ -262,12 +262,14 @@ def test_sass_int8_cholesky_uses_tcgen05_tmem_and_tma(built_lib):
     body = sass[beg:end if end > 0 else None]
     for mnemonic in ("UTCIMMA", "LDTM", "UTMALDG.4D", "UTCBAR", "FENCE.VIEW.ASYNC.G", "DMMA.8x8x4"):
         assert mnemonic in body, mnemonic
-    # the second-moment SYRK of the Ylm moments (syrk_i8.cu) runs on the same machinery
-    beg = sass.index("syrk_i8_kernel")
-    end = sass.find("Function :", beg)
-    body = sass[beg:end if end > 0 else None]
-    for mnemonic in ("UTCIMMA", "LDTM", "UTMALDG.4D", "UTCBAR"):
-        assert mnemonic in body, mnemonic
+    # the second-moment SYRK of the Ylm moments and the lower-triangle (A Sigma) A^T (syrk_i8.cu) run on the
+    # same machinery
+    for kernel in ("syrk_i8_kernel", "gemm_i8_lower_kernel"):
+        beg = sass.index(kernel)
+        end = sass.find("Function :", beg)
+        body = sass[beg:end if end > 0 else None]
+        for mnemonic in ("UTCIMMA", "LDTM", "UTMALDG.4D", "UTCBAR"):
+            assert mnemonic in body, (kernel, mnemonic)
 
 
 def test_uniform_time_stamp_detection():

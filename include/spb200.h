@@ -313,6 +313,52 @@ int spb_cholesky_solve_rows(spb_context *ctx, int nt, const double *L, int ldk, 
                             int ldr, double *quad, void *stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Rank-31 conditional log-likelihood, linear in nt (DESIGN.md section 4.6).  Replaces, for a static
+ * process conditional on inclination with scalar / per-point data_cov and a scalar / per-element
+ * baseline_var, the dense chain flux.py:335-343 (K = A cov_ylm A^T), sp.py:705-727 (normalisation)
+ * and sp.py:1052-1188 (noise terms, Cholesky, lnlike).  Every design-matrix row is
+ * Phi(t) B_inc with Phi = [1, cos(m theta), sin(m theta)] (m = 1..15, theta = 2 pi frac(t / p)),
+ * padded to 32 columns, so K = Phi C~ Phi^T + D with C~ of size 32.  Nothing of size nt^2 or
+ * nt x 256 is formed; an element's result does not depend on the batch it is evaluated in.
+ *
+ * spb_lowrank_inclination : B_inc (I, 32, 256) for inclinations inc_rad (I) and the flux operator
+ *                           rTA1 (rTA1_stride 0 | 256, as spb_design_matrix); workspace of
+ *                           spb_lowrank_inclination_workspace_bytes(I) bytes, 16-byte aligned.
+ * spb_lowrank_basis       : once per (t, period, data_cov), for any batch: the thin QR
+ *                           D^-1/2 Phi = Q R (Householder TSQR; Q (nt, 32) with orthonormal
+ *                           columns, R (32, 32), possibly singular) and
+ *                           phi_aux (65) = [Phi^T 1 (32) | Phi(t_0) (32) | sum log D].
+ *                           data_kind 0: data_cov is one value; 1: (nt) values.  nt >= 31.
+ * spb_lowrank_lnlike      : per element, C = B_inc cov_ylm B_inc^T (Binc_stride 0 = shared, or
+ *                           32 * 256), the GP mean (A mean_ylm)[0], the normalisation of
+ *                           spb_assemble_* (noise->normalized, same z, SPB_INFO_Z_RANGE), the
+ *                           baseline variance (noise->baseline_var, base_kind 0, base_stride 0 | 1),
+ *                           N = I + R C~ R^T, its Cholesky factor (SPB_INFO_NOT_PD), and
+ *                             lnlike = -1/2 sum_m (|y - Q w|^2 + w^T N^-1 w) - M/2 logdet K - nt M/2 log 2 pi
+ *                           with y = D^-1/2 (flux - mean - baseline_mean), w = Q^T y; -inf where info != 0.
+ *                           noise->data_kind / data_cov must be the ones given to spb_lowrank_basis
+ *                           (data_stride 0).  flux: (M, ldf) shared (flux_stride 0) or per element
+ *                           (flux_stride elements between elements); baseline_mean: NULL | one value
+ *                           (bm_stride 0) | one per element (bm_stride 1).  quad (B, M), logdet (B)
+ *                           (= logdet K), z_out (B) may be NULL.
+ * ------------------------------------------------------------------------------------------- */
+size_t spb_lowrank_inclination_workspace_bytes(const spb_context *ctx, int I);
+int spb_lowrank_inclination(spb_context *ctx, int I, const double *inc_rad, const double *rTA1,
+                            int rTA1_stride, double *Binc, void *workspace, size_t workspace_bytes,
+                            void *stream);
+size_t spb_lowrank_basis_workspace_bytes(const spb_context *ctx, int nt);
+int spb_lowrank_basis(spb_context *ctx, int nt, const double *t, double period, int data_kind,
+                      const double *data_cov, double *Q, double *R, double *phi_aux, void *workspace,
+                      size_t workspace_bytes, void *stream);
+size_t spb_lowrank_lnlike_workspace_bytes(const spb_context *ctx, int B, int M, int nt);
+int spb_lowrank_lnlike(spb_context *ctx, int B, int nt, const double *Binc, long long Binc_stride,
+                       const double *mean_ylm, const double *cov_ylm, const double *Q, const double *R,
+                       const double *phi_aux, const spb_noise_model *noise, int M, const double *flux,
+                       int ldf, long long flux_stride, const double *baseline_mean, long long bm_stride,
+                       double *lnlike, double *quad, double *logdet, double *z_out, int32_t *info,
+                       void *workspace, size_t workspace_bytes, void *stream);
+
+/* ---------------------------------------------------------------------------------------------
  * (f-2) building blocks of predict / sample / sample_conditional / sample_ylm_conditional
  * (sp.py:518-641, 729-765, 767-1002).  Together with spb_cholesky_lnlike (whose "residual" rows are
  * any set of right-hand sides: out = L^{-1} rhs, one per row) they cover

@@ -85,7 +85,14 @@ PROTOTYPES = {
     "spb_cholesky_lnlike_i8": (_I, [_P, _I, _I, _P, _I, _LL, _c.POINTER(Affine), _I, _P, _I, _LL,
                                     _P, _P, _P, _P, _I, _D, _P, _SZ, _P]),
     "spb_cholesky_solve_rows": (_I, [_P, _I, _P, _I, _I, _P, _I, _P, _P]),
-    "spb_temporal_scale": (_I, [_P, _I, _I, _I, _P, _P, _I, _P, _LL, _P, _LL, _P, _I, _LL, _P]),
+    "spb_lowrank_inclination_workspace_bytes": (_SZ, [_P, _I]),
+    "spb_lowrank_inclination": (_I, [_P, _I, _P, _P, _I, _P, _P, _SZ, _P]),
+    "spb_lowrank_basis_workspace_bytes": (_SZ, [_P, _I]),
+    "spb_lowrank_basis": (_I, [_P, _I, _P, _D, _I, _P, _P, _P, _P, _P, _SZ, _P]),
+    "spb_lowrank_lnlike_workspace_bytes": (_SZ, [_P, _I, _I, _I]),
+    "spb_lowrank_lnlike": (_I, [_P, _I, _I, _P, _LL, _P, _P, _P, _P, _P, _c.POINTER(NoiseModel), _I, _P,
+                                _I, _LL, _P, _LL, _P, _P, _P, _P, _P, _P, _SZ, _P]),
+    "spb_temporal_scale":(_I, [_P, _I, _I, _I, _P, _P, _I, _P, _LL, _P, _LL, _P, _I, _LL, _P]),
     "spb_gemm_nt": (_I, [_P, _I, _I, _I, _I, _D, _P, _I, _LL, _P, _I, _LL, _D, _P, _I, _LL, _P]),
     "spb_tril": (_I, [_P, _I, _I, _P, _I, _LL, _P]),
     "spb_cross_marginal": (_I, [_P, _I, _I, _I, _P, _P, _D, _I, _P, _P, _LL, _P, _I, _LL, _P]),

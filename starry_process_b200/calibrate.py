@@ -19,11 +19,12 @@ __all__ = ["get_log_prob", "inclination_log_prob"]
 
 def get_log_prob(t, flux=None, ferr=1.0e-3, p=1.0, ydeg=15, baseline_log_var=0.0, baseline_mean=0.0,
                  apply_jac=True, normalized=True, marginalize_over_inclination=True, u=(0.0, 0.0),
-                 device=None):
+                 device=None, method="dense"):
     """calibrate/log_prob.py:7-106.  Returns ``log_prob(*args)`` with the reference's argument order
     ``[flux,] r, a, b, c, n [, m] [, v] [, i]`` (``flux`` only if it was not fixed here, ``m`` only if
     ``baseline_mean is None``, ``v`` only if ``baseline_log_var is None``, ``i`` only if
-    ``marginalize_over_inclination`` is false)."""
+    ``marginalize_over_inclination`` is false).  ``method``: as in ``StarryProcess.log_likelihood``
+    (``"lowrank"`` needs ``marginalize_over_inclination=False``)."""
     t = np.asarray(t, dtype=np.float64).reshape(-1)
     K = t.size
     free_flux = flux is None
@@ -51,7 +52,7 @@ def get_log_prob(t, flux=None, ferr=1.0e-3, p=1.0, ydeg=15, baseline_log_var=0.0
         else:
             bvar = torch.tensor(10.0 ** float(v), dtype=torch.float64)   # 10 ** 0 = 1 by default
         ll = gp.log_likelihood(t, fl, float(ferr) ** 2, i=inc, p=p, u=list(u), baseline_mean=m,
-                               baseline_var=bvar)
+                               baseline_var=bvar, method=method)
         if apply_jac:
             ll = ll + gp.log_jac()
         return ll
@@ -61,12 +62,13 @@ def get_log_prob(t, flux=None, ferr=1.0e-3, p=1.0, ydeg=15, baseline_log_var=0.0
 
 def inclination_log_prob(t, flux, samples, inc, ferr=1.0e-3, p=1.0, ydeg=15, baseline_log_var=0.0,
                          baseline_mean=0.0, apply_jac=True, normalized=True, u=(0.0, 0.0),
-                         device=None):
+                         device=None, method="dense"):
     """The (light curve x posterior sample x inclination) grid of conditional log-probabilities that
     calibrate/inclination.py:63-74 fills with ``nlc * ninc_samples * ninc_pts`` separate calls.
 
     ``flux``: ``(nlc, nt)``; ``samples``: ``(ns, 5)`` rows ``r, a, b, c, n`` (the posterior draws the
-    caller selected); ``inc``: ``(ninc,)`` degrees.  Returns ``lp`` of shape ``(nlc, ns, ninc)``."""
+    caller selected); ``inc``: ``(ninc,)`` degrees.  Returns ``lp`` of shape ``(nlc, ns, ninc)``.
+    ``method="lowrank"`` evaluates every element through the rank-31 form (DESIGN.md section 4.6)."""
     flux = torch.as_tensor(np.asarray(flux), dtype=torch.float64)
     samples = torch.as_tensor(np.asarray(samples), dtype=torch.float64)
     inc = torch.as_tensor(np.asarray(inc), dtype=torch.float64).reshape(-1)
@@ -78,7 +80,7 @@ def inclination_log_prob(t, flux, samples, inc, ferr=1.0e-3, p=1.0, ydeg=15, bas
     fl = flux[:, None, None, :].expand(nlc, ns, ninc, nt).reshape(-1, 1, nt)
     fn = get_log_prob(t, flux=None, ferr=ferr, p=p, ydeg=ydeg, baseline_log_var=baseline_log_var,
                       baseline_mean=baseline_mean, apply_jac=apply_jac, normalized=normalized,
-                      marginalize_over_inclination=False, u=u, device=device)
+                      marginalize_over_inclination=False, u=u, device=device, method=method)
     lp = fn(fl, hp[:, 0].contiguous(), hp[:, 1].contiguous(), hp[:, 2].contiguous(),
             hp[:, 3].contiguous(), hp[:, 4].contiguous(), ii.contiguous())
     return lp.reshape(nlc, ns, ninc)

@@ -241,6 +241,41 @@ __global__ void __launch_bounds__(256) design_v_kernel(int I, const double *rTA1
   *out = make_double2(acc, m < 0 ? -vb : vb);
 }
 
+// Inclination basis of the rank-31 conditional path (DESIGN.md section 4.6): a design-matrix row is
+// f(theta) . Rx(pi/2) with f[n] = VV.x[n] cos(|m_n| theta) + VV.y[n] sin(|m_n| theta), so
+//   A = Phi(t) B_inc,  Phi = [1, cos(m theta) (m = 1..15), sin(m theta) (m = 1..15)]
+//   B_inc[m]      = sum over |m_n| = m of VV.x[n] Rx90[n, :]      (rows 0..15)
+//   B_inc[15 + m] = sum over |m_n| = m of VV.y[n] Rx90[n, :]      (rows 16..30);  row 31 = 0.
+// One thread per output column n' = l^2 + j' (Rx(pi/2) is block-diagonal in l).
+__global__ void __launch_bounds__(256) lowrank_binc_kernel(int I, const double *VV, const double *Rx90,
+                                                           double *Binc) {
+  __shared__ double2 v[256];
+  const int c = threadIdx.x, ii = blockIdx.x;
+  if (ii >= I) return;
+  v[c] = reinterpret_cast<const double2 *>(VV)[(size_t)ii * 256 + c];
+  __syncthreads();
+  const int l = (int)floor(sqrt((double)c) + 1e-9);
+  const int jp = c - l * l, w = 2 * l + 1;
+  const double *rx = Rx90 + nwig(l - 1);
+  double *out = Binc + (size_t)ii * 32 * 256 + c;
+  for (int k = 0; k <= SPB_LMAX; ++k) {
+    double a = 0.0, b = 0.0;
+    if (k <= l) {
+      const int j1 = l + k;
+      a = v[l * l + j1].x * rx[j1 * w + jp];
+      b = v[l * l + j1].y * rx[j1 * w + jp];
+      if (k > 0) {
+        const int j2 = l - k;
+        a += v[l * l + j2].x * rx[j2 * w + jp];
+        b += v[l * l + j2].y * rx[j2 * w + jp];
+      }
+    }
+    out[k * 256] = a;
+    if (k > 0) out[(SPB_LMAX + k) * 256] = b;
+  }
+  out[31 * 256] = 0.0;
+}
+
 // Store path: the warp collects a (32 timestamps x 16 columns) tile in shared memory -- 128-byte rows
 // in the TMA 128B-swizzle layout, so the lanes' 16-byte stores are conflict-free -- and one elected
 // lane hands it to the TMA engine (cp.async.bulk.tensor.3d shared -> global through a tensor map of A,
@@ -407,6 +442,31 @@ extern "C" int spb_design_matrix(spb_context *ctx, int I, int nt, const double *
   });
   if (st) return st;
   design_rows_kernel<<<grid, DM_THREADS, smem, stream>>>(p, tmap);
+  SPB_LAUNCH_CHECK(ctx);
+  return 0;
+}
+
+extern "C" size_t spb_lowrank_inclination_workspace_bytes(const spb_context *ctx, int I) {
+  return spb_design_matrix_workspace_bytes(ctx, I, 0);
+}
+
+extern "C" int spb_lowrank_inclination(spb_context *ctx, int I, const double *inc_rad, const double *rTA1,
+                                       int rTA1_stride, double *Binc, void *workspace,
+                                       size_t workspace_bytes, void *stream_) {
+  SPB_REQUIRE(ctx != nullptr && I > 0, "lowrank_inclination: bad arguments");
+  SPB_REQUIRE(ctx->tables_count == SPB_TAB_TOTAL, "lowrank_inclination: context has no constant tables");
+  SPB_REQUIRE(workspace != nullptr && workspace_bytes >= spb_lowrank_inclination_workspace_bytes(ctx, I) &&
+                  ((uintptr_t)workspace % 16) == 0,
+              "lowrank_inclination: workspace too small or not 16-byte aligned");
+  cudaStream_t stream = (cudaStream_t)stream_;
+  SPB_CHECK_CUDA(cudaSetDevice(ctx->device));
+  double *VV = reinterpret_cast<double *>(workspace);          // (I, 512)
+  double *RxInc = VV + (size_t)I * 512;                        // (I, 5456)
+  rx_kernel<<<I, 256, 0, stream>>>(I, inc_rad, -1.0, RxInc);  // Rx(-i), flux.py:96
+  SPB_LAUNCH_CHECK(ctx);
+  design_v_kernel<<<I, 256, 0, stream>>>(I, rTA1, rTA1_stride, RxInc, VV);
+  SPB_LAUNCH_CHECK(ctx);
+  lowrank_binc_kernel<<<I, 256, 0, stream>>>(I, VV, ctx->d_tables + SPB_TAB_RX90, Binc);
   SPB_LAUNCH_CHECK(ctx);
   return 0;
 }

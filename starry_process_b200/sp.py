@@ -775,16 +775,29 @@ class StarryProcess(object):
     def log_likelihood(self, t, flux, data_cov, i=defaults["i"], p=defaults["p"], u=None,
                        baseline_mean=defaults["baseline_mean"],
                        baseline_var=defaults["baseline_var"], marginalize_over_inclination=None,
-                       return_grad=False):
+                       return_grad=False, method="dense"):
         """sp.py:1052-1188.  ``flux`` is ``(nt,)`` or ``(M, nt)`` (M light curves sharing period,
         limb darkening, inclination and noise, scored jointly); returns a scalar, or ``(B,)`` for a
         batch of hyperparameter samples.  Extension: ``flux`` of shape ``(B, M, nt)`` gives every
         batch element its own light curve(s) (the light-curve x sample x inclination batches of
-        calibrate/inclination.py:63-74)."""
+        calibrate/inclination.py:63-74).
+
+        ``method``: ``"dense"`` (default) factorises the ``(nt, nt)`` covariance of every element, as
+        the reference does.  ``"lowrank"`` evaluates the same conditional-branch likelihood through its
+        rank-31 form (DESIGN.md section 4.6): time and memory linear in ``nt``, so light curves of
+        1e5-1e6 points fit.  It covers the static process conditional on inclination with a scalar or
+        ``(nt,)`` positive ``data_cov`` and a scalar or ``(B,)`` ``baseline_var``, and raises
+        ``ValueError`` otherwise."""
+        if method not in ("dense", "lowrank"):
+            raise ValueError("unknown method %r: expected 'dense' or 'lowrank'" % (method,))
         if return_grad:
             return self.log_likelihood_and_grad(
                 t, flux, data_cov, i=i, p=p, u=u, baseline_mean=baseline_mean,
-                baseline_var=baseline_var, marginalize_over_inclination=marginalize_over_inclination)
+                baseline_var=baseline_var, marginalize_over_inclination=marginalize_over_inclination,
+                method=method)
+        if method == "lowrank":
+            return self._log_likelihood_lowrank(t, flux, data_cov, i, p, u, baseline_mean, baseline_var,
+                                                marginalize_over_inclination)
         marg, t, inc, rta1 = self._prep(t, i, p, u, marginalize_over_inclination)
         nt = t.numel()
         ldk = nt + (nt & 1)
@@ -876,11 +889,88 @@ class StarryProcess(object):
         self._z = torch.cat(zs)
         return self._out(lnlike)
 
+    def _log_likelihood_lowrank(self, t, flux, data_cov, i, p, u, baseline_mean, baseline_var,
+                                marginalize_over_inclination):
+        """``log_likelihood(method="lowrank")``: include/spb200.h spb_lowrank_*."""
+        marg = self._marginalize_over_inclination if marginalize_over_inclination is None \
+            else bool(marginalize_over_inclination)
+        if marg:
+            raise ValueError("method='lowrank' needs marginalize_over_inclination=False: the marginalised "
+                             "covariance is the cubic interpolant of flux.py:256-276, which is not low-rank")
+        if self._tkind:
+            raise ValueError("method='lowrank' does not cover time-variable surfaces (tau): the temporal "
+                             "kernel makes the covariance full-rank")
+        dc = data_cov if isinstance(data_cov, torch.Tensor) else np.asarray(data_cov, dtype=np.float64)
+        if dc.ndim > 1:
+            raise ValueError("method='lowrank' needs a scalar or (nt,) data_cov, not a full matrix")
+        if not (isinstance(dc, torch.Tensor) and dc.is_cuda):
+            if not np.all(np.asarray(dc.cpu() if isinstance(dc, torch.Tensor) else dc) > 0.0):
+                raise ValueError("method='lowrank' needs a positive data_cov (it whitens with D^-1/2)")
+        bv_in = baseline_var
+        if isinstance(bv_in, (torch.Tensor, np.ndarray)) and bv_in.ndim > 1:
+            raise ValueError("method='lowrank' needs a scalar or (B,) baseline_var, not a full matrix")
+        nt = torch.as_tensor(t).numel() if isinstance(t, torch.Tensor) else np.asarray(t).size
+        if nt < 31:
+            raise ValueError("method='lowrank' needs nt >= 31 time stamps (the rank of the phase basis)")
+        _, t, inc, rta1 = self._prep(t, i, p, u, False)
+        dev, B = self.device, self._B
+        f = torch.as_tensor(flux, dtype=torch.float64).to(dev)
+        if f.ndim == 1:
+            f = f[None]
+        per_element = f.ndim == 3
+        if per_element and f.shape[0] != B:
+            raise ValueError("per-element flux must have shape (B, M, nt)")
+        if f.shape[-1] != nt:
+            raise ValueError("flux must have shape (nt,), (M, nt) or (B, M, nt)")
+        f = f.contiguous()
+        M = f.shape[-2]
+        bm = torch.as_tensor(baseline_mean, dtype=torch.float64).to(dev).contiguous()
+        if bm.ndim == 1 and bm.numel() != B:
+            raise ValueError("a 1-D baseline_mean must have one entry per batch element")
+        bvar = None
+        if isinstance(bv_in, (torch.Tensor, np.ndarray)) or bv_in != 0.0:
+            bvar = bv_in
+        keep = []
+        nm = self._noise_model(nt, data_cov, bvar, keep)
+        lib, h = self._lib, self._ctx.handle
+        I = inc.numel()
+        lnlike = torch.empty(B, dtype=torch.float64, device=dev)
+        z = torch.zeros(B, dtype=torch.float64, device=dev)
+        with torch.cuda.device(dev):
+            ev = self._mark("lowrank_inclination")
+            Binc = torch.empty(I, 32, 256, dtype=torch.float64, device=dev)
+            nb = lib.spb_lowrank_inclination_workspace_bytes(h, I)
+            ws = torch.empty(nb, dtype=torch.uint8, device=dev)
+            _lib.check(lib.spb_lowrank_inclination(h, I, _ptr(inc), _ptr(rta1), 0, _ptr(Binc), _ptr(ws), nb,
+                                                   _stream()))
+            self._mark_end(ev)
+            ev = self._mark("lowrank_basis")
+            Q = torch.empty(nt, 32, dtype=torch.float64, device=dev)
+            R = torch.empty(32, 32, dtype=torch.float64, device=dev)
+            aux = torch.empty(65, dtype=torch.float64, device=dev)
+            nb = lib.spb_lowrank_basis_workspace_bytes(h, nt)
+            ws = torch.empty(nb, dtype=torch.uint8, device=dev)
+            _lib.check(lib.spb_lowrank_basis(h, nt, _ptr(t), float(p), nm.data_kind, ctypes.c_void_p(nm.data_cov),
+                                             _ptr(Q), _ptr(R), _ptr(aux), _ptr(ws), nb, _stream()))
+            self._mark_end(ev)
+            ev = self._mark("lowrank_lnlike")
+            nb = lib.spb_lowrank_lnlike_workspace_bytes(h, B, M, nt)
+            ws = torch.empty(nb, dtype=torch.uint8, device=dev)
+            _lib.check(lib.spb_lowrank_lnlike(
+                h, B, nt, _ptr(Binc), 0 if I == 1 else 32 * 256, _ptr(self._mean_ylm), _ptr(self._cov_ylm),
+                _ptr(Q), _ptr(R), _ptr(aux), ctypes.byref(nm), M, _ptr(f), nt, M * nt if per_element else 0,
+                _ptr(bm), 1 if bm.ndim == 1 else 0, _ptr(lnlike), None, None, _ptr(z), _ptr(self._info),
+                _ptr(ws), nb, _stream()))
+            self._mark_end(ev)
+            del ws, keep
+        self._z = z
+        return self._out(lnlike)
+
     # ------------------------------------------------------------------ SURVEY 8(f) rank 4: gradient
     def log_likelihood_and_grad(self, t, flux, data_cov, i=defaults["i"], p=defaults["p"], u=None,
                                 baseline_mean=defaults["baseline_mean"],
                                 baseline_var=defaults["baseline_var"],
-                                marginalize_over_inclination=None, rel_step=1e-4):
+                                marginalize_over_inclination=None, rel_step=1e-4, method="dense"):
         """``log_likelihood`` and its gradient with respect to the hyperparameters the process was
         built from -- ``r`` [deg], ``a`` and ``b`` (or ``mu`` and ``sigma`` [deg]), ``c``, ``n`` -- as
         ``(lnlike, {"r": ..., "a" | "mu": ..., "b" | "sigma": ..., "c": ..., "n": ...})``, one value
@@ -895,7 +985,8 @@ class StarryProcess(object):
         central difference along each tangent has a relative truncation error of ``rel_step**2``
         (the flux-side likelihood is smooth in the moments) and no eigen-solver noise, because the
         displaced sets share the base eigen-problem up to the smooth perturbation.  Measured against
-        the analytic oracle (oracle/sp_oracle_grad.py): <= 1e-6 relative."""
+        the analytic oracle (oracle/sp_oracle_grad.py): <= 1e-6 relative.  ``method`` selects the
+        likelihood evaluation of the 11 B elements, as in ``log_likelihood``."""
         if self._dr is not None or self._time_variable or not hasattr(self, "_r") or self._r is None:
             raise NotImplementedError("gradients: delta spot-size prior, static surfaces, a single "
                                       "process (not a sum)")
@@ -936,7 +1027,7 @@ class StarryProcess(object):
             ll_all = big.log_likelihood(
                 t, tile(flux, 3), data_cov, i=tile(i, 1), p=p, u=u, baseline_mean=tile(baseline_mean, 1),
                 baseline_var=tile(baseline_var, 1),
-                marginalize_over_inclination=marginalize_over_inclination).reshape(11, B)
+                marginalize_over_inclination=marginalize_over_inclination, method=method).reshape(11, B)
             self._z = None if big._z is None else big._z[:B]
             self._info = big._info[:B].clone()
             ll = ll_all[0]

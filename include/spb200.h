@@ -15,8 +15,10 @@
  *     stream), re-entrant across streams/devices, and performs no host synchronisation;
  *   - return value: 0 on success, non-zero on a usage / CUDA error (message: spb_last_error());
  *   - per-batch-element numerical failures (non positive-definite K, normalised process outside
- *     its validity range) never fail the call: they set info[b] != 0 and lnlike[b] = -inf, the
- *     batched analogue of the reference's NaN -> -inf convention (math.py:82-91, sp.py:1178-1188);
+ *     its validity range, hyperparameters out of bounds, a latitude eigen-solve that did not
+ *     converge) never fail the call: they set info[b] != 0 and lnlike[b] = -inf (the bits of
+ *     SPB_INFO_NEG_INF), the batched analogue of the reference's NaN -> -inf convention
+ *     (math.py:82-91, sp.py:1178-1188);
  *   - Ylm index n = l^2 + l + m; angles in radians at this level (the Python surface takes degrees).
  */
 #ifndef SPB200_H
@@ -42,6 +44,10 @@ typedef struct spb_context spb_context;
 #define SPB_INFO_BOUNDS 4       /* hyperparameter outside CheckBoundsOp range (ops/exceptions.py:30-48) */
 #define SPB_INFO_EIG_NOCONV 8   /* latitude eigen-solve did not converge (eigh.py:12-16 -> NaN) */
 #define SPB_INFO_I8_RANGE 16    /* transient: spb_cholesky_lnlike_i8 re-ran this matrix on the DMMA kernel */
+/* The bits that force lnlike[b] = -inf on every log-likelihood route (dense Cholesky kernels, the INT8
+ * Cholesky, the rank-31 route): each marks an element whose reference value is NaN (-> -inf).  A NaN
+ * lnlike maps to -inf as well.  SPB_INFO_I8_RANGE is not among them: it only records a re-run.          */
+#define SPB_INFO_NEG_INF (SPB_INFO_NOT_PD | SPB_INFO_Z_RANGE | SPB_INFO_BOUNDS | SPB_INFO_EIG_NOCONV)
 
 const char *spb_last_error(void);
 int spb_version(void);
@@ -293,9 +299,10 @@ int spb_cholesky_lnlike_affine(spb_context *ctx, int B, int nt, double *K, int l
  * plane products -- the fastest), 8 or 87 = eight planes of 7-bit digits (56 bits, 36 products), 7 or 77 =
  * seven planes of 7-bit digits (49 bits).  Replaces the same
  * reference lines as spb_cholesky_lnlike_affine (math.py:75-100, sp.py:1154-1188).  Differences:
- *   K is only READ (the factor is not returned);  a lower bound of the smallest eigenvalue of K' is
- *   needed to scale the right-hand-side rows: `lambda_min` > 0 (e.g. the white-noise variance already
- *   added to K), or, when lambda_min <= 0, min(affine->diag) (`affine` may be NULL otherwise);  workspace of
+ *   K is only READ (the factor is not returned);  a diagonal lower bound diag(d) <= K' is needed to
+ *   scale the right-hand-side rows (|y_k|^2 <= sum_k r_k^2 / d_k): d = `lambda_min` > 0 (e.g. the
+ *   white-noise variance already added to K), or, when lambda_min <= 0, the affine diagonal
+ *   affine->diag (`affine` may be NULL otherwise);  workspace of
  *   spb_cholesky_i8_workspace_bytes(B, nt, M, planes) bytes (digit planes + row scales);
  *   matrices whose digits overflow (SPB_INFO_I8_RANGE, never observed) are re-run through the FP64
  *   kernel, which overwrites THEIR K with L.
@@ -406,6 +413,8 @@ int spb_dmma_peak(spb_context *ctx, int iters, double *tflops_host, double *ms_h
  *                              (A Sigma) A^T of spb_flux_conditional_lower (flux.py:335-343) -- on the INT8
  *                              tensor cores (exact 7 x 8-bit digit planes, tcgen05 + TMEM; cov_ylm within
  *                              1e-15 of its maximum of the FP64 result) | on the FP64 (DMMA) tensor cores;
+ *                              on the INT8 form, entries of K that involve a row of A Sigma or A holding an
+ *                              inf / NaN, or an entry of magnitude >= 1e300, are NaN (DESIGN.md 4.4);
  *                              environment default SPB_SYRK_I8                                     */
 int spb_set_option(spb_context *ctx, const char *name, int value);
 int spb_launch_count(const spb_context *ctx, long long *count_host);

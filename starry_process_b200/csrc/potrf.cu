@@ -908,9 +908,9 @@ __global__ void __launch_bounds__(NTHREADS, 2)
       const bool bad = sm.bad != 0;
       double ll = -0.5 * quad - (double)rm.M * logdet -
                   0.5 * (double)p.n * (double)rm.M * 1.8378770664093453;  // log(2 pi)
-      // flags raised by earlier stages (bounds, normalisation range) also map to -inf
+      // flags raised by earlier stages (bounds, normalisation range, eigen-solve) also map to -inf
       const int prev = p.info ? (p.info[item] & ~(SPB_INFO_NOT_PD | p.only_flag)) : 0;
-      if (bad || (prev & (SPB_INFO_Z_RANGE | SPB_INFO_BOUNDS)) || ll != ll) ll = -INFINITY;
+      if (bad || (prev & SPB_INFO_NEG_INF) || ll != ll) ll = -INFINITY;
       if (p.lnlike) p.lnlike[item] = ll;
       if (p.logdet) p.logdet[item] = bad ? NAN : logdet;
       if (p.info) p.info[item] = prev | (bad ? SPB_INFO_NOT_PD : 0);
@@ -1091,7 +1091,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) potrf_cluster_kernel(PotrfParams 
     double ll = -0.5 * qtot - (double)rm.M * logdet -
                 0.5 * (double)p.n * (double)rm.M * 1.8378770664093453;  // log(2 pi)
     const int prev = p.info ? (p.info[item] & ~SPB_INFO_NOT_PD) : 0;
-    if (bad || (prev & (SPB_INFO_Z_RANGE | SPB_INFO_BOUNDS)) || ll != ll) ll = -INFINITY;
+    if (bad || (prev & SPB_INFO_NEG_INF) || ll != ll) ll = -INFINITY;
     if (p.lnlike) p.lnlike[item] = ll;
     if (p.logdet) p.logdet[item] = bad ? NAN : logdet;
     if (p.info) p.info[item] = prev | (bad ? SPB_INFO_NOT_PD : 0);

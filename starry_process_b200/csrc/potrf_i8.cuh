@@ -45,7 +45,7 @@ struct I8Params {
   long long strideQ;     // bytes per matrix
   int NR, LDQ;
   int store_factor;      // also write L (fp64) over K like the DMMA kernel
-  double lambda_min;     // > 0: lower bound of the smallest eigenvalue of K' (else min(aff.diag))
+  double lambda_min;     // > 0: K' >= lambda_min I (else K' >= diag(aff.diag)): bounds the right-hand-side rows
 };
 
 // Virtual rows of a panel for this kernel.  A tile's A operand must be ONE box of 128 consecutive plane
@@ -104,7 +104,6 @@ struct SmemI8 {
   double red[I8_NCT / 32];
   double dpiv[NB];
   double af[4];
-  double dgmin;
   uint64_t full[STAGES_], empty[STAGES_], tmem_full, tmem_empty;
   unsigned first[I8_MAXP + 1];   // sequence number of the first tile of every panel of this matrix
   uint32_t tmem_base;
@@ -148,20 +147,6 @@ __device__ __forceinline__ double block_sum_i8(SM &sm, double v) {
   double t = 0.0;
 #pragma unroll
   for (int w = 0; w < I8_NCT / 32; ++w) t += sm.red[w];
-  cbar256();
-  return t;
-}
-template <class SM>
-__device__ __forceinline__ double block_min_i8(SM &sm, double v) {
-  const int tid = threadIdx.x, pw = tid >> 5, lane = tid & 31;
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v = fmin(v, __shfl_xor_sync(0xffffffffu, v, o));
-  cbar256();
-  if (lane == 0) sm.red[pw] = v;
-  cbar256();
-  double t = sm.red[0];
-#pragma unroll
-  for (int w = 1; w < I8_NCT / 32; ++w) t = fmin(t, sm.red[w]);
   cbar256();
   return t;
 }
@@ -259,19 +244,8 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
       I8_PROF_DECL(tid == 0 ? 0 : -1);
       if (quad_out)
         for (int m = tid; m < rm.M; m += I8_NCT) quad_out[m] = 0.0;
-      // row scales: 2^e_i > 1.0101 sqrt(K'_ii) for the rows of L;  for the right-hand-side rows
-      // |y_k| <= |y| <= |r| / sqrt(lambda_min(K')) <= sqrt(nt) max|r| / sqrt(min diag) (x 4 of margin)
-      double dgm = 1e300;
-      if (ip.lambda_min > 0.0) {
-        dgm = ip.lambda_min;
-      } else if (af.dg) {
-        if (af.dg_vec) {
-          for (int r = tid; r < p.n; r += I8_NCT) dgm = fmin(dgm, af.dg[r]);
-        } else {
-          dgm = af.dg[0];
-        }
-      }
-      dgm = block_min_i8(sm, dgm);
+      // row scales: 2^e_i > 1.0101 sqrt(K'_ii) for the rows of L;  for the right-hand-side rows a bound of
+      // |y_k| (below)
       // 2^e (x 2 for balanced 8-bit digits); 1 (2) for a row without a finite positive bound
       const auto row_scale = [](double x) {
         int e;
@@ -297,8 +271,19 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
         for (int k = lane; k < p.n; k += 32) mx = fmax(mx, fabs(rr[k]));
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+        // |y_k| <= |y| = sqrt(r^T K'^-1 r) <= sqrt(sum_k r_k^2 / d_k) with d = lambda_min or the affine diagonal
+        // (K' >= diag(d)): unlike sqrt(nt) max|r| / sqrt(min d) it does not grow with a diagonal scaling of K'
+        // or with noise that varies along the light curve (x 4 of margin; summed relative to max|r|)
+        const double inv = (mx > 0.0) ? 1.0 / mx : 0.0;
+        double s = 0.0;
+        for (int k = lane; k < p.n; k += 32) {
+          const double x = rr[k] * inv;
+          s += x * x / ((ip.lambda_min > 0.0) ? ip.lambda_min : (af.dg_vec ? af.dg[k] : af.dg[0]));
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
         if (lane == 0)
-          Eb[n64 + m] = row_scale(4.0 * sqrt((double)p.n) * mx * rsqrt(dgm));
+          Eb[n64 + m] = row_scale(4.0 * mx * sqrt(s));
       }
       for (int r = p.n + tid; r < n64; r += I8_NCT) Eb[r] = 1.0;
       __threadfence_block();
@@ -562,7 +547,7 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
         double ll = -0.5 * quad - (double)rm.M * logdet -
                     0.5 * (double)p.n * (double)rm.M * 1.8378770664093453;  // log(2 pi)
         const int prev = p.info ? (p.info[item] & ~(SPB_INFO_NOT_PD | SPB_INFO_I8_RANGE)) : 0;
-        if (bad || (prev & (SPB_INFO_Z_RANGE | SPB_INFO_BOUNDS)) || ll != ll) ll = -INFINITY;
+        if (bad || (prev & SPB_INFO_NEG_INF) || ll != ll) ll = -INFINITY;
         if (p.lnlike) p.lnlike[item] = ll;
         if (p.logdet) p.logdet[item] = bad ? NAN : logdet;
         if (p.info)

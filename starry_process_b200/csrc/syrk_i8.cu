@@ -265,25 +265,34 @@ struct GemmLParams {
 };
 
 // digit planes of `rows` rows of 256 doubles: src (nb, rows, 256) -> Q (nb, 7, rows, 256), E (nb, rows)
+//   * a row holding an inf or a NaN, or whose maximum is 1e300 or more (2^e would not fit), gets E = NaN:
+//     every product touching it comes out NaN, as on the FP64 GEMM, instead of a finite value from
+//     digits that cannot represent it;
+//   * E >= 2^-1058, so that the epilogue's E 2^-16 does not underflow for rows of subnormals; such rows
+//     are scaled by 2^200 before the cut (x 2^56 / E alone would overflow below 2^-967), exactly.
 __global__ void __launch_bounds__(256) slice256_kernel(const double *src, long long stride_b, int rows, uint8_t *Q,
                                                        double *E) {
   const int b = blockIdx.y, row = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
   if (row >= rows) return;
   const double *xr = src + (size_t)b * stride_b + (size_t)row * 256;
   double v[2][4];
-  double mx = 0.0;
+  double mx = 0.0, nf = 0.0;   // nf: x - x summed over the entries, NaN iff one is inf or NaN
 #pragma unroll
   for (int j = 0; j < 2; ++j) {
     const double4 t = *reinterpret_cast<const double4 *>(xr + 4 * (lane + 32 * j));
     v[j][0] = t.x; v[j][1] = t.y; v[j][2] = t.z; v[j][3] = t.w;
     mx = fmax(mx, fmax(fmax(fabs(t.x), fabs(t.y)), fmax(fabs(t.z), fabs(t.w))));
+    nf += ((t.x - t.x) + (t.y - t.y)) + ((t.z - t.z) + (t.w - t.w));
   }
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+  const bool bad = __any_sync(0xffffffffu, nf != 0.0) || mx >= 1e300;
   int ex;
-  const double Ev = i8_scale_exp(mx, ex) ? ldexp(1.0, ex + 1) : 1.0;
+  double Ev = i8_scale_exp(mx, ex) ? ldexp(1.0, ex + 1 > -1058 ? ex + 1 : -1058) : 1.0;
+  if (bad) Ev = __longlong_as_double(0x7ff8000000000000ll);
   if (lane == 0) E[(size_t)b * rows + row] = Ev;
-  const double sinv = ldexp(1.0 / Ev, SY_RB * SY_S);
+  const double pre = (Ev < 0x1p-900) ? 0x1p+200 : 1.0;
+  const double sinv = ldexp(1.0 / (Ev * pre), SY_RB * SY_S);
   uint8_t *qrow = Q + ((size_t)b * SY_S * rows + row) * 256;
   const size_t pstride = (size_t)rows * 256;
 #pragma unroll
@@ -292,7 +301,7 @@ __global__ void __launch_bounds__(256) slice256_kernel(const double *src, long l
 #pragma unroll
     for (int s = 0; s < SY_S; ++s) W[s] = 0u;
 #pragma unroll
-    for (int c = 0; c < 4; ++c) (void)i8_cut<SY_S, SY_RB>(v[j][c] * sinv, 8 * c, W);
+    for (int c = 0; c < 4; ++c) (void)i8_cut<SY_S, SY_RB>(v[j][c] * pre * sinv, 8 * c, W);
 #pragma unroll
     for (int s = 0; s < SY_S; ++s)
       *reinterpret_cast<uint32_t *>(qrow + (size_t)s * pstride + 4 * (lane + 32 * j)) = i8_recentre<SY_RB>(s, W[s]);

@@ -348,6 +348,24 @@ int spb_cholesky_solve_rows(spb_context *ctx, int nt, const double *L, int ldk, 
  *                           (flux_stride elements between elements); baseline_mean: NULL | one value
  *                           (bm_stride 0) | one per element (bm_stride 1).  quad (B, M), logdet (B)
  *                           (= logdet K), z_out (B) may be NULL.
+ *
+ * Predictive distribution (predict / sample_conditional) of an unnormalised process given one light curve:
+ *   mean(ts) = gp_mean + Phi(ts) a,   cov(ts, ts) = Phi(ts) P Phi(ts)^T,   draws = mean + Phi(ts) G z1 + sqrt(eps) z2
+ * spb_lowrank_posterior   : per element, from the operands of spb_lowrank_lnlike with M = 1 and a flux (nt)
+ *                           shared by the batch (noise->normalized must be 0): a (B, 32) = C~ R^T N^-1 w,
+ *                           P (B, 32, 32) = C~ - V^T V with V = L_N^-1 R C~, G (B, 32, 32) with G G^T = P
+ *                           (eigenvectors scaled by sqrt(max(lambda, 0))), gp_mean (B).  info (B) in/out:
+ *                           SPB_INFO_NOT_PD is set where N is not PD (a, P and G are then NaN) or where
+ *                           P has an eigenvalue below -1e-10 max(lambda_max(P), max_k C~_kk) (G is then
+ *                           NaN: no draws; a and P stay valid).  Other bits are kept.
+ *                           Workspace of spb_lowrank_posterior_workspace_bytes(B, nt) bytes.
+ * spb_lowrank_predict_eval: for nts time stamps t_sample and the posterior above: mean (B, nts); var (B, nts)
+ *                           = diag(Phi P Phi^T) or NULL; cov (B, nts, ldc) = Phi P Phi^T or NULL (two DMMA
+ *                           products; P 16-byte aligned); with nsamples > 0, draws (B, nsamples, nts) from
+ *                           unit_normals (nsamples, 32 + nts) per draw [z1 (32) | z2 (nts)], shared by the
+ *                           batch (un_stride 0) or per element (un_stride nsamples * (32 + nts)).  Workspace of
+ *                           spb_lowrank_predict_eval_workspace_bytes(B, nts, nsamples, cov != NULL) bytes.
+ *                           Nothing of size nts^2 is formed unless cov is requested.
  * ------------------------------------------------------------------------------------------- */
 size_t spb_lowrank_inclination_workspace_bytes(const spb_context *ctx, int I);
 int spb_lowrank_inclination(spb_context *ctx, int I, const double *inc_rad, const double *rTA1,
@@ -364,6 +382,20 @@ int spb_lowrank_lnlike(spb_context *ctx, int B, int nt, const double *Binc, long
                        int ldf, long long flux_stride, const double *baseline_mean, long long bm_stride,
                        double *lnlike, double *quad, double *logdet, double *z_out, int32_t *info,
                        void *workspace, size_t workspace_bytes, void *stream);
+size_t spb_lowrank_posterior_workspace_bytes(const spb_context *ctx, int B, int nt);
+int spb_lowrank_posterior(spb_context *ctx, int B, int nt, const double *Binc, long long Binc_stride,
+                          const double *mean_ylm, const double *cov_ylm, const double *Q, const double *R,
+                          const double *phi_aux, const spb_noise_model *noise, const double *flux,
+                          const double *baseline_mean, long long bm_stride, double *a, double *P, double *G,
+                          double *gp_mean, int32_t *info, void *workspace, size_t workspace_bytes,
+                          void *stream);
+size_t spb_lowrank_predict_eval_workspace_bytes(const spb_context *ctx, int B, int nts, int nsamples,
+                                                int full_cov);
+int spb_lowrank_predict_eval(spb_context *ctx, int B, int nts, const double *t_sample, double period,
+                             const double *a, const double *P, const double *G, const double *gp_mean,
+                             int nsamples, const double *unit_normals, long long un_stride, double eps,
+                             double *mean, double *var, double *cov, int ldc, double *draws, void *workspace,
+                             size_t workspace_bytes, void *stream);
 
 /* ---------------------------------------------------------------------------------------------
  * (f-2) building blocks of predict / sample / sample_conditional / sample_ylm_conditional

@@ -92,6 +92,12 @@ PROTOTYPES = {
     "spb_lowrank_lnlike_workspace_bytes": (_SZ, [_P, _I, _I, _I]),
     "spb_lowrank_lnlike": (_I, [_P, _I, _I, _P, _LL, _P, _P, _P, _P, _P, _c.POINTER(NoiseModel), _I, _P,
                                 _I, _LL, _P, _LL, _P, _P, _P, _P, _P, _P, _SZ, _P]),
+    "spb_lowrank_posterior_workspace_bytes": (_SZ, [_P, _I, _I]),
+    "spb_lowrank_posterior": (_I, [_P, _I, _I, _P, _LL, _P, _P, _P, _P, _P, _c.POINTER(NoiseModel), _P, _P,
+                                   _LL, _P, _P, _P, _P, _P, _P, _SZ, _P]),
+    "spb_lowrank_predict_eval_workspace_bytes": (_SZ, [_P, _I, _I, _I, _I]),
+    "spb_lowrank_predict_eval": (_I, [_P, _I, _I, _P, _D, _P, _P, _P, _P, _I, _P, _LL, _D, _P, _P, _P, _I, _P,
+                                      _P, _SZ, _P]),
     "spb_temporal_scale":(_I, [_P, _I, _I, _I, _P, _P, _I, _P, _LL, _P, _LL, _P, _I, _LL, _P]),
     "spb_gemm_nt": (_I, [_P, _I, _I, _I, _I, _D, _P, _I, _LL, _P, _I, _LL, _D, _P, _I, _LL, _P]),
     "spb_tril": (_I, [_P, _I, _I, _P, _I, _LL, _P]),

@@ -541,6 +541,284 @@ __global__ void lowrank_final_kernel(int B, int M, int nt, int nch, const double
   lnlike[b] = flagged ? -INFINITY : ll;
 }
 
+// ---------------------------------------------------------------------------------------------------
+// Predictive distribution of the unnormalised process given one light curve.  K(ts, t) = Phi_s C~ Phi^T and
+// K(ts, ts) = Phi_s C~ Phi_s^T, so with (Q T Q^T + I)^-1 = I - Q (I - N^-1) Q^T:
+//   mean(ts) = gp_mean + Phi_s a,        a = C~ R^T N^-1 w
+//   cov(ts)  = Phi_s P Phi_s^T,          P = C~ - V^T V,  V = L_N^-1 R C~
+// and draws use G G^T = P (eigenvectors of P scaled by the square roots of its eigenvalues, negative ones
+// clipped to zero): any square root gives the same distribution, and this one exists for a singular P.
+// Row and column 31 of C~, and therefore of P, are the zero padding.
+// ---------------------------------------------------------------------------------------------------
+// An eigenvalue of P below -1e-10 max(lambda_max(P), max_k C~_kk) sets SPB_INFO_NOT_PD: the subtraction
+// C~ - V^T V rounds at eps max C~_kk, which can exceed 1e-10 lambda_max(P) where the data pin every mode down.
+constexpr double POST_NEG_TOL = 1e-10;
+constexpr int JACOBI_SWEEPS = 30;
+constexpr int EVAL_EB = 8;               // elements per CTA of the evaluation
+constexpr int EVAL_SB = 32;              // draws per CTA of the evaluation
+
+struct PostParams {
+  const double *Binc;
+  long long Binc_stride;
+  const double *mean_ylm;
+  const double *C;          // (B, 32, 32) = B_inc Sigma B_inc^T
+  const double *R;          // (32, 32)
+  const double *aux;        // s | Phi(t0) | sum log D
+  const double *bvar;       // baseline variance: NULL | one value (bv_stride 0) | one per element (1)
+  long long bv_stride;
+  const double *L;          // (B, 32, 32) Cholesky factor of N (lowrank_cov_kernel)
+  const double *w;          // (B, 32) Q^T y (lowrank_wsum_kernel)
+  double *a, *P, *G, *gp_mean;
+  int32_t *info;
+};
+
+__global__ void __launch_bounds__(256) lowrank_post_kernel(PostParams p) {
+  __shared__ double Cs[LR * QR_LD], Rs[LR * QR_LD], Ls[LR * QR_LD], Vs[LR * QR_LD];
+  __shared__ double bmv[LR], us[LR];
+  const int b = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const double *Bb = p.Binc + (size_t)b * p.Binc_stride;
+  double *ab = p.a + (size_t)b * LR, *Pb = p.P + (size_t)b * LR * LR, *Gb = p.G + (size_t)b * LR * LR;
+  // GP mean (A mean_ylm)[0], summed in the order of lowrank_cov_kernel
+  for (int k = warp; k < LR; k += 8) {
+    double v = 0.0;
+    for (int n = lane; n < 256; n += 32) v += Bb[k * 256 + n] * p.mean_ylm[(size_t)b * 256 + n];
+    v = warp_sum(v);
+    if (lane == 0) bmv[k] = v;
+  }
+  for (int idx = tid; idx < LR * LR; idx += 256) {
+    const int i = idx / LR, j = idx % LR;
+    Cs[i * QR_LD + j] = p.C[(size_t)b * LR * LR + (i >= j ? i * LR + j : j * LR + i)];
+    Rs[i * QR_LD + j] = p.R[idx];
+    Ls[i * QR_LD + j] = p.L[(size_t)b * LR * LR + idx];
+  }
+  __syncthreads();
+  if (tid == 0) {
+    double g = 0.0;
+    for (int k = 0; k < LR; ++k) g += p.aux[LR + k] * bmv[k];
+    p.gp_mean[b] = g;
+    if (p.bvar) Cs[0] += p.bvar[(size_t)b * p.bv_stride];
+  }
+  if (p.info[b] & SPB_INFO_NOT_PD) {   // N (hence K(t, t)) is not PD: no posterior
+    for (int idx = tid; idx < LR * LR; idx += 256) {
+      Pb[idx] = NAN;
+      Gb[idx] = NAN;
+      if (idx < LR) ab[idx] = NAN;
+    }
+    return;
+  }
+  __syncthreads();
+  if (warp == 0) {   // a = C~ R^T N^-1 w: forward and back substitution with L_N, lane = row
+    double x = p.w[(size_t)b * LR + lane];
+    for (int i = 0; i < LR; ++i) {
+      const double xi = __shfl_sync(0xffffffffu, x, i) / Ls[i * QR_LD + i];
+      if (lane == i) x = xi;
+      else if (lane > i) x -= Ls[lane * QR_LD + i] * xi;
+    }
+    for (int i = LR - 1; i >= 0; --i) {
+      const double xi = __shfl_sync(0xffffffffu, x, i) / Ls[i * QR_LD + i];
+      if (lane == i) x = xi;
+      else if (lane < i) x -= Ls[i * QR_LD + lane] * xi;
+    }
+    double u = 0.0;
+    for (int i = 0; i < LR; ++i) u += Rs[i * QR_LD + lane] * __shfl_sync(0xffffffffu, x, i);
+    us[lane] = u;
+    __syncwarp();
+    double av = 0.0;
+    for (int j = 0; j < LR; ++j) av += Cs[lane * QR_LD + j] * us[j];
+    ab[lane] = av;
+  }
+  // R C~, then V = L_N^-1 (R C~) (one column per thread)
+  for (int idx = tid; idx < LR * LR; idx += 256) {
+    const int i = idx / LR, j = idx % LR;
+    double v = 0.0;
+    for (int k = 0; k < LR; ++k) v += Rs[i * QR_LD + k] * Cs[k * QR_LD + j];
+    Vs[i * QR_LD + j] = v;
+  }
+  __syncthreads();
+  if (tid < LR) {
+    for (int i = 0; i < LR; ++i) {
+      double v = Vs[i * QR_LD + tid];
+      for (int k = 0; k < i; ++k) v -= Ls[i * QR_LD + k] * Vs[k * QR_LD + tid];
+      Vs[i * QR_LD + tid] = v / Ls[i * QR_LD + i];
+    }
+  }
+  __syncthreads();
+  // P = C~ - V^T V, exactly symmetric (entries (i, j) and (j, i) are the same products in the same order);
+  // it replaces R, and the eigenvectors replace L_N
+  for (int idx = tid; idx < LR * LR; idx += 256) {
+    const int i = idx / LR, j = idx % LR;
+    double v = 0.0;
+    for (int k = 0; k < LR; ++k) v += Vs[k * QR_LD + i] * Vs[k * QR_LD + j];
+    v = Cs[i * QR_LD + j] - v;
+    Rs[i * QR_LD + j] = v;
+    Pb[idx] = v;
+  }
+  __syncthreads();
+  if (warp == 0) {
+    // cyclic Jacobi on the leading 31 x 31 block (the round-robin of moments_k1b: 15 disjoint rotations per
+    // round, index 31 the bye), lane = column in the row phase and row in the column phase
+    double *A = Rs, *U = Ls;
+    for (int r = 0; r < LR; ++r) U[r * QR_LD + lane] = (r == lane) ? 1.0 : 0.0;
+    double amax = 0.0;
+    for (int k = 0; k < LR - 1; ++k) amax = fmax(amax, fabs(A[k * QR_LD + k]));
+    const double floor2 = (1e-20 * amax) * (1e-20 * amax);
+    __syncwarp();
+    for (int sweep = 0; sweep < JACOBI_SWEEPS; ++sweep) {
+      bool rotated = false;
+      for (int rnd = 0; rnd < LR - 1; ++rnd) {
+        double cl = 1.0, sl = 0.0;
+        if (lane >= 1 && lane < 16) {
+          int pk = rnd + lane, qk = rnd - lane + 31;
+          pk -= (pk >= 31) ? 31 : 0;
+          qk -= (qk >= 31) ? 31 : 0;
+          const int pi = min(pk, qk), qi = max(pk, qk);
+          const double apq = A[pi * QR_LD + qi], app = A[pi * QR_LD + pi], aqq = A[qi * QR_LD + qi];
+          if (apq * apq > fmax(floor2, 1.6e-29 * fabs(app * aqq))) {
+            const double tau = (aqq - app) / (2.0 * apq);
+            const double t = (tau >= 0.0 ? 1.0 : -1.0) / (fabs(tau) + sqrt(1.0 + tau * tau));
+            cl = 1.0 / sqrt(1.0 + t * t);
+            sl = t * cl;
+          }
+        }
+        rotated |= __any_sync(0xffffffffu, sl != 0.0);
+        int P_[15], Q_[15];
+        double C_[15], S_[15];
+#pragma unroll
+        for (int k = 0; k < 15; ++k) {
+          int pk = rnd + k + 1, qk = rnd - k - 1 + 31;
+          pk -= (pk >= 31) ? 31 : 0;
+          qk -= (qk >= 31) ? 31 : 0;
+          P_[k] = min(pk, qk);
+          Q_[k] = max(pk, qk);
+          C_[k] = __shfl_sync(0xffffffffu, cl, k + 1);
+          S_[k] = __shfl_sync(0xffffffffu, sl, k + 1);
+        }
+        __syncwarp();
+        // rows: A <- J^T A (lane = column); the 15 rotations touch disjoint pairs
+#pragma unroll
+        for (int k = 0; k < 15; ++k) {
+          const double ap = A[P_[k] * QR_LD + lane], aq = A[Q_[k] * QR_LD + lane];
+          A[P_[k] * QR_LD + lane] = C_[k] * ap - S_[k] * aq;
+          A[Q_[k] * QR_LD + lane] = S_[k] * ap + C_[k] * aq;
+        }
+        __syncwarp();
+        // columns: A <- A J, U <- U J (lane = row)
+#pragma unroll
+        for (int k = 0; k < 15; ++k) {
+          const double ap = A[lane * QR_LD + P_[k]], aq = A[lane * QR_LD + Q_[k]];
+          A[lane * QR_LD + P_[k]] = C_[k] * ap - S_[k] * aq;
+          A[lane * QR_LD + Q_[k]] = S_[k] * ap + C_[k] * aq;
+          const double up = U[lane * QR_LD + P_[k]], uq = U[lane * QR_LD + Q_[k]];
+          U[lane * QR_LD + P_[k]] = C_[k] * up - S_[k] * uq;
+          U[lane * QR_LD + Q_[k]] = S_[k] * up + C_[k] * uq;
+        }
+        __syncwarp();
+      }
+      if (!rotated) break;
+    }
+    const double lam = lane < LR - 1 ? A[lane * QR_LD + lane] : 0.0;
+    double lmax = lam, lmin = lam, cmax = fabs(Cs[lane * QR_LD + lane]);
+    for (int o = 16; o > 0; o >>= 1) {
+      lmax = fmax(lmax, __shfl_xor_sync(0xffffffffu, lmax, o));
+      lmin = fmin(lmin, __shfl_xor_sync(0xffffffffu, lmin, o));
+      cmax = fmax(cmax, __shfl_xor_sync(0xffffffffu, cmax, o));
+    }
+    // only the draws need the square root: a and P stay valid, G is NaN
+    const bool bad = !(lmin >= -POST_NEG_TOL * fmax(lmax, cmax));
+    const double sq = sqrt(fmax(lam, 0.0));
+    for (int k = 0; k < LR; ++k) {   // G[lane][k] = U[lane][k] sqrt(lambda_k)
+      const double g = U[lane * QR_LD + k] * __shfl_sync(0xffffffffu, sq, k);
+      Gb[lane * LR + k] = bad ? NAN : g;
+    }
+    if (lane == 0 && bad) p.info[b] |= SPB_INFO_NOT_PD;
+  }
+}
+
+// gz[b][s] = G_b z1 (the first 32 unit normals of draw s)
+__global__ void __launch_bounds__(256) lowrank_gz_kernel(int B, int S, int nts, const double *G, const double *z,
+                                                         long long z_stride, double *gz) {
+  const long long pr = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
+  const int lane = threadIdx.x & 31;
+  if (pr >= (long long)B * S) return;
+  const int b = (int)(pr / S), s = (int)(pr % S);
+  const double *zr = z + (size_t)b * z_stride + (size_t)s * (LR + nts);
+  const double *Gb = G + (size_t)b * LR * LR;
+  double v = 0.0;
+  for (int j = 0; j < LR; ++j) v += Gb[lane * LR + j] * zr[j];
+  gz[(size_t)pr * LR + lane] = v;
+}
+
+struct EvalParams {
+  int B, nts, S;
+  const double *ts;
+  double period;
+  const double *a, *P, *gp_mean;
+  const double *gz;         // (B, S, 32)
+  const double *z;          // unit normals (S, 32 + nts) per element, z_stride elements apart
+  long long z_stride;
+  double sq_eps;
+  double *mean, *var, *draws;
+};
+
+// CTA (256 output points x EVAL_EB elements x EVAL_SB draws).  Phi(ts) is rebuilt with phase_row (the
+// rounding of the basis rows); the mean and variance are written by the CTAs of the first draw group.
+__global__ void __launch_bounds__(256) lowrank_eval_kernel(EvalParams p) {
+  __shared__ double Ps[LR * LR];
+  __shared__ double as[LR];
+  const int tid = threadIdx.x;
+  const long long i = (long long)blockIdx.x * 256 + tid;
+  const bool have = i < p.nts;
+  const int e0 = blockIdx.y * EVAL_EB, s0 = blockIdx.z * EVAL_SB;
+  const int s1 = min(p.S, s0 + EVAL_SB);
+  const bool first = blockIdx.z == 0;
+  double row[LR];
+  phase_row(have ? p.ts[i] : 0.0, p.period, row);
+  for (int e = 0; e < EVAL_EB && e0 + e < p.B; ++e) {
+    const int b = e0 + e;
+    __syncthreads();
+    if (tid < LR) as[tid] = p.a[(size_t)b * LR + tid];
+    if (p.var && first)
+      for (int idx = tid; idx < LR * LR; idx += 256) Ps[idx] = p.P[(size_t)b * LR * LR + idx];
+    __syncthreads();
+    if (!have) continue;
+    double d = 0.0;
+#pragma unroll
+    for (int k = 0; k < LR; ++k) d += row[k] * as[k];
+    const double m = p.gp_mean[b] + d;
+    if (first) {
+      p.mean[(size_t)b * p.nts + i] = m;
+      if (p.var) {   // sum_k (Phi P)_k Phi_k: the association of the two products that form the full matrix
+        double v = 0.0;
+#pragma unroll
+        for (int k = 0; k < LR; ++k) {
+          double tk = 0.0;
+#pragma unroll
+          for (int j = 0; j < LR; ++j) tk += row[j] * Ps[k * LR + j];
+          v += tk * row[k];
+        }
+        p.var[(size_t)b * p.nts + i] = v;
+      }
+    }
+    for (int s = s0; s < s1; ++s) {
+      const double *g = p.gz + ((size_t)b * p.S + s) * LR;
+      double d2 = 0.0;
+#pragma unroll
+      for (int k = 0; k < LR; ++k) d2 += row[k] * g[k];
+      const double z2 = p.z[(size_t)b * p.z_stride + (size_t)s * (LR + p.nts) + LR + i];
+      p.draws[((size_t)b * p.S + s) * p.nts + i] = m + d2 + p.sq_eps * z2;
+    }
+  }
+}
+
+// Phi(ts) (n, 32), the left factor of the full predictive covariance
+__global__ void __launch_bounds__(256) lowrank_phi_kernel(int n, const double *t, double period, double *Phi) {
+  const long long i = (long long)blockIdx.x * 256 + threadIdx.x;
+  if (i >= n) return;
+  double row[LR];
+  phase_row(t[i], period, row);
+  for (int c = 0; c < LR; ++c) Phi[(size_t)i * LR + c] = row[c];
+}
+
 struct LnlikeLayout {
   double *T, *C, *L, *off, *logdet, *wpart, *w, *qn, *sqpart;
   size_t bytes;
@@ -561,6 +839,25 @@ LnlikeLayout lnlike_layout(void *ws, int B, int M, int nt) {
   return l;
 }
 
+// predict_eval workspace: G z1 (B, S, 32) | full covariance only: Phi(ts) (nts, 32) | Phi(ts) P (B, nts, 32)
+struct EvalLayout {
+  double *gz, *Phi, *T;
+  size_t bytes;
+};
+
+EvalLayout eval_layout(void *ws, int B, int nts, int S, int full_cov) {
+  const size_t sizes[3] = {(size_t)B * S * LR, full_cov ? (size_t)nts * LR : 0,
+                           full_cov ? (size_t)B * nts * LR : 0};
+  double *ptrs[3];
+  size_t off = 0;
+  for (int k = 0; k < 3; ++k) {
+    ptrs[k] = ws ? reinterpret_cast<double *>(reinterpret_cast<unsigned char *>(ws) + off) : nullptr;
+    off += ((sizes[k] * sizeof(double) + 255) / 256) * 256;
+  }
+  EvalLayout l = {ptrs[0], ptrs[1], ptrs[2], off};
+  return l;
+}
+
 constexpr size_t QR_SMEM = (2 * QR_ROWS * QR_LD + LR) * sizeof(double);
 constexpr size_t SOLVE_SMEM = (8 * 32 * QR_LD + 8 * SOLVE_EB * LR + SOLVE_EB * LR) * sizeof(double);
 
@@ -574,6 +871,98 @@ int set_smem_attributes(spb_context *ctx) {
                                         (int)SOLVE_SMEM));
     return 0;
   });
+}
+
+// The part of the conditional evaluation shared by the log-likelihood and the predictive posterior:
+// C = B_inc Sigma B_inc^T, lowrank_cov_kernel (GP mean, C~, Cholesky of N), pass 1 of the solve and the
+// w sums.  `sp` is left filled in for pass 2.
+int lowrank_front(spb_context *ctx, int B, int nt, const double *Binc, long long Binc_stride,
+                  const double *mean_ylm, const double *cov_ylm, const double *Q, const double *R,
+                  const double *phi_aux, const spb_noise_model *noise, int M, const double *flux, int ldf,
+                  long long flux_stride, const double *baseline_mean, long long bm_stride, double *z_out,
+                  int32_t *info, const LnlikeLayout &ly, SolveParams &sp, cudaStream_t stream) {
+  const int nch = (nt + SOLVE_CH - 1) / SOLVE_CH;
+  int st = set_smem_attributes(ctx);
+  if (st) return st;
+  // C[b] = B_inc (Sigma B_inc^T): each Sigma is read from HBM once, by the first product
+  for (int b0 = 0; b0 < B; b0 += COV_CHUNK) {
+    const int Bc = (B - b0 < COV_CHUNK) ? B - b0 : COV_CHUNK;
+    gnt::Desc d1 = {};
+    d1.A = Binc + (size_t)b0 * Binc_stride;
+    d1.strideA = Binc_stride;
+    d1.lda = 256;
+    d1.Bm = cov_ylm + (size_t)b0 * 65536;
+    d1.strideB = 65536;
+    d1.ldb = 256;
+    d1.C = ly.T;
+    d1.strideC = (long long)LR * 256;
+    d1.ldc = 256;
+    d1.M = LR;
+    d1.N = 256;
+    d1.K = 256;
+    d1.batch = Bc;
+    d1.ksplit = 1;
+    d1.alpha = 1.0;
+    st = gnt::launch<gnt::EPI_STORE>(ctx, d1, stream);
+    if (st) return st;
+    gnt::Desc d2 = {};
+    d2.A = ly.T;
+    d2.strideA = (long long)LR * 256;
+    d2.lda = 256;
+    d2.Bm = Binc + (size_t)b0 * Binc_stride;
+    d2.strideB = Binc_stride;
+    d2.ldb = 256;
+    d2.C = ly.C + (size_t)b0 * LR * LR;
+    d2.strideC = (long long)LR * LR;
+    d2.ldc = LR;
+    d2.M = LR;
+    d2.N = LR;
+    d2.K = 256;
+    d2.batch = Bc;
+    d2.ksplit = 1;
+    d2.alpha = 1.0;
+    st = gnt::launch<gnt::EPI_STORE>(ctx, d2, stream);
+    if (st) return st;
+  }
+  CovParams cp;
+  cp.nt = nt;
+  cp.Binc = Binc;
+  cp.Binc_stride = Binc_stride;
+  cp.mean_ylm = mean_ylm;
+  cp.C = ly.C;
+  cp.R = R;
+  cp.aux = phi_aux;
+  cp.nm = *noise;
+  cp.bmean = baseline_mean;
+  cp.bm_stride = bm_stride;
+  cp.L = ly.L;
+  cp.off = ly.off;
+  cp.logdet = ly.logdet;
+  cp.z_out = z_out;
+  cp.info = info;
+  lowrank_cov_kernel<<<B, 256, 0, stream>>>(cp);
+  SPB_LAUNCH_CHECK(ctx);
+  sp.B = B;
+  sp.nt = nt;
+  sp.M = M;
+  sp.nch = nch;
+  sp.Q = Q;
+  sp.flux = flux;
+  sp.ldf = ldf;
+  sp.flux_stride = flux_stride;
+  sp.data_kind = noise->data_kind;
+  sp.data_cov = noise->data_cov;
+  sp.off = ly.off;
+  sp.w = ly.w;
+  sp.wpart = ly.wpart;
+  sp.sqpart = ly.sqpart;
+  const dim3 grid(nch, (B + SOLVE_EB - 1) / SOLVE_EB);
+  lowrank_solve_kernel<false><<<grid, 256, SOLVE_SMEM, stream>>>(sp);
+  SPB_LAUNCH_CHECK(ctx);
+  const long long pairs = (long long)B * M;
+  lowrank_wsum_kernel<<<(unsigned)((pairs + 7) / 8), 256, 0, stream>>>(B, M, nch, ly.wpart, ly.L, ly.w, ly.qn);
+  SPB_LAUNCH_CHECK(ctx);
+  return 0;
 }
 
 }  // namespace
@@ -669,97 +1058,182 @@ extern "C" int spb_lowrank_lnlike(spb_context *ctx, int B, int nt, const double 
               "lowrank_lnlike: workspace too small");
   SPB_REQUIRE(((uintptr_t)Binc % 16) == 0 && ((uintptr_t)cov_ylm % 16) == 0,
               "lowrank_lnlike: Binc and cov_ylm must be 16-byte aligned");
+  SPB_REQUIRE((long long)B <= 65535LL * SOLVE_EB, "lowrank_lnlike: batch too large for one launch");
   cudaStream_t stream = (cudaStream_t)stream_;
   SPB_CHECK_CUDA(cudaSetDevice(ctx->device));
   void *ws = reinterpret_cast<void *>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255);
   const LnlikeLayout ly = lnlike_layout(ws, B, M, nt);
   const int nch = (nt + SOLVE_CH - 1) / SOLVE_CH;
-  int st = set_smem_attributes(ctx);
-  if (st) return st;
-  // C[b] = B_inc (Sigma B_inc^T): each Sigma is read from HBM once, by the first product
-  for (int b0 = 0; b0 < B; b0 += COV_CHUNK) {
-    const int Bc = (B - b0 < COV_CHUNK) ? B - b0 : COV_CHUNK;
-    gnt::Desc d1 = {};
-    d1.A = Binc + (size_t)b0 * Binc_stride;
-    d1.strideA = Binc_stride;
-    d1.lda = 256;
-    d1.Bm = cov_ylm + (size_t)b0 * 65536;
-    d1.strideB = 65536;
-    d1.ldb = 256;
-    d1.C = ly.T;
-    d1.strideC = (long long)LR * 256;
-    d1.ldc = 256;
-    d1.M = LR;
-    d1.N = 256;
-    d1.K = 256;
-    d1.batch = Bc;
-    d1.ksplit = 1;
-    d1.alpha = 1.0;
-    st = gnt::launch<gnt::EPI_STORE>(ctx, d1, stream);
-    if (st) return st;
-    gnt::Desc d2 = {};
-    d2.A = ly.T;
-    d2.strideA = (long long)LR * 256;
-    d2.lda = 256;
-    d2.Bm = Binc + (size_t)b0 * Binc_stride;
-    d2.strideB = Binc_stride;
-    d2.ldb = 256;
-    d2.C = ly.C + (size_t)b0 * LR * LR;
-    d2.strideC = (long long)LR * LR;
-    d2.ldc = LR;
-    d2.M = LR;
-    d2.N = LR;
-    d2.K = 256;
-    d2.batch = Bc;
-    d2.ksplit = 1;
-    d2.alpha = 1.0;
-    st = gnt::launch<gnt::EPI_STORE>(ctx, d2, stream);
-    if (st) return st;
-  }
-  CovParams cp;
-  cp.nt = nt;
-  cp.Binc = Binc;
-  cp.Binc_stride = Binc_stride;
-  cp.mean_ylm = mean_ylm;
-  cp.C = ly.C;
-  cp.R = R;
-  cp.aux = phi_aux;
-  cp.nm = *noise;
-  cp.bmean = baseline_mean;
-  cp.bm_stride = bm_stride;
-  cp.L = ly.L;
-  cp.off = ly.off;
-  cp.logdet = ly.logdet;
-  cp.z_out = z_out;
-  cp.info = info;
-  lowrank_cov_kernel<<<B, 256, 0, stream>>>(cp);
-  SPB_LAUNCH_CHECK(ctx);
   SolveParams sp;
-  sp.B = B;
-  sp.nt = nt;
-  sp.M = M;
-  sp.nch = nch;
-  sp.Q = Q;
-  sp.flux = flux;
-  sp.ldf = ldf;
-  sp.flux_stride = flux_stride;
-  sp.data_kind = noise->data_kind;
-  sp.data_cov = noise->data_cov;
-  sp.off = ly.off;
-  sp.w = ly.w;
-  sp.wpart = ly.wpart;
-  sp.sqpart = ly.sqpart;
-  SPB_REQUIRE((long long)B <= 65535LL * SOLVE_EB, "lowrank_lnlike: batch too large for one launch");
-  dim3 grid(nch, (B + SOLVE_EB - 1) / SOLVE_EB);
-  lowrank_solve_kernel<false><<<grid, 256, SOLVE_SMEM, stream>>>(sp);
-  SPB_LAUNCH_CHECK(ctx);
-  const long long pairs = (long long)B * M;
-  lowrank_wsum_kernel<<<(unsigned)((pairs + 7) / 8), 256, 0, stream>>>(B, M, nch, ly.wpart, ly.L, ly.w, ly.qn);
-  SPB_LAUNCH_CHECK(ctx);
+  int st = lowrank_front(ctx, B, nt, Binc, Binc_stride, mean_ylm, cov_ylm, Q, R, phi_aux, noise, M, flux, ldf,
+                         flux_stride, baseline_mean, bm_stride, z_out, info, ly, sp, stream);
+  if (st) return st;
+  const dim3 grid(nch, (B + SOLVE_EB - 1) / SOLVE_EB);
   lowrank_solve_kernel<true><<<grid, 256, SOLVE_SMEM, stream>>>(sp);
   SPB_LAUNCH_CHECK(ctx);
   lowrank_final_kernel<<<(B + 127) / 128, 128, 0, stream>>>(B, M, nt, nch, ly.sqpart, ly.qn, ly.logdet, info,
                                                             lnlike, quad, logdet);
   SPB_LAUNCH_CHECK(ctx);
+  return 0;
+}
+
+extern "C" size_t spb_lowrank_posterior_workspace_bytes(const spb_context *ctx, int B, int nt) {
+  return spb_lowrank_lnlike_workspace_bytes(ctx, B, 1, nt);
+}
+
+extern "C" int spb_lowrank_posterior(spb_context *ctx, int B, int nt, const double *Binc, long long Binc_stride,
+                                     const double *mean_ylm, const double *cov_ylm, const double *Q,
+                                     const double *R, const double *phi_aux, const spb_noise_model *noise,
+                                     const double *flux, const double *baseline_mean, long long bm_stride,
+                                     double *a, double *P, double *G, double *gp_mean, int32_t *info,
+                                     void *workspace, size_t workspace_bytes, void *stream_) {
+  SPB_REQUIRE(ctx != nullptr && B > 0 && nt >= SPB_NEIG && noise != nullptr, "lowrank_posterior: bad arguments");
+  SPB_REQUIRE(Binc && mean_ylm && cov_ylm && Q && R && phi_aux && flux && a && P && G && gp_mean && info,
+              "lowrank_posterior: missing operand");
+  SPB_REQUIRE(Binc_stride == 0 || Binc_stride == (long long)LR * 256,
+              "lowrank_posterior: Binc_stride must be 0 (shared) or 32 * 256");
+  SPB_REQUIRE(!noise->normalized, "lowrank_posterior: the predictive distribution of a normalised process is "
+                                  "not defined");
+  SPB_REQUIRE(noise->data_cov != nullptr && (noise->data_kind == 0 || noise->data_kind == 1) &&
+                  noise->data_stride == 0,
+              "lowrank_posterior: data_cov must be one scalar or one (nt) vector shared by the batch");
+  SPB_REQUIRE(noise->baseline_var == nullptr || noise->base_kind == 0,
+              "lowrank_posterior: baseline_var must be a scalar (or one per element)");
+  SPB_REQUIRE(noise->temporal_kind == 0, "lowrank_posterior: temporal kernels are not low-rank");
+  SPB_REQUIRE(workspace != nullptr && workspace_bytes >= spb_lowrank_posterior_workspace_bytes(ctx, B, nt),
+              "lowrank_posterior: workspace too small");
+  SPB_REQUIRE(((uintptr_t)Binc % 16) == 0 && ((uintptr_t)cov_ylm % 16) == 0,
+              "lowrank_posterior: Binc and cov_ylm must be 16-byte aligned");
+  SPB_REQUIRE((long long)B <= 65535LL * SOLVE_EB, "lowrank_posterior: batch too large for one launch");
+  cudaStream_t stream = (cudaStream_t)stream_;
+  SPB_CHECK_CUDA(cudaSetDevice(ctx->device));
+  void *ws = reinterpret_cast<void *>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255);
+  const LnlikeLayout ly = lnlike_layout(ws, B, 1, nt);
+  SolveParams sp;
+  int st = lowrank_front(ctx, B, nt, Binc, Binc_stride, mean_ylm, cov_ylm, Q, R, phi_aux, noise, 1, flux, nt, 0,
+                         baseline_mean, bm_stride, nullptr, info, ly, sp, stream);
+  if (st) return st;
+  PostParams pp;
+  pp.Binc = Binc;
+  pp.Binc_stride = Binc_stride;
+  pp.mean_ylm = mean_ylm;
+  pp.C = ly.C;
+  pp.R = R;
+  pp.aux = phi_aux;
+  pp.bvar = noise->baseline_var;
+  pp.bv_stride = noise->base_stride;
+  pp.L = ly.L;
+  pp.w = ly.w;
+  pp.a = a;
+  pp.P = P;
+  pp.G = G;
+  pp.gp_mean = gp_mean;
+  pp.info = info;
+  lowrank_post_kernel<<<B, 256, 0, stream>>>(pp);
+  SPB_LAUNCH_CHECK(ctx);
+  return 0;
+}
+
+extern "C" size_t spb_lowrank_predict_eval_workspace_bytes(const spb_context *ctx, int B, int nts, int nsamples,
+                                                           int full_cov) {
+  (void)ctx;
+  if (B < 1) B = 1;
+  if (nts < 1) nts = 1;
+  if (nsamples < 0) nsamples = 0;
+  return eval_layout(nullptr, B, nts, nsamples, full_cov).bytes + 256;
+}
+
+extern "C" int spb_lowrank_predict_eval(spb_context *ctx, int B, int nts, const double *t_sample, double period,
+                                        const double *a, const double *P, const double *G,
+                                        const double *gp_mean, int nsamples, const double *unit_normals,
+                                        long long un_stride, double eps, double *mean, double *var,
+                                        double *cov, int ldc, double *draws, void *workspace,
+                                        size_t workspace_bytes, void *stream_) {
+  SPB_REQUIRE(ctx != nullptr && B > 0 && nts > 0 && nsamples >= 0, "lowrank_predict_eval: bad arguments");
+  SPB_REQUIRE(t_sample && a && P && gp_mean && mean, "lowrank_predict_eval: missing operand");
+  SPB_REQUIRE(period > 0.0, "lowrank_predict_eval: period must be positive");
+  SPB_REQUIRE(nsamples == 0 || (G && unit_normals && draws && eps >= 0.0 &&
+                                (un_stride == 0 || un_stride == (long long)nsamples * (LR + nts))),
+              "lowrank_predict_eval: draws need G, unit normals (nsamples, 32 + nts) shared (un_stride 0) or "
+              "per element (un_stride nsamples * (32 + nts)) and eps >= 0");
+  SPB_REQUIRE(cov == nullptr || (ldc >= nts && ((uintptr_t)P % 16) == 0),
+              "lowrank_predict_eval: cov needs ldc >= nts and a 16-byte aligned P");
+  SPB_REQUIRE((long long)B <= 65535LL * EVAL_EB && (long long)nsamples <= 65535LL * EVAL_SB,
+              "lowrank_predict_eval: batch or draw count too large for one launch");
+  SPB_REQUIRE(workspace != nullptr &&
+                  workspace_bytes >= spb_lowrank_predict_eval_workspace_bytes(ctx, B, nts, nsamples, cov != nullptr),
+              "lowrank_predict_eval: workspace too small");
+  cudaStream_t stream = (cudaStream_t)stream_;
+  SPB_CHECK_CUDA(cudaSetDevice(ctx->device));
+  void *ws = reinterpret_cast<void *>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255);
+  const EvalLayout ly = eval_layout(ws, B, nts, nsamples, cov != nullptr);
+  if (nsamples > 0) {
+    const long long pairs = (long long)B * nsamples;
+    lowrank_gz_kernel<<<(unsigned)((pairs + 7) / 8), 256, 0, stream>>>(B, nsamples, nts, G, unit_normals, un_stride,
+                                                                       ly.gz);
+    SPB_LAUNCH_CHECK(ctx);
+  }
+  EvalParams ep;
+  ep.B = B;
+  ep.nts = nts;
+  ep.S = nsamples;
+  ep.ts = t_sample;
+  ep.period = period;
+  ep.a = a;
+  ep.P = P;
+  ep.gp_mean = gp_mean;
+  ep.gz = ly.gz;
+  ep.z = unit_normals;
+  ep.z_stride = un_stride;
+  ep.sq_eps = sqrt(eps);
+  ep.mean = mean;
+  ep.var = var;
+  ep.draws = draws;
+  dim3 grid((nts + 255) / 256, (B + EVAL_EB - 1) / EVAL_EB, nsamples > 0 ? (nsamples + EVAL_SB - 1) / EVAL_SB : 1);
+  lowrank_eval_kernel<<<grid, 256, 0, stream>>>(ep);
+  SPB_LAUNCH_CHECK(ctx);
+  if (cov) {   // Phi_s P Phi_s^T: T = Phi_s P (P symmetric), cov = T Phi_s^T
+    lowrank_phi_kernel<<<(nts + 255) / 256, 256, 0, stream>>>(nts, t_sample, period, ly.Phi);
+    SPB_LAUNCH_CHECK(ctx);
+    for (int b0 = 0; b0 < B; b0 += 65535) {
+      const int Bc = (B - b0 < 65535) ? B - b0 : 65535;
+      gnt::Desc d1 = {};
+      d1.A = ly.Phi;
+      d1.strideA = 0;
+      d1.lda = LR;
+      d1.Bm = P + (size_t)b0 * LR * LR;
+      d1.strideB = (long long)LR * LR;
+      d1.ldb = LR;
+      d1.C = ly.T;
+      d1.strideC = (long long)nts * LR;
+      d1.ldc = LR;
+      d1.M = nts;
+      d1.N = LR;
+      d1.K = LR;
+      d1.batch = Bc;
+      d1.ksplit = 1;
+      d1.alpha = 1.0;
+      int st = gnt::launch<gnt::EPI_STORE>(ctx, d1, stream);
+      if (st) return st;
+      gnt::Desc d2 = {};
+      d2.A = ly.T;
+      d2.strideA = (long long)nts * LR;
+      d2.lda = LR;
+      d2.Bm = ly.Phi;
+      d2.strideB = 0;
+      d2.ldb = LR;
+      d2.C = cov + (size_t)b0 * nts * ldc;
+      d2.strideC = (long long)nts * ldc;
+      d2.ldc = ldc;
+      d2.M = nts;
+      d2.N = nts;
+      d2.K = LR;
+      d2.batch = Bc;
+      d2.ksplit = 1;
+      d2.alpha = 1.0;
+      st = gnt::launch<gnt::EPI_STORE>(ctx, d2, stream);
+      if (st) return st;
+    }
+  }
   return 0;
 }

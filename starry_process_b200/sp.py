@@ -892,27 +892,10 @@ class StarryProcess(object):
     def _log_likelihood_lowrank(self, t, flux, data_cov, i, p, u, baseline_mean, baseline_var,
                                 marginalize_over_inclination):
         """``log_likelihood(method="lowrank")``: include/spb200.h spb_lowrank_*."""
-        marg = self._marginalize_over_inclination if marginalize_over_inclination is None \
-            else bool(marginalize_over_inclination)
-        if marg:
-            raise ValueError("method='lowrank' needs marginalize_over_inclination=False: the marginalised "
-                             "covariance is the cubic interpolant of flux.py:256-276, which is not low-rank")
-        if self._tkind:
-            raise ValueError("method='lowrank' does not cover time-variable surfaces (tau): the temporal "
-                             "kernel makes the covariance full-rank")
-        dc = data_cov if isinstance(data_cov, torch.Tensor) else np.asarray(data_cov, dtype=np.float64)
-        if dc.ndim > 1:
-            raise ValueError("method='lowrank' needs a scalar or (nt,) data_cov, not a full matrix")
-        if not (isinstance(dc, torch.Tensor) and dc.is_cuda):
-            if not np.all(np.asarray(dc.cpu() if isinstance(dc, torch.Tensor) else dc) > 0.0):
-                raise ValueError("method='lowrank' needs a positive data_cov (it whitens with D^-1/2)")
+        self._lowrank_checks("lowrank", t, data_cov, baseline_var, marginalize_over_inclination)
         bv_in = baseline_var
-        if isinstance(bv_in, (torch.Tensor, np.ndarray)) and bv_in.ndim > 1:
-            raise ValueError("method='lowrank' needs a scalar or (B,) baseline_var, not a full matrix")
-        nt = torch.as_tensor(t).numel() if isinstance(t, torch.Tensor) else np.asarray(t).size
-        if nt < 31:
-            raise ValueError("method='lowrank' needs nt >= 31 time stamps (the rank of the phase basis)")
         _, t, inc, rta1 = self._prep(t, i, p, u, False)
+        nt = t.numel()
         dev, B = self.device, self._B
         f = torch.as_tensor(flux, dtype=torch.float64).to(dev)
         if f.ndim == 1:
@@ -937,22 +920,7 @@ class StarryProcess(object):
         lnlike = torch.empty(B, dtype=torch.float64, device=dev)
         z = torch.zeros(B, dtype=torch.float64, device=dev)
         with torch.cuda.device(dev):
-            ev = self._mark("lowrank_inclination")
-            Binc = torch.empty(I, 32, 256, dtype=torch.float64, device=dev)
-            nb = lib.spb_lowrank_inclination_workspace_bytes(h, I)
-            ws = torch.empty(nb, dtype=torch.uint8, device=dev)
-            _lib.check(lib.spb_lowrank_inclination(h, I, _ptr(inc), _ptr(rta1), 0, _ptr(Binc), _ptr(ws), nb,
-                                                   _stream()))
-            self._mark_end(ev)
-            ev = self._mark("lowrank_basis")
-            Q = torch.empty(nt, 32, dtype=torch.float64, device=dev)
-            R = torch.empty(32, 32, dtype=torch.float64, device=dev)
-            aux = torch.empty(65, dtype=torch.float64, device=dev)
-            nb = lib.spb_lowrank_basis_workspace_bytes(h, nt)
-            ws = torch.empty(nb, dtype=torch.uint8, device=dev)
-            _lib.check(lib.spb_lowrank_basis(h, nt, _ptr(t), float(p), nm.data_kind, ctypes.c_void_p(nm.data_cov),
-                                             _ptr(Q), _ptr(R), _ptr(aux), _ptr(ws), nb, _stream()))
-            self._mark_end(ev)
+            Binc, Q, R, aux = self._lowrank_basis(t, inc, rta1, p, nm)
             ev = self._mark("lowrank_lnlike")
             nb = lib.spb_lowrank_lnlike_workspace_bytes(h, B, M, nt)
             ws = torch.empty(nb, dtype=torch.uint8, device=dev)
@@ -965,6 +933,56 @@ class StarryProcess(object):
             del ws, keep
         self._z = z
         return self._out(lnlike)
+
+    def _lowrank_checks(self, method, t, data_cov, baseline_var, marginalize_over_inclination):
+        """``method`` of ``log_likelihood`` / ``predict`` / ``sample_conditional``: False for ``"dense"``, True
+        for ``"lowrank"`` once the inputs are found to be covered by the rank-31 form (ValueError otherwise)."""
+        if method not in ("dense", "lowrank"):
+            raise ValueError("unknown method %r: expected 'dense' or 'lowrank'" % (method,))
+        if method == "dense":
+            return False
+        marg = self._marginalize_over_inclination if marginalize_over_inclination is None \
+            else bool(marginalize_over_inclination)
+        if marg:
+            raise ValueError("method='lowrank' needs marginalize_over_inclination=False: the marginalised "
+                             "covariance is the cubic interpolant of flux.py:256-276, which is not low-rank")
+        if self._tkind:
+            raise ValueError("method='lowrank' does not cover time-variable surfaces (tau): the temporal "
+                             "kernel makes the covariance full-rank")
+        dc = data_cov if isinstance(data_cov, torch.Tensor) else np.asarray(data_cov, dtype=np.float64)
+        if dc.ndim > 1:
+            raise ValueError("method='lowrank' needs a scalar or (nt,) data_cov, not a full matrix")
+        if not (isinstance(dc, torch.Tensor) and dc.is_cuda):
+            if not np.all(np.asarray(dc.cpu() if isinstance(dc, torch.Tensor) else dc) > 0.0):
+                raise ValueError("method='lowrank' needs a positive data_cov (it whitens with D^-1/2)")
+        if isinstance(baseline_var, (torch.Tensor, np.ndarray)) and baseline_var.ndim > 1:
+            raise ValueError("method='lowrank' needs a scalar or (B,) baseline_var, not a full matrix")
+        nt = torch.as_tensor(t).numel() if isinstance(t, torch.Tensor) else np.asarray(t).size
+        if nt < 31:
+            raise ValueError("method='lowrank' needs nt >= 31 time stamps (the rank of the phase basis)")
+        return True
+
+    def _lowrank_basis(self, t, inc, rta1, p, nm):
+        """B_inc (I, 32, 256) and the thin QR of the whitened phase basis, Q (nt, 32), R (32, 32), aux (65)."""
+        lib, h, dev = self._lib, self._ctx.handle, self.device
+        I, nt = inc.numel(), t.numel()
+        ev = self._mark("lowrank_inclination")
+        Binc = torch.empty(I, 32, 256, dtype=torch.float64, device=dev)
+        nb = lib.spb_lowrank_inclination_workspace_bytes(h, I)
+        ws = torch.empty(nb, dtype=torch.uint8, device=dev)
+        _lib.check(lib.spb_lowrank_inclination(h, I, _ptr(inc), _ptr(rta1), 0, _ptr(Binc), _ptr(ws), nb,
+                                               _stream()))
+        self._mark_end(ev)
+        ev = self._mark("lowrank_basis")
+        Q = torch.empty(nt, 32, dtype=torch.float64, device=dev)
+        R = torch.empty(32, 32, dtype=torch.float64, device=dev)
+        aux = torch.empty(65, dtype=torch.float64, device=dev)
+        nb = lib.spb_lowrank_basis_workspace_bytes(h, nt)
+        ws = torch.empty(nb, dtype=torch.uint8, device=dev)
+        _lib.check(lib.spb_lowrank_basis(h, nt, _ptr(t), float(p), nm.data_kind, ctypes.c_void_p(nm.data_cov),
+                                         _ptr(Q), _ptr(R), _ptr(aux), _ptr(ws), nb, _stream()))
+        self._mark_end(ev)
+        return Binc, Q, R, aux
 
     # ------------------------------------------------------------------ SURVEY 8(f) rank 4: gradient
     def log_likelihood_and_grad(self, t, flux, data_cov, i=defaults["i"], p=defaults["p"], u=None,
@@ -1175,24 +1193,41 @@ class StarryProcess(object):
 
     def predict(self, t, flux, data_cov, t_sample=None, i=defaults["i"], p=defaults["p"], u=None,
                 baseline_mean=defaults["baseline_mean"], baseline_var=defaults["baseline_var"],
-                marginalize_over_inclination=None):
+                marginalize_over_inclination=None, method="dense", return_cov="full"):
         """sp.py:767-922: mean ``(nts,)`` and covariance ``(nts, nts)`` of the light-curve
         distribution conditioned on ``flux`` (leading ``B`` axis for batched hyperparameters).
+        ``return_cov="diag"`` returns the predictive variance ``(nts,)`` (or ``(B, nts)``) in place of
+        the matrix.
 
         One augmented factorisation does the work: the rows ``[K(ts, t); y - mean]`` are appended
         to ``K(t, t)``, the Cholesky kernel returns ``V = (L^-1 K(t, ts))^T`` and ``w = L^-1 (y -
-        mean)``, and ``mu = mean + V w``, ``K = K(ts, ts) - V V^T`` are two tensor-core GEMMs."""
+        mean)``, and ``mu = mean + V w``, ``K = K(ts, ts) - V V^T`` are two tensor-core GEMMs.
+
+        ``method="lowrank"`` evaluates the same distribution through the rank-31 form of the conditional
+        branch (DESIGN.md section 4.6): time and memory linear in ``nt`` and, with ``return_cov="diag"``,
+        in ``nts``.  It covers what ``log_likelihood(method="lowrank")`` covers and raises ``ValueError``
+        otherwise."""
         if self._normalized:
             raise NotImplementedError("Method not implemented when the flux is normalized.")
+        if return_cov not in ("full", "diag"):
+            raise ValueError("unknown return_cov %r: expected 'full' or 'diag'" % (return_cov,))
+        lowrank = self._lowrank_checks(method, t, data_cov, baseline_var, marginalize_over_inclination)
         nt_ = int(np.size(t)) if not isinstance(t, torch.Tensor) else t.numel()
         ns_ = nt_ if t_sample is None else (
             int(np.size(t_sample)) if not isinstance(t_sample, torch.Tensor) else t_sample.numel())
-        out = self._chunked("predict", max(nt_, ns_), max(nt_, ns_), dict(
-            t=t, flux=flux, data_cov=data_cov, t_sample=t_sample, i=i, p=p, u=u,
-            baseline_mean=baseline_mean, baseline_var=baseline_var,
-            marginalize_over_inclination=marginalize_over_inclination))
-        if out is not None:
-            return out
+        if not (lowrank and return_cov == "diag"):   # the rank-31 route only forms nts^2 for "full"
+            n = ns_ if lowrank else max(nt_, ns_)
+            out = self._chunked("predict", n, n, dict(
+                t=t, flux=flux, data_cov=data_cov, t_sample=t_sample, i=i, p=p, u=u,
+                baseline_mean=baseline_mean, baseline_var=baseline_var,
+                marginalize_over_inclination=marginalize_over_inclination, method=method,
+                return_cov=return_cov))
+            if out is not None:
+                return out
+        if lowrank:
+            mu, cov, _ = self._predictive_lowrank(t, flux, data_cov, t_sample, i, p, u, baseline_mean,
+                                                  baseline_var, return_cov)
+            return self._out(mu), self._out(cov)
         marg, t, inc, rta1 = self._prep(t, i, p, u, marginalize_over_inclination)
         dev, B = self.device, self._B
         nt = t.numel()
@@ -1269,15 +1304,31 @@ class StarryProcess(object):
             mu = torch.where(bad[:, None], torch.full_like(mu, float("nan")), mu)
             Kc = Kss[:, :, :nts]
             Kc = torch.where(bad[:, None, None], torch.full_like(Kc, float("nan")), Kc)
+            if return_cov == "diag":
+                Kc = Kc.diagonal(dim1=1, dim2=2).contiguous()
         return self._out(mu), self._out(Kc)
 
     def sample_conditional(self, t, flux, data_cov, t_sample=None, i=defaults["i"],
                            p=defaults["p"], u=None, baseline_mean=defaults["baseline_mean"],
                            baseline_var=defaults["baseline_var"], nsamples=1, eps=defaults["eps"],
-                           unit_normals=None, generator=None, marginalize_over_inclination=None):
+                           unit_normals=None, generator=None, marginalize_over_inclination=None,
+                           method="dense"):
         """sp.py:924-1002: draws ``(nsamples, nts)`` from the conditional light-curve distribution.
         (The reference body reads an undefined name ``ts``; the intended ``ts = t_sample or t`` is
-        what is implemented.)"""
+        what is implemented.)  ``unit_normals``: ``(nts, nsamples)`` (or ``(B, nts, nsamples)``).
+
+        ``method="lowrank"`` draws ``mean + Phi(ts) G z1 + sqrt(eps) z2`` with ``G G^T`` the predictive
+        covariance in the 32-dimensional phase basis (DESIGN.md section 4.6), in time and memory linear in
+        ``nt`` and ``nts``.  Its ``unit_normals`` have shape ``(32 + nts, nsamples)`` (or ``(B, 32 + nts,
+        nsamples)``): 32 rows ``z1`` for the basis coefficients, then ``nts`` rows ``z2`` for the white
+        ``eps`` term.  The draws have the dense route's distribution but not its values for the same
+        normals: the square root of the covariance is a different one."""
+        if self._normalized and method == "lowrank":   # as predict: checked before the inputs
+            raise NotImplementedError("Method not implemented when the flux is normalized.")
+        if self._lowrank_checks(method, t, data_cov, baseline_var, marginalize_over_inclination):
+            _, _, out = self._predictive_lowrank(t, flux, data_cov, t_sample, i, p, u, baseline_mean,
+                                                 baseline_var, None, nsamples, eps, unit_normals, generator)
+            return self._out(out)
         nt_ = int(np.size(t)) if not isinstance(t, torch.Tensor) else t.numel()
         ns_ = nt_ if t_sample is None else (
             int(np.size(t_sample)) if not isinstance(t_sample, torch.Tensor) else t_sample.numel())
@@ -1285,7 +1336,7 @@ class StarryProcess(object):
             t=t, flux=flux, data_cov=data_cov, t_sample=t_sample, i=i, p=p, u=u,
             baseline_mean=baseline_mean, baseline_var=baseline_var, nsamples=nsamples, eps=eps,
             unit_normals=unit_normals, generator=generator,
-            marginalize_over_inclination=marginalize_over_inclination))
+            marginalize_over_inclination=marginalize_over_inclination, method=method))
         if out is not None:
             return out
         mu, K = self.predict(t, flux, data_cov, t_sample=t_sample, i=i, p=p, u=u,
@@ -1305,6 +1356,72 @@ class StarryProcess(object):
             out = torch.where(((info & 1) != 0)[:, None, None], torch.full_like(out, float("nan")),
                               out)
         return self._out(out)
+
+    def _predictive_lowrank(self, t, flux, data_cov, t_sample, i, p, u, baseline_mean, baseline_var,
+                            return_cov, nsamples=0, eps=0.0, unit_normals=None, generator=None):
+        """``predict`` / ``sample_conditional`` with ``method="lowrank"``: spb_lowrank_posterior, then
+        spb_lowrank_predict_eval.  Returns ``(mean, var | cov | None, draws | None)``, each with a leading
+        batch axis.  Elements whose ``K(t, t)`` is not PD are NaN throughout; elements whose predictive
+        covariance is not PSD beyond rounding have NaN draws only (include/spb200.h)."""
+        _, t, inc, rta1 = self._prep(t, i, p, u, False)
+        dev, B, nt = self.device, self._B, t.numel()
+        ts = t if t_sample is None else self._t(t_sample)
+        nts = ts.numel()
+        f = torch.as_tensor(flux, dtype=torch.float64).to(dev).reshape(-1).contiguous()
+        if f.numel() != nt:
+            raise ValueError("flux must have shape (nt,)")
+        bm = torch.as_tensor(baseline_mean, dtype=torch.float64).to(dev).contiguous()
+        if bm.ndim == 1 and bm.numel() != B:
+            raise ValueError("a 1-D baseline_mean must have one entry per batch element")
+        bvar = None
+        if isinstance(baseline_var, (torch.Tensor, np.ndarray)) or baseline_var != 0.0:
+            bvar = baseline_var
+        keep = []
+        nm = self._noise_model(nt, data_cov, bvar, keep)
+        lib, h = self._lib, self._ctx.handle
+        I = inc.numel()
+        f64 = dict(dtype=torch.float64, device=dev)
+        a = torch.empty(B, 32, **f64)
+        P = torch.empty(B, 32, 32, **f64)
+        G = torch.empty(B, 32, 32, **f64)
+        gp_mean = torch.empty(B, **f64)
+        info = torch.zeros(B, dtype=torch.int32, device=dev)
+        z = None
+        if unit_normals is not None:
+            z = torch.as_tensor(unit_normals, dtype=torch.float64).to(dev)
+            if z.ndim not in (2, 3) or z.shape[-2] != 32 + nts or (z.ndim == 3 and z.shape[0] != B):
+                raise ValueError("unit normals must have shape (%d, nsamples) or (B, %d, nsamples) for "
+                                 "method='lowrank': 32 basis coefficients, then nts white-noise terms"
+                                 % (32 + nts, 32 + nts))
+            nsamples = z.shape[-1]
+            z = z.transpose(-1, -2).contiguous()            # (S, 32 + nts) per draw
+        elif nsamples:
+            z = torch.randn(B, nsamples, 32 + nts, generator=generator, **f64)
+        with torch.cuda.device(dev):
+            Binc, Q, R, aux = self._lowrank_basis(t, inc, rta1, p, nm)
+            ev = self._mark("lowrank_posterior")
+            nb = lib.spb_lowrank_posterior_workspace_bytes(h, B, nt)
+            ws = torch.empty(nb, dtype=torch.uint8, device=dev)
+            _lib.check(lib.spb_lowrank_posterior(
+                h, B, nt, _ptr(Binc), 0 if I == 1 else 32 * 256, _ptr(self._mean_ylm), _ptr(self._cov_ylm),
+                _ptr(Q), _ptr(R), _ptr(aux), ctypes.byref(nm), _ptr(f), _ptr(bm), 1 if bm.ndim == 1 else 0,
+                _ptr(a), _ptr(P), _ptr(G), _ptr(gp_mean), _ptr(info), _ptr(ws), nb, _stream()))
+            self._mark_end(ev)
+            del ws, Q
+            ev = self._mark("lowrank_eval")
+            mean = torch.empty(B, nts, **f64)
+            var = torch.empty(B, nts, **f64) if return_cov == "diag" else None
+            cov = torch.empty(B, nts, nts, **f64) if return_cov == "full" else None
+            draws = torch.empty(B, nsamples, nts, **f64) if nsamples else None
+            nb = lib.spb_lowrank_predict_eval_workspace_bytes(h, B, nts, nsamples, cov is not None)
+            ws = torch.empty(nb, dtype=torch.uint8, device=dev)
+            _lib.check(lib.spb_lowrank_predict_eval(
+                h, B, nts, _ptr(ts), float(p), _ptr(a), _ptr(P), _ptr(G), _ptr(gp_mean), int(nsamples), _ptr(z),
+                0 if z is None or z.ndim == 2 else nsamples * (32 + nts), float(eps), _ptr(mean), _ptr(var),
+                _ptr(cov), nts, _ptr(draws), _ptr(ws), nb, _stream()))
+            self._mark_end(ev)
+            del ws, keep
+        return mean, (var if cov is None else cov), draws
 
     def sample_ylm_conditional(self, t, flux, data_cov, i=defaults["i"], p=defaults["p"], u=None,
                                baseline_mean=defaults["baseline_mean"],

@@ -122,6 +122,22 @@ def _is_batched(x):
         or isinstance(x, (list, tuple))
 
 
+def _nt(t):
+    """Number of time stamps of host or device ``t``."""
+    return t.numel() if isinstance(t, torch.Tensor) else int(np.size(t))
+
+
+def _four_arrays(n1, n2):
+    """Device bytes per element of ``sample``, ``predict`` and the conditional samplers: about four
+    (n1 x n2) arrays, and the moments."""
+    return 4 * n1 * (n2 + (n2 & 1)) * 8 + 4 * 256 * 256 * 8
+
+
+# arguments of a chunk body (StarryProcess._batch) that carry a leading batch axis of B entries when
+# they have this many dimensions
+_BATCH_NDIM = dict(inc=1, f=3, bm=1, bvar=1, unit_normals=3)
+
+
 def gauss2beta(mu, sigma, log_alpha_max=10, log_beta_max=10):
     """latitude.py:14-77 (host utility; accepts floats, arrays or tensors, angles in degrees)."""
     tens = isinstance(mu, torch.Tensor) or isinstance(sigma, torch.Tensor)
@@ -568,20 +584,59 @@ class StarryProcess(object):
         t = self._t(t)
         inc = self._inc(i)
         _check_bounds("p", p, 0, np.inf)
+        return self._design(t, inc, p, self._rTA1(u))
+
+    def _design(self, t, inc, p, rta1):
+        """``A (I, nt, 256)`` of the device time stamps ``t`` at the inclinations ``inc`` [rad]."""
+        lib, h, dev = self._lib, self._ctx.handle, self.device
         I, nt = inc.numel(), t.numel()
-        rta1 = self._rTA1(u)
-        with torch.cuda.device(self.device):
-            per = torch.full((I,), float(p), dtype=torch.float64, device=self.device)
-            A = torch.empty(I, nt, 256, dtype=torch.float64, device=self.device)
-            nbytes = self._lib.spb_design_matrix_workspace_bytes(self._ctx.handle, I, nt)
-            ws = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
-            _lib.check(self._lib.spb_design_matrix(self._ctx.handle, I, nt, _ptr(t), _ptr(inc),
-                                                   _ptr(per), _ptr(rta1), 0, _ptr(A), _ptr(ws),
-                                                   nbytes, _stream()))
+        with torch.cuda.device(dev):
+            per = torch.full((I,), float(p), dtype=torch.float64, device=dev)
+            A = torch.empty(I, nt, 256, dtype=torch.float64, device=dev)
+            nbytes = lib.spb_design_matrix_workspace_bytes(h, I, nt)
+            ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+            _lib.check(lib.spb_design_matrix(h, I, nt, _ptr(t), _ptr(inc), _ptr(per), _ptr(rta1), 0,
+                                             _ptr(A), _ptr(ws), nbytes, _stream()))
         return A
 
     # ------------------------------------------------------------------ flux mean / covariance
-    def _noise_model(self, nt, data_cov, baseline_var, keep, lower_only=False, b0=0):
+    def _curves(self, flux, baseline_mean, baseline_var, nt, M=None):
+        """The light-curve inputs of one call, on the device: ``(f, per_element, M, bm, bvar)`` with
+        ``f`` of shape ``(B, M, nt)`` when ``per_element``, else ``(1, M, nt)``; ``bm`` a scalar or
+        ``(B,)``; ``bvar`` a scalar, ``(B,)`` or ``(nt, nt)``, or None for zero.  ``M=1``: the
+        single light curve ``(nt,)`` of ``predict`` and the conditional samplers."""
+        dev, B = self.device, self._B
+        f = torch.as_tensor(flux, dtype=torch.float64).to(dev)
+        if M == 1:
+            if f.numel() != nt:
+                raise ValueError("flux must have shape (nt,)")
+            f = f.reshape(1, nt)
+        elif f.ndim == 1:
+            f = f[None]
+        per_element = f.ndim == 3
+        if per_element and f.shape[0] != B:
+            raise ValueError("per-element flux must have shape (B, M, nt)")
+        if f.shape[-1] != nt:
+            raise ValueError("flux must have shape (nt,), (M, nt) or (B, M, nt)")
+        f = (f if per_element else f[None]).contiguous()
+        bm = torch.as_tensor(baseline_mean, dtype=torch.float64).to(dev).contiguous()
+        if bm.ndim == 1 and bm.numel() != B:
+            raise ValueError("a 1-D baseline_mean must have one entry per batch element")
+        bvar = None
+        if isinstance(baseline_var, (torch.Tensor, np.ndarray)) or baseline_var != 0.0:
+            bvar = torch.as_tensor(baseline_var, dtype=torch.float64).to(dev).contiguous()
+            # extension: one baseline variance per batch element (the free `v` of
+            # calibrate/log_prob.py:70-74)
+            if bvar.ndim == 1 and bvar.numel() != B:
+                raise ValueError("a 1-D baseline_var must have one entry per batch element")
+            if bvar.ndim > 1 and tuple(bvar.shape) != (nt, nt):
+                raise ValueError("baseline_var must be a scalar or an (nt, nt) matrix")
+        return f, per_element, f.shape[1], bm, bvar
+
+    def _noise_model(self, nt, data_cov, baseline_var, keep, lower_only=False, uniform_dt=0.0):
+        """spb_noise_model of one assembly of ``nt`` time stamps; ``uniform_dt`` is their spacing
+        (``_spacing``; 0 takes the general kernel), ``baseline_var`` as ``_curves`` returns it.
+        ``keep`` collects the device buffers it points to."""
         nm = _lib.NoiseModel()
         nm.lower_only = 1 if lower_only else 0
         nm.defer = 0
@@ -593,8 +648,8 @@ class StarryProcess(object):
         nm.data_stride = 0
         nm.base_stride = 0
         nm.temporal_kind = self._tkind
-        nm.uniform_dt = float(getattr(self, "_udt", 0.0) or 0.0)
-        nm.tau = self._tau[b0:].data_ptr() if self._tkind else None
+        nm.uniform_dt = float(uniform_dt)
+        nm.tau = self._tau.data_ptr() if self._tkind else None
         nm.tau_stride = 1 if self._tkind else 0
         if data_cov is not None:
             d = torch.as_tensor(data_cov, dtype=torch.float64).to(self.device).contiguous()
@@ -615,122 +670,149 @@ class StarryProcess(object):
             if bv.ndim == 0:
                 nm.base_kind, bv = 0, bv.reshape(1)
             elif bv.ndim == 1:
-                # extension: one baseline variance per batch element (the free `v` of
-                # calibrate/log_prob.py:70-74)
-                if bv.numel() != self._B:
-                    raise ValueError("a 1-D baseline_var must have one entry per batch element")
                 nm.base_kind, nm.base_stride = 0, 1
-                bv = bv[b0:].contiguous()
             else:
-                if tuple(bv.shape) != (nt, nt):
-                    raise ValueError("baseline_var must be a scalar or an (nt, nt) matrix")
                 nm.base_kind = 2
             keep.append(bv)
             nm.baseline_var = bv.data_ptr()
         return nm
 
-    def _flux_cov_chunk(self, b0, b1, t, inc, p, rta1, marg, data_cov, baseline_var, ldk,
-                        lower_only=False, defer=False):
-        """GP mean (scalar per element) and the (noise-augmented) covariance for elements b0:b1.
-        Returns (gp_mean, K, z), or with ``defer`` (marginal branch, scalar / per-point noise terms)
-        (gp_mean, K_raw, z, affine, keepalive): the covariance is left raw and the normalisation +
-        noise are applied inside the Cholesky kernel (``spb_cholesky_lnlike_affine``)."""
+    def _flux_cov(self, t, inc, p, rta1, marg, udt, data_cov, baseline_var, ldk, lower_only=False,
+                  defer=False):
+        """GP mean (scalar per element) and the (noise-augmented) covariance of every batch element.
+        Returns ``(gp_mean, K, z, coef, affine)``: ``coef`` is the marginal kernel table ``(B, 4,
+        covpts + 1)`` (None in the conditional branch).  With ``defer`` (marginal branch, scalar /
+        per-point noise terms) the covariance is left raw and ``affine`` is the ``spb_cholesky_lnlike_affine``
+        argument that applies the normalisation + noise inside the Cholesky kernel; else it is None."""
         lib, h = self._lib, self._ctx.handle
-        Bc, nt = b1 - b0, t.numel()
+        B, nt = self._B, t.numel()
         dev = self.device
         keep = []
-        nm = self._noise_model(nt, data_cov, baseline_var, keep, lower_only and marg, b0=b0)
+        nm = self._noise_model(nt, data_cov, baseline_var, keep, lower_only and marg, udt)
         defer_req = bool(defer)
         defer = bool(defer and marg and lower_only and nm.data_kind != 2 and nm.base_kind != 2)
         nm.defer = 1 if defer else 0
-        mean_ylm = self._mean_ylm[b0:b1]
-        cov_ylm = self._cov_ylm[b0:b1]
-        info = self._info[b0:b1]
-        gp_mean = torch.empty(Bc, dtype=torch.float64, device=dev)
-        K = torch.empty(Bc, nt, ldk, dtype=torch.float64, device=dev)
-        z = torch.zeros(Bc, dtype=torch.float64, device=dev)
-        nb_as = lib.spb_assemble_workspace_bytes(h, Bc, nt)
+        gp_mean = torch.empty(B, dtype=torch.float64, device=dev)
+        K = torch.empty(B, nt, ldk, dtype=torch.float64, device=dev)
+        z = torch.zeros(B, dtype=torch.float64, device=dev)
+        nb_as = lib.spb_assemble_workspace_bytes(h, B, nt)
         ws_as = torch.empty(nb_as, dtype=torch.uint8, device=dev)
+        coef = None
         if marg:
             nc = self._covpts + 1
-            var = torch.empty(Bc, dtype=torch.float64, device=dev)
-            coef = torch.empty(Bc, 4, nc, dtype=torch.float64, device=dev)
-            nb = lib.spb_flux_marginal_workspace_bytes(h, Bc)
+            var = torch.empty(B, dtype=torch.float64, device=dev)
+            coef = torch.empty(B, 4, nc, dtype=torch.float64, device=dev)
+            nb = lib.spb_flux_marginal_workspace_bytes(h, B)
             ws = torch.empty(nb, dtype=torch.uint8, device=dev)
             ev = self._mark("flux_marginal")
-            _lib.check(lib.spb_flux_marginal(h, Bc, _ptr(mean_ylm), _ptr(cov_ylm), _ptr(rta1),
+            _lib.check(lib.spb_flux_marginal(h, B, _ptr(self._mean_ylm), _ptr(self._cov_ylm), _ptr(rta1),
                                              self._covpts, _ptr(gp_mean), _ptr(var), _ptr(coef),
                                              _ptr(ws), nb, _stream()))
             self._mark_end(ev)
-            self._last_coef = coef   # (Bc, 4, covpts + 1): predict's cross-covariance re-uses it
             ev = self._mark("assemble")
-            _lib.check(lib.spb_assemble_marginal(h, Bc, nt, _ptr(t), float(p), self._covpts,
+            _lib.check(lib.spb_assemble_marginal(h, B, nt, _ptr(t), float(p), self._covpts,
                                                  _ptr(coef), _ptr(var), _ptr(gp_mean),
-                                                 ctypes.byref(nm), _ptr(K), ldk, _ptr(z), _ptr(info),
-                                                 _ptr(ws_as), nb_as, _stream()))
+                                                 ctypes.byref(nm), _ptr(K), ldk, _ptr(z),
+                                                 _ptr(self._info), _ptr(ws_as), nb_as, _stream()))
             self._mark_end(ev)
         else:
-            inc_c = inc if inc.numel() == 1 else inc[b0:b1].contiguous()
-            Ic = inc_c.numel()
-            per = torch.full((Ic,), float(p), dtype=torch.float64, device=dev)
-            A = torch.empty(Ic, nt, 256, dtype=torch.float64, device=dev)
-            nbd = lib.spb_design_matrix_workspace_bytes(h, Ic, nt)
-            wsd = torch.empty(nbd, dtype=torch.uint8, device=dev)
-            _lib.check(lib.spb_design_matrix(h, Ic, nt, _ptr(t), _ptr(inc_c), _ptr(per), _ptr(rta1),
-                                             0, _ptr(A), _ptr(wsd), nbd, _stream()))
-            nb = lib.spb_flux_conditional_workspace_bytes(h, Bc, nt)
+            A = self._design(t, inc, p, rta1)
+            nb = lib.spb_flux_conditional_workspace_bytes(h, B, nt)
             ws = torch.empty(nb, dtype=torch.uint8, device=dev)
             # log-likelihood path of an unnormalised, static process: only the lower triangle is needed and
             # the noise terms are added inside the Cholesky kernel's loads (no read-modify-write pass)
             defer_c = bool(defer_req and lower_only and not self._normalized and not self._tkind
                            and nm.data_kind != 2 and nm.base_kind != 2)
             fc = lib.spb_flux_conditional_lower if defer_c else lib.spb_flux_conditional
-            _lib.check(fc(h, Bc, nt, _ptr(A), 0 if Ic == 1 else nt * 256, _ptr(mean_ylm), _ptr(cov_ylm),
-                          _ptr(gp_mean), _ptr(K), ldk, _ptr(ws), nb, _stream()))
+            _lib.check(fc(h, B, nt, _ptr(A), 0 if A.shape[0] == 1 else nt * 256, _ptr(self._mean_ylm),
+                          _ptr(self._cov_ylm), _ptr(gp_mean), _ptr(K), ldk, _ptr(ws), nb, _stream()))
             if defer_c:
                 defer = True
             elif self._tkind:   # sp.py:697-698
-                _lib.check(lib.spb_temporal_scale(h, Bc, nt, nt, _ptr(t), _ptr(t), self._tkind,
-                                                  _ptr(self._tau[b0:b1].contiguous()), 1, None, 0,
-                                                  _ptr(K), ldk, nt * ldk, _stream()))
+                _lib.check(lib.spb_temporal_scale(h, B, nt, nt, _ptr(t), _ptr(t), self._tkind,
+                                                  _ptr(self._tau), 1, None, 0, _ptr(K), ldk, nt * ldk,
+                                                  _stream()))
             if not defer_c:
-                _lib.check(lib.spb_assemble_conditional(h, Bc, nt, _ptr(gp_mean), ctypes.byref(nm),
-                                                        _ptr(K), ldk, _ptr(z), _ptr(info), _ptr(ws_as),
-                                                        nb_as, _stream()))
+                _lib.check(lib.spb_assemble_conditional(h, B, nt, _ptr(gp_mean), ctypes.byref(nm),
+                                                        _ptr(K), ldk, _ptr(z), _ptr(self._info),
+                                                        _ptr(ws_as), nb_as, _stream()))
+        affine = None
         if defer:
-            af = _lib.Affine()
+            affine = _lib.Affine()
             if self._normalized:
                 qp, sp_ = ctypes.c_void_p(), ctypes.c_void_p()
-                lib.spb_assemble_workspace_layout(Bc, nt, _ptr(ws_as), ctypes.byref(qp),
+                lib.spb_assemble_workspace_layout(B, nt, _ptr(ws_as), ctypes.byref(qp),
                                                   ctypes.byref(sp_))
-                af.q, af.scal = qp, sp_
-            af.diag = nm.data_cov
-            af.diag_kind = nm.data_kind
-            af.diag_stride = 0
-            af.offset = nm.baseline_var
-            af.offset_stride = nm.base_stride
-            return gp_mean, K, z, af, (keep, ws_as)
-        return gp_mean, K, z
+                affine.q, affine.scal = qp, sp_
+            affine.diag = nm.data_cov
+            affine.diag_kind = nm.data_kind
+            affine.diag_stride = 0
+            affine.offset = nm.baseline_var
+            affine.offset_stride = nm.base_stride
+            affine.keep = (keep, ws_as)   # the device buffers it points into
+        return gp_mean, K, z, coef, affine
 
-    def _chunks(self, nt, ldk):
-        # as few chunks as the memory bound allows (96 GB of covariance matrices by default: the
-        # B200 has 180 GB), of equal size: the Cholesky kernel claims matrices dynamically, so one
-        # long launch has a shorter tail than several short ones
+    # ---- batch chunking: every batched method runs its body on views of batch chunks
+    def _cov_bytes(self, nt, ldk):
+        """Device bytes per element of ``log_likelihood`` / ``mean`` / ``cov``: K, the moments and
+        the digit planes of the INT8 path, which live next to K."""
         per = nt * ldk * 8 + 4 * 256 * 256 * 8
-        if self._ctx.i8_planes(nt, self._B):   # digit planes of the INT8 path live next to K
-            code = self._ctx.i8_planes(nt, self._B)   # 7 | 8 | 77 | 78 | 87: the first digit is the plane count
+        code = self._ctx.i8_planes(nt, self._B)   # 7 | 8 | 77 | 78 | 87: the first digit is the plane count
+        if code:
             per += (code // 10 if code > 10 else code) * (nt + 64) * (nt + 64)
-        # (the assembly / GEMM kernels carry the batch in grid.y: at most 65535 elements a launch)
+        return per
+
+    def _chunks(self, per):
+        """Batch chunks ``(b0, b1)`` at ``per`` device bytes per element: as few as the memory bound
+        allows (96 GB by default: the B200 has 180 GB), and at most 65535 elements each (the assembly
+        and GEMM kernels carry the batch in grid.y), of equal size: the Cholesky kernel claims
+        matrices dynamically, so one long launch has a shorter tail than several short ones."""
         step = max(1, min(self._B, self._max_chunk_bytes // per, 65535))
         nchunks = -(-self._B // step)
         step = -(-self._B // nchunks)
         return [(b0, min(self._B, b0 + step)) for b0 in range(0, self._B, step)]
 
+    def _sub(self, b0, b1):
+        """A view of batch elements b0:b1 as a process of its own (moments already computed)."""
+        sub = object.__new__(type(self))
+        sub.__dict__.update(self.__dict__)
+        sub._B, sub._batched = b1 - b0, True
+        for k in ("_r", "_a", "_b", "_c", "_n", "_tau", "_dr", "_mean_ylm", "_cov_ylm", "_info"):
+            v = getattr(self, k, None)
+            setattr(sub, k, None if v is None else v[b0:b1])
+        sub._cho_cov_ylm = None if self._cho_cov_ylm is None else self._cho_cov_ylm[b0:b1]
+        if getattr(self, "_mu_sigma", None) is not None:
+            sub._mu_sigma = (self._mu_sigma[0][b0:b1], self._mu_sigma[1][b0:b1])
+        return sub
+
+    def _batch(self, per, run, **elem):
+        """``run(gp, **elem)`` over the chunks of the batch (``_chunks(per)``), ``gp`` the view of a
+        chunk (the process itself when one chunk holds the batch).  ``elem`` are the per-element
+        arguments, sliced to the chunk when they carry a batch axis.  Returns the outputs of the
+        chunks concatenated along the batch axis."""
+        bounds = self._chunks(per)
+        if len(bounds) == 1:
+            return run(self, **elem)
+        outs = []
+        for b0, b1 in bounds:
+            kw = {k: v[b0:b1] if getattr(v, "ndim", None) == _BATCH_NDIM[k] and v.shape[0] == self._B
+                  else v for k, v in elem.items()}
+            outs.append(run(self._sub(b0, b1), **kw))
+        if isinstance(outs[0], tuple):
+            return tuple(torch.cat(o) for o in zip(*outs))
+        return torch.cat(outs)
+
+    def _spacing(self, t):
+        """``spb_noise_model.uniform_dt`` of the time stamps ``t`` (0 with ``SPB200_NO_UNIFORM_T`` set),
+        also left in ``_udt`` as a record of the last call, as ``_z`` is."""
+        udt = 0.0 if os.environ.get("SPB200_NO_UNIFORM_T") is not None else self._uniform_dt(t)
+        self._udt = udt
+        return udt
+
     def _prep(self, t, i, p, u, marginalize_over_inclination):
         marg = self._marginalize_over_inclination if marginalize_over_inclination is None \
             else bool(marginalize_over_inclination)
         self._compute_moments()
-        self._udt = self._uniform_dt(t) if os.environ.get("SPB200_NO_UNIFORM_T") is None else 0.0
         t = self._t(t)
         inc = self._inc(i)
         if inc.numel() not in (1, self._B):
@@ -741,34 +823,33 @@ class StarryProcess(object):
 
     def mean(self, t, i=defaults["i"], p=defaults["p"], u=None, marginalize_over_inclination=None):
         """sp.py:643-672."""
+        udt = self._spacing(t)
         marg, t, inc, rta1 = self._prep(t, i, p, u, marginalize_over_inclination)
         nt = t.numel()
         if self._normalized:
             out = torch.zeros(self._B, nt, dtype=torch.float64, device=self.device)
             return self._out(out)
+        ldk = nt + (nt & 1)
         with torch.cuda.device(self.device):
-            gm = []
-            for b0, b1 in self._chunks(nt, nt + (nt & 1)):
-                g, _, _ = self._flux_cov_chunk(b0, b1, t, inc, p, rta1, marg, None, None,
-                                               nt + (nt & 1))
-                gm.append(g)
-            g = torch.cat(gm)
+            g = self._batch(self._cov_bytes(nt, ldk),
+                            lambda gp, inc: gp._flux_cov(t, inc, p, rta1, marg, udt, None, None, ldk)[0],
+                            inc=inc)
         return self._out(g[:, None].expand(self._B, nt).contiguous())
 
     def cov(self, t, i=defaults["i"], p=defaults["p"], u=None, marginalize_over_inclination=None):
         """sp.py:674-703: the (normalised, if requested) GP flux covariance, ``(nt, nt)`` or
         ``(B, nt, nt)``."""
+        udt = self._spacing(t)
         marg, t, inc, rta1 = self._prep(t, i, p, u, marginalize_over_inclination)
         nt = t.numel()
         ldk = nt + (nt & 1)
-        outs, zs = [], []
+
+        def run(gp, inc):
+            _, K, z, _, _ = gp._flux_cov(t, inc, p, rta1, marg, udt, None, None, ldk)
+            return K[:, :, :nt], z
+
         with torch.cuda.device(self.device):
-            for b0, b1 in self._chunks(nt, ldk):
-                _, K, z = self._flux_cov_chunk(b0, b1, t, inc, p, rta1, marg, None, None, ldk)
-                outs.append(K[:, :, :nt])
-                zs.append(z)
-        self._z = torch.cat(zs)
-        K = torch.cat(outs) if len(outs) > 1 else outs[0]
+            K, self._z = self._batch(self._cov_bytes(nt, ldk), run, inc=inc)
         return self._out(K)
 
     # ------------------------------------------------------------------ log likelihood
@@ -788,38 +869,19 @@ class StarryProcess(object):
         1e5-1e6 points fit.  It covers the static process conditional on inclination with a scalar or
         ``(nt,)`` positive ``data_cov`` and a scalar or ``(B,)`` ``baseline_var``, and raises
         ``ValueError`` otherwise."""
-        if method not in ("dense", "lowrank"):
-            raise ValueError("unknown method %r: expected 'dense' or 'lowrank'" % (method,))
+        lowrank = self._lowrank_checks(method, t, data_cov, baseline_var, marginalize_over_inclination)
         if return_grad:
             return self.log_likelihood_and_grad(
                 t, flux, data_cov, i=i, p=p, u=u, baseline_mean=baseline_mean,
                 baseline_var=baseline_var, marginalize_over_inclination=marginalize_over_inclination,
                 method=method)
-        if method == "lowrank":
-            return self._log_likelihood_lowrank(t, flux, data_cov, i, p, u, baseline_mean, baseline_var,
-                                                marginalize_over_inclination)
+        if lowrank:
+            return self._log_likelihood_lowrank(t, flux, data_cov, i, p, u, baseline_mean, baseline_var)
+        udt = self._spacing(t)
         marg, t, inc, rta1 = self._prep(t, i, p, u, marginalize_over_inclination)
         nt = t.numel()
         ldk = nt + (nt & 1)
-        dev = self.device
-        f = torch.as_tensor(flux, dtype=torch.float64).to(dev)
-        if f.ndim == 1:
-            f = f[None]
-        per_element = f.ndim == 3
-        if per_element and f.shape[0] != self._B:
-            raise ValueError("per-element flux must have shape (B, M, nt)")
-        if f.shape[-1] != nt:
-            raise ValueError("flux must have shape (nt,), (M, nt) or (B, M, nt)")
-        M = f.shape[-2]
-        bm = torch.as_tensor(baseline_mean, dtype=torch.float64).to(dev)
-        if bm.ndim == 1 and bm.numel() != self._B:
-            raise ValueError("a 1-D baseline_mean must have one entry per batch element")
-        bvar = None
-        if isinstance(baseline_var, (torch.Tensor, np.ndarray)) or baseline_var != 0.0:
-            bvar = baseline_var
-        lnlike = torch.empty(self._B, dtype=torch.float64, device=dev)
-        zs = []
-        lib, h = self._lib, self._ctx.handle
+        f, _, _, bm, bvar = self._curves(flux, baseline_mean, baseline_var, nt)
         # white-noise floor of K (a lower bound of its smallest eigenvalue): scales the right-hand-side
         # digit planes of the INT8 path when the noise was already added by the assembly kernels
         lam_min, noise_free = 0.0, False
@@ -827,94 +889,83 @@ class StarryProcess(object):
                 isinstance(data_cov, (torch.Tensor, np.ndarray)) and data_cov.ndim == 0):
             lam_min = float(data_cov)
             noise_free = not (lam_min > 0.0)   # no white-noise floor: nothing bounds the solved rows
-        with torch.cuda.device(dev):
-            for b0, b1 in self._chunks(nt, ldk):
-                Bc = b1 - b0
-                out = self._flux_cov_chunk(b0, b1, t, inc, p, rta1, marg, data_cov, bvar, ldk,
-                                           lower_only=True, defer=True)
-                gp_mean, K, z = out[:3]
-                affine = out[3] if len(out) > 3 else None
-                zs.append(z)
-                # r = flux - (gp_mean + baseline_mean)  (sp.py:1157-1161); normalised: mean == 0
-                resid = torch.zeros(Bc, M, ldk, dtype=torch.float64, device=dev)
-                fc = f[b0:b1] if per_element else f[None]
-                bmc = bm[b0:b1, None, None] if bm.ndim == 1 else bm   # (B,) baseline means
-                if self._normalized:
-                    resid[:, :, :nt] = fc - bmc
-                else:
-                    resid[:, :, :nt] = fc - (gp_mean[:, None, None] + bmc)
-                ev = self._mark("cholesky")
-                if Bc == 1 and M >= 64:
-                    # one factorisation + many right-hand sides (ensemble of light curves sharing
-                    # K): factor on one CTA, then spread the RHS rows over the whole GPU
-                    logdet = torch.empty(1, dtype=torch.float64, device=dev)
-                    quad = torch.empty(M, dtype=torch.float64, device=dev)
-                    if affine is not None:
-                        _lib.check(lib.spb_cholesky_lnlike_affine(
-                            h, 1, nt, _ptr(K), ldk, nt * ldk, ctypes.byref(affine), 0, None, ldk, 0,
-                            None, None, _ptr(logdet), _ptr(self._info[b0:b1]), _stream()))
-                    else:
-                        _lib.check(lib.spb_cholesky_lnlike(
-                            h, 1, nt, _ptr(K), ldk, nt * ldk, 0, None, ldk, 0, None, None,
-                            _ptr(logdet), _ptr(self._info[b0:b1]), _stream()))
-                    _lib.check(lib.spb_cholesky_solve_rows(h, nt, _ptr(K), ldk, M, _ptr(resid), ldk,
-                                                           _ptr(quad), _stream()))
-                    ll = -0.5 * quad.sum() - M * logdet[0] - 0.5 * nt * M * math.log(2 * math.pi)
-                    flagged = (self._info[b0:b1] != 0) | torch.isnan(ll)
-                    lnlike[b0:b1] = torch.where(flagged, torch.full_like(ll, -float("inf")), ll)
-                elif self._ctx.i8_planes(nt, Bc) and nt > 64 and not noise_free and (
-                        (affine is not None and affine.diag) or lam_min > 0.0):
-                    # factorisation on the INT8 tensor cores (K is only read; potrf_i8.cuh)
-                    planes = self._ctx.i8_planes(nt, Bc)
-                    nb_i8 = lib.spb_cholesky_i8_workspace_bytes(Bc, nt, M, planes)
-                    ws_i8 = torch.empty(nb_i8, dtype=torch.uint8, device=dev)
-                    _lib.check(lib.spb_cholesky_lnlike_i8(
-                        h, Bc, nt, _ptr(K), ldk, nt * ldk,
-                        ctypes.byref(affine) if affine is not None else None, M, _ptr(resid), ldk,
-                        M * ldk, _ptr(lnlike[b0:b1]), None, None, _ptr(self._info[b0:b1]), planes,
-                        0.0 if affine is not None and affine.diag else lam_min, _ptr(ws_i8), nb_i8,
-                        _stream()))
-                    del ws_i8
-                elif affine is not None:
-                    _lib.check(lib.spb_cholesky_lnlike_affine(
-                        h, Bc, nt, _ptr(K), ldk, nt * ldk, ctypes.byref(affine), M, _ptr(resid), ldk,
-                        M * ldk, _ptr(lnlike[b0:b1]), None, None, _ptr(self._info[b0:b1]),
-                        _stream()))
-                else:
-                    _lib.check(lib.spb_cholesky_lnlike(
-                        h, Bc, nt, _ptr(K), ldk, nt * ldk, M, _ptr(resid), ldk, M * ldk,
-                        _ptr(lnlike[b0:b1]), None, None, _ptr(self._info[b0:b1]), _stream()))
-                self._mark_end(ev)
-                del K, resid, out
-        self._z = torch.cat(zs)
+        with torch.cuda.device(self.device):
+            lnlike, self._z = self._batch(
+                self._cov_bytes(nt, ldk),
+                lambda gp, inc, f, bm, bvar: gp._log_likelihood_dense(
+                    t, inc, p, rta1, marg, udt, f, bm, data_cov, bvar, lam_min, noise_free),
+                inc=inc, f=f, bm=bm, bvar=bvar)
         return self._out(lnlike)
 
-    def _log_likelihood_lowrank(self, t, flux, data_cov, i, p, u, baseline_mean, baseline_var,
-                                marginalize_over_inclination):
+    def _log_likelihood_dense(self, t, inc, p, rta1, marg, udt, f, bm, data_cov, bvar, lam_min,
+                              noise_free):
+        """``(lnlike, z)`` of every batch element: assembly, then one of the Cholesky kernels."""
+        dev, Bc = self.device, self._B
+        nt, M = t.numel(), f.shape[1]
+        ldk = nt + (nt & 1)
+        lib, h = self._lib, self._ctx.handle
+        gp_mean, K, z, _, affine = self._flux_cov(t, inc, p, rta1, marg, udt, data_cov, bvar, ldk,
+                                                  lower_only=True, defer=True)
+        lnlike = torch.empty(Bc, dtype=torch.float64, device=dev)
+        # r = flux - (gp_mean + baseline_mean)  (sp.py:1157-1161); normalised: mean == 0
+        resid = torch.zeros(Bc, M, ldk, dtype=torch.float64, device=dev)
+        bmc = bm[:, None, None] if bm.ndim == 1 else bm   # (B,) baseline means
+        if self._normalized:
+            resid[:, :, :nt] = f - bmc
+        else:
+            resid[:, :, :nt] = f - (gp_mean[:, None, None] + bmc)
+        ev = self._mark("cholesky")
+        if Bc == 1 and M >= 64:
+            # one factorisation + many right-hand sides (ensemble of light curves sharing
+            # K): factor on one CTA, then spread the RHS rows over the whole GPU
+            logdet = torch.empty(1, dtype=torch.float64, device=dev)
+            quad = torch.empty(M, dtype=torch.float64, device=dev)
+            if affine is not None:
+                _lib.check(lib.spb_cholesky_lnlike_affine(
+                    h, 1, nt, _ptr(K), ldk, nt * ldk, ctypes.byref(affine), 0, None, ldk, 0,
+                    None, None, _ptr(logdet), _ptr(self._info), _stream()))
+            else:
+                _lib.check(lib.spb_cholesky_lnlike(
+                    h, 1, nt, _ptr(K), ldk, nt * ldk, 0, None, ldk, 0, None, None,
+                    _ptr(logdet), _ptr(self._info), _stream()))
+            _lib.check(lib.spb_cholesky_solve_rows(h, nt, _ptr(K), ldk, M, _ptr(resid), ldk,
+                                                   _ptr(quad), _stream()))
+            ll = -0.5 * quad.sum() - M * logdet[0] - 0.5 * nt * M * math.log(2 * math.pi)
+            flagged = (self._info != 0) | torch.isnan(ll)
+            lnlike[:] = torch.where(flagged, torch.full_like(ll, -float("inf")), ll)
+        elif self._ctx.i8_planes(nt, Bc) and nt > 64 and not noise_free and (
+                (affine is not None and affine.diag) or lam_min > 0.0):
+            # factorisation on the INT8 tensor cores (K is only read; potrf_i8.cuh)
+            planes = self._ctx.i8_planes(nt, Bc)
+            nb_i8 = lib.spb_cholesky_i8_workspace_bytes(Bc, nt, M, planes)
+            ws_i8 = torch.empty(nb_i8, dtype=torch.uint8, device=dev)
+            _lib.check(lib.spb_cholesky_lnlike_i8(
+                h, Bc, nt, _ptr(K), ldk, nt * ldk,
+                ctypes.byref(affine) if affine is not None else None, M, _ptr(resid), ldk,
+                M * ldk, _ptr(lnlike), None, None, _ptr(self._info), planes,
+                0.0 if affine is not None and affine.diag else lam_min, _ptr(ws_i8), nb_i8,
+                _stream()))
+            del ws_i8
+        elif affine is not None:
+            _lib.check(lib.spb_cholesky_lnlike_affine(
+                h, Bc, nt, _ptr(K), ldk, nt * ldk, ctypes.byref(affine), M, _ptr(resid), ldk,
+                M * ldk, _ptr(lnlike), None, None, _ptr(self._info), _stream()))
+        else:
+            _lib.check(lib.spb_cholesky_lnlike(
+                h, Bc, nt, _ptr(K), ldk, nt * ldk, M, _ptr(resid), ldk, M * ldk,
+                _ptr(lnlike), None, None, _ptr(self._info), _stream()))
+        self._mark_end(ev)
+        return lnlike, z
+
+    def _log_likelihood_lowrank(self, t, flux, data_cov, i, p, u, baseline_mean, baseline_var):
         """``log_likelihood(method="lowrank")``: include/spb200.h spb_lowrank_*."""
-        self._lowrank_checks("lowrank", t, data_cov, baseline_var, marginalize_over_inclination)
-        bv_in = baseline_var
+        udt = self._spacing(t)
         _, t, inc, rta1 = self._prep(t, i, p, u, False)
         nt = t.numel()
         dev, B = self.device, self._B
-        f = torch.as_tensor(flux, dtype=torch.float64).to(dev)
-        if f.ndim == 1:
-            f = f[None]
-        per_element = f.ndim == 3
-        if per_element and f.shape[0] != B:
-            raise ValueError("per-element flux must have shape (B, M, nt)")
-        if f.shape[-1] != nt:
-            raise ValueError("flux must have shape (nt,), (M, nt) or (B, M, nt)")
-        f = f.contiguous()
-        M = f.shape[-2]
-        bm = torch.as_tensor(baseline_mean, dtype=torch.float64).to(dev).contiguous()
-        if bm.ndim == 1 and bm.numel() != B:
-            raise ValueError("a 1-D baseline_mean must have one entry per batch element")
-        bvar = None
-        if isinstance(bv_in, (torch.Tensor, np.ndarray)) or bv_in != 0.0:
-            bvar = bv_in
+        f, per_element, M, bm, bvar = self._curves(flux, baseline_mean, baseline_var, nt)
         keep = []
-        nm = self._noise_model(nt, data_cov, bvar, keep)
+        nm = self._noise_model(nt, data_cov, bvar, keep, uniform_dt=udt)
         lib, h = self._lib, self._ctx.handle
         I = inc.numel()
         lnlike = torch.empty(B, dtype=torch.float64, device=dev)
@@ -957,8 +1008,7 @@ class StarryProcess(object):
                 raise ValueError("method='lowrank' needs a positive data_cov (it whitens with D^-1/2)")
         if isinstance(baseline_var, (torch.Tensor, np.ndarray)) and baseline_var.ndim > 1:
             raise ValueError("method='lowrank' needs a scalar or (B,) baseline_var, not a full matrix")
-        nt = torch.as_tensor(t).numel() if isinstance(t, torch.Tensor) else np.asarray(t).size
-        if nt < 31:
+        if _nt(t) < 31:
             raise ValueError("method='lowrank' needs nt >= 31 time stamps (the rank of the phase basis)")
         return True
 
@@ -1026,12 +1076,10 @@ class StarryProcess(object):
             self._mark_end(ev)
             del ws
             # an 11 B-wide process over the displaced moments; everything else is shared
-            big = object.__new__(StarryProcess)
-            big.__dict__.update(self.__dict__)
-            big._B, big._batched = 11 * B, True
+            big = self._sub(0, B)
+            big._B = 11 * B
             big._mean_ylm, big._cov_ylm, big._cho_cov_ylm = mean, cov, None
             big._info = info.repeat(11).contiguous()
-            big._rTA1_cache = self._rTA1_cache
 
             def tile(x, per_dim):
                 """Per-element arguments (leading dimension B) are repeated for the 11 variants."""
@@ -1121,74 +1169,32 @@ class StarryProcess(object):
                    alpha=1.0, beta=1.0)
         return out
 
-    # ---- batch chunking of the methods that materialise several (nt x nt) arrays per element
-    def _sub(self, b0, b1):
-        """A view of batch elements b0:b1 as a process of its own (moments already computed)."""
-        sub = object.__new__(type(self))
-        sub.__dict__.update(self.__dict__)
-        sub._B, sub._batched = b1 - b0, True
-        for k in ("_r", "_a", "_b", "_c", "_n", "_tau", "_dr", "_mean_ylm", "_cov_ylm", "_info"):
-            v = getattr(self, k, None)
-            setattr(sub, k, None if v is None else v[b0:b1])
-        sub._cho_cov_ylm = None if self._cho_cov_ylm is None else self._cho_cov_ylm[b0:b1]
-        if getattr(self, "_mu_sigma", None) is not None:
-            sub._mu_sigma = (self._mu_sigma[0][b0:b1], self._mu_sigma[1][b0:b1])
-        return sub
-
-    def _chunked(self, method, n1, n2, kwargs,
-                 per_element=("i", "unit_normals", "baseline_mean", "baseline_var")):
-        """Runs ``method`` over batch chunks when the whole batch would not fit ``max_chunk_bytes``
-        (about four (n1 x n2) arrays per element) or one launch (65535 elements: the assembly and
-        GEMM kernels carry the batch in grid.y).  Returns None when no chunking is needed."""
-        per = 4 * n1 * (n2 + (n2 & 1)) * 8 + 4 * 256 * 256 * 8
-        step = max(1, min(self._B, self._max_chunk_bytes // per, 65535))
-        if step >= self._B:
-            return None
-        self._compute_moments()
-        outs = []
-        for b0 in range(0, self._B, step):
-            b1 = min(self._B, b0 + step)
-            kw = dict(kwargs)
-            for k in per_element:
-                v = kw.get(k, None)
-                if isinstance(v, (torch.Tensor, np.ndarray)) and v.ndim >= 1 and v.shape[0] == self._B \
-                        and v.ndim == (3 if k == "unit_normals" else 1):
-                    kw[k] = v[b0:b1]
-            outs.append(getattr(self._sub(b0, b1), method)(**kw))
-        if isinstance(outs[0], tuple):
-            return tuple(torch.cat([o[k] for o in outs]) for k in range(len(outs[0])))
-        return torch.cat(outs)
-
     def sample(self, t, i=defaults["i"], p=defaults["p"], u=None, nsamples=1, eps=defaults["eps"],
                unit_normals=None, generator=None, marginalize_over_inclination=None):
         """sp.py:729-765: draws from the prior over light curves, ``(nsamples, nt)`` (or
         ``(B, nsamples, nt)``).  ``unit_normals`` optionally supplies the reference's
         ``random_normal(self.random, (nt, nsamples))``."""
-        nt_ = int(np.size(t)) if not isinstance(t, torch.Tensor) else t.numel()
-        out = self._chunked("sample", nt_, nt_, dict(
-            t=t, i=i, p=p, u=u, nsamples=nsamples, eps=eps, unit_normals=unit_normals,
-            generator=generator, marginalize_over_inclination=marginalize_over_inclination))
-        if out is not None:
-            return out
+        udt = self._spacing(t)
         marg, t, inc, rta1 = self._prep(t, i, p, u, marginalize_over_inclination)
         nt = t.numel()
         ldk = nt + (nt & 1)
-        B = self._B
-        with torch.cuda.device(self.device):
+
+        def run(gp, inc, unit_normals):
             # eps I is the scalar "data covariance" of the assembly (added after the normalisation,
             # as sp.py:762 adds it to the output of cov())
-            gp_mean, K, _ = self._flux_cov_chunk(0, B, t, inc, p, rta1, marg, float(eps), None, ldk)
-            info = self._factor_rows(K, nt, ldk)
-            _lib.check(self._lib.spb_tril(self._ctx.handle, B, nt, _ptr(K), ldk, nt * ldk,
-                                          _stream()))
+            gp_mean, K, _, _, _ = gp._flux_cov(t, inc, p, rta1, marg, udt, float(eps), None, ldk)
+            info = gp._factor_rows(K, nt, ldk)
+            _lib.check(gp._lib.spb_tril(gp._ctx.handle, gp._B, nt, _ptr(K), ldk, nt * ldk, _stream()))
             if nt & 1:
                 K[:, :, nt:] = 0.0
-            mu = torch.zeros(B, nt, dtype=torch.float64, device=self.device)
-            if not self._normalized:
+            mu = torch.zeros(gp._B, nt, dtype=torch.float64, device=gp.device)
+            if not gp._normalized:
                 mu += gp_mean[:, None]
-            out = self._draw(mu, K, nt, ldk, nsamples, unit_normals, generator)
-            out = torch.where(((info & 1) != 0)[:, None, None], torch.full_like(out, float("nan")),
-                              out)
+            out = gp._draw(mu, K, nt, ldk, nsamples, unit_normals, generator)
+            return torch.where(((info & 1) != 0)[:, None, None], torch.full_like(out, float("nan")), out)
+
+        with torch.cuda.device(self.device):
+            out = self._batch(_four_arrays(nt, nt), run, inc=inc, unit_normals=unit_normals)
         return self._out(out)
 
     def predict(self, t, flux, data_cov, t_sample=None, i=defaults["i"], p=defaults["p"], u=None,
@@ -1197,7 +1203,7 @@ class StarryProcess(object):
         """sp.py:767-922: mean ``(nts,)`` and covariance ``(nts, nts)`` of the light-curve
         distribution conditioned on ``flux`` (leading ``B`` axis for batched hyperparameters).
         ``return_cov="diag"`` returns the predictive variance ``(nts,)`` (or ``(B, nts)``) in place of
-        the matrix.
+        the matrix.  Extension: a ``(B,)`` ``baseline_mean`` gives every batch element its own.
 
         One augmented factorisation does the work: the rows ``[K(ts, t); y - mean]`` are appended
         to ``K(t, t)``, the Cholesky kernel returns ``V = (L^-1 K(t, ts))^T`` and ``w = L^-1 (y -
@@ -1212,101 +1218,97 @@ class StarryProcess(object):
         if return_cov not in ("full", "diag"):
             raise ValueError("unknown return_cov %r: expected 'full' or 'diag'" % (return_cov,))
         lowrank = self._lowrank_checks(method, t, data_cov, baseline_var, marginalize_over_inclination)
-        nt_ = int(np.size(t)) if not isinstance(t, torch.Tensor) else t.numel()
-        ns_ = nt_ if t_sample is None else (
-            int(np.size(t_sample)) if not isinstance(t_sample, torch.Tensor) else t_sample.numel())
-        if not (lowrank and return_cov == "diag"):   # the rank-31 route only forms nts^2 for "full"
-            n = ns_ if lowrank else max(nt_, ns_)
-            out = self._chunked("predict", n, n, dict(
-                t=t, flux=flux, data_cov=data_cov, t_sample=t_sample, i=i, p=p, u=u,
-                baseline_mean=baseline_mean, baseline_var=baseline_var,
-                marginalize_over_inclination=marginalize_over_inclination, method=method,
-                return_cov=return_cov))
-            if out is not None:
-                return out
-        if lowrank:
-            mu, cov, _ = self._predictive_lowrank(t, flux, data_cov, t_sample, i, p, u, baseline_mean,
-                                                  baseline_var, return_cov)
-            return self._out(mu), self._out(cov)
+        marg, t, inc, rta1, udt, ts, udt_s, f, bm, bvar = self._conditional_inputs(
+            t, flux, t_sample, i, p, u, baseline_mean, baseline_var,
+            False if lowrank else marginalize_over_inclination)
+        nt, nts = t.numel(), ts.numel()
+        with torch.cuda.device(self.device):
+            if lowrank:
+                def run(gp, inc, bm, bvar):
+                    return gp._predictive_lowrank(t, ts, inc, p, rta1, udt, f, bm, bvar, data_cov,
+                                                  return_cov)[:2]
+
+                if return_cov == "diag":   # linear in nts as well: one launch sequence for the batch
+                    mu, cov = run(self, inc, bm, bvar)
+                else:
+                    mu, cov = self._batch(_four_arrays(nts, nts), run, inc=inc, bm=bm, bvar=bvar)
+            else:
+                def run(gp, inc, bm, bvar):
+                    mu, K = gp._predict_dense(t, ts, inc, p, rta1, marg, udt, udt_s, f, bm, bvar, data_cov)
+                    return mu, (K.diagonal(dim1=1, dim2=2).contiguous() if return_cov == "diag" else K)
+
+                n = max(nt, nts)
+                mu, cov = self._batch(_four_arrays(n, n), run, inc=inc, bm=bm, bvar=bvar)
+        return self._out(mu), self._out(cov)
+
+    def _conditional_inputs(self, t, flux, t_sample, i, p, u, baseline_mean, baseline_var,
+                            marginalize_over_inclination):
+        """``_prep`` plus the prediction grid ``ts`` and its spacing, and the one light curve
+        ``f (nt,)`` with its baseline terms (``_curves``) of ``predict`` / ``sample_conditional``."""
+        udt_s = None if t_sample is None else self._spacing(t_sample)
+        udt = self._spacing(t)           # second, so that _udt records the spacing of t
         marg, t, inc, rta1 = self._prep(t, i, p, u, marginalize_over_inclination)
+        ts, udt_s = (t, udt) if t_sample is None else (self._t(t_sample), udt_s)
+        f, _, _, bm, bvar = self._curves(flux, baseline_mean, baseline_var, t.numel(), M=1)
+        return marg, t, inc, rta1, udt, ts, udt_s, f.reshape(-1), bm, bvar
+
+    def _predict_dense(self, t, ts, inc, p, rta1, marg, udt, udt_s, f, bm, bvar, data_cov):
+        """Predictive mean ``(B, nts)`` and covariance ``(B, nts, nts)`` of every batch element (NaN
+        where ``K(t, t)`` is not positive definite)."""
         dev, B = self.device, self._B
-        nt = t.numel()
-        ldk = nt + (nt & 1)
-        ts = t if t_sample is None else self._t(t_sample)
-        nts = ts.numel()
-        lds = nts + (nts & 1)
-        bvar = None
-        if isinstance(baseline_var, (torch.Tensor, np.ndarray)) or baseline_var != 0.0:
-            bvar = torch.as_tensor(baseline_var, dtype=torch.float64).to(dev)
+        nt, nts = t.numel(), ts.numel()
+        ldk, lds = nt + (nt & 1), nts + (nts & 1)
         # scalar (or one value per batch element) vs. a full (nt, nt) matrix of extra covariance
         scalar_bvar = bvar is None or bvar.ndim <= 1
-        f = torch.as_tensor(flux, dtype=torch.float64).to(dev).reshape(-1)
-        if f.numel() != nt:
-            raise ValueError("flux must have shape (nt,)")
-        bm = torch.as_tensor(baseline_mean, dtype=torch.float64).to(dev)
         lib, h = self._lib, self._ctx.handle
-        with torch.cuda.device(dev):
-            # K(ts, ts) + baseline_var first (the marginal kernel table is shared by both calls)
-            _, Kss, _ = self._flux_cov_chunk(0, B, ts, inc, p, rta1, marg, None,
-                                             bvar if (scalar_bvar or nts == nt) else None, lds)
-            gp_mean, Ktt, _ = self._flux_cov_chunk(0, B, t, inc, p, rta1, marg, data_cov, bvar, ldk)
-            # right-hand sides: rows 0..nts-1 = K(ts, t) + baseline_var, row nts = y - mean
-            R = torch.zeros(B, nts + 1, ldk, dtype=torch.float64, device=dev)
-            rstride = (nts + 1) * ldk
+        # K(ts, ts) + baseline_var first (the marginal kernel table is shared by both calls)
+        _, Kss, _, _, _ = self._flux_cov(ts, inc, p, rta1, marg, udt_s, None,
+                                         bvar if (scalar_bvar or nts == nt) else None, lds)
+        gp_mean, Ktt, _, coef, _ = self._flux_cov(t, inc, p, rta1, marg, udt, data_cov, bvar, ldk)
+        # right-hand sides: rows 0..nts-1 = K(ts, t) + baseline_var, row nts = y - mean
+        R = torch.zeros(B, nts + 1, ldk, dtype=torch.float64, device=dev)
+        rstride = (nts + 1) * ldk
+        off = None
+        if bvar is not None and scalar_bvar:
+            off = bvar.reshape(-1).contiguous()
+        off_s = 0 if off is None or off.numel() == 1 else 1
+        late_off = off if self._tkind else None   # K(ts,t) *= k_temporal BEFORE + baseline_var
+        if self._tkind:
             off = None
-            if bvar is not None and scalar_bvar:
-                off = bvar.reshape(-1).contiguous()
-            off_s = 0 if off is None or off.numel() == 1 else 1
-            late_off = off if self._tkind else None   # K(ts,t) *= k_temporal BEFORE + baseline_var
-            if self._tkind:
-                off = None
-            if marg:
-                _lib.check(lib.spb_cross_marginal(
-                    h, B, nts, nt, _ptr(ts), _ptr(t), float(p), self._covpts,
-                    _ptr(self._last_coef), _ptr(off), off_s, _ptr(R), ldk, rstride, _stream()))
-            else:
-                I = inc.numel()
-                per = torch.full((I,), float(p), dtype=torch.float64, device=dev)
-                A2 = []
-                for tt_, n_ in ((ts, nts), (t, nt)):
-                    A_ = torch.empty(I, n_, 256, dtype=torch.float64, device=dev)
-                    nbd = lib.spb_design_matrix_workspace_bytes(h, I, n_)
-                    wsd = torch.empty(nbd, dtype=torch.uint8, device=dev)
-                    _lib.check(lib.spb_design_matrix(h, I, n_, _ptr(tt_), _ptr(inc), _ptr(per),
-                                                     _ptr(rta1), 0, _ptr(A_), _ptr(wsd), nbd,
-                                                     _stream()))
-                    A2.append(A_)
-                A_ts, A_t = A2
-                T = torch.empty(B, nts, 256, dtype=torch.float64, device=dev)
-                # T = A_ts Sigma (Sigma symmetric), K(ts, t) = T A_t^T   (sp.py:903-906)
-                self._gemm(B, nts, 256, 256, A_ts, 256, 0 if I == 1 else nts * 256, self._cov_ylm,
-                           256, 65536, T, 256, nts * 256)
-                if off is not None:
-                    R[:, :nts, :nt] = off.reshape(-1, 1, 1)
-                self._gemm(B, nts, nt, 256, T, 256, nts * 256, A_t, 256, 0 if I == 1 else nt * 256,
-                           R, ldk, rstride, alpha=1.0, beta=1.0)
-            if self._tkind:   # sp.py:893-895
-                _lib.check(lib.spb_temporal_scale(h, B, nts, nt, _ptr(ts), _ptr(t), self._tkind,
-                                                  _ptr(self._tau), 1, _ptr(late_off), off_s,
-                                                  _ptr(R), ldk, rstride, _stream()))
-            if bvar is not None and not scalar_bvar:
-                R[:, :nts, :nt] += bvar
-            R[:, nts, :nt] = (f - bm)[None, :] - gp_mean[:, None]
-            info = self._factor_rows(Ktt, nt, ldk, rows=R)
-            # mu = mean + V w ; K = K(ts, ts) - V V^T
-            mu = gp_mean[:, None].expand(B, nts).contiguous()
-            wrow = R.data_ptr() + nts * ldk * 8
-            self._gemm(B, nts, 1, ldk, R, ldk, rstride, wrow, ldk, rstride, mu, 1, nts,
-                       alpha=1.0, beta=1.0)
-            self._gemm(B, nts, nts, ldk, R, ldk, rstride, R, ldk, rstride, Kss, lds, nts * lds,
-                       alpha=-1.0, beta=1.0)
-            bad = ((info & 1) != 0)
-            mu = torch.where(bad[:, None], torch.full_like(mu, float("nan")), mu)
-            Kc = Kss[:, :, :nts]
-            Kc = torch.where(bad[:, None, None], torch.full_like(Kc, float("nan")), Kc)
-            if return_cov == "diag":
-                Kc = Kc.diagonal(dim1=1, dim2=2).contiguous()
-        return self._out(mu), self._out(Kc)
+        if marg:
+            _lib.check(lib.spb_cross_marginal(
+                h, B, nts, nt, _ptr(ts), _ptr(t), float(p), self._covpts,
+                _ptr(coef), _ptr(off), off_s, _ptr(R), ldk, rstride, _stream()))
+        else:
+            I = inc.numel()
+            A_ts, A_t = self._design(ts, inc, p, rta1), self._design(t, inc, p, rta1)
+            T = torch.empty(B, nts, 256, dtype=torch.float64, device=dev)
+            # T = A_ts Sigma (Sigma symmetric), K(ts, t) = T A_t^T   (sp.py:903-906)
+            self._gemm(B, nts, 256, 256, A_ts, 256, 0 if I == 1 else nts * 256, self._cov_ylm,
+                       256, 65536, T, 256, nts * 256)
+            if off is not None:
+                R[:, :nts, :nt] = off.reshape(-1, 1, 1)
+            self._gemm(B, nts, nt, 256, T, 256, nts * 256, A_t, 256, 0 if I == 1 else nt * 256,
+                       R, ldk, rstride, alpha=1.0, beta=1.0)
+        if self._tkind:   # sp.py:893-895
+            _lib.check(lib.spb_temporal_scale(h, B, nts, nt, _ptr(ts), _ptr(t), self._tkind,
+                                              _ptr(self._tau), 1, _ptr(late_off), off_s,
+                                              _ptr(R), ldk, rstride, _stream()))
+        if bvar is not None and not scalar_bvar:
+            R[:, :nts, :nt] += bvar
+        R[:, nts, :nt] = (f[None, :] - (bm[:, None] if bm.ndim == 1 else bm)) - gp_mean[:, None]
+        info = self._factor_rows(Ktt, nt, ldk, rows=R)
+        # mu = mean + V w ; K = K(ts, ts) - V V^T
+        mu = gp_mean[:, None].expand(B, nts).contiguous()
+        wrow = R.data_ptr() + nts * ldk * 8
+        self._gemm(B, nts, 1, ldk, R, ldk, rstride, wrow, ldk, rstride, mu, 1, nts,
+                   alpha=1.0, beta=1.0)
+        self._gemm(B, nts, nts, ldk, R, ldk, rstride, R, ldk, rstride, Kss, lds, nts * lds,
+                   alpha=-1.0, beta=1.0)
+        bad = ((info & 1) != 0)
+        mu = torch.where(bad[:, None], torch.full_like(mu, float("nan")), mu)
+        Kc = Kss[:, :, :nts]
+        return mu, torch.where(bad[:, None, None], torch.full_like(Kc, float("nan")), Kc)
 
     def sample_conditional(self, t, flux, data_cov, t_sample=None, i=defaults["i"],
                            p=defaults["p"], u=None, baseline_mean=defaults["baseline_mean"],
@@ -1325,59 +1327,44 @@ class StarryProcess(object):
         normals: the square root of the covariance is a different one."""
         if self._normalized and method == "lowrank":   # as predict: checked before the inputs
             raise NotImplementedError("Method not implemented when the flux is normalized.")
-        if self._lowrank_checks(method, t, data_cov, baseline_var, marginalize_over_inclination):
-            _, _, out = self._predictive_lowrank(t, flux, data_cov, t_sample, i, p, u, baseline_mean,
-                                                 baseline_var, None, nsamples, eps, unit_normals, generator)
-            return self._out(out)
-        nt_ = int(np.size(t)) if not isinstance(t, torch.Tensor) else t.numel()
-        ns_ = nt_ if t_sample is None else (
-            int(np.size(t_sample)) if not isinstance(t_sample, torch.Tensor) else t_sample.numel())
-        out = self._chunked("sample_conditional", max(nt_, ns_), max(nt_, ns_), dict(
-            t=t, flux=flux, data_cov=data_cov, t_sample=t_sample, i=i, p=p, u=u,
-            baseline_mean=baseline_mean, baseline_var=baseline_var, nsamples=nsamples, eps=eps,
-            unit_normals=unit_normals, generator=generator,
-            marginalize_over_inclination=marginalize_over_inclination, method=method))
-        if out is not None:
-            return out
-        mu, K = self.predict(t, flux, data_cov, t_sample=t_sample, i=i, p=p, u=u,
-                             baseline_mean=baseline_mean, baseline_var=baseline_var,
-                             marginalize_over_inclination=marginalize_over_inclination)
-        if not self._batched:
-            mu, K = mu[None], K[None]
-        B, nts = mu.shape
+        lowrank = self._lowrank_checks(method, t, data_cov, baseline_var, marginalize_over_inclination)
+        if self._normalized:
+            raise NotImplementedError("Method not implemented when the flux is normalized.")
+        marg, t, inc, rta1, udt, ts, udt_s, f, bm, bvar = self._conditional_inputs(
+            t, flux, t_sample, i, p, u, baseline_mean, baseline_var,
+            False if lowrank else marginalize_over_inclination)
+        nt, nts = t.numel(), ts.numel()
         lds = nts + (nts & 1)
         with torch.cuda.device(self.device):
-            Kp = torch.zeros(B, nts, lds, dtype=torch.float64, device=self.device)
-            Kp[:, :, :nts] = K
-            info = self._factor_rows(Kp, nts, lds, diag_add=eps)
-            _lib.check(self._lib.spb_tril(self._ctx.handle, B, nts, _ptr(Kp), lds, nts * lds,
-                                          _stream()))
-            out = self._draw(mu.contiguous(), Kp, nts, lds, nsamples, unit_normals, generator)
-            out = torch.where(((info & 1) != 0)[:, None, None], torch.full_like(out, float("nan")),
-                              out)
+            if lowrank:
+                _, _, out = self._predictive_lowrank(t, ts, inc, p, rta1, udt, f, bm, bvar, data_cov, None,
+                                                     nsamples, eps, unit_normals, generator)
+                return self._out(out)
+
+            def run(gp, inc, bm, bvar, unit_normals):
+                mu, K = gp._predict_dense(t, ts, inc, p, rta1, marg, udt, udt_s, f, bm, bvar, data_cov)
+                Kp = torch.zeros(gp._B, nts, lds, dtype=torch.float64, device=gp.device)
+                Kp[:, :, :nts] = K
+                info = gp._factor_rows(Kp, nts, lds, diag_add=eps)
+                _lib.check(gp._lib.spb_tril(gp._ctx.handle, gp._B, nts, _ptr(Kp), lds, nts * lds, _stream()))
+                out = gp._draw(mu, Kp, nts, lds, nsamples, unit_normals, generator)
+                return torch.where(((info & 1) != 0)[:, None, None], torch.full_like(out, float("nan")),
+                                   out)
+
+            n = max(nt, nts)
+            out = self._batch(_four_arrays(n, n), run, inc=inc, bm=bm, bvar=bvar,
+                              unit_normals=unit_normals)
         return self._out(out)
 
-    def _predictive_lowrank(self, t, flux, data_cov, t_sample, i, p, u, baseline_mean, baseline_var,
-                            return_cov, nsamples=0, eps=0.0, unit_normals=None, generator=None):
+    def _predictive_lowrank(self, t, ts, inc, p, rta1, udt, f, bm, bvar, data_cov, return_cov, nsamples=0,
+                            eps=0.0, unit_normals=None, generator=None):
         """``predict`` / ``sample_conditional`` with ``method="lowrank"``: spb_lowrank_posterior, then
         spb_lowrank_predict_eval.  Returns ``(mean, var | cov | None, draws | None)``, each with a leading
         batch axis.  Elements whose ``K(t, t)`` is not PD are NaN throughout; elements whose predictive
         covariance is not PSD beyond rounding have NaN draws only (include/spb200.h)."""
-        _, t, inc, rta1 = self._prep(t, i, p, u, False)
-        dev, B, nt = self.device, self._B, t.numel()
-        ts = t if t_sample is None else self._t(t_sample)
-        nts = ts.numel()
-        f = torch.as_tensor(flux, dtype=torch.float64).to(dev).reshape(-1).contiguous()
-        if f.numel() != nt:
-            raise ValueError("flux must have shape (nt,)")
-        bm = torch.as_tensor(baseline_mean, dtype=torch.float64).to(dev).contiguous()
-        if bm.ndim == 1 and bm.numel() != B:
-            raise ValueError("a 1-D baseline_mean must have one entry per batch element")
-        bvar = None
-        if isinstance(baseline_var, (torch.Tensor, np.ndarray)) or baseline_var != 0.0:
-            bvar = baseline_var
+        dev, B, nt, nts = self.device, self._B, t.numel(), ts.numel()
         keep = []
-        nm = self._noise_model(nt, data_cov, bvar, keep)
+        nm = self._noise_model(nt, data_cov, bvar, keep, uniform_dt=udt)
         lib, h = self._lib, self._ctx.handle
         I = inc.numel()
         f64 = dict(dtype=torch.float64, device=dev)
@@ -1397,30 +1384,29 @@ class StarryProcess(object):
             z = z.transpose(-1, -2).contiguous()            # (S, 32 + nts) per draw
         elif nsamples:
             z = torch.randn(B, nsamples, 32 + nts, generator=generator, **f64)
-        with torch.cuda.device(dev):
-            Binc, Q, R, aux = self._lowrank_basis(t, inc, rta1, p, nm)
-            ev = self._mark("lowrank_posterior")
-            nb = lib.spb_lowrank_posterior_workspace_bytes(h, B, nt)
-            ws = torch.empty(nb, dtype=torch.uint8, device=dev)
-            _lib.check(lib.spb_lowrank_posterior(
-                h, B, nt, _ptr(Binc), 0 if I == 1 else 32 * 256, _ptr(self._mean_ylm), _ptr(self._cov_ylm),
-                _ptr(Q), _ptr(R), _ptr(aux), ctypes.byref(nm), _ptr(f), _ptr(bm), 1 if bm.ndim == 1 else 0,
-                _ptr(a), _ptr(P), _ptr(G), _ptr(gp_mean), _ptr(info), _ptr(ws), nb, _stream()))
-            self._mark_end(ev)
-            del ws, Q
-            ev = self._mark("lowrank_eval")
-            mean = torch.empty(B, nts, **f64)
-            var = torch.empty(B, nts, **f64) if return_cov == "diag" else None
-            cov = torch.empty(B, nts, nts, **f64) if return_cov == "full" else None
-            draws = torch.empty(B, nsamples, nts, **f64) if nsamples else None
-            nb = lib.spb_lowrank_predict_eval_workspace_bytes(h, B, nts, nsamples, cov is not None)
-            ws = torch.empty(nb, dtype=torch.uint8, device=dev)
-            _lib.check(lib.spb_lowrank_predict_eval(
-                h, B, nts, _ptr(ts), float(p), _ptr(a), _ptr(P), _ptr(G), _ptr(gp_mean), int(nsamples), _ptr(z),
-                0 if z is None or z.ndim == 2 else nsamples * (32 + nts), float(eps), _ptr(mean), _ptr(var),
-                _ptr(cov), nts, _ptr(draws), _ptr(ws), nb, _stream()))
-            self._mark_end(ev)
-            del ws, keep
+        Binc, Q, R, aux = self._lowrank_basis(t, inc, rta1, p, nm)
+        ev = self._mark("lowrank_posterior")
+        nb = lib.spb_lowrank_posterior_workspace_bytes(h, B, nt)
+        ws = torch.empty(nb, dtype=torch.uint8, device=dev)
+        _lib.check(lib.spb_lowrank_posterior(
+            h, B, nt, _ptr(Binc), 0 if I == 1 else 32 * 256, _ptr(self._mean_ylm), _ptr(self._cov_ylm),
+            _ptr(Q), _ptr(R), _ptr(aux), ctypes.byref(nm), _ptr(f), _ptr(bm), 1 if bm.ndim == 1 else 0,
+            _ptr(a), _ptr(P), _ptr(G), _ptr(gp_mean), _ptr(info), _ptr(ws), nb, _stream()))
+        self._mark_end(ev)
+        del ws, Q
+        ev = self._mark("lowrank_eval")
+        mean = torch.empty(B, nts, **f64)
+        var = torch.empty(B, nts, **f64) if return_cov == "diag" else None
+        cov = torch.empty(B, nts, nts, **f64) if return_cov == "full" else None
+        draws = torch.empty(B, nsamples, nts, **f64) if nsamples else None
+        nb = lib.spb_lowrank_predict_eval_workspace_bytes(h, B, nts, nsamples, cov is not None)
+        ws = torch.empty(nb, dtype=torch.uint8, device=dev)
+        _lib.check(lib.spb_lowrank_predict_eval(
+            h, B, nts, _ptr(ts), float(p), _ptr(a), _ptr(P), _ptr(G), _ptr(gp_mean), int(nsamples), _ptr(z),
+            0 if z is None or z.ndim == 2 else nsamples * (32 + nts), float(eps), _ptr(mean), _ptr(var),
+            _ptr(cov), nts, _ptr(draws), _ptr(ws), nb, _stream()))
+        self._mark_end(ev)
+        del ws, keep
         return mean, (var if cov is None else cov), draws
 
     def sample_ylm_conditional(self, t, flux, data_cov, i=defaults["i"], p=defaults["p"], u=None,
@@ -1428,7 +1414,8 @@ class StarryProcess(object):
                                baseline_var=defaults["baseline_var"], nsamples=1,
                                unit_normals=None, generator=None):
         """sp.py:518-641: draws ``(nsamples, 256)`` of the Ylm coefficients conditioned on the
-        observed flux (the inclination is always used).
+        observed flux (the inclination is always used).  ``baseline_mean`` and ``baseline_var`` are
+        shared by the batch (``baseline_var`` may be an ``(nt, nt)`` matrix).
 
         With ``C = data_cov + baseline_var = L_C L_C^T``, ``G = (L_C^-1 A)^T`` and ``Y = L_y^-T``
         (``cov_ylm = L_y L_y^T``):  ``W = G G^T + Y Y^T``,  ``rhs = G L_C^-1 (f - b) + Y L_y^-1 mu``,
@@ -1440,28 +1427,20 @@ class StarryProcess(object):
             raise NotImplementedError("Method not implemented for time-variable maps.")
         if self._nylm != 256:
             raise NotImplementedError("sample_ylm_conditional is implemented at ydeg = 15")
-        nt_ = int(np.size(t)) if not isinstance(t, torch.Tensor) else t.numel()
-        out = self._chunked("sample_ylm_conditional", nt_, 256, dict(
-            t=t, flux=flux, data_cov=data_cov, i=i, p=p, u=u, baseline_mean=baseline_mean,
-            baseline_var=baseline_var, nsamples=nsamples, unit_normals=unit_normals,
-            generator=generator))
-        if out is not None:
-            return out
-        self._compute_moments()
-        dev, B = self.device, self._B
-        t = self._t(t)
+        _, t, inc, rta1 = self._prep(t, i, p, u, None)
         nt = t.numel()
         ldk = nt + (nt & 1)
-        f = torch.as_tensor(flux, dtype=torch.float64).to(dev).reshape(-1)
-        if f.numel() != nt:
-            raise ValueError("flux must have shape (nt,)")
-        bm = torch.as_tensor(baseline_mean, dtype=torch.float64).to(dev)
-        lib, h = self._lib, self._ctx.handle
-        with torch.cuda.device(dev):
-            A = self._design_full(t, i, p, u)
+        f, _, _, bm, bvar = self._curves(flux, baseline_mean, baseline_var, nt, M=1)
+        if bm.ndim == 1 or (bvar is not None and bvar.ndim == 1):
+            raise ValueError("sample_ylm_conditional factorises one noise covariance and one residual for "
+                             "the whole batch: baseline_mean and baseline_var cannot be per element")
+        f = f.reshape(-1)
+
+        def run(gp, inc, unit_normals):
+            dev, B = gp.device, gp._B
+            lib, h = gp._lib, gp._ctx.handle
+            A = gp._design(t, inc, p, rta1)
             I = A.shape[0]
-            if I not in (1, B):
-                raise ValueError("`i` must be a scalar or have one entry per batch element")
             # C = data_cov (+ baseline_var on every entry): input assembly, sp.py:594-607
             d = torch.as_tensor(data_cov, dtype=torch.float64).to(dev)
             C = torch.zeros(1, nt, ldk, dtype=torch.float64, device=dev)
@@ -1471,8 +1450,9 @@ class StarryProcess(object):
                 C[0, :, :nt].diagonal().copy_(d)
             else:
                 C[0, :, :nt] = d
-            C[0, :, :nt] += torch.as_tensor(baseline_var, dtype=torch.float64).to(dev)
-            infoC = self._factor_rows(C, nt, ldk)
+            if bvar is not None:
+                C[0, :, :nt] += bvar
+            infoC = gp._factor_rows(C, nt, ldk)
             # rows: A^T (256 per inclination) and the residual, all against the one factor of C
             R = torch.zeros(I * 256 + 1, ldk, dtype=torch.float64, device=dev)
             R[: I * 256, :nt] = A.transpose(1, 2).reshape(I * 256, nt)
@@ -1482,33 +1462,36 @@ class StarryProcess(object):
                                                    _ptr(quad), _stream()))
             grow = R.data_ptr() + I * 256 * ldk * 8
             # cov_ylm = L_y L_y^T with rows [I; mu] appended: Y = L_y^-T (as rows), wmu = L_y^-1 mu
-            Ly = self._cov_ylm.clone()
+            Ly = gp._cov_ylm.clone()
             Ry = torch.zeros(B, 257, 256, dtype=torch.float64, device=dev)
             Ry[:, :256, :] = torch.eye(256, dtype=torch.float64, device=dev)
-            Ry[:, 256, :] = self._mean_ylm
-            infoY = self._factor_rows(Ly, 256, 256, rows=Ry)
+            Ry[:, 256, :] = gp._mean_ylm
+            infoY = gp._factor_rows(Ly, 256, 256, rows=Ry)
             sY = 257 * 256
             W = torch.empty(B, 256, 256, dtype=torch.float64, device=dev)
             sG = 0 if I == 1 else 256 * ldk
-            self._gemm(B, 256, 256, ldk, R, ldk, sG, R, ldk, sG, W, 256, 65536)
-            self._gemm(B, 256, 256, 256, Ry, 256, sY, Ry, 256, sY, W, 256, 65536, beta=1.0)
+            gp._gemm(B, 256, 256, ldk, R, ldk, sG, R, ldk, sG, W, 256, 65536)
+            gp._gemm(B, 256, 256, 256, Ry, 256, sY, Ry, 256, sY, W, 256, 65536, beta=1.0)
             # rhs = Y wmu + G g, appended (with the identity) to the factorisation of W
             Rw = torch.zeros(B, 257, 256, dtype=torch.float64, device=dev)
             Rw[:, :256, :] = torch.eye(256, dtype=torch.float64, device=dev)
             rhs = Rw.data_ptr() + 256 * 256 * 8
-            self._gemm(B, 256, 1, 256, Ry, 256, sY, Ry.data_ptr() + 256 * 256 * 8, 256, sY, rhs, 1, sY)
-            self._gemm(B, 256, 1, ldk, R, ldk, sG, grow, ldk, 0, rhs, 1, sY, beta=1.0)
-            infoW = self._factor_rows(W, 256, 256, rows=Rw)
+            gp._gemm(B, 256, 1, 256, Ry, 256, sY, Ry.data_ptr() + 256 * 256 * 8, 256, sY, rhs, 1, sY)
+            gp._gemm(B, 256, 1, ldk, R, ldk, sG, grow, ldk, 0, rhs, 1, sY, beta=1.0)
+            infoW = gp._factor_rows(W, 256, 256, rows=Rw)
             # ycov = Y_W Y_W^T, ymu = Y_W (L_W^-1 rhs)
             ycov = torch.empty(B, 256, 256, dtype=torch.float64, device=dev)
-            self._gemm(B, 256, 256, 256, Rw, 256, sY, Rw, 256, sY, ycov, 256, 65536)
+            gp._gemm(B, 256, 256, 256, Rw, 256, sY, Rw, 256, sY, ycov, 256, 65536)
             ymu = torch.empty(B, 256, dtype=torch.float64, device=dev)
-            self._gemm(B, 256, 1, 256, Rw, 256, sY, rhs, 256, sY, ymu, 1, 256)
-            infoS = self._factor_rows(ycov, 256, 256)
+            gp._gemm(B, 256, 1, 256, Rw, 256, sY, rhs, 256, sY, ymu, 1, 256)
+            infoS = gp._factor_rows(ycov, 256, 256)
             _lib.check(lib.spb_tril(h, B, 256, _ptr(ycov), 256, 65536, _stream()))
-            out = self._draw(ymu, ycov, 256, 256, nsamples, unit_normals, generator)
+            out = gp._draw(ymu, ycov, 256, 256, nsamples, unit_normals, generator)
             bad = (((infoY | infoW | infoS) & 1) != 0) | ((infoC & 1) != 0)
-            out = torch.where(bad[:, None, None], torch.full_like(out, float("nan")), out)
+            return torch.where(bad[:, None, None], torch.full_like(out, float("nan")), out)
+
+        with torch.cuda.device(self.device):
+            out = self._batch(_four_arrays(nt, 256), run, inc=inc, unit_normals=unit_normals)
         return self._out(out)
 
     # ------------------------------------------------------------------ SURVEY 8(f) rank 3

@@ -163,6 +163,47 @@ def test_gpu_predict_batched_and_errors(spb, golden):
         spb.StarryProcess(normalized=True, **FID).sample_ylm_conditional(g["t"], g["flux"], 1e-6)
 
 
+HP3 = dict(r=[10.0, 15.0, 20.0], mu=[30.0, 40.0, 50.0], sigma=[5.0, 8.0, 10.0], c=[0.1, 0.08, 0.05],
+           n=[10.0, 5.0, 3.0])
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("marg", [False, True])
+def test_gpu_predict_per_element_baseline_mean(spb, golden, marg):
+    """A (B,) baseline_mean gives every batch element its own: element b of the batched predict and
+    sample_conditional equals, bit for bit, the same call with the scalar baseline_mean[b]."""
+    import torch
+
+    g = golden("predict_nt200.npz")
+    gp = spb.StarryProcess(normalized=False, marginalize_over_inclination=marg, **HP3)
+    bm = np.array([-2e-4, 0.0, 3e-4])
+    un = np.random.default_rng(0).standard_normal((120, 2))
+    kw = dict(t_sample=g["t_sample"], i=60.0, p=1.0, u=U_LD, baseline_var=1e-5)
+    args = (g["t"], g["flux"], g["data_cov_vec"])
+    mu, K = gp.predict(*args, baseline_mean=bm, **kw)
+    s = gp.sample_conditional(*args, baseline_mean=bm, unit_normals=un, **kw)
+    assert tuple(mu.shape) == (3, 120) and tuple(s.shape) == (3, 2, 120)
+    for b in range(3):
+        mu_b, K_b = gp.predict(*args, baseline_mean=float(bm[b]), **kw)
+        s_b = gp.sample_conditional(*args, baseline_mean=float(bm[b]), unit_normals=un, **kw)
+        assert torch.equal(mu[b], mu_b[b]) and torch.equal(K[b], K_b[b]) and torch.equal(s[b], s_b[b])
+
+
+@pytest.mark.gpu
+def test_gpu_sample_ylm_conditional_rejects_per_element_baseline(spb, golden):
+    """sample_ylm_conditional factorises one noise covariance and one residual for the whole batch:
+    a (B,) baseline_mean or baseline_var raises ValueError before any kernel launch."""
+    g = golden("predict_nt200.npz")
+    gp = spb.StarryProcess(normalized=False, marginalize_over_inclination=False, **HP3)
+    gp.design_matrix(g["t"], **KW)          # moments and flux operator computed ahead
+    gp.mean_ylm
+    n0 = gp._ctx.launches()
+    for bad in (dict(baseline_mean=np.array([0.0, 1e-4, 2e-4])), dict(baseline_var=np.full(3, 1e-5))):
+        with pytest.raises(ValueError, match="whole batch"):
+            gp.sample_ylm_conditional(g["t"], g["flux"], 1e-6, **KW, **bad)
+    assert gp._ctx.launches() == n0
+
+
 @pytest.mark.gpu
 @pytest.mark.parametrize("marg", [False, True])
 def test_gpu_predict_odd_sizes_vs_live_oracle(spb, oracle, golden, marg):

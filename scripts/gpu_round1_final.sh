@@ -8,8 +8,6 @@ timeout 900 python bench.py --impl reference --steps 3 --warmup 1 > gpurun_out/b
 timeout 900 python bench.py > gpurun_out/bench_sweep.json 2> gpurun_out/bench_sweep.err
 timeout 600 python bench.py --workload ensemble > gpurun_out/bench_ensemble.json 2> gpurun_out/bench_ensemble.err
 timeout 900 python scripts/gpu_configs.py > gpurun_out/configs.log 2>&1
-timeout 300 python scripts/gpu_potrf_prof.py > gpurun_out/potrf_prof.log 2>&1
-timeout 300 python scripts/gpu_k1_prof.py > gpurun_out/k1_prof.log 2>&1
 timeout 600 python scripts/gpu_check_potrf.py > gpurun_out/potrf_check.log 2>&1
 timeout 600 ncu --metrics gpu__time_duration.sum --clock-control none -c 400 --csv \
    --log-file gpurun_out/launches_sweep.csv python scripts/prof_driver.py sweep 1184 2 > gpurun_out/ncu_list.log 2>&1

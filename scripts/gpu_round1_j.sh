@@ -1,11 +1,10 @@
 #!/bin/bash
-# potrf iteration pass: tests, LAPACK check, phase timers, default bench
+# potrf iteration pass: tests, LAPACK check, default bench
 mkdir -p gpurun_out
 ( timeout 900 python -m pytest tests -m gpu -x -q ) > gpurun_out/pytest_gpu.log 2>&1
 echo "pytest exit $?" >> gpurun_out/pytest_gpu.log
 tail -3 gpurun_out/pytest_gpu.log
 timeout 600 python scripts/gpu_check_potrf.py > gpurun_out/potrf_check.log 2>&1; tail -25 gpurun_out/potrf_check.log
-timeout 300 python scripts/gpu_potrf_prof.py > gpurun_out/potrf_prof.log 2>&1; cat gpurun_out/potrf_prof.log
 timeout 900 python bench.py > gpurun_out/bench_sweep.json 2> gpurun_out/bench_sweep.err
 python - <<'PY'
 import json

@@ -4,8 +4,7 @@ import ctypes
 import os
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-# SPB200_LIB selects an instrumented debug build of the same library (scripts/gpu_potrf_prof.py)
-LIB_PATH = os.environ.get("SPB200_LIB") or os.path.join(HERE, "libspb200.so")
+LIB_PATH = os.path.join(HERE, "libspb200.so")
 
 _c = ctypes
 _P = _c.c_void_p

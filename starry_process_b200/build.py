@@ -38,30 +38,25 @@ def _digest():
     return h.hexdigest()
 
 
-def build(force=False, verbose=False, defines=(), lib=None):
-    """``defines``/``lib``: instrumented debug variants (e.g. the phase-timer build used by
-    scripts/gpu_potrf_prof.py, loaded through SPB200_LIB); the product library takes neither."""
+def build(force=False, verbose=False):
     nvcc = os.environ.get("NVCC", "nvcc")
-    if lib is not None:
-        return _compile(nvcc, lib, os.path.join(HERE, "build_" + os.path.basename(lib)), verbose,
-                        ["-D" + d for d in defines])
     dig = _digest()
     if (not force and os.path.exists(LIB) and os.path.exists(STAMP)
             and open(STAMP).read().strip() == dig):
         return LIB
-    _compile(nvcc, LIB, os.path.join(HERE, "build"), verbose, [])
+    _compile(nvcc, LIB, os.path.join(HERE, "build"), verbose)
     with open(STAMP, "w") as fh:
         fh.write(dig)
     return LIB
 
 
-def _compile(nvcc, LIB, objdir, verbose, extra):
+def _compile(nvcc, LIB, objdir, verbose):
     os.makedirs(objdir, exist_ok=True)
     objs = []
     procs = []
     for src in _sources():
         obj = os.path.join(objdir, os.path.basename(src)[:-3] + ".o")
-        flags = list(NVCC_FLAGS) + list(extra)
+        flags = list(NVCC_FLAGS)
         if os.path.basename(src) in NO_FMA:
             flags += ["-fmad=false"]
         if verbose:
@@ -85,11 +80,4 @@ def _compile(nvcc, LIB, objdir, verbose, extra):
 
 
 if __name__ == "__main__":
-    if "--prof-nomma" in sys.argv:
-        print(build(defines=["SPB_POTRF_PROF", "SPB_I8_NOMMA"], lib=os.path.join(HERE, "libspb200_prof.so"),
-                    verbose="-v" in sys.argv))
-    elif "--prof" in sys.argv:
-        print(build(defines=["SPB_POTRF_PROF"], lib=os.path.join(HERE, "libspb200_prof.so"),
-                    verbose="-v" in sys.argv))
-    else:
-        print(build(force="--force" in sys.argv, verbose="-v" in sys.argv))
+    print(build(force="--force" in sys.argv, verbose="-v" in sys.argv))

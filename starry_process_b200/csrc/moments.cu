@@ -134,14 +134,6 @@ int k1_upload_perm(int device) {
   return 0;
 }
 
-#ifdef SPB_POTRF_PROF
-__device__ unsigned long long g_k1a_prof[8];
-__device__ unsigned long long g_k1b_prof[8];
-#define K1PROF(k) do { __syncthreads(); if (threadIdx.x == 0) { unsigned long long _n = clock64(); atomicAdd(&g_k1a_prof[k], _n - _pt); _pt = _n; } } while (0)
-#else
-#define K1PROF(k)
-#endif
-
 // ---- sm.Bk (61 raw moments, or one of their derivative lanes) -> sm.tt (term table) -> sm.Y = Q Z
 // -> sm.A = S = Z^T Q Z symmetrised (31 x 31 padded to 32).  Shared by the value kernel (K1a) and the
 // tangent kernel (K1a_tan: the same linear chain applied to dB/dalpha, dB/dbeta).
@@ -316,9 +308,6 @@ __global__ void __launch_bounds__(NT1, 2) moments_k1a(K1Params p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   K1Smem &sm = *reinterpret_cast<K1Smem *>(smem_raw);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-#ifdef SPB_POTRF_PROF
-  unsigned long long _pt = clock64();
-#endif
   const int b = blockIdx.x;
   const double *tab = p.tab;
 
@@ -432,7 +421,6 @@ __global__ void __launch_bounds__(NT1, 2) moments_k1a(K1Params p) {
     if (lane == 0) sm.qs[row] = acc;
   }
 
-  K1PROF(0);
   // ---- Beta moments, latitude.py:197-200 and latitude.h:48-60
   if (tid == 0) {
     const double alpha0 = exp(aa * p.lam);
@@ -448,11 +436,9 @@ __global__ void __launch_bounds__(NT1, 2) moments_k1a(K1Params p) {
   }
   __syncthreads();
 
-  K1PROF(1);
   k1a_S_from_moments(sm, tab, tid, warp, lane);
   int l1, m1;
   lm_of(tid, l1, m1);
-  K1PROF(4);
   // S goes to the eigen-solve kernel
   for (int idx = tid; idx < 32 * 32; idx += NT1) p.Sred[(size_t)b * 1024 + idx] = sm.A[idx >> 5][idx & 31];
   if (tid < 16) p.qs[(size_t)b * 16 + tid] = sm.qs[tid];
@@ -488,7 +474,6 @@ __global__ void __launch_bounds__(NT1, 2) moments_k1a(K1Params p) {
     p.scale[b] = (pi * cc) * (pi * cc) * nn;  // contrast.py:23-25
     p.info[b] = bad ? SPB_INFO_BOUNDS : 0;
   }
-  K1PROF(5);
 }
 
 
@@ -758,12 +743,6 @@ __global__ void __launch_bounds__(32 * K1B_WARPS) moments_k1b(K1Params p) {
     sm.V[a][lane] = (a == lane) ? 1.0 : 0.0;
   }
   __syncwarp();
-#ifdef SPB_POTRF_PROF
-  unsigned long long _pt = clock64(), _acc[4] = {0, 0, 0, 0};
-#define K1BPROF(k) do { unsigned long long _n = clock64(); _acc[k] += _n - _pt; _pt = _n; } while (0)
-#else
-#define K1BPROF(k)
-#endif
   double amax = 0.0;
   for (int a = 0; a < 31; ++a) amax = fmax(amax, fabs(sm.A[a][a]));
   const double rot_tol = 1e-20 * amax;
@@ -772,7 +751,6 @@ __global__ void __launch_bounds__(32 * K1B_WARPS) moments_k1b(K1Params p) {
     if (lane == 0) sm.rotated = 0;
     __syncwarp();
     for (int rnd = 0; rnd < 31; ++rnd) {
-      K1BPROF(3);
       double cth_l = 1.0, sth_l = 0.0;
       if (lane < 16) {
         int pi, qi;
@@ -831,7 +809,6 @@ __global__ void __launch_bounds__(32 * K1B_WARPS) moments_k1b(K1Params p) {
         C[k] = __shfl_sync(0xffffffffu, cth_l, k);
         S[k] = __shfl_sync(0xffffffffu, sth_l, k);
       }
-      K1BPROF(0);
       // The 16 rotations of a round touch disjoint row (column) pairs, so all operands are loaded
       // first and all results stored last: the compiler cannot prove the shared-memory accesses of
       // different rotations independent, and would otherwise serialise load -> FP64 -> store 16x.
@@ -858,7 +835,6 @@ __global__ void __launch_bounds__(32 * K1B_WARPS) moments_k1b(K1Params p) {
         }
       }
       __syncwarp();
-      K1BPROF(1);
       // columns: A <- A J, V <- V J   (lane = row)
       {
         double ap[16], aq[16];
@@ -900,10 +876,6 @@ __global__ void __launch_bounds__(32 * K1B_WARPS) moments_k1b(K1Params p) {
         }
       }
       __syncwarp();
-      K1BPROF(2);
-#ifdef SPB_POTRF_PROF
-      if (lane == 0) atomicAdd(&g_k1b_prof[6], 1ull);
-#endif
     }
     converged = (sm.rotated == 0);
     __syncwarp();
@@ -933,14 +905,6 @@ __global__ void __launch_bounds__(32 * K1B_WARPS) moments_k1b(K1Params p) {
     }
     Sg[a * 32 + lane] = v;
   }
-#ifdef SPB_POTRF_PROF
-  if (lane == 0) {
-    atomicAdd(&g_k1b_prof[0], _acc[0]);
-    atomicAdd(&g_k1b_prof[1], _acc[1]);
-    atomicAdd(&g_k1b_prof[2], _acc[2]);
-    atomicAdd(&g_k1b_prof[3], _acc[3]);
-  }
-#endif
   if (lane == 0) {
     p.rkeep[b] = rk;
     if (!converged) atomicOr(&p.info[b], SPB_INFO_EIG_NOCONV);
@@ -1474,15 +1438,3 @@ extern "C" int spb_ylm_moments_grad(spb_context *ctx, int B, const double *r_deg
                                  stream));
   return 0;
 }
-
-#ifdef SPB_POTRF_PROF
-extern "C" int spb_k1a_prof(unsigned long long *out_host) {
-  if (cudaDeviceSynchronize() != cudaSuccess) return 1;
-  if (cudaMemcpyFromSymbol(out_host, g_k1a_prof, sizeof(unsigned long long) * 8) != cudaSuccess) return 1;
-  if (cudaMemcpyFromSymbol(out_host + 8, g_k1b_prof, sizeof(unsigned long long) * 8) != cudaSuccess) return 1;
-  unsigned long long z[8] = {0};
-  if (cudaMemcpyToSymbol(g_k1a_prof, z, sizeof(z)) != cudaSuccess) return 1;
-  if (cudaMemcpyToSymbol(g_k1b_prof, z, sizeof(z)) != cudaSuccess) return 1;
-  return 0;
-}
-#endif

@@ -142,27 +142,7 @@ struct Smem {
   uint64_t empty[STAGES];  // chunk consumed: 8 arrivals (one per warp)
   int bad;
   int next_item;
-#ifdef SPB_POTRF_PROF
-  unsigned long long prof[2][16];
-#endif
 };
-
-#ifdef SPB_POTRF_PROF
-// Phase timers (debug build only, scripts/gpu_potrf_prof.py): lane 0 of warp 0 (diagonal rows) and of
-// warp 4 (rows below) accumulate clock64 deltas per phase in shared memory.
-__device__ unsigned long long g_potrf_prof[2][16];
-__device__ unsigned long long g_potrf_clk[4];  // CTA 0: clock64 and globaltimer at start / end
-__device__ __forceinline__ unsigned long long gtimer() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  return t;
-}
-#define PROF_DECL unsigned long long _pt = clock64(); const int _pw = (threadIdx.x == 0) ? 0 : ((threadIdx.x == 96) ? 1 : -1)
-#define PROF_MARK(sm, k) do { if (_pw >= 0) { unsigned long long _n = clock64(); (sm).prof[_pw][k] += _n - _pt; _pt = _n; } } while (0)
-#else
-#define PROF_DECL
-#define PROF_MARK(sm, k)
-#endif
 
 static_assert(offsetof(Smem, Dv) == offsetof(Smem, Ld) + sizeof(double) * NB * LS,
               "Ld and Dv must be adjacent (copied as one block by the cluster kernel)");
@@ -195,10 +175,49 @@ struct AffRow {
   bool norm;         // s1, s2, s3 present
 };
 
+// AffRow of matrix `item`; thread 0 stores its scalars s1, s2, s3, offset in sm.af (the identity map
+// when p.aff_on == 0).
+template <class SM>
+__device__ __forceinline__ AffRow aff_setup(const PotrfParams &p, int item, SM &sm, int tid) {
+  AffRow af;
+  af.q = nullptr;
+  af.dg = nullptr;
+  af.dg_vec = 0;
+  af.norm = false;
+  if (p.aff_on) {
+    af.norm = (p.aff.scal != nullptr) && (p.aff.q != nullptr);
+    if (af.norm) af.q = p.aff.q + (size_t)item * p.n;
+    if (p.aff.diag) {
+      af.dg = p.aff.diag + (size_t)item * p.aff.diag_stride;
+      af.dg_vec = (p.aff.diag_kind == 1);
+    }
+  }
+  if (tid == 0) {
+    const double *sc = af.norm ? p.aff.scal + 4 * (size_t)item : nullptr;
+    sm.af[0] = sc ? sc[0] : 1.0;
+    sm.af[1] = sc ? sc[1] : 0.0;
+    sm.af[2] = sc ? sc[2] : 0.0;
+    sm.af[3] = (p.aff_on && p.aff.offset) ? p.aff.offset[(size_t)item * p.aff.offset_stride] : 0.0;
+  }
+  return af;
+}
+
 // K' = s1 K + s2 (1 - q_i)(1 - q_j) - s3 q_i q_j + offset  ==  s1 K + C_i - D_i q_j  with the per-row
 // constants C_i = s2 (1 - q_i) + offset and D_i = s2 (1 - q_i) + s3 q_i: two FMAs per entry on the
 // accumulator-load path (the re-association moves K' by a few 1e-16 of the rank-one terms, which are
 // themselves ~1e-3 of K: far below the 1e-8 lnlike tolerance).
+template <class SM>
+__device__ __forceinline__ void aff_row_consts(const SM &sm, const AffRow &af, int gi, double &Ci, double &Di) {
+  Ci = sm.af[3];
+  Di = 0.0;
+  if (af.norm) {
+    const double qi = af.q[gi];
+    const double a = sm.af[1] * (1.0 - qi);
+    Ci += a;
+    Di = a + sm.af[2] * qi;
+  }
+}
+
 template <class SM>
 __device__ __forceinline__ double aff_apply(const SM &sm, const AffRow &af, double k, double Ci,
                                             double Di, bool diag_row, int gi, int gc) {
@@ -262,15 +281,7 @@ __device__ __forceinline__ void init_acc(const SM &sm, const RM &rm, const AffRo
   const bool cov_row = aff_on && (kind == KIND_DIAG || kind == KIND_BELOW);
   const int gi = c0 + v;  // global row of a covariance row (diagonal-block and below rows alike)
   double Ci = 0.0, Di = 0.0;
-  if (cov_row) {
-    Ci = sm.af[3];
-    if (af.norm) {
-      const double qi = af.q[gi];
-      const double a = sm.af[1] * (1.0 - qi);
-      Ci += a;
-      Di = a + sm.af[2] * qi;
-    }
-  }
+  if (cov_row) aff_row_consts(sm, af, gi, Ci, Di);
   const bool diag_row = (kind == KIND_DIAG);
   if (full) {
     if (p == nullptr) p = rm.Kb;
@@ -342,10 +353,8 @@ __device__ __forceinline__ void gemm_tile(Smem &sm, const RowMap &rm, int v0, in
   const int nchunks = c0 / KC;
   const bool diag_warp = diag_tile && warp < 4;
   const int lim0 = diag_warp ? 2 * warp + 2 : 8;
-  PROF_DECL;
   if (nchunks == 0) {
     init();
-    PROF_MARK(sm, 1);
     return;
   }
   const bool warp_live = diag_warp || (v0 + warp * 16) < nvirt;
@@ -408,13 +417,10 @@ __device__ __forceinline__ void gemm_tile(Smem &sm, const RowMap &rm, int v0, in
 #pragma unroll
   for (int kk = 0; kk < KC / 4; ++kk) koff[kk] = swz(g, kk * 4 + tg);
 
-  PROF_MARK(sm, 9);
 #pragma unroll
   for (int j = 0; j < LA; ++j)
     if (j < nchunks) issue(j, it + j, true);
-  PROF_MARK(sm, 0);
   init();
-  PROF_MARK(sm, 1);
   for (int ch = 0; ch < nchunks; ++ch) {
     const unsigned x = it + ch;
     const unsigned st = x % STAGES;
@@ -424,9 +430,6 @@ __device__ __forceinline__ void gemm_tile(Smem &sm, const RowMap &rm, int v0, in
     bool early = false;
     if (ch + LA < nchunks) early = issue(ch + LA, x + LA, false);
     mbar_wait(&sm.full[st], (x / STAGES) & 1u);  // chunk ch landed, for every thread's copies
-#ifdef SPB_POTRF_PROF
-    if (ch == 0) PROF_MARK(sm, 2);
-#endif
     if (warp_live) {
       const double *Bw = &sm.Bs[st][g][0];
       const double *Aw = &sm.As[st][warp * 16 + g][0];
@@ -465,7 +468,6 @@ __device__ __forceinline__ void gemm_tile(Smem &sm, const RowMap &rm, int v0, in
     if (!early && ch + LA < nchunks) issue(ch + LA, x + LA, true);
   }
   it += nchunks;
-  PROF_MARK(sm, 3);
 }
 
 // Accumulator fragment (8x8, C layout) -> A fragment of its k-block q (columns 4q..4q+3).
@@ -663,10 +665,8 @@ __device__ __forceinline__ void potf2_regs(SM &sm, double (&acc)[2][8][2], int w
   // in columns 0 .. 8 b + 7
   const int rb[2] = {2 * warp, 2 * warp + 1};
   bool bad = false;
-  PROF_DECL;
 #pragma unroll
   for (int s = 0; s < 8; ++s) {
-    PROF_MARK(sm, 14);
     // owner of diagonal tile s: warp s / 2, m-tile s % 2
     if (warp == (s >> 1)) {
       double w0, w1;
@@ -675,7 +675,6 @@ __device__ __forceinline__ void potf2_regs(SM &sm, double (&acc)[2][8][2], int w
       *reinterpret_cast<double2 *>(&sm.Ld.at(8 * s + g, 8 * s + 2 * tg)) = make_double2(t0, t1);
       *reinterpret_cast<double2 *>(&sm.Dv[8 * s + g][2 * tg]) = make_double2(w0, w1);
       if (tg == 0) sm.dpiv[8 * s + g] = dg;
-      PROF_MARK(sm, 11);
     }
     // deferred part of the previous sub-panel's update: columns beyond s.  The A fragments are
     // re-read from the published X (no registers held across the barriers).
@@ -696,7 +695,6 @@ __device__ __forceinline__ void potf2_regs(SM &sm, double (&acc)[2][8][2], int w
       }
     }
     bar_diag();  // L_ss^-1 published
-    PROF_MARK(sm, 12);
     double xa[2][2] = {{0.0, 0.0}, {0.0, 0.0}};  // -X fragments of this sub-panel
     {
       const double d0 = sm.Dv[8 * s + g][tg], d1 = sm.Dv[8 * s + g][4 + tg];
@@ -718,7 +716,6 @@ __device__ __forceinline__ void potf2_regs(SM &sm, double (&acc)[2][8][2], int w
       }
     }
     bar_diag();  // column block s of L_jj published
-    PROF_MARK(sm, 13);
     if (s < 7) {  // critical path: column s + 1 only
 #pragma unroll
       for (int q = 0; q < 2; ++q) {
@@ -731,25 +728,46 @@ __device__ __forceinline__ void potf2_regs(SM &sm, double (&acc)[2][8][2], int w
     }
   }
   if (bad) sm.bad = 1;
-  PROF_MARK(sm, 14);
 }
 
-__device__ __forceinline__ double block_sum(Smem &sm, double v) {
+// the 8 compute warps of the INT8 kernel (named barrier 2: its producer and issuer warps stay out)
+__device__ __forceinline__ void cbar256() { asm volatile("bar.sync 2, 256;\n" ::: "memory"); }
+
+// Sum of v over the 8 warps (256 threads) of a kernel: the whole CTA of the FP64 kernels, the compute
+// warps of the INT8 kernel (I8: they meet at cbar256 instead of __syncthreads).
+template <bool I8, class SM>
+__device__ __forceinline__ double block_sum(SM &sm, double v) {
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   v = warp_sum(v);
-  __syncthreads();
+  if (I8) cbar256(); else __syncthreads();
   if (lane == 0) sm.red[warp] = v;
-  __syncthreads();
+  if (I8) cbar256(); else __syncthreads();
   double t = 0.0;
 #pragma unroll
   for (int w = 0; w < NTHREADS / 32; ++w) t += sm.red[w];
-  __syncthreads();
+  if (I8) cbar256(); else __syncthreads();
   return t;
 }
 
+// lnlike, logdet and info of matrix `item` (MODE_FACTOR; called by one thread).  Flags raised by earlier
+// stages (bounds, normalisation range, eigen-solve) also map to -inf; the `clear` bits belong to this
+// launch and are recomputed: SPB_INFO_NOT_PD from `bad`, plus the bits in `set`.
+__device__ __forceinline__ void lnlike_epilogue(const PotrfParams &p, int item, double quad, double logdet,
+                                                bool bad, int clear, int set) {
+  const int M = p.R ? p.M : 0;
+  double ll = -0.5 * quad - (double)M * logdet - 0.5 * (double)p.n * (double)M * 1.8378770664093453;  // log(2 pi)
+  const int prev = p.info ? (p.info[item] & ~clear) : 0;
+  if (bad || (prev & SPB_INFO_NEG_INF) || ll != ll) ll = -INFINITY;
+  if (p.lnlike) p.lnlike[item] = ll;
+  if (p.logdet) p.logdet[item] = bad ? NAN : logdet;
+  if (p.info) p.info[item] = prev | (bad ? SPB_INFO_NOT_PD : 0) | set;
+}
+
+// dynamic shared memory of the three Cholesky kernels (TMA 128-byte swizzle: 1 KB aligned)
+extern __shared__ __align__(1024) unsigned char smem_raw[];
+
 __global__ void __launch_bounds__(NTHREADS, 2)
     potrf_lnlike_kernel(PotrfParams p, const __grid_constant__ CUtensorMap tmK) {
-  extern __shared__ __align__(1024) unsigned char smem_raw[];   // TMA 128-byte swizzle: 1 KB aligned
   Smem &sm = *reinterpret_cast<Smem *>(smem_raw);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, tg = lane & 3;
 
@@ -764,16 +782,8 @@ __global__ void __launch_bounds__(NTHREADS, 2)
       mbar_init(&sm.empty[s], NTHREADS / 32);
     }
   }
-#ifdef SPB_POTRF_PROF
-  if (tid < 32) sm.prof[tid / 16][tid % 16] = 0;
-  if (tid == 0 && blockIdx.x == 0) {
-    g_potrf_clk[0] = clock64();
-    g_potrf_clk[1] = gtimer();
-  }
-#endif
   __syncthreads();
   unsigned it = 0;  // running k-chunk count of this CTA (ring slot / barrier phase)
-  PROF_DECL;
 
   // Work items (matrices) beyond the first wave are claimed from a global counter: the two CTAs of
   // an SM drift in and out of phase (tensor-pipe phases overlapping or not), so CTA run times for
@@ -807,25 +817,7 @@ __global__ void __launch_bounds__(NTHREADS, 2)
       rm.nrhs = min(p.rows_per_cta, p.M - rm.rb);
       quad_out = p.quad;
     }
-    AffRow af;
-    af.q = nullptr;
-    af.dg = nullptr;
-    af.dg_vec = 0;
-    af.norm = false;
-    if (p.aff_on && p.mode == MODE_FACTOR) {
-      af.norm = (p.aff.scal != nullptr) && (p.aff.q != nullptr);
-      if (af.norm) af.q = p.aff.q + (size_t)item * p.n;
-      if (p.aff.diag) {
-        af.dg = p.aff.diag + (size_t)item * p.aff.diag_stride;
-        af.dg_vec = (p.aff.diag_kind == 1);
-      }
-      if (tid == 0) {
-        sm.af[0] = af.norm ? p.aff.scal[4 * (size_t)item + 0] : 1.0;
-        sm.af[1] = af.norm ? p.aff.scal[4 * (size_t)item + 1] : 0.0;
-        sm.af[2] = af.norm ? p.aff.scal[4 * (size_t)item + 2] : 0.0;
-        sm.af[3] = p.aff.offset ? p.aff.offset[(size_t)item * p.aff.offset_stride] : 0.0;
-      }
-    }
+    const AffRow af = aff_setup(p, item, sm, tid);   // aff_on == 0 in MODE_SOLVE
     if (tid == 0) sm.bad = 0;
     if (quad_out) {
       if (p.mode == MODE_FACTOR) {
@@ -867,14 +859,8 @@ __global__ void __launch_bounds__(NTHREADS, 2)
           for (int mt = 0; mt < 2; ++mt)
             init_acc(sm, rm, af, p.aff_on != 0, v0 + warp * 16 + mt * 8 + g, c0, tg, full_panel, acc[mt]);
         }, p.use_tma ? &tmK : nullptr, item);   // acc = K - L L^T = P
-#ifdef SPB_POTRF_PROF
-        _pt = clock64();
-#endif
         if (diag_tile) {
           if (warp < 4) potf2_regs(sm, acc, warp, lane);
-#ifdef SPB_POTRF_PROF
-          _pt = clock64();
-#endif
           __syncthreads();  // L_jj and the inverses of its diagonal tiles are in shared memory
           if (tid < min(NB, p.n - c0)) logdet_part += 0.5 * log(sm.dpiv[tid]);
           // write L_jj back (lower triangle, valid rows/cols only)
@@ -882,15 +868,12 @@ __global__ void __launch_bounds__(NTHREADS, 2)
             const int i = idx >> 6, j = idx & 63;
             if (j <= i && c0 + i < p.n) rm.Kb[(size_t)(c0 + i) * p.ld + c0 + j] = sm.Ld.at(i, j);
           }
-          PROF_MARK(sm, 4);
         }
         if (!(diag_tile && warp < 4) && (v0 + warp * 16) < nvirt) {
           trsm_warp(sm, acc, lane);
-          PROF_MARK(sm, 5);
 #pragma unroll
           for (int mt = 0; mt < 2; ++mt)
             store_rows(rm, v0 + warp * 16 + mt * 8 + g, c0, tg, acc[mt], quad_part, quad_out);
-          PROF_MARK(sm, 6);
         }
       }
       // this thread's st.global of the panel (store_rows, the L_jj write-back) must be visible to the
@@ -898,39 +881,17 @@ __global__ void __launch_bounds__(NTHREADS, 2)
       fence_proxy_async_global();
       __syncthreads();  // Ld/Dv are rewritten by the next panel; global writes of this panel done
       __threadfence_block();
-      PROF_MARK(sm, 7);
     }
 
     // ---- reductions -> lnlike
-    const double quad = block_sum(sm, quad_part);
-    const double logdet = block_sum(sm, logdet_part);
-    if (p.mode == MODE_FACTOR && tid == 0) {
-      const bool bad = sm.bad != 0;
-      double ll = -0.5 * quad - (double)rm.M * logdet -
-                  0.5 * (double)p.n * (double)rm.M * 1.8378770664093453;  // log(2 pi)
-      // flags raised by earlier stages (bounds, normalisation range, eigen-solve) also map to -inf
-      const int prev = p.info ? (p.info[item] & ~(SPB_INFO_NOT_PD | p.only_flag)) : 0;
-      if (bad || (prev & SPB_INFO_NEG_INF) || ll != ll) ll = -INFINITY;
-      if (p.lnlike) p.lnlike[item] = ll;
-      if (p.logdet) p.logdet[item] = bad ? NAN : logdet;
-      if (p.info) p.info[item] = prev | (bad ? SPB_INFO_NOT_PD : 0);
-    }
+    const double quad = block_sum<false>(sm, quad_part);
+    const double logdet = block_sum<false>(sm, logdet_part);
+    if (p.mode == MODE_FACTOR && tid == 0)
+      lnlike_epilogue(p, item, quad, logdet, sm.bad != 0, SPB_INFO_NOT_PD | p.only_flag, 0);
     if (tid == 0) sm.next_item = (int)gridDim.x + (int)atomicAdd(p.counter, 1u);
     __syncthreads();
     item = sm.next_item;
-    PROF_MARK(sm, 8);
-#ifdef SPB_POTRF_PROF
-    if (_pw >= 0) sm.prof[_pw][10] += 1;
-#endif
   }
-#ifdef SPB_POTRF_PROF
-  __syncthreads();
-  if (tid < 32) atomicAdd(&g_potrf_prof[tid / 16][tid % 16], sm.prof[tid / 16][tid % 16]);
-  if (tid == 0 && blockIdx.x == 0) {
-    g_potrf_clk[2] = clock64();
-    g_potrf_clk[3] = gtimer();
-  }
-#endif
 }
 
 #include "potrf_i8.cuh"
@@ -949,8 +910,6 @@ __global__ void __launch_bounds__(NTHREADS, 2)
 // TRSM.  Same device functions, same operands per tile as the batch kernel: the factor and the
 // solved rows are bit-identical to it (lnlike to rounding: |y|^2 is summed per CTA).
 // ------------------------------------------------------------------------------------------
-constexpr int CLUSTER_MAX = 8;   // portable cluster size; 4 and 2 serve mid-sized batches
-
 __device__ __forceinline__ unsigned cluster_rank() {
   unsigned r;
   asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
@@ -963,7 +922,6 @@ __device__ __forceinline__ void cluster_barrier() {
 
 template <int CLUSTER>
 __global__ void __launch_bounds__(NTHREADS, 1) potrf_cluster_kernel(PotrfParams p) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
   Smem &sm = *reinterpret_cast<Smem *>(smem_raw);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, tg = lane & 3;
   const int rank = (int)cluster_rank();
@@ -990,25 +948,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) potrf_cluster_kernel(PotrfParams 
   rm.rb = 0;
   rm.nrhs = rm.M;
   double *quad_out = p.quad ? p.quad + (size_t)item * p.M : nullptr;
-  AffRow af;
-  af.q = nullptr;
-  af.dg = nullptr;
-  af.dg_vec = 0;
-  af.norm = false;
-  if (p.aff_on) {
-    af.norm = (p.aff.scal != nullptr) && (p.aff.q != nullptr);
-    if (af.norm) af.q = p.aff.q + (size_t)item * p.n;
-    if (p.aff.diag) {
-      af.dg = p.aff.diag + (size_t)item * p.aff.diag_stride;
-      af.dg_vec = (p.aff.diag_kind == 1);
-    }
-    if (tid == 0) {
-      sm.af[0] = af.norm ? p.aff.scal[4 * (size_t)item + 0] : 1.0;
-      sm.af[1] = af.norm ? p.aff.scal[4 * (size_t)item + 1] : 0.0;
-      sm.af[2] = af.norm ? p.aff.scal[4 * (size_t)item + 2] : 0.0;
-      sm.af[3] = p.aff.offset ? p.aff.offset[(size_t)item * p.aff.offset_stride] : 0.0;
-    }
-  }
+  const AffRow af = aff_setup(p, item, sm, tid);
   // per-RHS accumulators are zeroed by CTA 0 before the first "L_jj published" barrier; every
   // contribution is added after it
   if (quad_out && rank == 0)
@@ -1077,8 +1017,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) potrf_cluster_kernel(PotrfParams 
     cluster_barrier();   // panel complete: its columns are visible to every CTA of the cluster
   }
 
-  const double quad = block_sum(sm, quad_part);
-  const double logdet = block_sum(sm, logdet_part);   // non-zero in CTA 0 only
+  const double quad = block_sum<false>(sm, quad_part);
+  const double logdet = block_sum<false>(sm, logdet_part);   // non-zero in CTA 0 only
   // deterministic reduction: one partial per CTA, summed by CTA 0 in rank order
   if (tid == 0) p.scratch[(size_t)item * CLUSTER + rank] = quad;
   __threadfence();
@@ -1087,16 +1027,17 @@ __global__ void __launch_bounds__(NTHREADS, 1) potrf_cluster_kernel(PotrfParams 
     double qtot = 0.0;
 #pragma unroll
     for (int r = 0; r < CLUSTER; ++r) qtot += __ldcg(p.scratch + (size_t)item * CLUSTER + r);
-    const bool bad = sm.bad != 0;
-    double ll = -0.5 * qtot - (double)rm.M * logdet -
-                0.5 * (double)p.n * (double)rm.M * 1.8378770664093453;  // log(2 pi)
-    const int prev = p.info ? (p.info[item] & ~SPB_INFO_NOT_PD) : 0;
-    if (bad || (prev & SPB_INFO_NEG_INF) || ll != ll) ll = -INFINITY;
-    if (p.lnlike) p.lnlike[item] = ll;
-    if (p.logdet) p.logdet[item] = bad ? NAN : logdet;
-    if (p.info) p.info[item] = prev | (bad ? SPB_INFO_NOT_PD : 0);
+    lnlike_epilogue(p, item, qtot, logdet, sm.bad != 0, SPB_INFO_NOT_PD | p.only_flag, 0);
   }
 }
+
+// cluster sizes of potrf_cluster_kernel, largest first (the order of spb_context::max_active_clusters)
+struct ClusterKernel {
+  int size;
+  void (*kernel)(PotrfParams);
+};
+constexpr ClusterKernel CLUSTER_KERNELS[3] = {
+    {8, potrf_cluster_kernel<8>}, {4, potrf_cluster_kernel<4>}, {2, potrf_cluster_kernel<2>}};
 
 // ------------------------------------------------------------------------------------------
 // DMMA peak micro-benchmark: 8 warps x 16 independent accumulator tiles, operands in registers.
@@ -1118,7 +1059,33 @@ __global__ void __launch_bounds__(256, 2) dmma_peak_kernel(int iters, double *si
 
 }  // namespace
 
-static int potrf_launch(spb_context *ctx, PotrfParams &p, void *stream) {
+// PotrfParams of a MODE_FACTOR launch; affine == nullptr: no fused affine map
+static PotrfParams factor_params(int B, int nt, double *K, int ldk, long long K_stride,
+                                 const spb_affine *affine, int M, double *resid, int ldr,
+                                 long long resid_stride, double *lnlike, double *quad, double *logdet,
+                                 int32_t *info) {
+  PotrfParams p = {};
+  p.K = K;
+  p.n = nt;
+  p.ld = ldk;
+  p.strideK = K_stride;
+  p.R = (M > 0) ? resid : nullptr;
+  p.M = M;
+  p.ldr = ldr;
+  p.strideR = resid_stride;
+  p.lnlike = lnlike;
+  p.quad = quad;
+  p.logdet = logdet;
+  p.info = info;
+  p.B = B;
+  p.mode = MODE_FACTOR;
+  p.aff = affine ? *affine : spb_affine{};
+  p.aff_on = affine ? 1 : 0;
+  return p;
+}
+
+// the layout every kernel of this file assumes: 16-byte loads of (column, column + 1) pairs
+static int check_layout(const PotrfParams &p) {
   SPB_REQUIRE(p.n > 0 && p.B > 0, "cholesky: empty problem");
   SPB_REQUIRE(p.ld >= p.n && (p.ld % 2) == 0, "cholesky: ldk must be even and >= nt");
   SPB_REQUIRE(((uintptr_t)p.K % 16) == 0 && (p.strideK % 2) == 0,
@@ -1128,6 +1095,18 @@ static int potrf_launch(spb_context *ctx, PotrfParams &p, void *stream) {
     SPB_REQUIRE(((uintptr_t)p.R % 16) == 0 && (p.strideR % 2) == 0,
                 "cholesky: resid must be 16-byte aligned with an even batch stride");
   }
+  return 0;
+}
+
+// the next work counter of the context's ring, zeroed in-stream
+static int claim_counter(spb_context *ctx, void *stream, unsigned int **counter) {
+  *counter = ctx->d_counters + (__atomic_fetch_add(&ctx->counter_next, 1u, __ATOMIC_RELAXED) % SPB_NUM_COUNTERS);
+  SPB_CHECK_CUDA(cudaMemsetAsync(*counter, 0, sizeof(unsigned int), (cudaStream_t)stream));
+  return 0;
+}
+
+static int potrf_launch(spb_context *ctx, PotrfParams &p, void *stream) {
+  if (const int st = check_layout(p)) return st;
   SPB_CHECK_CUDA(cudaSetDevice(ctx->device));
   p.scratch = nullptr;
   const size_t smem = sizeof(Smem);   // batch and cluster kernel
@@ -1138,20 +1117,17 @@ static int potrf_launch(spb_context *ctx, PotrfParams &p, void *stream) {
                                           (int)smem));
       SPB_CHECK_CUDA(cudaFuncSetAttribute(potrf_lnlike_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
                                           cudaSharedmemCarveoutMaxShared));
-      SPB_CHECK_CUDA(cudaFuncSetAttribute(potrf_cluster_kernel<8>,
-                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      SPB_CHECK_CUDA(cudaFuncSetAttribute(potrf_cluster_kernel<4>,
-                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      SPB_CHECK_CUDA(cudaFuncSetAttribute(potrf_cluster_kernel<2>,
-                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      for (const ClusterKernel &ck : CLUSTER_KERNELS)
+        SPB_CHECK_CUDA(cudaFuncSetAttribute(ck.kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       return 0;
     });
     if (st) return st;
   }
   int nitems = (p.mode == MODE_FACTOR) ? p.B : (p.M + p.rows_per_cta - 1) / p.rows_per_cta;
-  // few matrices: one 8-CTA cluster per matrix instead of one CTA (see potrf_cluster_kernel)
-  int cs = 0;
-  if (!ctx->opt_no_cluster && p.mode == MODE_FACTOR && p.n > 2 * 128 && ctx->d_scratch &&
+  // few matrices: one 8-CTA cluster per matrix instead of one CTA (see potrf_cluster_kernel).  The
+  // cluster kernel factors every matrix of the batch: never for a pass restricted by only_flag.
+  int k_cs = -1;
+  if (!ctx->opt_no_cluster && p.mode == MODE_FACTOR && p.only_flag == 0 && p.n > 2 * 128 && ctx->d_scratch &&
       p.B * 2 <= ctx->num_sms) {
     // largest cluster size whose clusters are all co-resident (a second wave of clusters would
     // cost more than a smaller cluster: GPCs host a whole number of clusters), asked of the driver
@@ -1160,7 +1136,7 @@ static int potrf_launch(spb_context *ctx, PotrfParams &p, void *stream) {
       std::lock_guard<std::mutex> lock(occ_mu);
       if (ctx->max_active_clusters[0] < 0) {
         for (int k = 0; k < 3; ++k) {
-          const int c = 8 >> k;
+          const int c = CLUSTER_KERNELS[k].size;
           cudaLaunchConfig_t q = {};
           q.gridDim = dim3((unsigned)(c * ctx->num_sms));
           q.blockDim = dim3(NTHREADS);
@@ -1173,9 +1149,7 @@ static int potrf_launch(spb_context *ctx, PotrfParams &p, void *stream) {
           q.attrs = a;
           q.numAttrs = 1;
           int n = 0;
-          cudaError_t e = (c == 8)   ? cudaOccupancyMaxActiveClusters(&n, potrf_cluster_kernel<8>, &q)
-                          : (c == 4) ? cudaOccupancyMaxActiveClusters(&n, potrf_cluster_kernel<4>, &q)
-                                     : cudaOccupancyMaxActiveClusters(&n, potrf_cluster_kernel<2>, &q);
+          const cudaError_t e = cudaOccupancyMaxActiveClusters(&n, CLUSTER_KERNELS[k].kernel, &q);
           ctx->max_active_clusters[k] = (e == cudaSuccess) ? n : 0;
         }
         (void)cudaGetLastError();
@@ -1183,10 +1157,11 @@ static int potrf_launch(spb_context *ctx, PotrfParams &p, void *stream) {
     }
     // a cluster size is eligible only if its per-CTA partial sums fit the launch's scratch slot;
     // otherwise fall through to the next size and finally to the one-CTA-per-matrix kernel
-    for (int k = 0; k < 3 && !cs; ++k)
-      if (p.B <= ctx->max_active_clusters[k] && (8 >> k) * p.B <= SPB_SCRATCH_PER_SLOT) cs = 8 >> k;
+    for (int k = 0; k < 3 && k_cs < 0; ++k)
+      if (p.B <= ctx->max_active_clusters[k] && CLUSTER_KERNELS[k].size * p.B <= SPB_SCRATCH_PER_SLOT) k_cs = k;
   }
-  if (cs) {
+  if (k_cs >= 0) {
+    const int cs = CLUSTER_KERNELS[k_cs].size;
     const unsigned slot = __atomic_fetch_add(&ctx->counter_next, 1u, __ATOMIC_RELAXED) % SPB_NUM_COUNTERS;
     p.scratch = ctx->d_scratch + (size_t)slot * SPB_SCRATCH_PER_SLOT;
     p.counter = nullptr;
@@ -1202,9 +1177,7 @@ static int potrf_launch(spb_context *ctx, PotrfParams &p, void *stream) {
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    if (cs == 8) SPB_CHECK_CUDA(cudaLaunchKernelEx(&cfg, potrf_cluster_kernel<8>, p));
-    else if (cs == 4) SPB_CHECK_CUDA(cudaLaunchKernelEx(&cfg, potrf_cluster_kernel<4>, p));
-    else SPB_CHECK_CUDA(cudaLaunchKernelEx(&cfg, potrf_cluster_kernel<2>, p));
+    SPB_CHECK_CUDA(cudaLaunchKernelEx(&cfg, CLUSTER_KERNELS[k_cs].kernel, p));
     SPB_LAUNCH_CHECK(ctx);
     return 0;
   }
@@ -1221,9 +1194,7 @@ static int potrf_launch(spb_context *ctx, PotrfParams &p, void *stream) {
                                     NB, 1);
     p.use_tma = (st == 0) ? 1 : 0;   // an unencodable layout simply keeps the cp.async path
   }
-  p.counter = ctx->d_counters +
-      (__atomic_fetch_add(&ctx->counter_next, 1u, __ATOMIC_RELAXED) % SPB_NUM_COUNTERS);
-  SPB_CHECK_CUDA(cudaMemsetAsync(p.counter, 0, sizeof(unsigned int), (cudaStream_t)stream));
+  if (const int st = claim_counter(ctx, stream, &p.counter)) return st;
   potrf_lnlike_kernel<<<grid, NTHREADS, smem, (cudaStream_t)stream>>>(p, tmK);
   SPB_LAUNCH_CHECK(ctx);
   return 0;
@@ -1234,25 +1205,8 @@ extern "C" int spb_cholesky_lnlike(spb_context *ctx, int B, int nt, double *K, i
                                    long long resid_stride, double *lnlike, double *quad,
                                    double *logdet, int32_t *info, void *stream) {
   SPB_REQUIRE(ctx != nullptr, "null context");
-  PotrfParams p;
-  p.only_flag = 0;
-  p.K = K;
-  p.n = nt;
-  p.ld = ldk;
-  p.strideK = K_stride;
-  p.R = (M > 0) ? resid : nullptr;
-  p.M = M;
-  p.ldr = ldr;
-  p.strideR = resid_stride;
-  p.lnlike = lnlike;
-  p.quad = quad;
-  p.logdet = logdet;
-  p.info = info;
-  p.B = B;
-  p.mode = MODE_FACTOR;
-  p.rows_per_cta = 0;
-  p.aff = spb_affine{};
-  p.aff_on = 0;
+  PotrfParams p = factor_params(B, nt, K, ldk, K_stride, nullptr, M, resid, ldr, resid_stride, lnlike, quad,
+                                logdet, info);
   return potrf_launch(ctx, p, stream);
 }
 
@@ -1264,25 +1218,8 @@ extern "C" int spb_cholesky_lnlike_affine(spb_context *ctx, int B, int nt, doubl
   SPB_REQUIRE(ctx != nullptr && affine != nullptr, "cholesky_lnlike_affine: null argument");
   SPB_REQUIRE((affine->scal == nullptr) == (affine->q == nullptr),
               "cholesky_lnlike_affine: scal and q must be given together");
-  PotrfParams p;
-  p.only_flag = 0;
-  p.K = K;
-  p.n = nt;
-  p.ld = ldk;
-  p.strideK = K_stride;
-  p.R = (M > 0) ? resid : nullptr;
-  p.M = M;
-  p.ldr = ldr;
-  p.strideR = resid_stride;
-  p.lnlike = lnlike;
-  p.quad = quad;
-  p.logdet = logdet;
-  p.info = info;
-  p.B = B;
-  p.mode = MODE_FACTOR;
-  p.rows_per_cta = 0;
-  p.aff = *affine;
-  p.aff_on = 1;
+  PotrfParams p = factor_params(B, nt, K, ldk, K_stride, affine, M, resid, ldr, resid_stride, lnlike, quad,
+                                logdet, info);
   return potrf_launch(ctx, p, stream);
 }
 
@@ -1319,49 +1256,20 @@ extern "C" int spb_cholesky_lnlike_i8(spb_context *ctx, int B, int nt, double *K
   SPB_REQUIRE(affine == nullptr || (affine->scal == nullptr) == (affine->q == nullptr),
               "cholesky_lnlike_i8: scal and q must be given together");
   int rb = 0;
-  const int planes_arg = planes;
   planes = i8_decode(planes, &rb);
   SPB_REQUIRE(planes != 0, "cholesky_lnlike_i8: planes must be 7, 8, 77, 78 or 87");
   SPB_REQUIRE(info != nullptr, "cholesky_lnlike_i8: info is required");
   SPB_REQUIRE(nt > NB && nt <= NB * I8_MAXP, "cholesky_lnlike_i8: nt out of range (64 < nt <= 16384)");
   SPB_REQUIRE(workspace != nullptr && workspace_bytes >= spb_cholesky_i8_workspace_bytes(B, nt, M, planes),
               "cholesky_lnlike_i8: workspace too small");
-  PotrfParams p;
-  p.only_flag = 0;
-  p.K = K;
-  p.n = nt;
-  p.ld = ldk;
-  p.strideK = K_stride;
-  p.R = (M > 0) ? resid : nullptr;
-  p.M = M;
-  p.ldr = ldr;
-  p.strideR = resid_stride;
-  p.lnlike = lnlike;
-  p.quad = quad;
-  p.logdet = logdet;
-  p.info = info;
-  p.B = B;
-  p.mode = MODE_FACTOR;
-  p.rows_per_cta = 0;
-  p.aff = affine ? *affine : spb_affine{};
-  p.aff_on = affine ? 1 : 0;
-  p.scratch = nullptr;
-  p.use_tma = 0;
-  SPB_REQUIRE(p.n > 0 && p.B > 0, "cholesky: empty problem");
-  SPB_REQUIRE(p.ld >= p.n && (p.ld % 2) == 0, "cholesky: ldk must be even and >= nt");
-  SPB_REQUIRE(((uintptr_t)p.K % 16) == 0 && (p.strideK % 2) == 0,
-              "cholesky: K must be 16-byte aligned with an even batch stride");
-  if (p.R) {
-    SPB_REQUIRE(p.ldr >= p.n && (p.ldr % 2) == 0, "cholesky: ldr must be even and >= nt");
-    SPB_REQUIRE(((uintptr_t)p.R % 16) == 0 && (p.strideR % 2) == 0,
-                "cholesky: resid must be 16-byte aligned with an even batch stride");
-  }
+  PotrfParams p = factor_params(B, nt, K, ldk, K_stride, affine, M, resid, ldr, resid_stride, lnlike, quad,
+                                logdet, info);
+  if (const int st = check_layout(p)) return st;
   SPB_CHECK_CUDA(cudaSetDevice(ctx->device));
   I8Params ip;
   const int n64 = i8_n64(nt);
   ip.NR = n64 + M;
   ip.LDQ = n64;
-  ip.store_factor = 0;
   ip.lambda_min = lambda_min;
   uintptr_t w = ((uintptr_t)workspace + 255) & ~(uintptr_t)255;
   ip.Q = reinterpret_cast<uint8_t *>(w);
@@ -1398,16 +1306,12 @@ extern "C" int spb_cholesky_lnlike_i8(spb_context *ctx, int B, int nt, double *K
       SPB_I8_ATTR(7, 2, 7, true);
       SPB_I8_ATTR(7, 2, 8, true);
 #undef SPB_I8_ATTR
-      SPB_CHECK_CUDA(cudaFuncSetAttribute(potrf_lnlike_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                          (int)sizeof(Smem)));
       return 0;
     });
     if (st) return st;
   }
   const int grid = B < ctx->num_sms ? B : ctx->num_sms;
-  p.counter = ctx->d_counters +
-      (__atomic_fetch_add(&ctx->counter_next, 1u, __ATOMIC_RELAXED) % SPB_NUM_COUNTERS);
-  SPB_CHECK_CUDA(cudaMemsetAsync(p.counter, 0, sizeof(unsigned int), (cudaStream_t)stream));
+  if (const int st = claim_counter(ctx, stream, &p.counter)) return st;
   // 7-plane kernels, nt <= 1536: two ring stages + the cp.async prefetch of the next K tile (the per-tile
   // chain dominates there); larger nt: three ring stages (the MMA stream dominates, -8 % with two)
   const bool kpre = (planes == 7) && nt <= 1536;
@@ -1421,60 +1325,29 @@ extern "C" int spb_cholesky_lnlike_i8(spb_context *ctx, int B, int nt, double *K
 #undef SPB_I8_GO
   SPB_LAUNCH_CHECK(ctx);
   // safety net: matrices flagged SPB_INFO_I8_RANGE go through the FP64 kernel (their K is intact)
-  {
-    PotrfParams f = p;
-    f.only_flag = SPB_INFO_I8_RANGE;
-    f.counter = ctx->d_counters +
-        (__atomic_fetch_add(&ctx->counter_next, 1u, __ATOMIC_RELAXED) % SPB_NUM_COUNTERS);
-    SPB_CHECK_CUDA(cudaMemsetAsync(f.counter, 0, sizeof(unsigned int), (cudaStream_t)stream));
-    CUtensorMap tmK;
-    memset(&tmK, 0, sizeof(tmK));
-    const int g2 = B < 2 * ctx->num_sms ? B : 2 * ctx->num_sms;
-    potrf_lnlike_kernel<<<g2, NTHREADS, sizeof(Smem), (cudaStream_t)stream>>>(f, tmK);
-    SPB_LAUNCH_CHECK(ctx);
-  }
-  return 0;
+  p.only_flag = SPB_INFO_I8_RANGE;
+  return potrf_launch(ctx, p, stream);
 }
 
 extern "C" int spb_cholesky_solve_rows(spb_context *ctx, int nt, const double *L, int ldk, int M,
                                        double *resid, int ldr, double *quad, void *stream) {
   SPB_REQUIRE(ctx != nullptr, "null context");
   SPB_REQUIRE(M > 0 && resid != nullptr, "solve_rows: no right-hand sides");
-  PotrfParams p;
-  p.only_flag = 0;
+  PotrfParams p = {};   // no lnlike / logdet / info, no affine map
   p.K = const_cast<double *>(L);
   p.n = nt;
   p.ld = ldk;
-  p.strideK = 0;
   p.R = resid;
   p.M = M;
   p.ldr = ldr;
-  p.strideR = 0;
-  p.lnlike = nullptr;
   p.quad = quad;
-  p.logdet = nullptr;
-  p.info = nullptr;
   p.B = 1;
-  p.aff = spb_affine{};
-  p.aff_on = 0;
   p.mode = MODE_SOLVE;
   // one full 128-row tile per work item (a tile costs the same DMMA time however many of its
   // rows are live, so smaller items would only replicate the streaming of L)
   p.rows_per_cta = TM;
   return potrf_launch(ctx, p, stream);
 }
-
-#ifdef SPB_POTRF_PROF
-// debug build only: read (and reset) the phase timers; out[2][16]
-extern "C" int spb_potrf_prof(unsigned long long *out_host) {
-  SPB_CHECK_CUDA(cudaDeviceSynchronize());
-  SPB_CHECK_CUDA(cudaMemcpyFromSymbol(out_host, g_potrf_prof, sizeof(unsigned long long) * 32));
-  unsigned long long z[32] = {0};
-  SPB_CHECK_CUDA(cudaMemcpyToSymbol(g_potrf_prof, z, sizeof(z)));
-  SPB_CHECK_CUDA(cudaMemcpyFromSymbol(out_host + 32, g_potrf_clk, sizeof(unsigned long long) * 4));
-  return 0;
-}
-#endif
 
 extern "C" int spb_dmma_peak(spb_context *ctx, int iters, double *tflops_host, double *ms_host) {
   SPB_REQUIRE(ctx != nullptr, "null context");

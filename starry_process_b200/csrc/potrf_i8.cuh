@@ -28,14 +28,6 @@
 // SPB_INFO_I8_RANGE for the matrix; the launcher then re-runs exactly those matrices through the DMMA
 // kernel (K is untouched, so nothing is lost).
 
-#ifdef SPB_POTRF_PROF
-#define I8_PROF_DECL(row_) unsigned long long _it = clock64(); const int _ir = (row_)
-#define I8_PROF(sm, k) do { if (_ir >= 0) { unsigned long long _n = clock64(); (sm).prof[_ir][k] += _n - _it; _it = _n; } } while (0)
-#else
-#define I8_PROF_DECL(row_)
-#define I8_PROF(sm, k)
-#endif
-
 constexpr int I8_MAXP = 256;         // panels per matrix (nt <= 16384)
 static_assert(NB == I8_TN, "a panel is one TMEM block wide");
 
@@ -44,7 +36,6 @@ struct I8Params {
   double *E;             // (B, NR) row scales 2^e
   long long strideQ;     // bytes per matrix
   int NR, LDQ;
-  int store_factor;      // also write L (fp64) over K like the DMMA kernel
   double lambda_min;     // > 0: K' >= lambda_min I (else K' >= diag(aff.diag)): bounds the right-hand-side rows
 };
 
@@ -111,12 +102,7 @@ struct SmemI8 {
   int bad;
   int bad_range;
   int next_item;
-#ifdef SPB_POTRF_PROF
-  unsigned long long prof[2][16];
-#endif
 };
-
-__device__ __forceinline__ void cbar256() { asm volatile("bar.sync 2, 256;\n" ::: "memory"); }
 
 // The fused affine map (spb_affine) of one accumulator row that holds RAW values of a full panel (the
 // arithmetic half of init_acc; used when the values come from the cp.async prefetch buffer).
@@ -127,28 +113,9 @@ __device__ __forceinline__ void i8_apply_aff(const SM &sm, const RowMapI8 &rm, c
   (void)rm.row(v, kind);
   if (kind != KIND_DIAG && kind != KIND_BELOW) return;
   const int gi = c0 + v;
-  double Ci = sm.af[3], Di = 0.0;
-  if (af.norm) {
-    const double qi = af.q[gi];
-    const double a = sm.af[1] * (1.0 - qi);
-    Ci += a;
-    Di = a + sm.af[2] * qi;
-  }
+  double Ci, Di;
+  aff_row_consts(sm, af, gi, Ci, Di);
   aff_full_row(sm, af, kind == KIND_DIAG, gi, v, c0, tg, Ci, Di, accrow);
-}
-
-template <class SM>
-__device__ __forceinline__ double block_sum_i8(SM &sm, double v) {
-  const int tid = threadIdx.x, pw = tid >> 5, lane = tid & 31;
-  v = warp_sum(v);
-  cbar256();
-  if (lane == 0) sm.red[pw] = v;
-  cbar256();
-  double t = 0.0;
-#pragma unroll
-  for (int w = 0; w < I8_NCT / 32; ++w) t += sm.red[w];
-  cbar256();
-  return t;
 }
 
 // number of 128-row tiles of the panel starting at column c0 (NR = nt + M virtual rows in total)
@@ -164,7 +131,6 @@ template <int S, int STAGES, int RB, bool KPRE>
 __global__ void __launch_bounds__(I8_NTHREADS, 1)
     potrf_i8_kernel(PotrfParams p, I8Params ip, const __grid_constant__ CUtensorMap tmA,
                     const __grid_constant__ CUtensorMap tmB) {
-  extern __shared__ __align__(1024) unsigned char smem_raw[];
   using SM = SmemI8<S, STAGES, KPRE>;
   SM &sm = *reinterpret_cast<SM *>(smem_raw);
   const int tid = threadIdx.x, pw = tid >> 5, lane = tid & 31, g = lane >> 2, tg = lane & 3;
@@ -179,9 +145,6 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
     sm.stored = 0;
     fence_mbarrier_init();
   }
-#ifdef SPB_POTRF_PROF
-  if (tid < 32) sm.prof[tid / 16][tid % 16] = 0;
-#endif
   if (pw == I8_ISSUER_WARP) i8_tmem_alloc(&sm.tmem_base);
   tc_fence_before();
   __syncthreads();
@@ -205,26 +168,10 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
     const int M_ = p.R ? p.M : 0;
     const bool gap = (M_ <= n64 - p.n);   // also true when M = 0; false when nt is a multiple of 64 and M > 0
     double *quad_out = p.quad ? p.quad + (size_t)item * p.M : nullptr;
-    AffRow af;
-    af.q = nullptr;
-    af.dg = nullptr;
-    af.dg_vec = 0;
-    af.norm = false;
-    if (p.aff_on) {
-      af.norm = (p.aff.scal != nullptr) && (p.aff.q != nullptr);
-      if (af.norm) af.q = p.aff.q + (size_t)item * p.n;
-      if (p.aff.diag) {
-        af.dg = p.aff.diag + (size_t)item * p.aff.diag_stride;
-        af.dg_vec = (p.aff.diag_kind == 1);
-      }
-    }
+    const AffRow af = aff_setup(p, item, sm, tid);
     double *Eb = ip.E + (size_t)item * NR;
     uint8_t *Qb = ip.Q + (size_t)item * ip.strideQ;
     if (tid == 0) {
-      sm.af[0] = af.norm ? p.aff.scal[4 * (size_t)item + 0] : 1.0;
-      sm.af[1] = af.norm ? p.aff.scal[4 * (size_t)item + 1] : 0.0;
-      sm.af[2] = af.norm ? p.aff.scal[4 * (size_t)item + 2] : 0.0;
-      sm.af[3] = (p.aff_on && p.aff.offset) ? p.aff.offset[(size_t)item * p.aff.offset_stride] : 0.0;
       sm.bad = 0;
       sm.bad_range = 0;
       unsigned f = seq_base;
@@ -241,7 +188,6 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
 
     if (pw < 8) {
       // ============================================================== COMPUTE WARPS
-      I8_PROF_DECL(tid == 0 ? 0 : -1);
       if (quad_out)
         for (int m = tid; m < rm.M; m += I8_NCT) quad_out[m] = 0.0;
       // row scales: 2^e_i > 1.0101 sqrt(K'_ii) for the rows of L;  for the right-hand-side rows a bound of
@@ -254,13 +200,8 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
       for (int r = tid; r < p.n; r += I8_NCT) {
         double kd = rm.Kb[(size_t)r * p.ld + r];
         if (p.aff_on) {
-          double Ci = sm.af[3], Di = 0.0;
-          if (af.norm) {
-            const double qi = af.q[r];
-            const double a = sm.af[1] * (1.0 - qi);
-            Ci += a;
-            Di = a + sm.af[2] * qi;
-          }
+          double Ci, Di;
+          aff_row_consts(sm, af, r, Ci, Di);
           kd = aff_apply(sm, af, kd, Ci, Di, true, r, r);
         }
         Eb[r] = row_scale(sqrt(kd));
@@ -288,7 +229,6 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
       for (int r = p.n + tid; r < n64; r += I8_NCT) Eb[r] = 1.0;
       __threadfence_block();
       cbar256();
-      I8_PROF(sm, 8);
 
       double logdet_part = 0.0, quad_part = 0.0;
       double acc[2][8][2];
@@ -364,10 +304,6 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
               }
             }
           }
-#ifdef SPB_POTRF_PROF
-          if (tid == 0 && c0 == 0) sm.prof[0][9] += clock64() - _it;   // K loads of panel 0 (no MMA / TMA in flight)
-#endif
-          I8_PROF(sm, 0);
           if (nchunks > 0) {
             // scales of this thread's rows (plane row = c0 + virtual row for matrix and RHS rows alike)
             double si[2];
@@ -382,7 +318,6 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
             }
             mbar_wait_sleep(&sm.tmem_full, tq & 1u, 50);
             tc_fence_after();
-            I8_PROF(sm, 1);
             const uint32_t tw = tmem + ((uint32_t)(32 * (pw & 3) + 16 * ((pw >> 2) & 1)) << 16);
 #pragma unroll
             for (int cq = 0; cq < 4; ++cq) {
@@ -408,45 +343,28 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
             __syncwarp();
             if (lane == 0) mbar_arrive(&sm.tmem_empty);
             ++tq;
-            I8_PROF(sm, 2);
           }
           const int lw = warp;
           if (diag_tile) {
-            if (lw < 4) {
-#ifdef SPB_POTRF_PROF
-              const unsigned long long t8_before = sm.prof[0][11];
-#endif
-              potf2_regs(sm, acc, lw, lane);
-#ifdef SPB_POTRF_PROF
-              if (tid == 0 && c0 == 0) sm.prof[0][15] += sm.prof[0][11] - t8_before;   // pivot chains of panel 0
-#endif
-            }
+            if (lw < 4) potf2_regs(sm, acc, lw, lane);
             cbar256();   // L_jj and the inverses of its diagonal tiles are in shared memory
             if (tid < min(NB, p.n - c0)) logdet_part += 0.5 * log(sm.dpiv[tid]);
-            if (ip.store_factor) {
-              for (int idx = tid; idx < NB * NB; idx += I8_NCT) {
-                const int i = idx >> 6, j = idx & 63;
-                if (j <= i && c0 + i < p.n) rm.Kb[(size_t)(c0 + i) * p.ld + c0 + j] = sm.Ld.at(i, j);
-              }
-            }
           }
-          I8_PROF(sm, 3);
           // a matrix already found not positive definite turns into NaNs from here on: its digits
           // overflow, but there is nothing to rescue by re-running it on the FP64 kernel
           const bool already_bad = (*(volatile int *)&sm.bad) != 0;
           const int vr2 = v0 + lw * 16;             // first tile row of this warp from here on
           if (!(diag_tile && lw < 4) && vr2 < nvirt) {
             trsm_warp(sm, acc, lane);
-            I8_PROF(sm, 4);
 #pragma unroll
             for (int mt = 0; mt < 2; ++mt) {
               const int v = vr2 + mt * 8 + g;
               int kind;
               double *prow = rm.row(v, kind);
               const bool live = (kind == KIND_BELOW || kind == KIND_RHS);
-              // ---- fp64: y rows always (output), rows of L only on request
+              // ---- fp64: the y rows (output); the rows of L are kept only as digit planes
               double q = 0.0;
-              if (live && (kind == KIND_RHS || ip.store_factor)) {
+              if (kind == KIND_RHS) {
 #pragma unroll
                 for (int nt = 0; nt < 8; ++nt) {
                   const int gc = c0 + nt * 8 + 2 * tg;
@@ -523,7 +441,6 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
           }
           // the planes (generic-proxy stores) must be visible to the TMA engine before the producer is
           // told about them; the barrier also protects Ld / Dv against the next panel's potf2
-          I8_PROF(sm, 5);
           fence_proxy_async_global();
           __threadfence_block();
           cbar256();
@@ -531,33 +448,20 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
             __threadfence_block();   // the barrier's view of the other warps' stores before the counter moves
             sm.stored = seq + 1;
           }
-          I8_PROF(sm, 6);
         }
       }
       if (bad_range) sm.bad_range = 1;
       // ---- reductions -> lnlike
-      const double quad = block_sum_i8(sm, quad_part);
-      const double logdet = block_sum_i8(sm, logdet_part);
-      I8_PROF(sm, 7);
-#ifdef SPB_POTRF_PROF
-      if (tid == 0) sm.prof[0][10] += 1;
-#endif
+      const double quad = block_sum<true>(sm, quad_part);
+      const double logdet = block_sum<true>(sm, logdet_part);
       if (tid == 0) {
-        const bool bad = sm.bad != 0;
-        double ll = -0.5 * quad - (double)rm.M * logdet -
-                    0.5 * (double)p.n * (double)rm.M * 1.8378770664093453;  // log(2 pi)
-        const int prev = p.info ? (p.info[item] & ~(SPB_INFO_NOT_PD | SPB_INFO_I8_RANGE)) : 0;
-        if (bad || (prev & SPB_INFO_NEG_INF) || ll != ll) ll = -INFINITY;
-        if (p.lnlike) p.lnlike[item] = ll;
-        if (p.logdet) p.logdet[item] = bad ? NAN : logdet;
-        if (p.info)
-          p.info[item] = prev | (bad ? SPB_INFO_NOT_PD : 0) | (sm.bad_range ? SPB_INFO_I8_RANGE : 0);
+        lnlike_epilogue(p, item, quad, logdet, sm.bad != 0, SPB_INFO_NOT_PD | SPB_INFO_I8_RANGE,
+                        sm.bad_range ? SPB_INFO_I8_RANGE : 0);
         sm.next_item = (int)gridDim.x + (int)atomicAdd(p.counter, 1u);
       }
     } else if (pw == I8_PRODUCER_WARP) {
       // ============================================================== TMA PRODUCER (one thread)
       if (lane == 0) {
-        I8_PROF_DECL(1);
         unsigned known = sm.stored;
         for (int c0 = NB; c0 < p.n; c0 += NB) {
           const int nvirt = i8_nvirt(p.n, n64, M_, gap, c0);
@@ -579,16 +483,13 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
                 vP = vlast + (c0 - P);
               }
               const unsigned need = sm.first[P / NB] + (unsigned)(vP / I8_TM) + 1u;
-              I8_PROF(sm, 10);
               if ((int)(known - need) < 0) {
                 while ((int)((known = sm.stored) - need) < 0) __nanosleep(100);
                 __threadfence_block();
                 fence_proxy_async_global();
               }
-              I8_PROF(sm, 8);
               const unsigned st = xchunk % STAGES;
               if (xchunk >= (unsigned)STAGES) mbar_wait_sleep(&sm.empty[st], ((xchunk / STAGES) + 1u) & 1u, 100);
-              I8_PROF(sm, 9);
               mbar_arrive_expect_tx(&sm.full[st], (unsigned)(S * (I8_TM + NB) * I8_KCH));
               tma_load_4d(&sm.A[st][0][0][0], &tmA, &sm.full[st], ch * I8_KCH, c0 + v0, 0, item);
               tma_load_4d(&sm.B[st][0][0][0], &tmB, &sm.full[st], ch * I8_KCH, c0, 0, item);
@@ -599,24 +500,17 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
     } else if (pw == I8_ISSUER_WARP) {
       // ============================================================== MMA ISSUER (one thread)
       if (lane == 0) {
-        I8_PROF_DECL(1);
         for (int c0 = NB; c0 < p.n; c0 += NB) {
           const int nvirt = i8_nvirt(p.n, n64, M_, gap, c0);
           const int nchunks = c0 / I8_KCH;
           for (int v0 = 0; v0 < nvirt; v0 += I8_TM, ++tq) {
-            I8_PROF(sm, 2);
             if (tq > 0) mbar_wait_sleep(&sm.tmem_empty, (tq + 1u) & 1u, 100);   // the warps have drained TMEM
             tc_fence_after();
-            I8_PROF(sm, 0);
             for (int ch = 0; ch < nchunks; ++ch, ++xchunk) {
               const unsigned st = xchunk % STAGES;
-              I8_PROF(sm, 2);
               mbar_wait_sleep(&sm.full[st], (xchunk / STAGES) & 1u, 50);
               tc_fence_after();
-              I8_PROF(sm, 1);
-#ifndef SPB_I8_NOMMA
               i8_issue_chunk<S>(tmem, sm.A[st], sm.B[st], ch > 0);
-#endif
               i8_commit(&sm.empty[st]);
             }
             i8_commit(&sm.tmem_full);
@@ -630,8 +524,5 @@ __global__ void __launch_bounds__(I8_NTHREADS, 1)
   }
   tc_fence_before();
   __syncthreads();
-#ifdef SPB_POTRF_PROF
-  if (tid < 32) atomicAdd(&g_potrf_prof[tid / 16][tid % 16], sm.prof[tid / 16][tid % 16]);
-#endif
   if (pw == I8_ISSUER_WARP) i8_tmem_dealloc(tmem);
 }

@@ -74,6 +74,11 @@ def _both_kernels(spb, B, n, M, planes, seed, dg=1e-4, poison=None, not_pd=None)
             torch.cuda.synchronize()
             if poison is None and not_pd is None:
                 assert torch.equal(Kc, K), "the INT8 path must leave K untouched"
+            elif poison is not None:
+                # only the flagged matrix goes through the FP64 safety net, which stores its factor over K
+                keep = [i for i in range(B) if i != poison[0]]
+                assert torch.equal(Kc[keep], K[keep]), "the safety net must re-run only the flagged matrix"
+                assert not torch.equal(Kc[poison[0]], K[poison[0]]), "the flagged matrix was not re-run"
         torch.cuda.synchronize()
         out[name] = dict(ll=ll.cpu().numpy(), quad=quad.cpu().numpy(), logdet=logdet.cpu().numpy(),
                          info=info.cpu().numpy(), y=rc.cpu().numpy()[:, :M, :n])

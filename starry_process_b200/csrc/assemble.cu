@@ -52,48 +52,14 @@ __device__ __forceinline__ double temporal_k(int kind, double ti, double tj, dou
   return exp(-(dt * dt) / (2.0 * tau));
 }
 
-// theta_i = 2 pi mod(t_i / p, 1)  (flux.py:261)
-__device__ __forceinline__ double phase_of(double t, double period) {
-  const double x = t / period;
-  return 2.0 * 3.14159265358979323846 * (x - floor(x));
-}
-
-// ---- pass A (normalised only): row sums of the raw covariance -------------------------------
+// ---- pass A (normalised conditional): row sums of K -----------------------------------------
 __global__ void __launch_bounds__(256) rowsum_kernel(AsmParams p) {
-  extern __shared__ double sh[];  // coef (4*nc) | theta (nt) | t (nt, time-variable only)
   const int b = blockIdx.y;
-  const int nc = p.covpts + 1;
-  double *cf = sh, *th = sh + 4 * nc, *tm = th + p.nt;
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int tkind = p.nm.temporal_kind;
-  const double tau = tkind ? p.nm.tau[(size_t)b * p.nm.tau_stride] : 1.0;
-  if (p.marginal) {
-    for (int k = tid; k < 4 * nc; k += 256) cf[k] = p.coef[(size_t)b * 4 * nc + k];
-    for (int k = tid; k < p.nt; k += 256) th[k] = phase_of(p.t[k], p.period);
-    if (tkind)
-      for (int k = tid; k < p.nt; k += 256) tm[k] = p.t[k];
-  }
-  __syncthreads();
-  const double dx = (double)p.covpts / (2.0 * 3.14159265358979323846);  // 1 / dx
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   for (int i = blockIdx.x * 8 + warp; i < p.nt; i += gridDim.x * 8) {
+    const double *row = p.K + ((size_t)b * p.nt + i) * p.ldk;
     double s = 0.0;
-    if (p.marginal) {
-      if (p.nt == 1) {
-        s = (lane == 0) ? p.var[b] : 0.0;
-      } else {
-        const double thi = th[i];
-        if (tkind) {
-          const double ti = tm[i];
-          for (int j = lane; j < p.nt; j += 32)
-            s += interp_cov(cf, nc, dx, thi, th[j]) * temporal_k(tkind, ti, tm[j], tau);
-        } else {
-          for (int j = lane; j < p.nt; j += 32) s += interp_cov(cf, nc, dx, thi, th[j]);
-        }
-      }
-    } else {
-      const double *row = p.K + ((size_t)b * p.nt + i) * p.ldk;
-      for (int j = lane; j < p.nt; j += 32) s += row[j];
-    }
+    for (int j = lane; j < p.nt; j += 32) s += row[j];
     s = warp_sum(s);
     if (lane == 0) p.rowq[(size_t)b * p.nt + i] = s;
   }
@@ -108,23 +74,100 @@ __global__ void __launch_bounds__(256) rowsum_kernel(AsmParams p) {
 constexpr int RS_G = 8;      // CTAs per sample
 constexpr int RS_CB = 512;   // columns per register block (16 per lane: 3 CTAs per SM)
 
-// TEMPORAL is a compile-time switch: the time-variable branch must not cost the static path (the
-// bench workload) registers or predicated instructions in its inner loop.
-template <bool TEMPORAL>
+// How an entry v(i, j) of the raw covariance is obtained: one policy per kind of light curve, each a
+// compile-time parameter of rowsum_sym_kernel so that no policy costs another registers or predicated
+// instructions in the inner loop.  A policy stages its shared-memory tables (stage: per time stamp, beside
+// the phase table; tables: once that is complete, together with its per-CTA constants, whose FP64 divisions
+// then overlap the latency of the staging loads), fixes the row (row) and returns v(i, j) for j < i
+// (operator()) and v(i, i) for nt > 1 (diag).
+//
+// General time stamps: the cubic interpolant of flux.py:256-276 at |theta_i - theta_j|.
+struct GeneralEntry {
+  const double *cf, *th;
+  int nc;
+  double inv_dx, thi;
+  __device__ GeneralEntry(const AsmParams &p, int b, const double *cf_, const double *th_, double *tail)
+      : cf(cf_), th(th_), nc(p.covpts + 1) {}
+  __device__ void stage(int k, double wraps) {}
+  __device__ void tables(const AsmParams &p) { inv_dx = (double)p.covpts / (2.0 * 3.14159265358979323846); }
+  __device__ void row(int i) { thi = th[i]; }
+  __device__ double operator()(int i, int j) const { return interp_cov(cf, nc, inv_dx, thi, th[j]); }
+  __device__ double diag() const { return interp_cov(cf, nc, inv_dx, thi, thi); }
+};
+
+// Time-variable surfaces: the interpolant times the temporal kernel (which is 1 on the diagonal).
+struct TemporalEntry : GeneralEntry {
+  const double *t;
+  double *tm;   // tail: t (nt)
+  int tkind;
+  double tau, ti;
+  __device__ TemporalEntry(const AsmParams &p, int b, const double *cf_, const double *th_, double *tail)
+      : GeneralEntry(p, b, cf_, th_, tail), t(p.t), tm(tail), tkind(p.nm.temporal_kind),
+        tau(p.nm.tau[(size_t)b * p.nm.tau_stride]) {}
+  __device__ void stage(int k, double wraps) { tm[k] = t[k]; }
+  __device__ void row(int i) {
+    GeneralEntry::row(i);
+    ti = tm[i];
+  }
+  __device__ double operator()(int i, int j) const {
+    return GeneralEntry::operator()(i, j) * temporal_k(tkind, ti, tm[j], tau);
+  }
+};
+
+// EQUALLY SPACED time stamps (spb_noise_model.uniform_dt).
+// theta_i - theta_j = 2 pi ((t_i - t_j) / p - (floor(t_i / p) - floor(t_j / p))) = 2 pi (d dt / p - m) with
+// d = i - j and m one of floor(d dt / p), floor(d dt / p) + 1: the interpolant is tabulated once per CTA
+// for the 2 nt possible arguments (G[0][d], G[1][d]) and an entry costs two conflict-free shared-memory
+// loads (the wrap count of column j and the table value) instead of the phase load and four coefficient
+// gathers of the general policy, which is bound by exactly those (shared-memory LSU 77 %).  Entries whose
+// wrap count is neither of the two candidates (cannot happen in exact arithmetic) take the general formula.
+struct UniformEntry : GeneralEntry {
+  double *G;      // tail: G (2 nt) | wraps (nt ints) | m0 (nt ints)
+  int *fl, *m0t;  // floor(t_k / p) per stamp, floor(d dt / p) per lag
+  int nt, fli;
+  __device__ UniformEntry(const AsmParams &p, int b, const double *cf_, const double *th_, double *tail)
+      : GeneralEntry(p, b, cf_, th_, tail), G(tail), fl(reinterpret_cast<int *>(tail + 2 * p.nt)), m0t(fl + p.nt),
+        nt(p.nt) {}
+  __device__ void stage(int k, double wraps) { fl[k] = (int)wraps; }
+  __device__ void tables(const AsmParams &p) {
+    GeneralEntry::tables(p);
+    const double dtp = p.nm.uniform_dt / p.period;
+    for (int d = threadIdx.x; d < nt; d += 256) {
+      const double x = (double)d * dtp, m0 = floor(x);
+      G[d] = interp_cov(cf, nc, inv_dx, 2.0 * 3.14159265358979323846 * (x - m0), 0.0);
+      G[nt + d] = interp_cov(cf, nc, inv_dx, 2.0 * 3.14159265358979323846 * (m0 + 1.0 - x), 0.0);
+      m0t[d] = (int)m0;
+    }
+    __syncthreads();
+  }
+  __device__ void row(int i) {
+    GeneralEntry::row(i);
+    fli = fl[i];
+  }
+  __device__ double operator()(int i, int j) const {
+    const int d = i - j;
+    const int w = (fli - fl[j]) - m0t[d];   // 0 or 1
+    return ((unsigned)w <= 1u) ? G[w * nt + d] : GeneralEntry::operator()(i, j);
+  }
+  __device__ double diag() const { return G[0]; }
+};
+
+template <class Entry>
 __global__ void __launch_bounds__(256, 3) rowsum_sym_kernel(AsmParams p) {
-  extern __shared__ double sh[];  // coef (4*nc) | theta (nt) | part (8 x RS_CB) | t (nt, optional)
+  extern __shared__ double sh[];  // coef (4*nc) | theta (nt) | part (8 x RS_CB) | the entry's own tables
   const int b = blockIdx.y, c = blockIdx.x;
   const int nc = p.covpts + 1;
-  double *cf = sh, *th = sh + 4 * nc, *part = th + p.nt, *tm = part + 8 * RS_CB;
+  double *cf = sh, *th = sh + 4 * nc, *part = th + p.nt;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int tkind = TEMPORAL ? p.nm.temporal_kind : 0;
-  const double tau = tkind ? p.nm.tau[(size_t)b * p.nm.tau_stride] : 1.0;
+  Entry e(p, b, cf, th, part + 8 * RS_CB);
   for (int k = tid; k < 4 * nc; k += 256) cf[k] = p.coef[(size_t)b * 4 * nc + k];
-  for (int k = tid; k < p.nt; k += 256) th[k] = phase_of(p.t[k], p.period);
-  if (TEMPORAL)
-    for (int k = tid; k < p.nt; k += 256) tm[k] = p.t[k];
+  for (int k = tid; k < p.nt; k += 256) {
+    double wraps;
+    th[k] = spb_phase(p.t[k], p.period, &wraps);
+    e.stage(k, wraps);
+  }
   __syncthreads();
-  const double dx = (double)p.covpts / (2.0 * 3.14159265358979323846);  // 1 / dx
+  e.tables(p);
   double *rowq = p.rowq + (size_t)b * p.nt;
   double *colp = p.colpart + ((size_t)b * RS_G + c) * p.nt;
   for (int cb0 = 0; cb0 < p.nt; cb0 += RS_CB) {
@@ -133,8 +176,7 @@ __global__ void __launch_bounds__(256, 3) rowsum_sym_kernel(AsmParams p) {
     for (int k = 0; k < RS_CB / 32; ++k) cs[k] = 0.0;
     for (int i = c * 8 + warp; i < p.nt; i += RS_G * 8) {
       if (i < cb0) continue;
-      const double thi = th[i];
-      const double ti = TEMPORAL ? tm[i] : 0.0;
+      e.row(i);
       double *Krow = p.K + ((size_t)b * p.nt + i) * p.ldk;
       double rs = 0.0;
 #pragma unroll
@@ -142,13 +184,12 @@ __global__ void __launch_bounds__(256, 3) rowsum_sym_kernel(AsmParams p) {
         const int j = cb0 + 32 * k + lane;
         if (cb0 + 32 * k <= i) {        // warp-uniform
           if (j < i) {
-            double v = interp_cov(cf, nc, dx, thi, th[j]);
-            if (TEMPORAL) v *= temporal_k(tkind, ti, tm[j], tau);
+            const double v = e(i, j);
             rs += v;
             cs[k] += v;
             if (p.nm.defer) Krow[j] = v;   // raw covariance, written once (coalesced along j)
           } else if (j == i) {
-            const double v = (p.nt == 1) ? p.var[b] : interp_cov(cf, nc, dx, thi, thi);
+            const double v = (p.nt == 1) ? p.var[b] : e.diag();
             rs += v;
             if (p.nm.defer) Krow[j] = v;
           }
@@ -164,85 +205,6 @@ __global__ void __launch_bounds__(256, 3) rowsum_sym_kernel(AsmParams p) {
       double t = 0.0;
 #pragma unroll
       for (int w = 0; w < 8; ++w) t += part[w * RS_CB + j];
-      colp[cb0 + j] = t;
-    }
-    __syncthreads();
-  }
-}
-
-// ---- pass A'' : the same symmetric pass for EQUALLY SPACED time stamps (spb_noise_model.uniform_dt).
-// theta_i - theta_j = 2 pi ((t_i - t_j) / p - (floor(t_i / p) - floor(t_j / p))) = 2 pi (d dt / p - m) with
-// d = i - j and m one of floor(d dt / p), floor(d dt / p) + 1: the interpolant is tabulated once per CTA
-// for the 2 nt possible arguments (G[0][d], G[1][d]) and an entry costs two conflict-free shared-memory
-// loads (the wrap count of column j and the table value) instead of the phase load and four coefficient
-// gathers of the general kernel, which is bound by exactly those (shared-memory LSU 77 %).  Entries whose
-// wrap count is neither of the two candidates (cannot happen in exact arithmetic) take the general formula.
-constexpr int RSU_CB = 512;   // columns per register block of the uniform kernel (16 per lane: 3 CTAs per SM)
-__global__ void __launch_bounds__(256, 3) rowsum_sym_uniform_kernel(AsmParams p) {
-  extern __shared__ double sh[];  // coef (4*nc) | theta (nt) | part (8 x RSU_CB) | G (2 nt) | wraps (nt ints) | m0 (nt ints)
-  const int b = blockIdx.y, c = blockIdx.x;
-  const int nc = p.covpts + 1;
-  double *cf = sh, *th = sh + 4 * nc, *part = th + p.nt, *G = part + 8 * RSU_CB;
-  int *fl = reinterpret_cast<int *>(G + 2 * p.nt);
-  int *m0t = fl + p.nt;          // floor(d dt / p) per lag d
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  for (int k = tid; k < 4 * nc; k += 256) cf[k] = p.coef[(size_t)b * 4 * nc + k];
-  for (int k = tid; k < p.nt; k += 256) {
-    th[k] = phase_of(p.t[k], p.period);
-    fl[k] = (int)floor(p.t[k] / p.period);
-  }
-  __syncthreads();
-  const double dx = (double)p.covpts / (2.0 * 3.14159265358979323846);  // 1 / dx
-  const double dtp = p.nm.uniform_dt / p.period;
-  for (int d = tid; d < p.nt; d += 256) {
-    const double x = (double)d * dtp, m0 = floor(x);
-    G[d] = interp_cov(cf, nc, dx, 2.0 * 3.14159265358979323846 * (x - m0), 0.0);
-    G[p.nt + d] = interp_cov(cf, nc, dx, 2.0 * 3.14159265358979323846 * (m0 + 1.0 - x), 0.0);
-    m0t[d] = (int)m0;
-  }
-  __syncthreads();
-  double *rowq = p.rowq + (size_t)b * p.nt;
-  double *colp = p.colpart + ((size_t)b * RS_G + c) * p.nt;
-  for (int cb0 = 0; cb0 < p.nt; cb0 += RSU_CB) {
-    double cs[RSU_CB / 32];
-#pragma unroll
-    for (int k = 0; k < RSU_CB / 32; ++k) cs[k] = 0.0;
-    for (int i = c * 8 + warp; i < p.nt; i += RS_G * 8) {
-      if (i < cb0) continue;
-      const double thi = th[i];
-      const int fli = fl[i];
-      double *Krow = p.K + ((size_t)b * p.nt + i) * p.ldk;
-      double rs = 0.0;
-#pragma unroll
-      for (int k = 0; k < RSU_CB / 32; ++k) {
-        const int j = cb0 + 32 * k + lane;
-        if (cb0 + 32 * k <= i) {        // warp-uniform
-          if (j < i) {
-            const int d = i - j;
-            const int w = (fli - fl[j]) - m0t[d];   // 0 or 1
-            double v;
-            if ((unsigned)w <= 1u) v = G[w * p.nt + d];
-            else v = interp_cov(cf, nc, dx, thi, th[j]);
-            rs += v;
-            cs[k] += v;
-            if (p.nm.defer) Krow[j] = v;
-          } else if (j == i) {
-            const double v = (p.nt == 1) ? p.var[b] : G[0];
-            rs += v;
-            if (p.nm.defer) Krow[j] = v;
-          }
-        }
-      }
-      rs = warp_sum(rs);
-      if (lane == 0) rowq[i] = (cb0 == 0) ? rs : rowq[i] + rs;
-    }
-#pragma unroll
-    for (int k = 0; k < RSU_CB / 32; ++k) part[warp * RSU_CB + 32 * k + lane] = cs[k];
-    __syncthreads();
-    for (int j = tid; j < RSU_CB && cb0 + j < p.nt; j += 256) {
-      double t = 0.0;
-#pragma unroll
-      for (int w = 0; w < 8; ++w) t += part[w * RSU_CB + j];
       colp[cb0 + j] = t;
     }
     __syncthreads();
@@ -271,24 +233,10 @@ __global__ void __launch_bounds__(256) norm_scalars_kernel(AsmParams p) {
     for (int k = 0; k < 8; ++k) tot += red[k];
     const double K = (double)p.nt;
     const double m = tot / (K * K);             // tt.mean(Sig)
-    const double mu = 1.0 + p.gp_mean[b];       // sp.py:700-701
-    const double z = m / (mu * mu);
-    double fac = 1.0, alpha = 0.0, beta = 0.0;  // norm.py:26-44
-    for (int n = 0; n <= p.nm.normalization_order; ++n) {
-      alpha += fac;
-      beta += 2 * n * fac;
-      fac *= z * (2 * n + 3);
-    }
-    p.scal[4 * b + 0] = alpha / (mu * mu);
-    p.scal[4 * b + 1] = z * (alpha + beta);
-    p.scal[4 * b + 2] = z * alpha;
-    p.scal[4 * b + 3] = m;
-    if (p.z_out) p.z_out[b] = z;
-    // re-evaluated on every call, as the reference does (sp.py:1178-1183): z depends on t, i, p, u,
-    // so the bit is WRITTEN, not OR-ed into the process' persistent flags (one writer per element)
-    if (p.info)
-      p.info[b] = (p.info[b] & ~SPB_INFO_Z_RANGE) | ((z > p.nm.normalization_zmax) ? SPB_INFO_Z_RANGE : 0);
     mshare = m;
+    p.scal[4 * b + 3] = m;
+    spb_norm_series(m, p.gp_mean[b], p.nm.normalization_order, p.nm.normalization_zmax, p.scal + 4 * b,
+                    p.z_out ? p.z_out + b : nullptr, p.info ? p.info + b : nullptr);
   }
   __syncthreads();
   const double km = (double)p.nt * mshare;
@@ -326,7 +274,7 @@ __global__ void __launch_bounds__(256) write_kernel(AsmParams p) {
   const double tau = tkind ? p.nm.tau[(size_t)b * p.nm.tau_stride] : 1.0;
   if (p.marginal) {
     for (int k = tid; k < 4 * nc; k += 256) cf[k] = p.coef[(size_t)b * 4 * nc + k];
-    for (int k = tid; k < p.nt; k += 256) th[k] = phase_of(p.t[k], p.period);
+    for (int k = tid; k < p.nt; k += 256) th[k] = spb_phase(p.t[k], p.period);
     if (TEMPORAL && tkind)
       for (int k = tid; k < p.nt; k += 256) tm[k] = p.t[k];
   }
@@ -385,17 +333,15 @@ int run_assemble(spb_context *ctx, AsmParams &p, void *workspace, size_t workspa
   static spb_once_flag attr_once;   // function attributes are per device
   {
     const int st = spb_once_per_device(attr_once, ctx->device, [&]() -> int {
-      SPB_CHECK_CUDA(cudaFuncSetAttribute(rowsum_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                          200 * 1024));
       SPB_CHECK_CUDA(cudaFuncSetAttribute(write_kernel<false>,
                                           cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
       SPB_CHECK_CUDA(cudaFuncSetAttribute(write_kernel<true>,
                                           cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-      SPB_CHECK_CUDA(cudaFuncSetAttribute(rowsum_sym_kernel<false>,
+      SPB_CHECK_CUDA(cudaFuncSetAttribute(rowsum_sym_kernel<GeneralEntry>,
                                           cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-      SPB_CHECK_CUDA(cudaFuncSetAttribute(rowsum_sym_kernel<true>,
+      SPB_CHECK_CUDA(cudaFuncSetAttribute(rowsum_sym_kernel<TemporalEntry>,
                                           cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-      SPB_CHECK_CUDA(cudaFuncSetAttribute(rowsum_sym_uniform_kernel,
+      SPB_CHECK_CUDA(cudaFuncSetAttribute(rowsum_sym_kernel<UniformEntry>,
                                           cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
       return 0;
     });
@@ -406,15 +352,14 @@ int run_assemble(spb_context *ctx, AsmParams &p, void *workspace, size_t workspa
       const size_t smS = smA + (size_t)8 * RS_CB * sizeof(double);
       SPB_REQUIRE(smS <= 200 * 1024, "assemble: nt too large for the shared-memory staging");
       dim3 gridS(RS_G, p.B);
-      const size_t smU = smA + (size_t)8 * RSU_CB * sizeof(double) +
-                         (size_t)p.nt * (2 * sizeof(double) + 2 * sizeof(int)) + 16;
-      if (p.nm.temporal_kind) rowsum_sym_kernel<true><<<gridS, 256, smS, stream>>>(p);
+      const size_t smU = smS + (size_t)p.nt * (2 * sizeof(double) + 2 * sizeof(int)) + 16;
+      if (p.nm.temporal_kind) rowsum_sym_kernel<TemporalEntry><<<gridS, 256, smS, stream>>>(p);
       else if (p.nm.uniform_dt > 0.0 && p.nt > 1 && smU <= 200 * 1024)
-        rowsum_sym_uniform_kernel<<<gridS, 256, smU, stream>>>(p);
-      else rowsum_sym_kernel<false><<<gridS, 256, smS, stream>>>(p);
+        rowsum_sym_kernel<UniformEntry><<<gridS, 256, smU, stream>>>(p);
+      else rowsum_sym_kernel<GeneralEntry><<<gridS, 256, smS, stream>>>(p);
     } else {
       dim3 gridA(min((p.nt + 7) / 8, 16), p.B);
-      rowsum_kernel<<<gridA, 256, smA, stream>>>(p);
+      rowsum_kernel<<<gridA, 256, 0, stream>>>(p);
     }
     SPB_LAUNCH_CHECK(ctx);
     norm_scalars_kernel<<<p.B, 256, 0, stream>>>(p);
@@ -459,12 +404,12 @@ __global__ void __launch_bounds__(256) cross_marginal_kernel(int nts, int nt, in
   double *cf = sh, *th = sh + 4 * nc;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   for (int k = tid; k < 4 * nc; k += 256) cf[k] = coef[(size_t)b * 4 * nc + k];
-  for (int k = tid; k < nt; k += 256) th[k] = phase_of(t[k], period);
+  for (int k = tid; k < nt; k += 256) th[k] = spb_phase(t[k], period);
   __syncthreads();
   const double inv_dx = (double)covpts / (2.0 * 3.14159265358979323846);
   const double off = offset ? offset[(size_t)b * offset_stride] : 0.0;
   for (int i = blockIdx.x * 8 + warp; i < nts; i += gridDim.x * 8) {
-    const double thi = phase_of(ts[i], period);
+    const double thi = spb_phase(ts[i], period);
     double *row = out + (size_t)b * out_stride + (size_t)i * ld;
     for (int j = lane; j < ld; j += 32)
       row[j] = (j < nt) ? interp_cov(cf, nc, inv_dx, thi, th[j]) + off : 0.0;

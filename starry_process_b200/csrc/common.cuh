@@ -199,3 +199,50 @@ __device__ __forceinline__ double warp_sum(double v) {
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
   return v;
 }
+
+// ---- phase basis of the light curve: every kernel that evaluates a function of the phase ---------
+// theta = 2 pi mod(t / p, 1) (flux.py:261); *wraps, if given, receives floor(t / p).
+__device__ __forceinline__ double spb_phase(double t, double period, double *wraps = nullptr) {
+  const double x = t / period;
+  const double w = floor(x);
+  if (wraps) *wraps = w;
+  return 2.0 * 3.14159265358979323846 * (x - w);
+}
+
+// cs[m] = cos(m theta), sn[m] = sin(m theta) for m <= SPB_LMAX by the Chebyshev recurrences of wigner.h:311-316.
+// The design matrix (wigner.cu, -fmad=false) and the rank-31 basis Phi(t) (lowrank.cu, -fmad=true) must round
+// identically, since Phi B_inc is exactly the design matrix: the product is rounded on its own (__dmul_rn), so
+// no translation unit can fuse it into the subtraction; the doubling is exact.
+__device__ __forceinline__ void spb_harmonics(double theta, double *cs, double *sn) {
+  cs[0] = 1.0;
+  sn[0] = 0.0;
+  cs[1] = cos(theta);
+  sn[1] = sin(theta);
+#pragma unroll
+  for (int k = 2; k <= SPB_LMAX; ++k) {
+    cs[k] = __dmul_rn(2.0 * cs[k - 1], cs[1]) - cs[k - 2];
+    sn[k] = __dmul_rn(2.0 * sn[k - 1], cs[1]) - sn[k - 2];
+  }
+}
+
+// ---- normalisation series of the flux covariance (norm.py:26-44, sp.py:700-727) -------------------
+// From m, the mean of the raw covariance Sig, the normalised covariance is
+// s[0] Sig + s[1] (1 - q)(1 - q)^T - s[2] q q^T; *z (if given) receives z.  z depends on t, i, p and u, so
+// the SPB_INFO_Z_RANGE bit of *info (if given) is re-evaluated on every call, as the reference does
+// (sp.py:1178-1183): it is WRITTEN, not OR-ed into the process' persistent flags.
+__device__ __forceinline__ void spb_norm_series(double m, double gp_mean, int order, double zmax, double *s,
+                                                double *z_out, int32_t *info) {
+  const double mu = 1.0 + gp_mean;  // sp.py:700-701
+  const double z = m / (mu * mu);
+  double fac = 1.0, alpha = 0.0, beta = 0.0;
+  for (int n = 0; n <= order; ++n) {
+    alpha += fac;
+    beta += 2 * n * fac;
+    fac *= z * (2 * n + 3);
+  }
+  s[0] = alpha / (mu * mu);
+  s[1] = z * (alpha + beta);
+  s[2] = z * alpha;
+  if (z_out) *z_out = z;
+  if (info) *info = (*info & ~SPB_INFO_Z_RANGE) | ((z > zmax) ? SPB_INFO_Z_RANGE : 0);
+}

@@ -28,27 +28,14 @@ constexpr int SOLVE_CH = 2048;    // time stamps per CTA of the solve (8 warps x
 constexpr int SOLVE_EB = 8;       // batch elements per CTA of the solve
 constexpr int COV_CHUNK = 512;    // elements per (B_inc Sigma) workspace chunk
 
-// Phi(t) = [1, cos(m theta), sin(m theta)], theta = 2 pi frac(t / p) and the Chebyshev recurrences of
-// design_rows_kernel (wigner.h:311-316), unfused as there (wigner.cu is built with -fmad=false).
+// Phi(t) = [1, cos(m theta), sin(m theta), 0] (m = 1 .. 15): the phase basis of design_rows_kernel
 __device__ __forceinline__ void phase_row(double t, double period, double *row) {
-  const double x = t / period;
-  const double th = 2.0 * 3.14159265358979323846 * (x - floor(x));
-  const double c1 = cos(th), s1 = sin(th);
-  double cm2 = 1.0, sm2 = 0.0, cm1 = c1, sm1 = s1;
-  row[0] = 1.0;
-  row[1] = c1;
-  row[SPB_LMAX + 1] = s1;
+  double cs[SPB_LMAX + 1], sn[SPB_LMAX + 1];
+  spb_harmonics(spb_phase(t, period), cs, sn);
 #pragma unroll
-  for (int k = 2; k <= SPB_LMAX; ++k) {
-    const double c = __dsub_rn(__dmul_rn(__dmul_rn(2.0, cm1), c1), cm2);
-    const double s = __dsub_rn(__dmul_rn(__dmul_rn(2.0, sm1), c1), sm2);
-    row[k] = c;
-    row[SPB_LMAX + k] = s;
-    cm2 = cm1;
-    cm1 = c;
-    sm2 = sm1;
-    sm1 = s;
-  }
+  for (int k = 0; k <= SPB_LMAX; ++k) row[k] = cs[k];
+#pragma unroll
+  for (int k = 1; k <= SPB_LMAX; ++k) row[SPB_LMAX + k] = sn[k];
   row[LR - 1] = 0.0;
 }
 
@@ -247,15 +234,15 @@ size_t basis_ws_doubles(int nt) {
 }
 
 // ---------------------------------------------------------------------------------------------------
-// Per element: GP mean, normalisation (same series, z and SPB_INFO_Z_RANGE as norm_scalars_kernel),
-// C~, T = R C~ R^T, Cholesky of N = I + T, logdet.
+// Per element: GP mean, normalisation (spb_norm_series, as norm_scalars_kernel), C~ (written back over C for
+// lowrank_post_kernel), T = R C~ R^T, Cholesky of N = I + T, logdet.
 // ---------------------------------------------------------------------------------------------------
 struct CovParams {
   int nt;
   const double *Binc;
   long long Binc_stride;
   const double *mean_ylm;
-  const double *C;          // (B, 32, 32) = B_inc Sigma B_inc^T
+  double *C;                // (B, 32, 32) in: B_inc Sigma B_inc^T, out: C~
   const double *R;          // (32, 32)
   const double *aux;        // s | Phi(t0) | sum log D
   spb_noise_model nm;
@@ -264,6 +251,7 @@ struct CovParams {
   double *L;                // (B, 32, 32) out: Cholesky factor of N (lower)
   double *off;              // (B) out: residual offset (GP mean unless normalised, + baseline mean)
   double *logdet;           // (B) out: logdet K
+  double *gp_mean;          // (B) out, optional
   double *z_out;
   int32_t *info;
 };
@@ -294,6 +282,7 @@ __global__ void __launch_bounds__(256) lowrank_cov_kernel(CovParams p) {
     double g = 0.0;
     for (int k = 0; k < LR; ++k) g += s[LR + k] * bmv[k];   // (A mean_ylm)[0], flux.py:340
     sc[0] = g;
+    if (p.gp_mean) p.gp_mean[b] = g;
   }
   if (p.nm.normalized && tid < LR) {
     double v = 0.0;
@@ -309,20 +298,8 @@ __global__ void __launch_bounds__(256) lowrank_cov_kernel(CovParams p) {
       for (int k = 0; k < LR; ++k) tot += s[k] * cs[k];
       const double K = (double)p.nt;
       const double m = tot / (K * K);             // tt.mean(Sig)
-      const double mu = 1.0 + gp_mean;            // sp.py:700-701
-      const double z = m / (mu * mu);
-      double fac = 1.0, alpha = 0.0, beta = 0.0;  // norm.py:26-44
-      for (int n = 0; n <= p.nm.normalization_order; ++n) {
-        alpha += fac;
-        beta += 2 * n * fac;
-        fac *= z * (2 * n + 3);
-      }
-      sc[1] = alpha / (mu * mu);
-      sc[2] = z * (alpha + beta);
-      sc[3] = z * alpha;
-      if (p.z_out) p.z_out[b] = z;
-      if (p.info)
-        p.info[b] = (p.info[b] & ~SPB_INFO_Z_RANGE) | ((z > p.nm.normalization_zmax) ? SPB_INFO_Z_RANGE : 0);
+      spb_norm_series(m, gp_mean, p.nm.normalization_order, p.nm.normalization_zmax, sc + 1,
+                      p.z_out ? p.z_out + b : nullptr, p.info ? p.info + b : nullptr);
       sc[4] = K * m;
     }
     __syncthreads();
@@ -351,6 +328,7 @@ __global__ void __launch_bounds__(256) lowrank_cov_kernel(CovParams p) {
     double v = 0.0;
     for (int k = 0; k < LR; ++k) v += Rs[i * QR_LD + k] * Cs[k * QR_LD + j];
     Ps[i * QR_LD + j] = v;
+    p.C[(size_t)b * LR * LR + idx] = Cs[i * QR_LD + j];
   }
   __syncthreads();
   for (int idx = tid; idx < LR * LR; idx += 256) {
@@ -558,45 +536,24 @@ constexpr int EVAL_EB = 8;               // elements per CTA of the evaluation
 constexpr int EVAL_SB = 32;              // draws per CTA of the evaluation
 
 struct PostParams {
-  const double *Binc;
-  long long Binc_stride;
-  const double *mean_ylm;
-  const double *C;          // (B, 32, 32) = B_inc Sigma B_inc^T
+  const double *C;          // (B, 32, 32) C~ (lowrank_cov_kernel)
   const double *R;          // (32, 32)
-  const double *aux;        // s | Phi(t0) | sum log D
-  const double *bvar;       // baseline variance: NULL | one value (bv_stride 0) | one per element (1)
-  long long bv_stride;
   const double *L;          // (B, 32, 32) Cholesky factor of N (lowrank_cov_kernel)
   const double *w;          // (B, 32) Q^T y (lowrank_wsum_kernel)
-  double *a, *P, *G, *gp_mean;
+  double *a, *P, *G;
   int32_t *info;
 };
 
 __global__ void __launch_bounds__(256) lowrank_post_kernel(PostParams p) {
   __shared__ double Cs[LR * QR_LD], Rs[LR * QR_LD], Ls[LR * QR_LD], Vs[LR * QR_LD];
-  __shared__ double bmv[LR], us[LR];
+  __shared__ double us[LR];
   const int b = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const double *Bb = p.Binc + (size_t)b * p.Binc_stride;
   double *ab = p.a + (size_t)b * LR, *Pb = p.P + (size_t)b * LR * LR, *Gb = p.G + (size_t)b * LR * LR;
-  // GP mean (A mean_ylm)[0], summed in the order of lowrank_cov_kernel
-  for (int k = warp; k < LR; k += 8) {
-    double v = 0.0;
-    for (int n = lane; n < 256; n += 32) v += Bb[k * 256 + n] * p.mean_ylm[(size_t)b * 256 + n];
-    v = warp_sum(v);
-    if (lane == 0) bmv[k] = v;
-  }
   for (int idx = tid; idx < LR * LR; idx += 256) {
     const int i = idx / LR, j = idx % LR;
-    Cs[i * QR_LD + j] = p.C[(size_t)b * LR * LR + (i >= j ? i * LR + j : j * LR + i)];
+    Cs[i * QR_LD + j] = p.C[(size_t)b * LR * LR + idx];
     Rs[i * QR_LD + j] = p.R[idx];
     Ls[i * QR_LD + j] = p.L[(size_t)b * LR * LR + idx];
-  }
-  __syncthreads();
-  if (tid == 0) {
-    double g = 0.0;
-    for (int k = 0; k < LR; ++k) g += p.aux[LR + k] * bmv[k];
-    p.gp_mean[b] = g;
-    if (p.bvar) Cs[0] += p.bvar[(size_t)b * p.bv_stride];
   }
   if (p.info[b] & SPB_INFO_NOT_PD) {   // N (hence K(t, t)) is not PD: no posterior
     for (int idx = tid; idx < LR * LR; idx += 256) {
@@ -879,8 +836,8 @@ int set_smem_attributes(spb_context *ctx) {
 int lowrank_front(spb_context *ctx, int B, int nt, const double *Binc, long long Binc_stride,
                   const double *mean_ylm, const double *cov_ylm, const double *Q, const double *R,
                   const double *phi_aux, const spb_noise_model *noise, int M, const double *flux, int ldf,
-                  long long flux_stride, const double *baseline_mean, long long bm_stride, double *z_out,
-                  int32_t *info, const LnlikeLayout &ly, SolveParams &sp, cudaStream_t stream) {
+                  long long flux_stride, const double *baseline_mean, long long bm_stride, double *gp_mean,
+                  double *z_out, int32_t *info, const LnlikeLayout &ly, SolveParams &sp, cudaStream_t stream) {
   const int nch = (nt + SOLVE_CH - 1) / SOLVE_CH;
   int st = set_smem_attributes(ctx);
   if (st) return st;
@@ -938,6 +895,7 @@ int lowrank_front(spb_context *ctx, int B, int nt, const double *Binc, long long
   cp.L = ly.L;
   cp.off = ly.off;
   cp.logdet = ly.logdet;
+  cp.gp_mean = gp_mean;
   cp.z_out = z_out;
   cp.info = info;
   lowrank_cov_kernel<<<B, 256, 0, stream>>>(cp);
@@ -1066,7 +1024,7 @@ extern "C" int spb_lowrank_lnlike(spb_context *ctx, int B, int nt, const double 
   const int nch = (nt + SOLVE_CH - 1) / SOLVE_CH;
   SolveParams sp;
   int st = lowrank_front(ctx, B, nt, Binc, Binc_stride, mean_ylm, cov_ylm, Q, R, phi_aux, noise, M, flux, ldf,
-                         flux_stride, baseline_mean, bm_stride, z_out, info, ly, sp, stream);
+                         flux_stride, baseline_mean, bm_stride, nullptr, z_out, info, ly, sp, stream);
   if (st) return st;
   const dim3 grid(nch, (B + SOLVE_EB - 1) / SOLVE_EB);
   lowrank_solve_kernel<true><<<grid, 256, SOLVE_SMEM, stream>>>(sp);
@@ -1111,23 +1069,16 @@ extern "C" int spb_lowrank_posterior(spb_context *ctx, int B, int nt, const doub
   const LnlikeLayout ly = lnlike_layout(ws, B, 1, nt);
   SolveParams sp;
   int st = lowrank_front(ctx, B, nt, Binc, Binc_stride, mean_ylm, cov_ylm, Q, R, phi_aux, noise, 1, flux, nt, 0,
-                         baseline_mean, bm_stride, nullptr, info, ly, sp, stream);
+                         baseline_mean, bm_stride, gp_mean, nullptr, info, ly, sp, stream);
   if (st) return st;
   PostParams pp;
-  pp.Binc = Binc;
-  pp.Binc_stride = Binc_stride;
-  pp.mean_ylm = mean_ylm;
   pp.C = ly.C;
   pp.R = R;
-  pp.aux = phi_aux;
-  pp.bvar = noise->baseline_var;
-  pp.bv_stride = noise->base_stride;
   pp.L = ly.L;
   pp.w = ly.w;
   pp.a = a;
   pp.P = P;
   pp.G = G;
-  pp.gp_mean = gp_mean;
   pp.info = info;
   lowrank_post_kernel<<<B, 256, 0, stream>>>(pp);
   SPB_LAUNCH_CHECK(ctx);

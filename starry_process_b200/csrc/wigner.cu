@@ -310,18 +310,8 @@ __global__ void __launch_bounds__(DM_THREADS, 3)
   for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
     const int t = tile * DM_THREADS + tid;
     // rows past nt are computed on a clamped timestamp and clipped by the tensor map
-    const double x = p.t[t < p.nt ? t : p.nt - 1] / per;
-    const double theta = 2.0 * 3.14159265358979323846 * (x - floor(x));  // tt.mod(t/p, 1)
-    double cs[16], sn[16];
-    cs[0] = 1.0;
-    sn[0] = 0.0;
-    cs[1] = cos(theta);
-    sn[1] = sin(theta);
-#pragma unroll
-    for (int k = 2; k <= SPB_LMAX; ++k) {  // wigner.h:311-316
-      cs[k] = 2.0 * cs[k - 1] * cs[1] - cs[k - 2];
-      sn[k] = 2.0 * sn[k - 1] * cs[1] - sn[k - 2];
-    }
+    double cs[SPB_LMAX + 1], sn[SPB_LMAX + 1];
+    spb_harmonics(spb_phase(p.t[t < p.nt ? t : p.nt - 1], per), cs, sn);
     const int trow0 = tile * DM_THREADS + warp * 32;   // first timestamp of this warp's tile
     double o0, o1, o2, o3;
 #define RS2(q) Rs2[q]

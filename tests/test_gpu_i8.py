@@ -234,7 +234,7 @@ def test_moments_syrk_on_int8_tensor_cores_matches_fp64_syrk(spb, golden):
 
 def test_uniform_time_stamps_fast_path_matches_general_assembly(spb, monkeypatch):
     """flux.py:256-276 for equally spaced time stamps: the tabulated interpolant (spb_noise_model.uniform_dt,
-    rowsum_sym_uniform_kernel) against the per-entry evaluation -- several periods (0, few and many wraps per
+    rowsum_sym_kernel<UniformEntry>) against the per-entry evaluation -- several periods (0, few and many wraps per
     light curve), a shifted grid, and an irregular grid, which must not take the fast path."""
     import bench
 

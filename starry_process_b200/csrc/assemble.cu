@@ -457,7 +457,11 @@ extern "C" int spb_cross_marginal(spb_context *ctx, int B, int nts, int nt, cons
                                   const double *t, double period, int covpts, const double *coef,
                                   const double *offset, long long offset_stride, double *K_ts_t,
                                   int ld, long long K_stride, void *stream) {
-  SPB_REQUIRE(ctx != nullptr && B > 0 && nts > 0 && nt > 0 && ld >= nt, "cross_marginal: bad arguments");
+  SPB_REQUIRE(ctx != nullptr && ts != nullptr && t != nullptr && coef != nullptr && K_ts_t != nullptr,
+              "cross_marginal: null argument");
+  SPB_REQUIRE(B > 0 && nts > 0 && nt > 0 && ld >= nt, "cross_marginal: bad arguments");
+  SPB_REQUIRE(covpts >= 4, "cross_marginal: covpts must be >= 4");
+  SPB_REQUIRE(period > 0.0, "cross_marginal: period must be positive");
   SPB_REQUIRE(B <= 65535, "cross_marginal: batch too large for one launch");
   SPB_CHECK_CUDA(cudaSetDevice(ctx->device));
   const size_t smem = (size_t)(4 * (covpts + 1) + nt) * sizeof(double);

@@ -206,7 +206,8 @@ __global__ void __launch_bounds__(NTHREADS, 2) gemm_nt_kernel(Desc d) {
         if (n >= d.N) continue;
         double v = acc[mt][nt][e];
         if (EPI == EPI_STORE) {
-          Cb[(size_t)m * d.ldc + n] = d.alpha * v;
+          // lower_only: the strict upper triangle of a diagonal tile stays untouched
+          if (!d.lower_only || n <= m) Cb[(size_t)m * d.ldc + n] = d.alpha * v;
         } else if (EPI == EPI_AXPBY) {
           double *c = Cb + (size_t)m * d.ldc + n;
           *c = (d.beta == 0.0) ? d.alpha * v : fma(d.alpha, v, d.beta * *c);
@@ -241,6 +242,8 @@ inline int launch(spb_context *ctx, const Desc &d, cudaStream_t stream) {
   SPB_REQUIRE(d.M > 0 && d.N > 0 && d.K > 0 && d.batch > 0, "gemm_nt: empty problem");
   SPB_REQUIRE((d.lda % 2) == 0 && (d.ldb % 2) == 0 && (d.K % 2) == 0,
               "gemm_nt: K and the operand leading dimensions must be even");
+  SPB_REQUIRE(d.lda >= d.K && d.ldb >= d.K && d.ldc >= d.N,
+              "gemm_nt: leading dimensions must be lda >= K, ldb >= K and ldc >= N");
   SPB_REQUIRE(((uintptr_t)d.A % 16) == 0 && ((uintptr_t)d.Bm % 16) == 0 &&
                   (d.strideA % 2) == 0 && (d.strideB % 2) == 0,
               "gemm_nt: operands must be 16-byte aligned");

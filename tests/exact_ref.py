@@ -4,7 +4,9 @@ tests/test_gpu_i8_exact.py checks the kernels against them.
 
 * ``exact_dot_rows``: the correctly rounded fp64 value of sum_k X[i,k] Y[j,k] for sampled (i, j);
 * ``woodbury_lnlike``: log det K, r^T K^-1 r and the Gaussian log-likelihood for K = diag(d) + U U^T with a
-  thin U, in 50-digit arithmetic, independent of any Cholesky factorisation.
+  thin U, in 50-digit arithmetic, independent of any Cholesky factorisation;
+* ``phase_fp64``, ``interp_cov_mp``, ``temporal_k_mp``: the phase of spb_phase bit for bit, and the marginal
+  interpolant and the temporal kernels in mpmath, for the predict building blocks (tests/test_gpu_dmma_exact.py).
 """
 import math
 
@@ -106,6 +108,43 @@ def woodbury_lnlike(d, U, R, dps=50):
         M = len(quad)
         ll = -mpmath.fsum(quad) / 2 - M * logdet / 2 - mpmath.mpf(nt * M) / 2 * mpmath.log(2 * mpmath.pi)
     return logdet, quad, ll
+
+
+TWO_PI = 2.0 * 3.14159265358979323846   # the fp64 constant of spb_phase (pi rounded, doubled exactly)
+
+
+def phase_fp64(t, period):
+    """spb_phase (csrc/common.cuh) bit for bit: x = fl(t / p), w = floor(x), theta = fl(TWO_PI fl(x - w)), the
+    same three IEEE roundings as on the device.  x - w is exact for x >= 0; for x just below a negative
+    integer it rounds up to exactly 1 and theta to exactly TWO_PI."""
+    x = np.asarray(t, dtype=np.float64) / np.float64(period)
+    return TWO_PI * (x - np.floor(x))
+
+
+def interp_cov_mp(cf, covpts, s):
+    """The cubic interpolant of flux.py:256-276 (csrc/assemble.cu interp_cov) evaluated exactly (mpmath at the
+    working precision) on a coefficient table cf (4, covpts + 1) at the scaled lag s = |dtheta| covpts / 2pi:
+    bin ind = floor(s) (at most covpts), x0 = s - ind, value sum_k cf[k][ind] x0^k."""
+    import mpmath
+
+    s = mpmath.mpf(s)
+    ind = min(int(mpmath.floor(s)), covpts)
+    x0 = s - ind
+    return mpmath.fsum(mpmath.mpf(float(cf[k][ind])) * x0 ** k for k in range(4)), ind
+
+
+def temporal_k_mp(kind, dt, tau):
+    """temporal.py:8-16 in mpmath at the working precision, on the fp64 inputs dt = |t1 - t2| (exact) and tau:
+    kind 1 Matern-3/2 (1 + x) e^-x with x = sqrt(3) dt / tau, kind 2 exp(-dt^2 / (2 tau)).  Also returns the
+    condition number x |d ln k / dx| of k in its argument: x^2 / (1 + x) for kind 1, dt^2 / (2 tau) for kind 2."""
+    import mpmath
+
+    dt, tau = mpmath.mpf(dt), mpmath.mpf(tau)
+    if kind == 1:
+        x = mpmath.sqrt(3) * dt / tau
+        return (1 + x) * mpmath.exp(-x), x * x / (1 + x)
+    a = dt * dt / (2 * tau)
+    return mpmath.exp(-a), a
 
 
 def _forward(L, w, k):

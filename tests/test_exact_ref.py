@@ -7,7 +7,55 @@ from fractions import Fraction
 
 import numpy as np
 
-from exact_ref import exact_dot_rows, woodbury_lnlike
+from exact_ref import TWO_PI, exact_dot_rows, interp_cov_mp, phase_fp64, temporal_k_mp, woodbury_lnlike
+
+
+def test_phase_fp64_against_fractions():
+    """theta = fl(TWO_PI fl(x - floor(x))), x = fl(t / p), each step correctly rounded; t just below a negative
+    multiple of p gives exactly TWO_PI."""
+    rng = np.random.default_rng(6)
+    t = np.r_[rng.uniform(-50, 50, 200), 0.0, 3.0, -3.0, -3.0 * (1 + 2.0 ** -52), -1e-20]
+    p = 1.5
+    th = phase_fp64(t, p)
+    for tv, g in zip(t, th):
+        x = float(Fraction(tv) / Fraction(p))
+        frac = float(Fraction(x) - math.floor(x))
+        assert g == float(Fraction(TWO_PI) * Fraction(frac)), tv
+    assert th[-1] == TWO_PI and th[-5] == 0.0
+    assert np.all((th >= 0) & (th <= TWO_PI))
+
+
+def test_interp_cov_mp_against_fractions():
+    """The interpolant at rational lags, against the cubic evaluated in rational arithmetic; the bin of a lag on
+    a knot is the upper one, and s = covpts takes the last bin with x0 = 0."""
+    import mpmath
+
+    rng = np.random.default_rng(7)
+    covpts = 6
+    cf = rng.standard_normal((4, covpts + 1))
+    with mpmath.workdps(40):
+        for s in (Fraction(0), Fraction(1, 3), Fraction(2), Fraction(47, 10), Fraction(covpts)):
+            v, ind = interp_cov_mp(cf, covpts, mpmath.mpf(s.numerator) / s.denominator)
+            i = min(math.floor(s), covpts)
+            x0 = s - i
+            want = sum(Fraction(float(cf[k][i])) * x0 ** k for k in range(4))
+            assert ind == i
+            assert abs(v - mpmath.mpf(want.numerator) / want.denominator) <= mpmath.mpf(10) ** -35 * (1 + abs(v))
+
+
+def test_temporal_k_mp_closed_forms():
+    """Matern-3/2 at x = 1 is 2/e, the squared exponential at dt^2 / (2 tau) = 1 is 1/e, both are 1 at dt = 0;
+    the condition numbers are x^2 / (1 + x) and dt^2 / (2 tau)."""
+    import mpmath
+
+    with mpmath.workdps(40):
+        k, c = temporal_k_mp(1, 2.0, 2.0 * math.sqrt(3))   # x = sqrt(3) 2 / fl(2 sqrt 3) = 1 (1 + O(u))
+        x = mpmath.sqrt(3) * 2 / mpmath.mpf(2.0 * math.sqrt(3))
+        assert abs(k - (1 + x) * mpmath.exp(-x)) < mpmath.mpf(10) ** -38
+        assert abs(k - 2 / mpmath.e) < 1e-15 and abs(c - mpmath.mpf(1) / 2) < 1e-15
+        k, c = temporal_k_mp(2, 2.0, 2.0)
+        assert abs(k - 1 / mpmath.e) < mpmath.mpf(10) ** -38 and c == 1
+        assert temporal_k_mp(1, 0.0, 3.0)[0] == 1 and temporal_k_mp(2, 0.0, 3.0)[0] == 1
 
 
 def _adversarial_rows(rng, K):

@@ -194,21 +194,53 @@ def test_cholesky_cluster_and_batch_kernels_agree(spb):
 
 
 def test_solve_rows_many_rhs(spb):
+    """y = L^-1 r for M rows against one factor, nt in {1, 2, 127, 129, 1000, 4097} (odd nt with an even, padded
+    ld) x M in {1, 31, 300}.  Backward error of each solved row, the residual L y - r formed by exact dot
+    products: a triangular solve returns the exact solution of (L + dL) y = r with |dL| <= gamma_nt |L|, so
+    |L y - r|_i <= gamma_nt (|L||y|)_i; doubled (c = 2) for the reciprocal-times-multiply division, plus u for
+    the correctly rounded residual.  quad against math.fsum(y^2) of the returned y within gamma_nt (a sum of
+    nt non-negative squares, each rounded)."""
+    import math
+
     import scipy.linalg as sl
 
+    from exact_ref import exact_dot_rows
+
     ctx = spb.get_context(0)
-    rng = np.random.default_rng(5)
-    n, M = 1000, 300
-    A = rng.standard_normal((n, 50))
-    L = np.linalg.cholesky(A @ A.T / 50 + 0.5 * np.eye(n))
-    Lt = torch.tensor(L, device="cuda")
-    Rh = rng.standard_normal((M, n))
-    R = torch.tensor(Rh, device="cuda")
-    quad = torch.zeros(M, dtype=torch.float64, device="cuda")
-    assert ctx.lib.spb_cholesky_solve_rows(ctx.handle, n, P(Lt), n, M, P(R), n, P(quad), None) == 0
-    y = sl.solve_triangular(L, Rh.T, lower=True)
-    assert np.abs(R.cpu().numpy() - y.T).max() <= 1e-11
-    assert np.abs(quad.cpu().numpy() - (y ** 2).sum(0)).max() <= 1e-9
+    u = 2.0 ** -53
+
+    def gam(k):
+        return k * u / (1 - k * u)
+
+    for n in (1, 2, 127, 129, 1000, 4097):
+        rng = np.random.default_rng(n)
+        ld = n + (n & 1)
+        A = rng.standard_normal((n, 50))
+        L = np.linalg.cholesky(A @ A.T / 50 + 0.5 * np.eye(n))
+        Lp = np.zeros((n, ld))
+        Lp[:, :n] = L
+        Lt = torch.tensor(Lp, device="cuda")
+        for M in (1, 31, 300):
+            Rh = rng.standard_normal((M, n))
+            Rp = np.zeros((M, ld))
+            Rp[:, :n] = Rh
+            R = torch.tensor(Rp, device="cuda")
+            quad = torch.zeros(M, dtype=torch.float64, device="cuda")
+            assert ctx.lib.spb_cholesky_solve_rows(ctx.handle, n, P(Lt), ld, M, P(R), ld, P(quad), None) == 0
+            Y = R.cpu().numpy()[:, :n]
+            q = quad.cpu().numpy()
+            if n == 1000 and M == 300:   # the original scipy comparison
+                y = sl.solve_triangular(L, Rh.T, lower=True)
+                assert np.abs(Y - y.T).max() <= 1e-11
+            rows = sorted({0, 1, 63, 64, 127, 128, n - 1} & set(range(n)) | set(int(x) for x in rng.integers(0, n, 8)))
+            for m in sorted({0, M - 1, M // 2}):
+                X = np.concatenate([L, Rh[m][:, None]], axis=1)   # (L y - r)_i = [L_i, r_i] . [y, -1]
+                yv = np.concatenate([Y[m], [-1.0]])[None]
+                res = exact_dot_rows(X, yv, [(i, 0) for i in rows])
+                LY = exact_dot_rows(np.abs(L), np.abs(Y[m:m + 1]), [(i, 0) for i in rows])
+                assert np.all(np.abs(res) <= (2 * gam(n) + u) * LY * (1 + 2 * u)), (n, M, m)
+                fs = math.fsum((Y[m] ** 2).tolist())   # each square rounded once more on the host: gamma_{n+1}
+                assert abs(q[m] - fs) <= gam(n + 1) * fs, (n, M, m, q[m], fs)
 
 
 # --------------------------------------------------------------------------------------- moments
